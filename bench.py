@@ -69,7 +69,14 @@ def parse_args():
                     help="MAX_RADIANCE_RAY_DEPTH of the strong-scaling frame (BASELINE config 3 is '2-bounce'; the reference's shaders are 1)")
     ap.add_argument("--radiance-depth", type=int, default=1, choices=[1, 2], help="MAX_RADIANCE_RAY_DEPTH of the headline workload (1 = reference)")
     ap.add_argument("--no-target-scene", action="store_true", help="skip the 1.31 M-triangle incoherent-ray target measurement")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame buffers of the last timed step to DIR/<name>.npy (float32; see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed (--impl ours)")
+    return args
 
 
 def load_workload(args):
@@ -289,6 +296,10 @@ def run_ours(args):
     torch.cuda.synchronize()
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:  # before the measurements below dispatch into the same buffers again
+        frame = reduced_t if world > 1 else out_t
+        named = {"direct": frame, "indirect_specular": outs[1], "denoised": dn["out"]} if wl.realtime else {"accumulation": frame}
+        dump_outputs(args.dump_outputs, {k: v.cpu().numpy() for k, v in named.items()}, W, H)
     clock_info = clocks.stop() if rank == 0 else None
     launches = ctx.launches() - launches0  # this rank's own kernels; NCCL's reduce kernels are not counted
     rc = ctx.ray_counts(reset=True)
@@ -351,6 +362,23 @@ def run_ours(args):
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_LIMIT_BYTES = 64 * 2**20
+
+
+def dump_outputs(path, arrays, W, H):
+    """Writes each RGBA float32 frame of `arrays` to path/<name>.npy: the whole (H, W, 4) frame when all of them fit in
+    DUMP_LIMIT_BYTES, else the same fixed sample of pixels from each, an (n, 4) array whose rows are the pixels
+    np.sort(np.random.Generator(np.random.PCG64(0)).choice(H * W, n, replace=False)) in row-major order."""
+    os.makedirs(path, exist_ok=True)
+    frames = {k: np.ascontiguousarray(v, np.float32).reshape(H * W, 4) for k, v in arrays.items()}
+    pix = None
+    if sum(v.nbytes for v in frames.values()) > DUMP_LIMIT_BYTES:
+        n = (DUMP_LIMIT_BYTES - 1024 * len(frames)) // (16 * len(frames))  # room for the .npy headers
+        pix = np.sort(np.random.Generator(np.random.PCG64(0)).choice(H * W, n, replace=False))
+    for k, v in frames.items():
+        np.save(os.path.join(path, k + ".npy"), v.reshape(H, W, 4) if pix is None else v[pix])
 
 
 def make_comm(rt, ctx, torch, dist, world, rank):

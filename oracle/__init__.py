@@ -3,9 +3,12 @@
 TEST INFRASTRUCTURE, NOT PRODUCT — see oracle/oracle.h.  Importable only from tests/, from
 ``__graft_entry__.smoke()`` and from ``bench.py``'s cpu_baseline / ``--impl reference`` legs.
 """
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -25,15 +28,18 @@ def build(force: bool = False) -> str:
 
 
 def use_native() -> str:
-    """CPU-baseline build of the same sources: -O3 -march=native, compiled ON THE MACHINE THAT RUNS IT (oracle/_native/
-    is git- and gpurun-ignored, so a library built for another CPU never travels).  Must be called before the first
-    lib() call; falls back to the portable -O2 library if the compile fails.  Returns the flags in use."""
+    """CPU-baseline build of the same sources: -O3 -march=native, compiled ON THE MACHINE THAT RUNS IT, into a temporary
+    directory removed at exit (the tree is left untouched and may be read-only, and a library built for another CPU
+    never travels with it).  Must be called before the first lib() call; falls back to the portable -O2 library if the
+    compile fails.  Returns the flags in use."""
     global _SO
     if _lib is not None:  # already loaded: report what is in use
         return "-O3 -march=native -ffp-contract=off" if _SO.endswith("liboracle_native.so") else "-O2 -ffp-contract=off"
+    out_dir = tempfile.mkdtemp(prefix="oracle_native_")
+    atexit.register(shutil.rmtree, out_dir, ignore_errors=True)
     try:
-        subprocess.run(["make", "-C", _DIR, "-s", "native"], check=True, capture_output=True, timeout=600)
-        _SO = os.path.join(_DIR, "_native", "liboracle_native.so")
+        subprocess.run(["make", "-C", _DIR, "-s", "native", f"NATIVE_DIR={out_dir}"], check=True, capture_output=True, timeout=600)
+        _SO = os.path.join(out_dir, "liboracle_native.so")
         return "-O3 -march=native -ffp-contract=off"
     except Exception:
         return "-O2 -ffp-contract=off (native build failed)"

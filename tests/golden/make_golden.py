@@ -1,6 +1,6 @@
 """Regenerates tests/golden/*.npz from the CPU oracle.
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py [REFERENCE_CHECKOUT]
 
 The reference cannot be executed here (Windows/D3D12), so these vectors are NOT reference outputs: they freeze the
 oracle's answers (which tests/test_oracle_reference_kats.py pins against the reference's own test logic) so that
@@ -99,11 +99,10 @@ def main():
     np.savez_compressed(os.path.join(HERE, "rng.npz"), seeds=seeds, rands=rands)
     np.savez_compressed(os.path.join(HERE, "hitgroups_mixed.npz"), **hit_group_vectors(oracle))
     # a 192 x 128 crop of the reference's own mock denoiser inputs (src/DenoiseCompositor.cpp:52-60 loads
-    # assets/textures/{DirectLighting,IndirectSpecular}.PNG, 1922 x 1126, 8-bit) around the busiest region: a fixture that
-    # travels to the GPU box, where /root/reference does not exist.  tests/test_independent_answers.py checks the crop
-    # against the full files whenever they are present.
-    tex = "/root/reference/assets/textures"
-    if os.path.exists(os.path.join(tex, "DirectLighting.PNG")):
+    # assets/textures/{DirectLighting,IndirectSpecular}.PNG, 1922 x 1126, 8-bit) around the busiest region: the repository
+    # does not carry the full files, so it is rewritten only when the path of a reference checkout is given.
+    tex = os.path.join(sys.argv[1], "assets", "textures") if len(sys.argv) > 1 else ""
+    if tex and os.path.exists(os.path.join(tex, "DirectLighting.PNG")):
         from PIL import Image
         y0, x0, hh, ww = 128, 832, 128, 192
         d = np.asarray(Image.open(os.path.join(tex, "DirectLighting.PNG")).convert("RGBA"))[y0:y0 + hh, x0:x0 + ww]

@@ -26,7 +26,7 @@ def test_library_exports_every_declared_symbol(rt):
     assert set(names) <= exported
 
 
-def test_header_is_plain_c_and_cites_the_reference():
+def test_header_is_plain_c_and_cites_the_reference(tmp_path):
     hdr = open(os.path.join(ROOT, "include", "rt_core.h")).read()
     types = open(os.path.join(ROOT, "include", "rt_types.h")).read()
     for text in (hdr, types):
@@ -38,7 +38,7 @@ def test_header_is_plain_c_and_cites_the_reference():
         assert anchor in hdr, anchor
     # the header compiles as C99
     src = '#include "rt_core.h"\nint main(void){ rt_per_frame_constants f; (void)f; return sizeof(rt_hit) == 32 ? 0 : 1; }\n'
-    exe = "/tmp/rt_core_c99_check"
+    exe = str(tmp_path / "rt_core_c99_check")
     subprocess.run(["gcc", "-std=c99", "-Wall", "-Werror", "-I", os.path.join(ROOT, "include"), "-x", "c", "-", "-o", exe],
                    input=src, text=True, check=True)
     assert subprocess.run([exe]).returncode == 0

@@ -13,7 +13,6 @@ from dxrexperiments_b200 import scenes, types as T
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REF_TEX = "/root/reference/assets/textures"
 
 
 # ---------------------------------------------------------------------------------------------- RNG
@@ -125,33 +124,9 @@ def test_oracle_denoiser_matches_the_independent_statement(k, mode, tonemap, gam
     np.testing.assert_allclose(out[..., :3], final, rtol=3e-5, atol=3e-6)
 
 
-def _load_reference_mock_inputs():
-    """The reference's own mock denoiser inputs (src/DenoiseCompositor.cpp:52-60), 1922 x 1126, as WIC decodes them: 8-bit
-    UNORM -> float / 255.  Only present in the build container."""
-    from PIL import Image
-    d = np.asarray(Image.open(os.path.join(REF_TEX, "DirectLighting.PNG")).convert("RGBA"), np.float32) / np.float32(255.0)
-    s = np.asarray(Image.open(os.path.join(REF_TEX, "IndirectSpecular.PNG")).convert("RGBA"), np.float32) / np.float32(255.0)
-    return np.ascontiguousarray(d), np.ascontiguousarray(s)
-
-
-def test_oracle_denoiser_on_the_reference_mock_inputs_full_size(orc):
-    if not os.path.exists(os.path.join(REF_TEX, "DirectLighting.PNG")):
-        pytest.skip("reference checkout not present")
-    direct, spec = _load_reference_mock_inputs()
-    assert direct.shape == (1126, 1922, 4) and spec.shape == (1126, 1922, 4)
-    out, tmp = orc.denoise(direct, spec, T.DenoiserParams(1.0, 2.2, 1, 0, 12, 0), threads=8)
-    hp, final = cf.denoise_reference(direct, spec, k=12)
-    ok = np.isfinite(final).all(axis=-1)  # 0/0 where a whole window has zero weight: NaN on both sides
-    assert ok.mean() > 0.99
-    np.testing.assert_allclose(out[..., :3][ok], final[ok], rtol=3e-5, atol=3e-6)
-    # the committed crop (tests/golden/make_golden.py crops these very files) must be what the full-size run contains
-    g = np.load(os.path.join(GOLDEN, "denoise_mock_crop.npz"))
-    y0, x0 = int(g["origin"][0]), int(g["origin"][1])
-    hh, ww = g["direct_u8"].shape[:2]
-    np.testing.assert_array_equal((direct[y0:y0 + hh, x0:x0 + ww] * 255.0 + 0.5).astype(np.uint8), g["direct_u8"])
-
-
 def _mock_crop():
+    """A 192 x 128 crop of the reference's own mock denoiser inputs (src/DenoiseCompositor.cpp:52-60, 1922 x 1126 8-bit
+    PNGs), as WIC decodes them: 8-bit UNORM -> float / 255."""
     g = np.load(os.path.join(GOLDEN, "denoise_mock_crop.npz"))
     return g["direct_u8"].astype(np.float32) / np.float32(255.0), g["spec_u8"].astype(np.float32) / np.float32(255.0)
 
