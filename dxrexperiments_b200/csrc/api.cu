@@ -36,13 +36,6 @@ int rt_context_create(int device, rt_context **out) {
     cudaDeviceProp prop;
     RT_CUDA(cudaGetDeviceProperties(&prop, device));
     ctx->num_sms = prop.multiProcessorCount;
-    if (const char *g = getenv("RT_L2_FETCH_GRANULARITY")) {  // development knob (A/B of the build's gather passes): 32, 64 or 128 bytes
-        size_t before = 0, after = 0;
-        cudaDeviceGetLimit(&before, cudaLimitMaxL2FetchGranularity);
-        cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, size_t(atoi(g)));
-        cudaDeviceGetLimit(&after, cudaLimitMaxL2FetchGranularity);
-        fprintf(stderr, "rt_core: L2 fetch granularity %zu -> %zu\n", before, after);
-    }
     RT_CUDA(cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
     ctx->owns_stream = true;
     RT_CUDA(cudaMalloc(&ctx->status, 256));

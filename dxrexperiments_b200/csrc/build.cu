@@ -395,12 +395,6 @@ struct KarrasDev {
 #define RT_FIT_BLOCK 256
 #endif
 constexpr int kFitBlock = RT_FIT_BLOCK;
-#ifndef RT_FIT_LOCAL
-#define RT_FIT_LOCAL 1  // 0: the global-atomic k_fit for every level (A/B measurements)
-#endif
-#ifndef RT_LBVH_FUSED
-#define RT_LBVH_FUSED 1  // 0: k_hierarchy + k_fit_local + k_fit_exits also for PREFER_FAST_BUILD (A/B measurements)
-#endif
 __global__ void __launch_bounds__(kThreads) k_hierarchy(const uint32_t *codes, uint32_t n, rt_hierarchy_node *nodes, uint8_t *local) {
     int idx = blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= int(n) - 1) return;
@@ -444,20 +438,12 @@ __global__ void __launch_bounds__(kThreads) k_hierarchy(const uint32_t *codes, u
 }
 
 // ------------------------------------------------------------------------------------------ rearrange
-#ifndef RT_GATHER_L2_HINT
-#define RT_GATHER_L2_HINT 64  // ld.global.L2::64B for the random 48-byte record gather (A/B at 10 M triangles: 2.116 -> 2.069 ms); 0: ld.global.cs
-#endif
-#if RT_GATHER_L2_HINT
+// The 48-byte records are gathered in random order: L2::64B caps the L2 prefetch of each load at 64 bytes.
 __device__ __forceinline__ uint4 ld_gather16(const uint4 *p) {
     uint4 v;
-#if RT_GATHER_L2_HINT == 64
     asm volatile("ld.global.L2::64B.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-#else
-    asm volatile("ld.global.cs.L2::128B.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-#endif
     return v;
 }
-#endif
 // FL/RearrangeTriangles.hlsl:18-36: out[dst] = in[perm[dst]]; also emits the packed 48-byte triangle.
 __global__ void __launch_bounds__(kThreads) k_rearrange_tris(const rt_packed_tri *recs, const uint32_t *perm, uint32_t n,
                                                              rt_primitive *out_prims, rt_primitive_meta *out_meta, rt_packed_tri *packed) {
@@ -471,11 +457,7 @@ __global__ void __launch_bounds__(kThreads) k_rearrange_tris(const rt_packed_tri
         const uint32_t src = perm[b0 + threadIdx.x];
         const uint4 *q = reinterpret_cast<const uint4 *>(recs + src);
         // each record is read exactly once
-#if RT_GATHER_L2_HINT
         s_rec[3 * threadIdx.x] = ld_gather16(q), s_rec[3 * threadIdx.x + 1] = ld_gather16(q + 1), s_rec[3 * threadIdx.x + 2] = ld_gather16(q + 2);
-#else
-        s_rec[3 * threadIdx.x] = __ldcs(q), s_rec[3 * threadIdx.x + 1] = __ldcs(q + 1), s_rec[3 * threadIdx.x + 2] = __ldcs(q + 2);
-#endif
     }
     __syncthreads();
     const uint32_t *sw = reinterpret_cast<const uint32_t *>(s_rec);  // 12 words per element
@@ -1744,9 +1726,9 @@ static int build_common(rt_context *ctx, uint32_t n, bool top, uint32_t flags, u
     uint32_t *sort_cache = reinterpret_cast<uint32_t *>(result + R.sort_cache);
     uint32_t *parents = reinterpret_cast<uint32_t *>(result + R.parents);
     // one byte per internal node in the sort's dead ping-pong buffer (the sorted pairs end up in keysC / valsC)
-    uint8_t *fit_local = (!top && RT_FIT_LOCAL) ? scratch + L.keysB : nullptr;
+    uint8_t *fit_local = !top ? scratch + L.keysB : nullptr;
     // full bottom-level build without treelet passes or update caches: hierarchy emission and fit are one kernel (k_lbvh_fit)
-    const bool fused = !top && !update && RT_FIT_LOCAL && RT_LBVH_FUSED && treelet_passes(flags) == 0 && !allows_update(flags);
+    const bool fused = !top && !update && treelet_passes(flags) == 0 && !allows_update(flags);
     if (update) {
         k_invert_cache<<<grid, kThreads, 0, st>>>(sort_cache, n, perm);
         ctx->launches++;
@@ -1833,7 +1815,7 @@ static int build_common(rt_context *ctx, uint32_t n, bool top, uint32_t flags, u
     } else {
         if (update)
             k_fit<false, true><<<grid, kThreads, 0, st>>>(n, hier, counters, nodes, sp, nullptr, perm, wide, ext, parents);
-        else if (RT_FIT_LOCAL) {
+        else {
             // exit list in the sort's dead ping-pong buffers: node ids in valsB, subtree sizes (<= kFitBlock) behind the flags.
             // keysB holds 4n bytes; flags take n, the sizes 2 x (exit entries <= n) after a 256-byte round-up, and a build of
             // n <= kFitBlock primitives fits in one block and leaves no entries — so the 3n + 255 bytes used fit for every n
@@ -1851,8 +1833,6 @@ static int build_common(rt_context *ctx, uint32_t n, bool top, uint32_t flags, u
                 ctx->launches++;
             }
         }
-        else
-            k_fit<false, false><<<grid, kThreads, 0, st>>>(n, hier, counters, nodes, sp, nullptr, perm, wide, ext, parents);
     }
     ctx->launches++;
     if (n > 1 && !fitted_locally) {  // k_fit_local / k_fit_exits write the 4-wide nodes themselves

@@ -47,20 +47,12 @@ __device__ __forceinline__ float4 fetch(const float4 *img, int x, int y, int w, 
     return __ldg(img + size_t(y) * w + x);
 }
 
-[[maybe_unused]] __device__ __forceinline__ float range_weight(float sx, float sy, float sz, float cx, float cy, float cz) {
-    float dist = ((fabsf(sx - cx) + fabsf(sy - cy)) + fabsf(sz - cz)) * 10.0f;
-    return 1.0f - fminf(fmaxf(dist, 0.0f), 1.0f);
-}
-
 __device__ __forceinline__ int hpad(int c) { return c + (c >> 3); }
 
 // Packed fp32 pairs (sm_100 FADD2 / FMUL2 / FFMA2: two IEEE round-to-nearest operations per issue slot, each lane's result
 // bit-identical to the scalar instruction).  The kernel is issue-bound (ncu: 66 % of the issue slots, DRAM 16 %), so the
 // filter's (texel, output) work is done for two neighbouring outputs per instruction wherever the operation has a packed
 // form; |x| and saturate only exist as scalar operand modifiers and stay scalar.
-#ifndef RT_DENOISE_PACKED
-#define RT_DENOISE_PACKED 1
-#endif
 typedef unsigned long long f32x2;
 __device__ __forceinline__ f32x2 pk2(float lo, float hi) {
     f32x2 r;
@@ -99,8 +91,8 @@ __global__ void __launch_bounds__(kThreadsDn, 3) k_denoise(const __grid_constant
     float *pl = smem + 64;       // planes: in.r in.g in.b joint.r joint.g joint.b
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int k = A.k;
-    if (threadIdx.x < 64) {  // sW[RT_DENOISE_PACKED + jj] = weight of tap i = jj - k; zero outside the kernel
-        const int i = int(threadIdx.x) - RT_DENOISE_PACKED - k;
+    if (threadIdx.x < 64) {  // sW[1 + jj] = weight of tap i = jj - k; zero outside the kernel
+        const int i = int(threadIdx.x) - 1 - k;
         sW[threadIdx.x] = (i >= -k && i <= k) ? A.wts[i + MAX_EXTENT] : 0.0f;
     }
     // ---- stage the tile and the +-k halo along the filter axis
@@ -155,7 +147,6 @@ __global__ void __launch_bounds__(kThreadsDn, 3) k_denoise(const __grid_constant
         // the order i = -k .. k.  The tap weight w[jj - r] lives in ring slot (jj - r) & 7: a slot is written once, when
         // its texel is fetched (r = 0), and read by output r exactly r steps later, so with the jj loop unrolled by 8
         // all slot indices are compile-time constants — one weight fetch per texel instead of one per tap.
-#if RT_DENOISE_PACKED
         // Outputs r and r + 1 share every instruction that has a packed form.  A tap past an output's last one needs no
         // test: its weight sW[jj - r] is 0 there, and x + 0 * s is x (s is finite), so such a half-pair is value-neutral.
         f32x2 cx2[R / 2], cy2[R / 2], cz2[R / 2], ar2[R / 2], ag2[R / 2], ab2[R / 2], aw2[R / 2];
@@ -204,32 +195,6 @@ __global__ void __launch_bounds__(kThreadsDn, 3) k_denoise(const __grid_constant
             upk2(ar2[h], ar[2 * h], ar[2 * h + 1]), upk2(ag2[h], ag[2 * h], ag[2 * h + 1]);
             upk2(ab2[h], ab[2 * h], ab[2 * h + 1]), upk2(aw2[h], aw[2 * h], aw[2 * h + 1]);
         }
-#else
-        float ring[8];
-        auto block = [&](const int b, auto firstTag, auto checkTag) {
-            constexpr bool FIRST = decltype(firstTag)::value, CHECK = decltype(checkTag)::value;
-#pragma unroll
-            for (int p = 0; p < 8; ++p) {
-                const int jj = 8 * b + p;
-                const float *q = at(jj - k);
-                const float sx = q[0], sy = q[PLANE], sz = q[2 * PLANE], jx = q[3 * PLANE], jy = q[4 * PLANE], jz = q[5 * PLANE];
-                ring[p] = sW[jj];
-#pragma unroll
-                for (int r = 0; r < R; ++r) {
-                    if (FIRST && p < r) continue;          // jj - r < 0: before the first tap of output r
-                    if (CHECK && jj - r > 2 * k) continue;  // past its last tap
-                    const float bw = ring[(p - r) & 7] * range_weight(jx, jy, jz, cjx[r], cjy[r], cjz[r]);
-                    ar[r] = __fmaf_rn(sx, bw, ar[r]), ag[r] = __fmaf_rn(sy, bw, ag[r]), ab[r] = __fmaf_rn(sz, bw, ab[r]);
-                    aw[r] += bw;
-                }
-            }
-        };
-        const int nblocks = (2 * k + R + 7) / 8, nfull = (2 * k + 1) / 8;  // blocks b < nfull have jj <= 2k for every p
-        block(0, std::true_type{}, std::integral_constant<bool, true>{});
-        int b = 1;
-        for (; b < nfull; ++b) block(b, std::false_type{}, std::false_type{});
-        for (; b < nblocks; ++b) block(b, std::false_type{}, std::true_type{});
-#endif
     }
     if (PASS == 0) {
         // results go back through shared memory (the input planes are dead) so that the global stores are coalesced

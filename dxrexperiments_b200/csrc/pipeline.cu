@@ -139,14 +139,7 @@ __device__ __forceinline__ void flush_stats(const TraceCtr &c, uint32_t rays, un
 #ifndef RT_DISPATCH_BANDS
 #define RT_DISPATCH_BANDS 2  // pixel bands per dispatch (1 = off, at most RT_MAX_BANDS)
 #endif
-#ifndef RT_OVERLAP_SHADOW
-#define RT_OVERLAP_SHADOW 1
-#endif
 // ------------------------------------------------------------------------------------------------ K1
-#ifndef RT_PRIMARY_WIDE4
-#define RT_PRIMARY_WIDE4 1  // coherent camera rays over the 4-wide nodes at 6 blocks/SM (80 registers): with the treelet-optimised tree
-                           // 5.84 vs 5.40 Grays/s on C2, 3.29 vs 2.79 on 1.3 M triangles (before the treelet pass the BVH2 loop won on C2)
-#endif
 #ifndef RT_PRIMARY_MIN_BLOCKS
 #define RT_PRIMARY_MIN_BLOCKS 7  // 72 registers: the kernel is latency-bound (26 % of the warp slots active at 6 blocks); A/B round 2: 5 / 6 / 7 / 8
                                  // blocks per SM = 5363 / 5767 / 6103 / 5802 Mrays/s on C2, 3053 / 3160 / 3329 / 3035 on 1.31 M triangles
@@ -160,28 +153,13 @@ __global__ void __launch_bounds__(kBlock, RT_PRIMARY_MIN_BLOCKS) k_primary(const
     const uint32_t lx = (tile % tilesX) * 8 + (lane & 7), ly = (tile / tilesX) * 4 + (lane >> 3);
     const bool inside = lx < L.rw && ly < L.rh;
     TraceCtr ctr{0, 0, 0, 0};
-#if RT_PRIMARY_PHASES && RT_PRIMARY_WIDE4
-    if (!STATS) {  // warp-synchronous traversal: every lane takes part in the votes, lanes outside the image carry no ray
-        f3 o = mk3(0.0f, 0.0f, 0.0f), d = mk3(0.0f, 0.0f, 1.0f);
-        if (inside) primary_ray(L.f, L.width, L.height, L.x0 + lx, image_row(L, ly), L.jitterScale, o, d);
-        TraceAccel A = resolve_tlas(tlas, status);
-        TraceHit h;
-        trace_ray4(A, o.x, o.y, o.z, 0.0f, d.x, d.y, d.z, RT_RAY_MAX_T, RT_RAY_FLAG_CULL_BACK_FACING_TRIANGLES, 0xFF, 0, h, status, inside);
-        if (inside) {
-            const uint32_t p = ly * L.rw + lx;
-            ws.hitA[p] = make_float4(h.t, h.u, h.v, __uint_as_float(h.prim));
-            ws.hitRec[p] = h.record;
-        }
-        return;
-    }
-#endif
     if (inside) {
         const uint32_t x = L.x0 + lx, y = image_row(L, ly);
         f3 o, d;
         primary_ray(L.f, L.width, L.height, x, y, L.jitterScale, o, d);
         TraceAccel A = resolve_tlas(tlas, status);
         TraceHit h;
-        if (STATS || !RT_PRIMARY_WIDE4)  // instrumented: BVH2 in the reference's visit order
+        if (STATS)  // instrumented: BVH2 in the reference's visit order
             trace_ray<false, STATS>(A, o.x, o.y, o.z, 0.0f, d.x, d.y, d.z, RT_RAY_MAX_T, RT_RAY_FLAG_CULL_BACK_FACING_TRIANGLES, 0xFF, 0, 0, h,
                                     &ctr, status);
         else
@@ -244,9 +222,6 @@ __device__ __forceinline__ void write_pixel(const Launch &L, float *out, uint64_
 // memory inside the shading kernel (one global atomic per block); no pass over the queues, no extra launch.
 // The reference has no counterpart: the Fallback Layer traces in fixed 8x8 pixel groups and never reorders rays
 // (FL/UberShaderRayTracingProgram.cpp:268-272).
-#ifndef RT_COHERENCE_BINS
-#define RT_COHERENCE_BINS 1  // 0: slots in pixel order within the tile (A/B measurements)
-#endif
 constexpr int kShadeTile = 16;                     // pixels per tile edge
 constexpr int kShadeThreads = kShadeTile * kShadeTile;
 constexpr int kBins = 32;                          // 4 record classes x 8 octants
@@ -382,7 +357,6 @@ __global__ void __launch_bounds__(kShadeThreads) k_shade_primary(const __grid_co
     // ---- slot allocation: counting sort of the tile's hits by bin
     const int lane = threadIdx.x & 31;
     uint32_t slot = 0xffffffffu;
-#if RT_COHERENCE_BINS
     __syncthreads();  // s_count cleared
     uint32_t inWarp = 0, warpBase = 0;
     {
@@ -409,9 +383,6 @@ __global__ void __launch_bounds__(kShadeThreads) k_shade_primary(const __grid_co
     }
     __syncthreads();
     if (isHit) slot = s_base + s_offset[bin] + warpBase + inWarp;
-#else
-    slot = warp_alloc(isHit, &ws.counters[0]);
-#endif
     if (isHit) {
         const size_t pl = ws.plane;
         for (uint32_t k = 0; k < L.shadowsPerHit; ++k)
@@ -959,7 +930,7 @@ static int dispatch_band(rt_context *ctx, rt_program *prog, const Launch &L, con
     // k_shade_primary and meet again in k_resolve.  Outside the instrumented / per-stage-timed modes the shadow wave
     // runs on a side stream: its persistent blocks move in as the other kernels' blocks drain, so the tails of the
     // trace kernels (8-20 % of each launch with warps running out of rays, ncu sm__warps_active) overlap.
-    const bool overlap = RT_OVERLAP_SHADOW && !timing && !stats && side != nullptr;
+    const bool overlap = !timing && !stats && side != nullptr;
     if (overlap) {
         RT_CUDA(cudaEventRecord(ev_fork, st));
         RT_CUDA(cudaStreamWaitEvent(side, ev_fork, 0));

@@ -54,26 +54,12 @@ struct RayPre {  // GetRayData: TraverseFunction.hlsli:438-460
 // Component k of (x, y, z) as two select instructions.  Written as the nested conditional `k == 0 ? x : (k == 1 ? y : z)`
 // nvcc 12.9 emits a BRANCH per pick (BSSY / ISETP / BRA / MOV / BSYNC): ncu attributed 31 % of the closest-hit kernel's warp
 // instructions to the nine picks of the watertight triangle test, executed at 7-8 lanes.
-#ifndef RT_PUSH_BRANCHFREE
-#define RT_PUSH_BRANCHFREE 0  // 1: wide4_step stores every candidate and lets the stack pointer keep it or not, no branches.  Measured: the
-                              // unconditional local-memory stores cost far more than the branches (C2 primary 6744 -> 5570, incoherent 4816 -> 4436)
-#endif
-#ifndef RT_TRIANGLE_BRANCHFREE
-#define RT_TRIANGLE_BRANCHFREE 1  // 0: the reference's chain of early exits (A/B on C2: incoherent 4739 -> 4816, shadow 5242 -> 5280 Mrays/s)
-#endif
-#ifndef RT_PICK_SELP
-#define RT_PICK_SELP 1  // 0: the nested conditional (A/B)
-#endif
 __device__ __forceinline__ float pick(float x, float y, float z, int k) {
-#if RT_PICK_SELP
     float r;
     asm("{\n\t.reg .pred p0, p1;\n\tsetp.eq.s32 p0, %4, 0;\n\tsetp.eq.s32 p1, %4, 1;\n\tselp.f32 %0, %2, %3, p1;\n\tselp.f32 %0, %1, %0, p0;\n\t}"
         : "=f"(r)
         : "f"(x), "f"(y), "f"(z), "r"(k));
     return r;
-#else
-    return k == 0 ? x : (k == 1 ? y : z);
-#endif
 }
 
 // The part of GetRayData the ray/box test needs: o, 1/d, o*(1/d).
@@ -153,7 +139,6 @@ __device__ __forceinline__ bool ray_triangle(float &hitT, float &bu, float &bv, 
     float V = sub_(mul_(Ax, Cy), mul_(Ay, Cx));
     float W = sub_(mul_(Bx, Ay), mul_(By, Ax));
     float det = add_(add_(U, V), W);
-#if RT_TRIANGLE_BRANCHFREE
     // The reference's early exits (:236-262) as ONE exit: a lane that leaves early only waits for the other lanes of its
     // warp, and every exit costs a convergence barrier.  min / max of (U, V, W) give "some edge function is negative /
     // positive" with the comparisons' own NaN behaviour (fminf / fmaxf return the non-NaN operand).
@@ -168,32 +153,31 @@ __device__ __forceinline__ bool ray_triangle(float &hitT, float &bu, float &bv, 
     const bool bad2 = T > 0.0f || T < hd, bad1 = T < 0.0f || T > hd, bad0 = sT < 0.0f || sT > had;
     bad = bad || (cull == 2 ? bad2 : (cull == 1 ? bad1 : bad0));
     if (bad) return false;
-#else
-    if (cull == 2) {
-        if (U > 0.0f || V > 0.0f || W > 0.0f) return false;
-    } else if (cull == 1) {
-        if (U < 0.0f || V < 0.0f || W < 0.0f) return false;
-    } else {
-        if ((U < 0.0f || V < 0.0f || W < 0.0f) && (U > 0.0f || V > 0.0f || W > 0.0f)) return false;
-    }
-    if (det == 0.0f) return false;
-    Az = mul_(r.sz, Az), Bz = mul_(r.sz, Bz), Cz = mul_(r.sz, Cz);
-    float T = add_(add_(mul_(U, Az), mul_(V, Bz)), mul_(W, Cz));
-    if (cull == 2) {
-        if (T > 0.0f || T < mul_(hitT, det)) return false;
-    } else if (cull == 1) {
-        if (T < 0.0f || T > mul_(hitT, det)) return false;
-    } else {
-        float s = fabsf(T);
-        if ((T > 0.0f) != (det > 0.0f)) s = -s;
-        if (s < 0.0f || s > mul_(hitT, fabsf(det))) return false;
-    }
-#endif
     float rcpDet = div_(1.0f, det);
     bu = mul_(V, rcpDet);
     bv = mul_(W, rcpDet);
     hitT = mul_(T, rcpDet);
     return true;
+}
+
+// The `cull` argument of ray_triangle for a ray entering an instance: TraverseFunction.hlsli:215-220.
+__device__ __forceinline__ int cull_mode(uint32_t instFlags, uint32_t rayFlags) {
+    const bool useCulling = !(instFlags & RT_INSTANCE_FLAG_TRIANGLE_CULL_DISABLE);
+    const bool flip = (instFlags & RT_INSTANCE_FLAG_TRIANGLE_FRONT_COUNTERCLOCKWISE) != 0;
+    const uint32_t backFlag = flip ? RT_RAY_FLAG_CULL_FRONT_FACING_TRIANGLES : RT_RAY_FLAG_CULL_BACK_FACING_TRIANGLES;
+    const uint32_t frontFlag = flip ? RT_RAY_FLAG_CULL_BACK_FACING_TRIANGLES : RT_RAY_FLAG_CULL_FRONT_FACING_TRIANGLES;
+    return (useCulling && (rayFlags & frontFlag)) ? 2 : ((useCulling && (rayFlags & backFlag)) ? 1 : 0);
+}
+
+// IsOpaque(): TraverseFunction.hlsli:119-134.  The geometry flag, overridden by the instance's FORCE_(NON_)OPAQUE,
+// overridden by the ray's.
+__device__ __forceinline__ bool is_opaque(uint32_t geomFlags, uint32_t instFlags, uint32_t rayFlags) {
+    bool opaque = (geomFlags & RT_GEOMETRY_FLAG_OPAQUE) != 0;
+    if (instFlags & RT_INSTANCE_FLAG_FORCE_OPAQUE) opaque = true;
+    else if (instFlags & RT_INSTANCE_FLAG_FORCE_NON_OPAQUE) opaque = false;
+    if (rayFlags & RT_RAY_FLAG_FORCE_OPAQUE) opaque = true;
+    else if (rayFlags & RT_RAY_FLAG_FORCE_NON_OPAQUE) opaque = false;
+    return opaque;
 }
 
 // `status` != nullptr: the caller's kernels know triangles only (hit groups of type TRIANGLES).  A TLAS that reaches
@@ -218,17 +202,7 @@ __device__ __forceinline__ TraceAccel resolve_tlas(const void *tlas_result, uint
     return a;
 }
 
-#ifndef RT_PRIMARY_PHASES
-#define RT_PRIMARY_PHASES 0  // 1: trace_ray4 votes per iteration between a box step and a triangle step (see there)
-#endif
-#ifndef RT_PRIMARY_LEAF_THRESHOLD
-#define RT_PRIMARY_LEAF_THRESHOLD 8
-#endif
 #define RT_SENTINEL 0x7fffffffu  // never a valid internal index (indices are < 2^24)
-
-#ifndef RT_LDG256
-#define RT_LDG256 1  // fetch 4-wide nodes with four 256-bit loads instead of eight 128-bit ones
-#endif
 
 // Sorting key of a child hit: the entry distance (>= 0, so its bits order like the float) with the slot number in
 // the two lowest mantissa bits; a miss sorts last.
@@ -253,58 +227,32 @@ __device__ __forceinline__ uint32_t ref_of(uint32_t key, uint32_t r0, uint32_t r
 // One internal step over a 4-wide node: test the four child boxes (RayBoxTest arithmetic unchanged), order the
 // hits near-to-far with a 5-exchange network on integer keys, return the nearest and push the others farthest
 // first.  WITH_T: also record each pushed node's entry distance so that it can be dropped at pop time.
-#ifndef RT_SHADOW_UNSORTED
-#define RT_SHADOW_UNSORTED 1  // any-hit rays take the children in slot order: no sorting network (A/B: shadow rays 3.44 -> 4.55 Grays/s on C2;
-                              // reverse slot order, area-ordered slots and "nearest first, rest unsorted" for closest hits all measured worse)
-#endif
 // The traversal stack is a policy type S with  bool room(sp, n)  and  void push(sp, ref, key):
-//   LocalStack  — 64 entries (+ entry distances) in local memory: the one-thread-one-ray loops (k_primary)
-//   the persistent kernels' stack keeps its first entries in shared memory (trace_persistent.cuh).
+//   LocalStack   — 64 entries (+ entry distances) in local memory: the one-thread-one-ray loop (k_primary)
+//   PersistStack — 64 entries, no distances: the persistent kernels (trace_persistent.cuh)
 struct LocalStack {
     uint32_t ref[RT_STACK_SIZE], key[RT_STACK_SIZE];
     __device__ __forceinline__ bool room(int sp, int n) const { return sp + n <= RT_STACK_SIZE; }
     __device__ __forceinline__ void push(int &sp, uint32_t r, uint32_t k) { ref[sp] = r, key[sp] = k, ++sp; }
-    // store always, keep the slot only if `keep`: no branch (the caller has checked room())
-    __device__ __forceinline__ void push_if(int &sp, uint32_t r, uint32_t k, bool keep) { ref[sp] = r, key[sp] = k, sp += keep ? 1 : 0; }
 };
 
 template <bool WITH_T, bool SORTED = true, class S>
 __device__ __forceinline__ uint32_t wide4_step(const rt_wide4_node *nodes, uint32_t ref, const RayPre &cur, float tCur, S &stk, int &sp,
                                                uint32_t *status) {
     const float4 *np = reinterpret_cast<const float4 *>(nodes + ref);
-#if RT_LDG256
     float4 c0, h0, c1, h1, c2, h2, c3, h3;
     ldg256(np, c0, h0), ldg256(np + 2, c1, h1), ldg256(np + 4, c2, h2), ldg256(np + 6, c3, h3);
-#else
-    const float4 c0 = __ldg(np), h0 = __ldg(np + 1), c1 = __ldg(np + 2), h1 = __ldg(np + 3);
-    const float4 c2 = __ldg(np + 4), h2 = __ldg(np + 5), c3 = __ldg(np + 6), h3 = __ldg(np + 7);
-#endif
     float t0, t1, t2, t3;
     const bool b0 = ray_box(t0, tCur, cur, c0.x, c0.y, c0.z, h0.x, h0.y, h0.z);
     const bool b1 = ray_box(t1, tCur, cur, c1.x, c1.y, c1.z, h1.x, h1.y, h1.z);
     const bool b2 = ray_box(t2, tCur, cur, c2.x, c2.y, c2.z, h2.x, h2.y, h2.z);
     const bool b3 = ray_box(t3, tCur, cur, c3.x, c3.y, c3.z, h3.x, h3.y, h3.z);
     const uint32_t r0 = __float_as_uint(c0.w), r1 = __float_as_uint(c1.w), r2 = __float_as_uint(c2.w), r3 = __float_as_uint(c3.w);
-#if RT_SHADOW_UNSORTED
     if (!SORTED) {
         // any-hit rays: visibility does not depend on the visiting order, so the children are taken in slot order
         uint32_t first = RT_SENTINEL;
         const bool v[4] = {b0, b1, b2 && r2 != RT_WIDE4_EMPTY, b3 && r3 != RT_WIDE4_EMPTY};
         const uint32_t r[4] = {r0, r1, r2, r3};
-#if RT_PUSH_BRANCHFREE
-        // Hits leave in slot order: the lowest hit slot is visited next, the others are pushed highest first.  Written
-        // without branches: every candidate is STORED at the top of the stack and the stack pointer keeps it or not
-        // (the nested conditionals were 8 % of the shadow kernel's warp instructions, most of them convergence barriers).
-        if (stk.room(sp, 3)) {
-            first = select_u32(v[3], r[3], first);
-#pragma unroll
-            for (int k = 2; k >= 0; --k) {
-                stk.push_if(sp, first, 0u, v[k] && first != RT_SENTINEL);
-                first = select_u32(v[k], r[k], first);
-            }
-            return first;
-        }
-#endif
 #pragma unroll
         for (int k = 3; k >= 0; --k) {
             if (v[k]) {
@@ -317,21 +265,12 @@ __device__ __forceinline__ uint32_t wide4_step(const rt_wide4_node *nodes, uint3
         }
         return first;
     }
-#endif
     // slots 2 and 3 may be empty; their half = -1 box fails the slab test of every ray except one whose slabs are all
     // NaN (a zero direction passes every box, in the reference too), hence the explicit check
     uint32_t k0 = hit_key(b0, t0, 0), k1 = hit_key(b1, t1, 1), k2 = hit_key(b2 && r2 != RT_WIDE4_EMPTY, t2, 2),
              k3 = hit_key(b3 && r3 != RT_WIDE4_EMPTY, t3, 3);
     key_cas(k0, k1), key_cas(k2, k3), key_cas(k0, k2), key_cas(k1, k3), key_cas(k1, k2);
     if (k0 == 0xffffffffu) return RT_SENTINEL;
-#if RT_PUSH_BRANCHFREE
-    if (stk.room(sp, 3)) {  // the other hits, farthest first: stored unconditionally, kept if they are hits
-        stk.push_if(sp, ref_of(k3, r0, r1, r2, r3), k3, k3 != 0xffffffffu);
-        stk.push_if(sp, ref_of(k2, r0, r1, r2, r3), k2, k2 != 0xffffffffu);
-        stk.push_if(sp, ref_of(k1, r0, r1, r2, r3), k1, k1 != 0xffffffffu);
-        return ref_of(k0, r0, r1, r2, r3);
-    }
-#endif
     if (k1 != 0xffffffffu) {  // push the other hits, farthest first
         if (!stk.room(sp, 3)) {
             atomicOr(status, 1u);
@@ -349,30 +288,19 @@ __device__ __forceinline__ uint32_t wide4_step(const rt_wide4_node *nodes, uint3
 // any-hit / opaque-flag handling: the caller's rays carry only cull flags (RayGen: CULL_BACK_FACING_TRIANGLES).
 __device__ __forceinline__ bool trace_ray4(const TraceAccel &A, float ox, float oy, float oz, float tmin, float dx, float dy, float dz,
                                            float tmax, uint32_t rayFlags, uint32_t mask, uint32_t rayContribution, TraceHit &hit,
-                                           uint32_t *status, bool valid = true) {
+                                           uint32_t *status) {
     hit.prim = RT_NO_HIT;
     hit.t = tmax;
     hit.u = hit.v = 0.0f;
     hit.inst_index = hit.geom_index = hit.inst_id = hit.leaf_slot = hit.record = 0;
-#if RT_PRIMARY_PHASES
-    // Warp-synchronous variant: EVERY lane of the warp calls (valid = false for lanes without a ray) and the warp votes,
-    // per iteration, between a box step for the lanes at internal nodes and a triangle step for the lanes at leaves,
-    // instead of running both sides of the branch with complementary lane masks.
-    bool alive = valid && A.count != 0;
-#else
     if (A.count == 0) return false;
-#endif
     LocalStack stk;
     int sp = 0, blasBase = -1;
     float tCur = tmax;
     RayPre cur;
     ray_pre_box<true>(cur, ox, oy, oz, dx, dy, dz);
     float tUnused;
-#if RT_PRIMARY_PHASES
-    alive = alive && ray_box(tUnused, tCur, cur, A.root_c[0], A.root_c[1], A.root_c[2], A.root_h[0], A.root_h[1], A.root_h[2]);
-#else
     if (!ray_box(tUnused, tCur, cur, A.root_c[0], A.root_c[1], A.root_c[2], A.root_h[0], A.root_h[1], A.root_h[2])) return false;
-#endif
     const bool plain = [&] {
         const float v[6] = {ox, oy, oz, dx, dy, dz};
         bool p = true;
@@ -389,19 +317,8 @@ __device__ __forceinline__ bool trace_ray4(const TraceAccel &A, float ox, float 
     uint32_t instIndex = 0, instOffset = 0, instId = 0;
     int cull = 0;
     uint32_t ref = A.root_ref;
-#if RT_PRIMARY_PHASES
-    while (true) {
-        const unsigned aliveMask = __ballot_sync(0xffffffffu, alive);
-        if (aliveMask == 0) break;
-        const bool atLeaf = alive && (ref & RT_NODE_LEAF_FLAG);
-        const unsigned leafMask = __ballot_sync(0xffffffffu, atLeaf);
-        const bool leafPhase = (aliveMask & ~leafMask) == 0 || __popc(leafMask) >= RT_PRIMARY_LEAF_THRESHOLD;
-        if (leafPhase ? !atLeaf : (!alive || atLeaf)) continue;  // lanes of the other kind wait for their phase
-        if (leafPhase) {
-#else
     while (true) {
         if (ref & RT_NODE_LEAF_FLAG) {
-#endif
             const uint32_t slot = ref & 0x00ffffffu;
             ref = RT_SENTINEL;
             if (!bottom) {
@@ -409,13 +326,8 @@ __device__ __forceinline__ bool trace_ray4(const TraceAccel &A, float ox, float 
                 const uint4 m3 = __ldg(ip + 3);
                 if ((m3.x >> 24) & mask) {
                     const uint4 m4 = __ldg(ip + 4);
-                    const uint32_t instFlags = m3.y >> 24;
                     instIndex = m3.z, instOffset = m3.y & 0x00ffffffu, instId = m3.x & 0x00ffffffu;
-                    const bool useCulling = !(instFlags & RT_INSTANCE_FLAG_TRIANGLE_CULL_DISABLE);
-                    const bool flip = (instFlags & RT_INSTANCE_FLAG_TRIANGLE_FRONT_COUNTERCLOCKWISE) != 0;
-                    const uint32_t backFlag = flip ? RT_RAY_FLAG_CULL_FRONT_FACING_TRIANGLES : RT_RAY_FLAG_CULL_BACK_FACING_TRIANGLES;
-                    const uint32_t frontFlag = flip ? RT_RAY_FLAG_CULL_BACK_FACING_TRIANGLES : RT_RAY_FLAG_CULL_FRONT_FACING_TRIANGLES;
-                    cull = (useCulling && (rayFlags & frontFlag)) ? 2 : ((useCulling && (rayFlags & backFlag)) ? 1 : 0);
+                    cull = cull_mode(m3.y >> 24, rayFlags);
                     sameSpace = plain && (m3.y & RT_PACKED_INSTANCE_IDENTITY);
                     if (sameSpace) {
                         ray_pre_shear(cur, dx, dy, dz);
@@ -468,11 +380,7 @@ __device__ __forceinline__ bool trace_ray4(const TraceAccel &A, float ox, float 
                 ref = stk.ref[sp];
                 break;
             }
-#if RT_PRIMARY_PHASES
-            if (done) alive = false;
-#else
             if (done) break;
-#endif
         }
     }
     return hit.prim != RT_NO_HIT;
@@ -604,14 +512,7 @@ __device__ __forceinline__ bool trace_ray(const TraceAccel &A, float ox, float o
                     const float4 r2 = __ldg(reinterpret_cast<const float4 *>(ip + 2));
                     const uint4 m4 = __ldg(ip + 4);
                     instFlags = m3.y >> 24;
-                    // cull mode: TraverseFunction.hlsli:215-220
-                    {
-                        bool useCulling = !(instFlags & RT_INSTANCE_FLAG_TRIANGLE_CULL_DISABLE);
-                        bool flip = (instFlags & RT_INSTANCE_FLAG_TRIANGLE_FRONT_COUNTERCLOCKWISE) != 0;
-                        uint32_t backFlag = flip ? RT_RAY_FLAG_CULL_FRONT_FACING_TRIANGLES : RT_RAY_FLAG_CULL_BACK_FACING_TRIANGLES;
-                        uint32_t frontFlag = flip ? RT_RAY_FLAG_CULL_BACK_FACING_TRIANGLES : RT_RAY_FLAG_CULL_FRONT_FACING_TRIANGLES;
-                        cull = (useCulling && (rayFlags & frontFlag)) ? 2 : ((useCulling && (rayFlags & backFlag)) ? 1 : 0);
-                    }
+                    cull = cull_mode(instFlags, rayFlags);
                     const float m[12] = {r0.x, r0.y, r0.z, r0.w, r1.x, r1.y, r1.z, r1.w, r2.x, r2.y, r2.z, r2.w};
                     f3 o2 = xform_point(m, mk3(ox, oy, oz));
                     f3 d2 = xform_vector(m, mk3(dx, dy, dz));
@@ -629,11 +530,7 @@ __device__ __forceinline__ bool trace_ray(const TraceAccel &A, float ox, float o
                 const float4 *tp = reinterpret_cast<const float4 *>(tris + slot);
                 const float4 p0 = __ldg(tp), p1 = __ldg(tp + 1), p2 = __ldg(tp + 2);
                 const uint32_t gflags = __float_as_uint(p2.w);
-                bool opaque = (gflags & RT_GEOMETRY_FLAG_OPAQUE) != 0;  // IsOpaque(): :119-134
-                if (instFlags & RT_INSTANCE_FLAG_FORCE_OPAQUE) opaque = true;
-                else if (instFlags & RT_INSTANCE_FLAG_FORCE_NON_OPAQUE) opaque = false;
-                if (rayFlags & RT_RAY_FLAG_FORCE_OPAQUE) opaque = true;
-                else if (rayFlags & RT_RAY_FLAG_FORCE_NON_OPAQUE) opaque = false;
+                const bool opaque = is_opaque(gflags, instFlags, rayFlags);
                 const bool culled = (opaque && (rayFlags & RT_RAY_FLAG_CULL_OPAQUE)) || (!opaque && (rayFlags & RT_RAY_FLAG_CULL_NON_OPAQUE));
                 ref = RT_SENTINEL;
                 if (HOOKS) {

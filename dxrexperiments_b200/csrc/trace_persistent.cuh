@@ -8,7 +8,7 @@
 //     refills exactly those lanes (Aila & Laine's "dynamic fetch", warp-synchronous via __ballot_sync);
 //   * internal-node steps and leaf steps are separate warp-wide phases: a lane that reaches a leaf parks until
 //     kLeafThreshold lanes hold one (or nobody can advance), so the triangle test never runs for 1-2 lanes;
-//   * an internal step reads ONE 128-byte rt_wide4_node (eight 16-byte loads) and tests four boxes, i.e. two BVH2
+//   * an internal step reads ONE 128-byte rt_wide4_node (four 32-byte loads) and tests four boxes, i.e. two BVH2
 //     levels per dependent memory round trip — the kernel was latency-bound on the chain of node fetches
 //     (profiles/r1_ncu_trace_persistent.md); hits are ordered near-to-far with a 5-exchange network on integer keys;
 //   * the ray constants are only recomputed when the instance transform actually changes them.
@@ -27,9 +27,6 @@
 #endif
 #ifndef RT_INT_UNROLL
 #define RT_INT_UNROLL 2  // internal-node steps per phase selection (A/B on C2 / C1M: 2 = +3.8 / +4.4 % on incoherent rays, +5.3 / +2.9 % on shadow rays; 3 and 4 lose again)
-#endif
-#ifndef RT_LEAF_UNROLL
-#define RT_LEAF_UNROLL 1  // leaf steps per phase selection
 #endif
 constexpr int kFetchThreshold = RT_FETCH_THRESHOLD;  // refill when >= this many lanes are idle
 constexpr int kLeafThreshold = RT_LEAF_THRESHOLD;    // run a leaf phase when >= this many lanes hold a leaf
@@ -51,37 +48,14 @@ struct TraceSink {  // where results go; only the members of the kernel's MODE a
 #ifndef RT_PERSIST_MIN_BLOCKS
 #define RT_PERSIST_MIN_BLOCKS 8
 #endif
-#ifndef RT_PERSIST_WIDE4
-#define RT_PERSIST_WIDE4 1  // 1: traverse the 4-wide nodes (rt_wide4_node); 0: the BVH2 wide nodes (A/B measurements)
-#endif
-#ifndef RT_SMEM_STACK
-#define RT_SMEM_STACK 0  // > 0: the first RT_SMEM_STACK entries of every lane's stack in shared memory ([entry][thread], conflict free),
-                         // deeper ones in local memory.  Measured (profiles/r2_trace_ab.md): 8 entries in shared memory cost 6-9 % on
-                         // C2 / C1M — the kernel is issue-bound and the extra select between the two homes costs more than the
-                         // cheaper access saves; local memory is L1-resident on-chip SRAM already, so the default keeps the stack there
-#endif
 constexpr int kPersistThreads = 128;
 
-// Stack policy of wide4_step (trace.cuh) for the persistent lanes.
+// Stack policy of wide4_step (trace.cuh) for the persistent lanes.  It stays in local memory: the kernel is
+// issue-bound, and local memory is L1-resident on-chip SRAM already (profiles/r2_trace_ab.md).
 struct PersistStack {
-#if RT_SMEM_STACK > 0
-    uint32_t *sm;  // &s_stack[0][threadIdx.x]
-    uint32_t lm[RT_STACK_SIZE - RT_SMEM_STACK];
-    __device__ __forceinline__ void push(int &sp, uint32_t r, uint32_t) {
-        if (sp < RT_SMEM_STACK) sm[sp * kPersistThreads] = r;
-        else lm[sp - RT_SMEM_STACK] = r;
-        ++sp;
-    }
-    __device__ __forceinline__ void push_if(int &sp, uint32_t r, uint32_t k, bool keep) {
-        if (keep) push(sp, r, k);
-    }
-    __device__ __forceinline__ uint32_t at(int sp) const { return sp < RT_SMEM_STACK ? sm[sp * kPersistThreads] : lm[sp - RT_SMEM_STACK]; }
-#else
     uint32_t lm[RT_STACK_SIZE];
     __device__ __forceinline__ void push(int &sp, uint32_t r, uint32_t) { lm[sp++] = r; }
-    __device__ __forceinline__ void push_if(int &sp, uint32_t r, uint32_t, bool keep) { lm[sp] = r, sp += keep ? 1 : 0; }
     __device__ __forceinline__ uint32_t at(int sp) const { return lm[sp]; }
-#endif
     __device__ __forceinline__ bool room(int sp, int n) const { return sp + n <= RT_STACK_SIZE; }
 };
 
@@ -105,10 +79,6 @@ k_trace_persistent(const void *tlas, const rt_ray *rays, const uint32_t *count, 
     constexpr uint32_t rayContribution = MODE == 1 ? 1u : 0u;  // shadow rays use hit group 1 (S/RaytracingCommon.hlsli:94)
 
     PersistStack stk;
-#if RT_SMEM_STACK > 0
-    __shared__ uint32_t s_stack[RT_SMEM_STACK][kPersistThreads];
-    stk.sm = &s_stack[0][threadIdx.x];
-#endif
     // per-lane ray state
     bool alive = false;
     uint32_t rayIdx = 0, ref = RT_SENTINEL;
@@ -120,13 +90,8 @@ k_trace_persistent(const void *tlas, const rt_ray *rays, const uint32_t *count, 
     RayPre cur;
     cur.ox = cur.oy = cur.oz = cur.ix = cur.iy = cur.iz = cur.oix = cur.oiy = cur.oiz = cur.sx = cur.sy = cur.sz = 0;
     cur.kx = 0, cur.ky = 1, cur.kz = 2;
-#if RT_PERSIST_WIDE4
     const rt_wide4_node *const topNodes = A.wide4;
     const rt_wide4_node *nodes = topNodes;
-#else
-    const rt_wide_node *const topNodes = A.wide;
-    const rt_wide_node *nodes = topNodes;
-#endif
     const rt_packed_tri *tris = nullptr;
     uint32_t instFlags = 0, instOffset = 0;
     int cull = 0;
@@ -222,11 +187,7 @@ k_trace_persistent(const void *tlas, const rt_ray *rays, const uint32_t *count, 
         const unsigned intMask = aliveMask & ~leafMask;
         if (intMask == 0 || __popc(leafMask) >= kLeafThreshold) {
             // ---------------------------------------------------------------- leaf phase
-            // RT_LEAF_UNROLL > 1: a lane that pops straight into another leaf (the sibling triangle) tests it right away
-#pragma unroll
-            for (int lu = 0; lu < RT_LEAF_UNROLL; ++lu) {
-            if (lu > 0) pop();
-            if (alive && ref != RT_SENTINEL && (ref & RT_NODE_LEAF_FLAG) && (lu == 0 || bottom)) {
+            if (alive && ref != RT_SENTINEL && (ref & RT_NODE_LEAF_FLAG)) {
                 const uint32_t slot = ref & 0x00ffffffu;
                 ref = RT_SENTINEL;
                 if (!bottom) {
@@ -238,13 +199,7 @@ k_trace_persistent(const void *tlas, const rt_ray *rays, const uint32_t *count, 
                         instFlags = m3.y >> 24;
                         instOffset = m3.y & 0x00ffffffu;
                         if (GENERAL) instIndex = m3.z, instId = m3.x & 0x00ffffffu;
-                        {
-                            const bool useCulling = !(instFlags & RT_INSTANCE_FLAG_TRIANGLE_CULL_DISABLE);
-                            const bool flip = (instFlags & RT_INSTANCE_FLAG_TRIANGLE_FRONT_COUNTERCLOCKWISE) != 0;
-                            const uint32_t backFlag = flip ? RT_RAY_FLAG_CULL_FRONT_FACING_TRIANGLES : RT_RAY_FLAG_CULL_BACK_FACING_TRIANGLES;
-                            const uint32_t frontFlag = flip ? RT_RAY_FLAG_CULL_BACK_FACING_TRIANGLES : RT_RAY_FLAG_CULL_FRONT_FACING_TRIANGLES;
-                            cull = (useCulling && (rayFlags & frontFlag)) ? 2 : ((useCulling && (rayFlags & backFlag)) ? 1 : 0);
-                        }
+                        cull = cull_mode(instFlags, rayFlags);
                         sameSpace = plain && (m3.y & RT_PACKED_INSTANCE_IDENTITY);
                         if (sameSpace) {
                             ray_pre_shear(cur, wdx, wdy, wdz);
@@ -257,11 +212,7 @@ k_trace_persistent(const void *tlas, const rt_ray *rays, const uint32_t *count, 
                             const f3 d2 = xform_vector(m, mk3(wdx, wdy, wdz));
                             cur = make_ray_pre<true>(o2.x, o2.y, o2.z, d2.x, d2.y, d2.z);
                         }
-#if RT_PERSIST_WIDE4
                         nodes = reinterpret_cast<const rt_wide4_node *>(__ldg(reinterpret_cast<const unsigned long long *>(ip + 5)));
-#else
-                        nodes = reinterpret_cast<const rt_wide_node *>(uintptr_t(uint64_t(m4.x) | (uint64_t(m4.y) << 32)));
-#endif
                         tris = reinterpret_cast<const rt_packed_tri *>(uintptr_t(uint64_t(m4.z) | (uint64_t(m4.w) << 32)));
                         bottom = true;
                         blasBase = sp;
@@ -273,12 +224,7 @@ k_trace_persistent(const void *tlas, const rt_ray *rays, const uint32_t *count, 
                     const float4 p0 = __ldg(tp), p1 = __ldg(tp + 1), p2 = __ldg(tp + 2);
                     bool culled = false;
                     if (GENERAL) {  // IsOpaque() and the CULL_(NON_)OPAQUE ray flags (:119-134); the pipelines' rays carry none
-                        const uint32_t gflags = __float_as_uint(p2.w);
-                        bool opaque = (gflags & RT_GEOMETRY_FLAG_OPAQUE) != 0;
-                        if (instFlags & RT_INSTANCE_FLAG_FORCE_OPAQUE) opaque = true;
-                        else if (instFlags & RT_INSTANCE_FLAG_FORCE_NON_OPAQUE) opaque = false;
-                        if (rayFlags & RT_RAY_FLAG_FORCE_OPAQUE) opaque = true;
-                        else if (rayFlags & RT_RAY_FLAG_FORCE_NON_OPAQUE) opaque = false;
+                        const bool opaque = is_opaque(__float_as_uint(p2.w), instFlags, rayFlags);
                         culled = (opaque && (rayFlags & RT_RAY_FLAG_CULL_OPAQUE)) || (!opaque && (rayFlags & RT_RAY_FLAG_CULL_NON_OPAQUE));
                     }
                     float t0 = tCur, bu, bv;
@@ -291,7 +237,6 @@ k_trace_persistent(const void *tlas, const rt_ray *rays, const uint32_t *count, 
                     }
                 }
             }
-            }
         } else {
             // ---------------------------------------------------------------- internal phase
             // RT_INT_UNROLL > 1: a lane whose step (or the pop after it) ends at another internal node takes the next
@@ -301,27 +246,8 @@ k_trace_persistent(const void *tlas, const rt_ray *rays, const uint32_t *count, 
             for (int u = 0; u < RT_INT_UNROLL; ++u) {
                 if (u > 0) pop();
                 if (alive && ref != RT_SENTINEL && !(ref & RT_NODE_LEAF_FLAG)) {
-#if RT_PERSIST_WIDE4
                     // one 128-byte node = four child boxes (two BVH2 levels per dependent fetch)
                     ref = wide4_step<false, MODE != 1>(nodes, ref, cur, tCur, stk, sp, status);
-#else
-                    const float4 *np = reinterpret_cast<const float4 *>(nodes + ref);
-                    const float4 n0 = __ldg(np), n1 = __ldg(np + 1), n2 = __ldg(np + 2), n3 = __ldg(np + 3);
-                    float lt, rt;
-                    const bool lh = ray_box(lt, tCur, cur, n0.x, n0.y, n0.z, n1.x, n1.y, n1.z);
-                    const bool rh = ray_box(rt, tCur, cur, n2.x, n2.y, n2.z, n3.x, n3.y, n3.z);
-                    const uint32_t l = __float_as_uint(n0.w), r = __float_as_uint(n1.w);
-                    if (lh && rh) {
-                        const bool rightFirst = rt < lt;
-                        if (stk.room(sp, 1)) stk.push(sp, rightFirst ? l : r, 0u);
-                        else atomicOr(status, 1u);
-                        ref = rightFirst ? r : l;
-                    } else if (lh || rh) {
-                        ref = rh ? r : l;
-                    } else {
-                        ref = RT_SENTINEL;
-                    }
-#endif
                 }
             }
         }

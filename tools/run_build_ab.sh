@@ -13,7 +13,6 @@ for f in 8 0; do
 echo "== default lib, flags $f"; probe $f
 for so in build/rt_*.so; do [ -e "$so" ] || continue; echo "== $so, flags $f"; RT_CORE_LIB=$PWD/$so probe $f; done
 done
-for g in 32 64 128; do echo "== default lib, flags 8, L2 fetch granularity $g"; RT_L2_FETCH_GRANULARITY=$g probe 8; done
 } > gpurun_out/${TAG}_ab.log 2>&1
 cat gpurun_out/${TAG}_ab.log
 ncu --metrics gpu__time_duration.sum,dram__bytes_read.sum,dram__bytes_write.sum --clock-control none -c 200 --csv --log-file gpurun_out/${TAG}_build_launches.csv python tools/probe_scale.py --build 10000000 --flags 8 --reps 1 > gpurun_out/${TAG}_ncu.log 2>&1
