@@ -254,6 +254,13 @@ int rt_set_output(rt_context *ctx, uint32_t slot, float *rgba, uint64_t pitch) {
     ctx->pitch[slot] = pitch;
     return RT_OK;
 }
+int rt_set_aov_output(rt_context *ctx, uint32_t aov, float *rgba, uint64_t pitch) {
+    RT_REQUIRE(ctx != nullptr && aov < RT_AOV_COUNT, "unknown AOV id");
+    RT_REQUIRE((uintptr_t(rgba) & 15) == 0 && pitch % 16 == 0, "AOV output alignment");
+    ctx->aov[aov] = rgba;
+    ctx->aov_pitch[aov] = pitch;
+    return RT_OK;
+}
 int rt_set_render_options(rt_context *ctx, const rt_render_options *o) {
     RT_REQUIRE(ctx && o, "null argument");
     RT_REQUIRE(o->max_radiance_ray_depth == 1 || o->max_radiance_ray_depth == 2, "max_radiance_ray_depth must be 1 or 2");

@@ -59,6 +59,8 @@ struct rt_context {
     rt_per_frame_constants frame{};
     float *output[2] = {nullptr, nullptr};
     uint64_t pitch[2] = {0, 0};
+    float *aov[RT_AOV_COUNT] = {};  // rt_set_aov_output: progressive AOV images, nullptr = unbound
+    uint64_t aov_pitch[RT_AOV_COUNT] = {};
     const void *tlas = nullptr;
     rt_render_options render_options{1u, 0u};
 

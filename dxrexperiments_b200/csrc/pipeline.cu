@@ -213,6 +213,34 @@ __device__ __forceinline__ void write_pixel(const Launch &L, float *out, uint64_
     *px = cur;
 }
 
+// AOV outputs of a progressive dispatch (rt_set_aov_output): one RGBA fp32 image per rt_aov id, bit k of `mask` set when
+// AOV k is bound.  Only the <true> instantiations of k_shade_primary and k_resolve read it.
+struct AovOut {
+    float *ptr[RT_AOV_COUNT];
+    uint64_t pitch[RT_AOV_COUNT];
+    uint32_t mask;
+};
+
+// AOVs 0-4 accumulate exactly as the beauty frame does, so each one equals the matching debug view bit for bit.
+__device__ __forceinline__ void write_aov(const Launch &L, const AovOut &a, int k, uint32_t x, uint32_t y, f3 c) {
+    if (a.mask & (1u << k)) write_pixel(L, a.ptr[k], a.pitch[k], x, y, c, true);
+}
+
+// The normal AOV: the running mean of (N, coverage) without write_pixel's clamp at 0, so that negative components
+// survive and `w` is the fraction of samples that hit.
+__device__ __forceinline__ void write_normal_aov(const Launch &L, const AovOut &a, uint32_t x, uint32_t y, f3 n, float coverage) {
+    if (!(a.mask & (1u << RT_AOV_NORMAL))) return;
+    float4 *px = reinterpret_cast<float4 *>(reinterpret_cast<uint8_t *>(a.ptr[RT_AOV_NORMAL]) + size_t(y) * a.pitch[RT_AOV_NORMAL]) + x;
+    const uint32_t cnt = L.f.cameraParams.accumCount;
+    const float4 prev = *px;
+    const float fn = float(cnt), fn1 = float(cnt + 1);
+    float4 cur = make_float4((fn * prev.x + n.x) / fn1, (fn * prev.y + n.y) / fn1, (fn * prev.z + n.z) / fn1, (fn * prev.w + coverage) / fn1);
+    if (L.halfTargets)
+        cur = make_float4(__half2float(__float2half_rn(cur.x)), __half2float(__float2half_rn(cur.y)), __half2float(__float2half_rn(cur.z)),
+                          __half2float(__float2half_rn(cur.w)));
+    *px = cur;
+}
+
 // ------------------------------------------------------------------------------------------------ K2
 // Coherence binning (north star: "rays compacted and sorted ... between bounces"): a block shades one 16x16 pixel tile
 // and hands out the tile's hit slots bin by bin, the bin being {hit-group record (material / instance), direction octant of
@@ -241,10 +269,12 @@ __device__ __forceinline__ uint32_t octant_of(f3 d) {
 #ifndef RT_RESOLVE_MIN_BLOCKS
 #define RT_RESOLVE_MIN_BLOCKS 12
 #endif
+// AOV: write the AOV outputs of the primary misses and the normal AOV of every pixel (progressive program only).
+template <bool AOV>
 __global__ void __launch_bounds__(kShadeThreads) k_shade_primary(const __grid_constant__ Launch L, WS ws, const rt_hit_record_dev *recs,
                                                                  uint32_t n_recs, const float *env, uint32_t envSize, float *out0,
                                                                  uint64_t pitch0, float *out1, uint64_t pitch1,
-                                                                 unsigned long long *rayCounts, uint32_t *status) {
+                                                                 unsigned long long *rayCounts, uint32_t *status, const AovOut aov) {
     __shared__ uint32_t s_count[kBins], s_offset[kBins], s_base;
     const uint32_t tilesX = (L.rw + kShadeTile - 1) / kShadeTile;
     const uint32_t lx = (blockIdx.x % tilesX) * kShadeTile + (threadIdx.x % kShadeTile);
@@ -268,6 +298,14 @@ __global__ void __launch_bounds__(kShadeThreads) k_shade_primary(const __grid_co
                 write_pixel(L, out1, pitch1, x, y, mk3(0, 0, 0), false);
             } else {
                 write_pixel(L, out0, pitch0, x, y, c, true);
+                if (AOV) {  // every debug view shows the environment for a miss
+                    write_aov(L, aov, RT_AOV_DIRECT, x, y, c);
+                    write_aov(L, aov, RT_AOV_INDIRECT_DIFFUSE, x, y, c);
+                    write_aov(L, aov, RT_AOV_INDIRECT_SPECULAR, x, y, c);
+                    write_aov(L, aov, RT_AOV_ALBEDO, x, y, c);
+                    write_aov(L, aov, RT_AOV_FRESNEL, x, y, c);
+                    write_normal_aov(L, aov, x, y, mk3(0, 0, 0), 0.0f);
+                }
             }
         }
     }
@@ -284,6 +322,7 @@ __global__ void __launch_bounds__(kShadeThreads) k_shade_primary(const __grid_co
         const rt_hit_record_dev &R = recs[rec];
         const uint32_t prim = __float_as_uint(hA.w);
         const f3 N = normalize3(interpolate_normal(R, prim, hA.y, hA.z));
+        if (AOV) write_normal_aov(L, aov, x, y, N, 1.0f);
         pos = o + hA.x * d;  // HitWorldPosition
         const rt_debug_options &opt = L.f.options;
         if (!L.realtime && opt.showAmbientOcclusionOnly) {
@@ -613,8 +652,10 @@ __device__ __forceinline__ f3 secondary_radiance(const Launch &L, const WS &ws, 
     return (mk3(m.emissive[0], m.emissive[1], m.emissive[2]) * m.emissive[3] + albedo * diffuseComponent) + specTerm;
 }
 
+// AOV: also write AOVs 0-4 of every hit slot (progressive program only).
+template <bool AOV>
 __global__ void __launch_bounds__(kBlock, RT_RESOLVE_MIN_BLOCKS) k_resolve(const __grid_constant__ Launch L, WS ws, const rt_hit_record_dev *recs, float *out0,
-                                                    uint64_t pitch0, float *out1, uint64_t pitch1) {
+                                                    uint64_t pitch0, float *out1, uint64_t pitch1, const AovOut aov) {
     const uint32_t n = ws.counters[0];
     for (uint32_t s = blockIdx.x * blockDim.x + threadIdx.x; s < n; s += gridDim.x * blockDim.x) {
         const uint4 info = ws.slotInfo[s];
@@ -670,6 +711,13 @@ __global__ void __launch_bounds__(kBlock, RT_RESOLVE_MIN_BLOCKS) k_resolve(const
             write_pixel(L, out0, pitch0, x, y, albedo * direct / RT_M_PI, false);
             write_pixel(L, out1, pitch1, x, y, m.reflectivity * spec * fres, false);
             continue;
+        }
+        if (AOV) {  // the expressions of the debug views below, so that each AOV equals its view bit for bit
+            write_aov(L, aov, RT_AOV_DIRECT, x, y, albedo * direct / RT_M_PI);
+            write_aov(L, aov, RT_AOV_INDIRECT_DIFFUSE, x, y, albedo * indirect / RT_M_PI);
+            write_aov(L, aov, RT_AOV_INDIRECT_SPECULAR, x, y, m.reflectivity * spec * fres);
+            write_aov(L, aov, RT_AOV_ALBEDO, x, y, albedo);
+            write_aov(L, aov, RT_AOV_FRESNEL, x, y, fres);
         }
         const rt_debug_options &opt = L.f.options;
         const f3 diffuseComponent = (direct + indirect) / RT_M_PI;
@@ -827,6 +875,14 @@ static int dispatch_impl(rt_context *ctx, rt_program *prog, uint32_t width, uint
     RT_REQUIRE(ctx->pitch[0] >= uint64_t(width) * 16, "output pitch");
     RT_REQUIRE(prog->kind != RT_PROGRAM_REALTIME || ctx->pitch[1] >= uint64_t(width) * 16, "output pitch of slot 1");
     RT_REQUIRE(prog->n_recs > 0, "no hit records bound (rt_bindings_set_hit_record)");
+    bool anyAov = false;
+    for (uint32_t k = 0; k < RT_AOV_COUNT; ++k) {
+        if (!ctx->aov[k]) continue;
+        anyAov = true;
+        RT_REQUIRE(ctx->aov_pitch[k] >= uint64_t(width) * 16, "AOV output pitch");
+    }
+    RT_REQUIRE(!anyAov || prog->kind != RT_PROGRAM_REALTIME, "AOV outputs bound for a realtime program (its outputs already are AOVs)");
+    RT_REQUIRE(!anyAov || !ctx->frame.options.showAmbientOcclusionOnly, "AOV outputs bound in the ambient-occlusion debug view");
     RT_CUDA(cudaSetDevice(ctx->device));
     const bool realtime = prog->kind == RT_PROGRAM_REALTIME;
     // RayGen early-out: S/ProgressiveRaytracing.hlsl:13-15
@@ -923,8 +979,17 @@ static int dispatch_band(rt_context *ctx, rt_program *prog, const Launch &L, con
     else k_primary<false><<<rt_div_up(tiles, kBlock / 32), kBlock, 0, st>>>(L, ctx->tlas, ws, ctx->status, sPrim);
     if (timing) RT_CUDA(cudaEventRecord(ctx->ev[1], st));
     const uint32_t shadeTiles = ((L.rw + kShadeTile - 1) / kShadeTile) * ((L.rh + kShadeTile - 1) / kShadeTile);
-    k_shade_primary<<<shadeTiles, kShadeThreads, 0, st>>>(L, ws, prog->dev_recs, prog->n_recs, prog->env_texels, prog->env_size,
-                                                             ctx->output[0], ctx->pitch[0], ctx->output[1], ctx->pitch[1], ctx->ray_counts, ctx->status);
+    AovOut aov{};
+    for (int k = 0; k < RT_AOV_COUNT; ++k) {
+        aov.ptr[k] = ctx->aov[k], aov.pitch[k] = ctx->aov_pitch[k];
+        if (ctx->aov[k]) aov.mask |= 1u << k;
+    }
+    if (aov.mask)
+        k_shade_primary<true><<<shadeTiles, kShadeThreads, 0, st>>>(L, ws, prog->dev_recs, prog->n_recs, prog->env_texels, prog->env_size,
+                                                                    ctx->output[0], ctx->pitch[0], ctx->output[1], ctx->pitch[1], ctx->ray_counts, ctx->status, aov);
+    else
+        k_shade_primary<false><<<shadeTiles, kShadeThreads, 0, st>>>(L, ws, prog->dev_recs, prog->n_recs, prog->env_texels, prog->env_size,
+                                                                     ctx->output[0], ctx->pitch[0], ctx->output[1], ctx->pitch[1], ctx->ray_counts, ctx->status, aov);
     if (timing) RT_CUDA(cudaEventRecord(ctx->ev[2], st));
     // The depth-0 shadow wave and the secondary-ray chain (trace -> shade -> depth-1 shadow wave) both depend only on
     // k_shade_primary and meet again in k_resolve.  Outside the instrumented / per-stage-timed modes the shadow wave
@@ -959,7 +1024,8 @@ static int dispatch_band(rt_context *ctx, rt_program *prog, const Launch &L, con
         ctx->launches += 2;
     }
     if (overlap) RT_CUDA(cudaStreamWaitEvent(st, ev_join, 0));
-    k_resolve<<<qgrid, kBlock, 0, st>>>(L, ws, prog->dev_recs, ctx->output[0], ctx->pitch[0], ctx->output[1], ctx->pitch[1]);
+    if (aov.mask) k_resolve<true><<<qgrid, kBlock, 0, st>>>(L, ws, prog->dev_recs, ctx->output[0], ctx->pitch[0], ctx->output[1], ctx->pitch[1], aov);
+    else k_resolve<false><<<qgrid, kBlock, 0, st>>>(L, ws, prog->dev_recs, ctx->output[0], ctx->pitch[0], ctx->output[1], ctx->pitch[1], aov);
     ctx->launches += 7;
     RT_LAUNCH_CHECK();
     if (timing) {

@@ -3,6 +3,8 @@
 // Both reference pipelines share almost all of their host code; here that code lives once in
 // RaytracingPipelineBase and the two classes differ in shader library, outputs and accumulation.
 #pragma once
+#include <array>
+
 #include "RaytracingPipeline.h"
 
 class RaytracingPipelineBase : public RaytracingPipeline {
@@ -34,6 +36,12 @@ public:
     // MAX_RADIANCE_RAY_DEPTH (1 in the reference's shaders; 2 = one more Phong-lobe bounce) and emulation of the
     // R16G16B16A16_FLOAT render targets createOutputResource() is asked for (rt_set_render_options); applied by render().
     void setRenderOptions(UINT maxRadianceRayDepth, bool halfRenderTargets) { mRenderOptions = {maxRadianceRayDepth, halfRenderTargets ? 1u : 0u}; }
+    // AOV outputs (rt_set_aov_output; progressive pipeline only): enableAov before createOutputResource, which allocates the
+    // enabled ones next to the beauty output; render() then accumulates them from the same rays.  getAovResource is null
+    // for an AOV that is not enabled.  render() binds all RT_AOV_COUNT slots on every call (null for disabled ones), so a
+    // pipeline without AOVs sharing the context with one that has them never dispatches into the other's buffers.
+    void enableAov(rt_aov aov) { mAovEnabled.at(aov) = true; }
+    DXRFramework::RtBuffer::SharedPtr getAovResource(rt_aov aov) const { return mAovResource.at(aov); }
 
     // Environment: a procedural sky by default; loadEnvironmentDDS replaces it with an R16G16B16A16F / R32G32B32A32F
     // cube map file such as the reference's assets/textures/CathedralRadiance.dds.
@@ -58,6 +66,8 @@ protected:
     std::vector<Material> mMaterials;
     std::shared_ptr<Math::Camera> mCamera;
     std::vector<DXRFramework::RtBuffer::SharedPtr> mOutputResource;
+    std::array<bool, RT_AOV_COUNT> mAovEnabled{};
+    std::array<DXRFramework::RtBuffer::SharedPtr, RT_AOV_COUNT> mAovResource;
     UINT mNumOutputs;
     PerFrameConstants mConstantBuffer{};
     DXRFramework::RtTexture::SharedPtr mEnvCube;

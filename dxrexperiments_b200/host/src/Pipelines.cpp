@@ -91,6 +91,12 @@ void RaytracingPipelineBase::createOutputResource(DXGI_FORMAT /*format*/, UINT w
         b->clear();
         mOutputResource.push_back(b);
     }
+    for (int k = 0; k < RT_AOV_COUNT; ++k) {
+        mAovResource[k] = nullptr;
+        if (!mAovEnabled[k]) continue;
+        mAovResource[k] = mRtContext->createBuffer(uint64_t(width) * height * 16);
+        mAovResource[k]->clear();
+    }
 }
 
 // calculateCameraVariables (src/ProgressiveRaytracingPipeline.cpp:151-168)
@@ -156,6 +162,9 @@ void RaytracingPipelineBase::render(UINT /*frameIndex*/, UINT width, UINT height
     ThrowIfFailed(rt_set_frame_constants(ctx, &mConstantBuffer), "rt_set_frame_constants");
     for (UINT i = 0; i < mNumOutputs; ++i)
         ThrowIfFailed(rt_set_output(ctx, i, static_cast<float *>(mOutputResource.at(i)->ptr()), uint64_t(width) * 16), "rt_set_output");
+    for (uint32_t k = 0; k < RT_AOV_COUNT; ++k)
+        ThrowIfFailed(rt_set_aov_output(ctx, k, mAovResource[k] ? static_cast<float *>(mAovResource[k]->ptr()) : nullptr, uint64_t(width) * 16),
+                      "rt_set_aov_output");
     ThrowIfFailed(rt_set_tlas(ctx, mRtScene->getTlasWrappedPtr()), "rt_set_tlas");
     ThrowIfFailed(rt_set_render_options(ctx, &mRenderOptions), "rt_set_render_options");
 
@@ -163,6 +172,8 @@ void RaytracingPipelineBase::render(UINT /*frameIndex*/, UINT width, UINT height
     else if (mStripGroups > 1) mRtContext->raytraceStrips(mRtBindings, mRtState, width, height, mStripRows, mStripGroups, mStripGroup);
     else mRtContext->raytrace(mRtBindings, mRtState, width, height, 3);
     for (auto &o : mOutputResource) mRtContext->insertUAVBarrier(o);
+    for (auto &o : mAovResource)
+        if (o) mRtContext->insertUAVBarrier(o);
 }
 
 // ------------------------------------------------------------------------------------------------ progressive

@@ -5,6 +5,8 @@
 //   dxr_headless --model scene.obj --pipeline progressive --spp 16 --width 1920 --height 1080 --out frame.pfm
 //   dxr_headless --scene cornell --pipeline realtime --out direct.pfm --out2 spec.pfm --denoise composite.pfm
 //   dxr_headless ... --exr frame.exr [--exr-half]        OpenEXR output (fp32, or HALF = the reference's R16G16B16A16_FLOAT)
+//   dxr_headless --pipeline progressive ... --aov albedo albedo.pfm --aov normal normal.exr   AOV outputs, accumulated from the
+//     same rays as --out (direct, indirect-diffuse, indirect-specular, albedo, fresnel, normal; EXR when the path ends in .exr)
 // Multi-GPU (one process per GPU, replicated scene; the frame's samples and strips are sharded, one NCCL reduce at the end):
 //   for r in 0 1; do dxr_headless ... --spp 64 --world 2 --rank $r --comm-file /tmp/id [--strip-groups 2] --out frame.pfm & done
 #include <chrono>
@@ -71,6 +73,7 @@ static int usage() {
               "             [--spp N] [--seed S] [--no-jitter] [--eye x y z] [--at x y z] [--light-pos x y z] [--env-dds file | --env-raw file size]\n"
               "             [--out file.pfm] [--out2 file.pfm] [--denoise file.pfm] [--exr file.exr [--exr-half]] [--dump-frames file.bin] [--device N]\n"
               "             [--radiance-depth 1|2] [--fp16-targets] [--denoise-mock direct.pfm specular.pfm --denoise out.pfm [--kernel-size K]]\n"
+              "             [--aov direct|indirect-diffuse|indirect-specular|albedo|fresnel|normal file.pfm|file.exr]...   (progressive only)\n"
               "             [--world N --rank R --comm-file path [--strip-groups G] [--strip-rows 32] [--band-shard]]   (one process per GPU)");
     return 0;
 }
@@ -177,6 +180,22 @@ int main(int argc, char **argv) {
             tex->cubemap = true;
             pipeline->setEnvironment(tex);
         }
+        // --aov NAME PATH, repeatable: names in rt_aov id order
+        static const char *const kAovNames[RT_AOV_COUNT] = {"direct", "indirect-diffuse", "indirect-specular", "albedo", "fresnel", "normal"};
+        std::vector<std::pair<int, std::string>> aovFiles;
+        if (a.has("aov")) {
+            const auto &v = a.kv.at("aov");
+            if (pipelineName == "realtime") throw std::runtime_error("--aov needs --pipeline progressive");
+            if (v.empty() || v.size() % 2) throw std::runtime_error("--aov takes a name and a path");
+            for (size_t i = 0; i < v.size(); i += 2) {
+                int id = -1;
+                for (int k = 0; k < RT_AOV_COUNT; ++k)
+                    if (v[i] == kAovNames[k]) id = k;
+                if (id < 0) throw std::runtime_error("unknown AOV name " + v[i]);
+                pipeline->enableAov(rt_aov(id));
+                aovFiles.emplace_back(id, v[i + 1]);
+            }
+        }
         pipeline->loadResources(3);
         pipeline->createOutputResource(DXGI_FORMAT_R16G16B16A16_FLOAT, width, height);
         pipeline->setRenderOptions(UINT(a.num("radiance-depth", 1)), a.has("fp16-targets"));
@@ -218,6 +237,9 @@ int main(int argc, char **argv) {
         // ---- the path's one collective: every output is summed onto rank 0, weighted by the rank's share of the samples
         std::vector<RtBuffer::SharedPtr> finalOut;
         for (int i = 0; i < pipeline->getNumOutputs(); ++i) finalOut.push_back(pipeline->getOutputResource(i));
+        // the AOVs are running means like the beauty output, so they reduce with the same weights
+        const size_t numBeauty = finalOut.size();
+        for (const auto &f : aovFiles) finalOut.push_back(pipeline->getAovResource(rt_aov(f.first)));
         std::shared_ptr<DenoiseCompositor> bandDenoiser;
         RtBuffer::SharedPtr bandFrame;
         if (bandShard) {
@@ -250,7 +272,8 @@ int main(int argc, char **argv) {
         };
         if (a.has("out")) save(finalOut[0], a.str("out", ""));
         if (a.has("exr")) save(finalOut[0], a.str("exr", ""));
-        if (a.has("out2") && finalOut.size() > 1) save(finalOut[1], a.str("out2", ""));
+        if (a.has("out2") && numBeauty > 1) save(finalOut[1], a.str("out2", ""));
+        for (size_t i = 0; i < aovFiles.size(); ++i) save(finalOut[numBeauty + i], aovFiles[i].second);
         if (bandShard) {
             save(bandFrame, a.str("denoise", ""));
         } else if (a.has("denoise") && rank == 0) {

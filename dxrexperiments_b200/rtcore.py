@@ -76,6 +76,7 @@ def _load():
         "rt_bindings_set_miss_record": (i32, [vp, u32, vp, u32]),
         "rt_set_frame_constants": (i32, [vp, vp]),
         "rt_set_output": (i32, [vp, u32, vp, u64]),
+        "rt_set_aov_output": (i32, [vp, u32, vp, u64]),
         "rt_set_tlas": (i32, [vp, vp]),
         "rt_set_render_options": (i32, [vp, vp]),
         "rt_dispatch_rays": (i32, [vp, vp, u32, u32, u32]),
@@ -610,11 +611,13 @@ class Renderer:
     """Convenience host for tests/bench: one scene (instances of meshes), one program, fp32 outputs on the device."""
 
     def __init__(self, ctx: Context, meshes, transforms, materials, env_texels, kind=PROGRESSIVE, width=256, height=256,
-                 outputs=None, instance_mesh=None, build_flags: int = 0):
+                 outputs=None, instance_mesh=None, build_flags: int = 0, aovs=()):
         """outputs: optional list of caller-owned device buffers (anything with .ptr, e.g. a wrapped torch tensor)
         of width*height RGBA fp32, one per output slot; allocated here when omitted.
         instance_mesh: optional list, one mesh index per transform (instancing: many instances of few BLASes);
-        by default instance i is mesh i."""
+        by default instance i is mesh i.
+        aovs: names from types.AOV_NAMES (progressive program only): each gets a zeroed width*height RGBA fp32 buffer
+        that every dispatch accumulates next to the beauty output (rt_set_aov_output); read it back with aov(name)."""
         self.ctx, self.width, self.height, self.kind = ctx, width, height, kind
         self.blases = [ctx.build_blas_from_mesh(m, build_flags=build_flags) for m in meshes]  # 0 = the application's flags (RtModel.cpp:86-118)
         if instance_mesh is None:
@@ -629,12 +632,19 @@ class Renderer:
         n_out = 2 if kind == REALTIME else 1
         self.out = list(outputs) if outputs is not None else [ctx.alloc(16 * width * height).zero() for _ in range(n_out)]
         assert len(self.out) == n_out
+        unknown = [a for a in aovs if a not in T.AOV_NAMES]
+        if unknown:
+            raise ValueError(f"unknown AOV names {unknown}; known: {T.AOV_NAMES}")
+        self.aovs = {a: ctx.alloc(16 * width * height).zero() for a in aovs}
 
     def dispatch(self, frame: T.PerFrameConstants, region=None, strips=None):
         """region: (x0, y0, x1, y1) pixel rectangle; strips: (strip_rows, groups, group) strip-interleaved shard."""
         # global root arguments are (re)bound per dispatch, as render() does (ProgressiveRaytracingPipeline.cpp:236-242)
         for slot, o in enumerate(self.out):
             check(lib.rt_set_output(self.ctx.handle, slot, o.ptr, 16 * self.width))
+        for k, name in enumerate(T.AOV_NAMES):  # all six, so that AOVs another Renderer bound on this context are unbound
+            buf = self.aovs.get(name)
+            check(lib.rt_set_aov_output(self.ctx.handle, k, buf.ptr if buf is not None else None, 16 * self.width if buf is not None else 0))
         check(lib.rt_set_tlas(self.ctx.handle, self.tlas.result.ptr))
         check(lib.rt_set_frame_constants(self.ctx.handle, C.byref(frame)))
         if strips is not None:
@@ -661,3 +671,7 @@ class Renderer:
 
     def image(self, slot=0) -> np.ndarray:
         return self.out[slot].download(np.float32).reshape(self.height, self.width, 4)
+
+    def aov(self, name: str) -> np.ndarray:
+        """The accumulated AOV `name` (one of the names passed as aovs=) as (height, width, 4) float32."""
+        return self.aovs[name].download(np.float32).reshape(self.height, self.width, 4)

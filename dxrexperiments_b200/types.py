@@ -140,6 +140,9 @@ PRIMITIVE_TYPE_TRIANGLE, PRIMITIVE_TYPE_PROCEDURAL = 1, 2
 ANYHIT_NONE, ANYHIT_ACCEPT, ANYHIT_IGNORE, ANYHIT_END_SEARCH, ANYHIT_CUTOUT = 0, 1, 2, 3, 4
 INTERSECTION_NONE, INTERSECTION_BOX, INTERSECTION_SPHERE = 0, 1, 2
 HIT_KIND_TRIANGLE_FRONT_FACE = 0xFE
+# rt_aov (include/rt_core.h): AOV outputs of the progressive program, in id order
+AOV_DIRECT, AOV_INDIRECT_DIFFUSE, AOV_INDIRECT_SPECULAR, AOV_ALBEDO, AOV_FRESNEL, AOV_NORMAL, AOV_COUNT = range(7)
+AOV_NAMES = ("direct", "indirect-diffuse", "indirect-specular", "albedo", "fresnel", "normal")
 
 
 def parse_blas_blob(blob: np.ndarray):

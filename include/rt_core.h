@@ -182,6 +182,34 @@ int rt_set_frame_constants(rt_context *ctx, const rt_per_frame_constants *frame)
  * RGBA fp32, pitch in bytes (>= width*16).  The reference's targets are R16G16B16A16_FLOAT
  * (src/DXRExperimentsApp.cpp:28); fp32 is a declared deviation (DESIGN.md). */
 int rt_set_output(rt_context *ctx, uint32_t slot, float *rgba, uint64_t pitch_bytes);
+/* AOV outputs of the progressive program (new work: the reference has no counterpart; its nearest relative is the
+ * DebugOptions switches, assets/shaders/RaytracingHlslCompat.h:64-77, each of which REPLACES the beauty frame with one
+ * component).  A bound AOV is accumulated next to gOutput from the same rays, with the same running mean and the same
+ * fp16 rounding under half_render_targets, so AOV k equals the beauty output of the same dispatches with debug view k
+ * switched on, bit for bit.  AOVs 0-4 hold, for a primary hit:
+ *   DIRECT             albedo * direct / pi            (showDirectLightingOnly)
+ *   INDIRECT_DIFFUSE   albedo * indirect / pi          (showIndirectDiffuseOnly)
+ *   INDIRECT_SPECULAR  reflectivity * spec * fresnel   (showIndirectSpecularOnly)
+ *   ALBEDO             albedo                          (showGBufferAlbedoOnly)
+ *   FRESNEL            fresnel                         (showFresnelTerm)
+ * and for a primary miss the environment times environmentStrength; they are clamped at 0 with alpha 1 like gOutput.
+ * NORMAL holds (N, 1) for a hit and (0, 0, 0, 0) for a miss, without the clamp, so its w is the fraction of samples that
+ * hit.  N is the normalised interpolated vertex normal exactly as shade() receives it: the OBJECT-space normal, which
+ * the reference does not transform by the instance.  Debug views change gOutput only; the AOVs keep these definitions. */
+typedef enum rt_aov {
+    RT_AOV_DIRECT = 0,
+    RT_AOV_INDIRECT_DIFFUSE = 1,
+    RT_AOV_INDIRECT_SPECULAR = 2,
+    RT_AOV_ALBEDO = 3,
+    RT_AOV_FRESNEL = 4,
+    RT_AOV_NORMAL = 5,
+    RT_AOV_COUNT = 6
+} rt_aov;
+/* Binds AOV `aov` (an rt_aov id; others are RT_ERR_INVALID_ARG) to a caller-owned RGBA fp32 image; NULL unbinds.  A
+ * dispatch checks pitch_bytes >= width*16 for every bound AOV.  A dispatch with any AOV bound is RT_ERR_INVALID_ARG for
+ * a realtime program (its outputs already are AOVs) and in the showAmbientOcclusionOnly view (which traces AO rays
+ * instead of lighting).  The maxIterations early-out leaves the AOVs untouched, as it leaves gOutput. */
+int rt_set_aov_output(rt_context *ctx, uint32_t aov, float *rgba, uint64_t pitch_bytes);
 int rt_set_tlas(rt_context *ctx, const void *tlas_result);
 /* Two things that are constants of the reference and options here (defaults = the reference's shaders / this library's
  * declared fp32 deviation):
