@@ -492,6 +492,8 @@ __global__ void __launch_bounds__(kThreads) k_rearrange_tris(const rt_packed_tri
 }
 
 // ------------------------------------------------------------------------------------------ bottom-up fit
+// The node rules, written once and used by every fit kernel: leaf box, child-box merge, root record, fitted parent
+// (child order, reference node, wide node, 4-wide node) and the 4-wide collapse.
 struct Box {
     float c[3], h[3];
 };
@@ -518,14 +520,179 @@ __device__ __forceinline__ Box load_node_box(const rt_aabb_node *nodes, uint32_t
     return r;
 }
 
-// FL/ComputeAABBs.hlsli:69-175.  One thread per leaf climbs; the second child to arrive at a parent
-// (atomic counter carrying triangle counts) fits the parent.  Children are ordered "smaller subtree
-// left"; on equal counts the reference is arrival-order dependent, pinned here as "keep Karras order".
-// TOP = false: leaf box from the sorted triangle (GetBoxDataFromTriangle, RayTracingHelper.hlsli:273-285).
-// TOP = true : leaf box = load-order instance box permuted by `perm`.
-// UPDATE = true (PERFORM_UPDATE, ComputeAABBs.hlsli:38-67): the topology is the one already in `nodes` — children
-// from each node's {flags, right} words, parents from the cached parent array — and only the boxes are re-fitted.
-// The subtree sizes are those of the original build, so the child order never changes (ties: pinned "no swap").
+// Leaf box of a sorted primitive from its nine floats: GetBoxDataFromTriangle (RayTracingHelper.hlsli:273-285) with
+// AABB_Min_Padding, or for a procedural primitive the AABB {min, max} as given (ComputeLeafAABB, procedural branch,
+// FL/BottomLevelComputeAABBs.hlsl:32-40).
+__device__ __forceinline__ Box leaf_box(const float *v, bool procedural) {
+    float mn[3], mx[3];
+    if (procedural) {
+#pragma unroll
+        for (int k = 0; k < 3; ++k) mn[k] = v[k], mx[k] = v[3 + k];
+    } else {
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            mn[k] = fminf(fminf(v[k], v[3 + k]), v[6 + k]);
+            mx[k] = fmaxf(fmaxf(v[k], v[3 + k]), v[6 + k]);
+            mn[k] = fminf(mn[k], mx[k] - 0.001f);  // AABB_Min_Padding
+        }
+    }
+    return aabb_to_box(mn, mx);
+}
+
+// GetBoxFromChildBoxes: FL/RayTracingHelper.hlsli:297-307.  `bl` is the child stored on the left: the reference's
+// operand order of min / max.
+__device__ __forceinline__ Box merge_boxes(const Box &bl, const Box &br) {
+    float mn[3], mx[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        mn[k] = fminf(bl.c[k] - bl.h[k], br.c[k] - br.h[k]);
+        mx[k] = fmaxf(bl.c[k] + bl.h[k], br.c[k] + br.h[k]);
+    }
+    return aabb_to_box(mn, mx);
+}
+
+__device__ __forceinline__ void store_root(rt_ext_header *ext, const Box &b) {
+    ext->root_center[0] = b.c[0], ext->root_center[1] = b.c[1], ext->root_center[2] = b.c[2];
+    ext->root_half[0] = b.h[0], ext->root_half[1] = b.h[1], ext->root_half[2] = b.h[2];
+}
+
+// A child reference of the traversal section: internal node i is i, leaf node nInternal + slot is LEAF_FLAG | slot.
+__device__ __forceinline__ uint32_t node_ref(uint32_t node, uint32_t nInternal) {
+    return node >= nInternal ? (RT_NODE_LEAF_FLAG | (node - nInternal)) : node;
+}
+
+// The two halves of an empty 4-wide slot: {0, 0, 0, RT_WIDE4_EMPTY}, {-1, -1, -1, 0}.
+__device__ __forceinline__ float4 wide4_empty(bool half) {
+    return half ? make_float4(-1.0f, -1.0f, -1.0f, 0.0f) : make_float4(0.0f, 0.0f, 0.0f, __uint_as_float(RT_WIDE4_EMPTY));
+}
+
+// BVH2 -> BVH4 for the traversal kernels.  A node's 4-wide node starts from its two (ordered) children and opens, twice,
+// the internal child with the largest surface area (half-extent product sum); strict >, so the lower slot wins a tie.
+// The opened child's left child takes its slot and its right child is appended.  `src` supplies the children: a
+// Src::Slot is one child, src.ref / src.half give its reference and half extents, and src.open(s, l, r) the two
+// children of the internal child s.  Returns the number of filled slots (2 to 4).
+template <class Src>
+__device__ __forceinline__ int collapse4(const Src &src, typename Src::Slot s[4]) {
+    int cnt = 2;
+#pragma unroll
+    for (int it = 0; it < 2; ++it) {
+        int best = -1;
+        float bestArea = -1.0f;
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            if (k < cnt && !(src.ref(s[k]) & RT_NODE_LEAF_FLAG)) {
+                const float3 h = src.half(s[k]);
+                const float a = h.x * h.y + h.y * h.z + h.z * h.x;
+                if (a > bestArea) bestArea = a, best = k;
+            }
+        }
+        if (best < 0) break;
+        typename Src::Slot opened = s[0], l, r;
+#pragma unroll
+        for (int k = 1; k < 4; ++k)
+            if (k == best) opened = s[k];
+        src.open(opened, l, r);
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            if (k == best) s[k] = l;
+            if (k == cnt) s[k] = r;
+        }
+        cnt++;
+    }
+    return cnt;
+}
+
+// collapse4's children from the finished BVH2 wide nodes in global memory.  Loads go through L2: the wide nodes were
+// written in the same kernel and published with a fence before the counter that let us fit the parent.
+struct WideChildren {
+    struct Slot {
+        float4 c, h;  // {center, ref}, {half, -}
+    };
+    const rt_wide_node *wide;
+    __device__ __forceinline__ uint32_t ref(const Slot &s) const { return __float_as_uint(s.c.w); }
+    __device__ __forceinline__ float3 half(const Slot &s) const { return make_float3(s.h.x, s.h.y, s.h.z); }
+    __device__ __forceinline__ void open(const Slot &s, Slot &l, Slot &r) const {
+        const float4 *w = reinterpret_cast<const float4 *>(wide + ref(s));
+        const float4 w0 = __ldcg(w), w1 = __ldcg(w + 1), w2 = __ldcg(w + 2), w3 = __ldcg(w + 3);
+        l.c = w0, l.h = w1;
+        r.c = make_float4(w2.x, w2.y, w2.z, w1.w), r.h = w3;
+    }
+};
+
+// The fit of one parent from its children l, r (Karras order) with subtree sizes lc, rc and boxes bl, br: the child
+// order, the reference node, the BVH2 wide node (both child boxes live in the parent), the 4-wide node when WIDE4 and,
+// for the root, the root record.  REORDER: smaller subtree on the left, ties keep the Karras order (on equal counts the
+// reference is arrival-order dependent, pinned here).  A refit (PERFORM_UPDATE) passes false: the topology and the child
+// order are those of the build it updates.  Every subtree below `parent` is complete and published (fence + counter).
+// Returns the parent's box.
+template <bool REORDER, bool WIDE4>
+__device__ __forceinline__ Box fit_parent(uint32_t parent, uint32_t l, uint32_t r, uint32_t lc, uint32_t rc, Box bl, Box br,
+                                          uint32_t nInternal, rt_aabb_node *nodes, rt_wide_node *wide, rt_wide4_node *wide4,
+                                          rt_ext_header *ext) {
+    if (REORDER && rc < lc) {
+        uint32_t t = l; l = r; r = t;
+        Box tb = bl; bl = br; br = tb;
+    }
+    const Box box = merge_boxes(bl, br);
+    store_node(nodes, parent, box, l & 0x00ffffffu, r);
+    const uint32_t lref = node_ref(l, nInternal), rref = node_ref(r, nInternal);
+    float4 *w = reinterpret_cast<float4 *>(wide + parent);
+    w[0] = make_float4(bl.c[0], bl.c[1], bl.c[2], __uint_as_float(lref));
+    w[1] = make_float4(bl.h[0], bl.h[1], bl.h[2], __uint_as_float(rref));
+    w[2] = make_float4(br.c[0], br.c[1], br.c[2], 0.0f);
+    w[3] = make_float4(br.h[0], br.h[1], br.h[2], 0.0f);
+    if (WIDE4) {
+        WideChildren::Slot s[4];
+        s[0].c = make_float4(bl.c[0], bl.c[1], bl.c[2], __uint_as_float(lref)), s[0].h = make_float4(bl.h[0], bl.h[1], bl.h[2], 0.0f);
+        s[1].c = make_float4(br.c[0], br.c[1], br.c[2], __uint_as_float(rref)), s[1].h = make_float4(br.h[0], br.h[1], br.h[2], 0.0f);
+        const int cnt = collapse4(WideChildren{wide}, s);
+        float4 *o = reinterpret_cast<float4 *>(wide4 + parent);
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            o[2 * k] = k < cnt ? s[k].c : wide4_empty(false);
+            o[2 * k + 1] = k < cnt ? make_float4(s[k].h.x, s[k].h.y, s[k].h.z, 0.0f) : wide4_empty(true);
+        }
+    }
+    if (parent == 0) store_root(ext, box);
+    return box;
+}
+
+// FL/ComputeAABBs.hlsli:69-175, through global memory: one thread carries a fitted node (its box and subtree size) up
+// the tree; the second child to arrive at a parent (atomic counter carrying subtree sizes) fits the parent.
+// UPDATE (PERFORM_UPDATE, ComputeAABBs.hlsli:38-67): the topology is the one already in `nodes` — children from each
+// node's {flags, right} words, parents from the cached parent array — and only the boxes are re-fitted.
+// WIDE4: write the 4-wide node of every parent fitted (k_fit_exits); k_fit leaves them to k_collapse4.
+template <bool UPDATE, bool WIDE4>
+__device__ __forceinline__ void climb(uint32_t node, uint32_t count, Box box, uint32_t nInternal, const rt_hierarchy_node *hier,
+                                      const uint32_t *parents, uint32_t *counters, rt_aabb_node *nodes, rt_wide_node *wide,
+                                      rt_wide4_node *wide4, rt_ext_header *ext) {
+    const uint32_t *hw = reinterpret_cast<const uint32_t *>(hier);
+    while (true) {
+        uint32_t parent, l = 0, r = 0;
+        if (UPDATE) {
+            parent = parents[node];
+        } else {
+            parent = __ldg(hw + 3 * size_t(node)) & ~treelet::kCollapseBit;
+            l = __ldg(hw + 3 * size_t(parent) + 1), r = __ldg(hw + 3 * size_t(parent) + 2);
+        }
+        __threadfence();
+        const uint32_t other = atomicAdd(&counters[parent], count);
+        if (other == 0) return;  // first to arrive: the sibling will fit the parent
+        __threadfence();
+        if (UPDATE) l = nodes[parent].flags & 0x00ffffffu, r = nodes[parent].right;
+        const bool isLeft = (l == node);
+        const Box sb = load_node_box(nodes, isLeft ? r : l);
+        box = fit_parent<!UPDATE, WIDE4>(parent, l, r, isLeft ? count : other, isLeft ? other : count, isLeft ? box : sb, isLeft ? sb : box,
+                                         nInternal, nodes, wide, wide4, ext);
+        if (parent == 0) return;
+        count += other;
+        node = parent;
+    }
+}
+
+// One thread per leaf: the leaf box, then the global climb.  TLAS builds and updates, and PERFORM_UPDATE refits of a BLAS;
+// their 4-wide nodes are written afterwards by k_collapse4.
+// TOP = false: leaf box from the sorted primitive.  TOP = true: leaf box = load-order instance box permuted by `perm`.
 template <bool TOP, bool UPDATE>
 __global__ void __launch_bounds__(kThreads) k_fit(uint32_t n, const rt_hierarchy_node *hier, uint32_t *counters,
                                                   rt_aabb_node *nodes, const rt_primitive *sorted_prims,
@@ -534,7 +701,6 @@ __global__ void __launch_bounds__(kThreads) k_fit(uint32_t n, const rt_hierarchy
     uint32_t slot = blockIdx.x * blockDim.x + threadIdx.x;
     if (slot >= n) return;
     const uint32_t nInternal = n - 1;
-    uint32_t node = nInternal + slot;
     Box box;
     uint32_t leafFlags = slot | RT_NODE_LEAF_FLAG;
     if (TOP) {
@@ -542,170 +708,210 @@ __global__ void __launch_bounds__(kThreads) k_fit(uint32_t n, const rt_hierarchy
         box.c[0] = s.center[0], box.c[1] = s.center[1], box.c[2] = s.center[2];
         box.h[0] = s.halfDim[0], box.h[1] = s.halfDim[1], box.h[2] = s.halfDim[2];
     } else {
-        const float *v = sorted_prims[slot].v;
-        float mn[3], mx[3];
-        if (*reinterpret_cast<const uint32_t *>(sorted_prims + slot) == RT_PRIMITIVE_TYPE_PROCEDURAL) {
-            // ComputeLeafAABB, procedural branch (FL/BottomLevelComputeAABBs.hlsl:32-40): the AABB as given, flagged
-#pragma unroll
-            for (int k = 0; k < 3; ++k) mn[k] = v[k], mx[k] = v[3 + k];
-            leafFlags |= RT_NODE_PROCEDURAL_FLAG;
-        } else {
-#pragma unroll
-            for (int k = 0; k < 3; ++k) {
-                mn[k] = fminf(fminf(v[k], v[3 + k]), v[6 + k]);
-                mx[k] = fmaxf(fmaxf(v[k], v[3 + k]), v[6 + k]);
-                mn[k] = fminf(mn[k], mx[k] - 0.001f);  // AABB_Min_Padding
-            }
-        }
-        box = aabb_to_box(mn, mx);
+        const bool procedural = *reinterpret_cast<const uint32_t *>(sorted_prims + slot) == RT_PRIMITIVE_TYPE_PROCEDURAL;
+        box = leaf_box(sorted_prims[slot].v, procedural);
+        if (procedural) leafFlags |= RT_NODE_PROCEDURAL_FLAG;
     }
-    store_node(nodes, node, box, leafFlags, 1u);
-    if (n == 1) {
-        ext->root_center[0] = box.c[0], ext->root_center[1] = box.c[1], ext->root_center[2] = box.c[2];
-        ext->root_half[0] = box.h[0], ext->root_half[1] = box.h[1], ext->root_half[2] = box.h[2];
-        return;
-    }
-    uint32_t count = 1;
-    while (true) {
-        const uint32_t parent = UPDATE ? parents[node] : (hier[node].parent & ~treelet::kCollapseBit);
-        __threadfence();
-        const uint32_t other = atomicAdd(&counters[parent], count);
-        if (other == 0) return;  // first to arrive: the sibling will fit the parent
-        __threadfence();
-        uint32_t l, r;
-        if (UPDATE) {
-            l = nodes[parent].flags & 0x00ffffffu, r = nodes[parent].right;
-        } else {
-            l = hier[parent].left, r = hier[parent].right;
-        }
-        const bool isLeft = (l == node);
-        const uint32_t lc = isLeft ? count : other, rc = isLeft ? other : count;
-        const uint32_t sibling = isLeft ? r : l;
-        Box sb = load_node_box(nodes, sibling);
-        Box bl = isLeft ? box : sb, br = isLeft ? sb : box;
-        if (!UPDATE && rc < lc) {  // smaller subtree on the left; ties keep the Karras order
-            uint32_t t = l; l = r; r = t;
-            Box tb = bl; bl = br; br = tb;
-        }
-        // GetBoxFromChildBoxes: FL/RayTracingHelper.hlsli:297-307
-        float mn[3], mx[3];
-#pragma unroll
-        for (int k = 0; k < 3; ++k) {
-            mn[k] = fminf(bl.c[k] - bl.h[k], br.c[k] - br.h[k]);
-            mx[k] = fmaxf(bl.c[k] + bl.h[k], br.c[k] + br.h[k]);
-        }
-        box = aabb_to_box(mn, mx);
-        store_node(nodes, parent, box, l & 0x00ffffffu, r);
-        // traversal section: both child boxes live in the parent
-        const uint32_t lref = l >= nInternal ? (RT_NODE_LEAF_FLAG | (l - nInternal)) : l;
-        const uint32_t rref = r >= nInternal ? (RT_NODE_LEAF_FLAG | (r - nInternal)) : r;
-        float4 *w = reinterpret_cast<float4 *>(wide + parent);
-        w[0] = make_float4(bl.c[0], bl.c[1], bl.c[2], __uint_as_float(lref));
-        w[1] = make_float4(bl.h[0], bl.h[1], bl.h[2], __uint_as_float(rref));
-        w[2] = make_float4(br.c[0], br.c[1], br.c[2], 0.0f);
-        w[3] = make_float4(br.h[0], br.h[1], br.h[2], 0.0f);
-        if (parent == 0) {
-            ext->root_center[0] = box.c[0], ext->root_center[1] = box.c[1], ext->root_center[2] = box.c[2];
-            ext->root_half[0] = box.h[0], ext->root_half[1] = box.h[1], ext->root_half[2] = box.h[2];
-            return;
-        }
-        count += other;
-        node = parent;
-    }
+    store_node(nodes, nInternal + slot, box, leafFlags, 1u);
+    if (n == 1) store_root(ext, box);
+    else climb<UPDATE, false>(nInternal + slot, 1u, box, nInternal, hier, parents, counters, nodes, wide, nullptr, ext);
 }
 
-// k_fit for a full bottom-level build with the lower levels of the tree fitted inside the thread block.  A block owns
-// kFitBlock consecutive sorted slots; a parent flagged `local` (k_hierarchy; kept valid by k_treelet_reorder) has its
-// whole subtree among them.  The block works in rounds over a shared-memory ready queue: a node enters the queue when
-// its second child has been fitted (shared arrival counter), and the nodes of a round are handed to consecutive
-// threads, so the warps stay dense where the one-thread-per-leaf climb of k_fit runs at 6-7 of 32 lanes (ncu) and pays
-// a global atomic plus two device-wide fences per level.  Child boxes and subtree sizes are exchanged through shared
-// memory.  Nodes whose parent is not local — about log2(n) per block — leave through an exit list and finish with
-// k_fit's global climb.  Results (reference nodes, wide nodes, child order) are those of k_fit, bit for bit: the child
-// order depends only on the subtree sizes and the Karras order, never on who arrives first.
-// The 4-wide node of `parent` from its two (already ordered) children and, through the children's finished wide nodes,
-// its grandchildren: open, twice, the internal child with the largest surface area — k_collapse4's rule.  Used by
-// k_fit_exits, where every subtree below `parent` is complete and published (fence + counter) before we got here.
-__device__ __forceinline__ void collapse4_store(uint32_t parent, const Box &bl, uint32_t lref, const Box &br, uint32_t rref,
-                                                const rt_wide_node *wide, rt_wide4_node *wide4) {
-    float4 c[4], h[4];
-    int cnt = 2;
-    c[0] = make_float4(bl.c[0], bl.c[1], bl.c[2], __uint_as_float(lref)), h[0] = make_float4(bl.h[0], bl.h[1], bl.h[2], 0.0f);
-    c[1] = make_float4(br.c[0], br.c[1], br.c[2], __uint_as_float(rref)), h[1] = make_float4(br.h[0], br.h[1], br.h[2], 0.0f);
-#pragma unroll
-    for (int it = 0; it < 2; ++it) {
-        int best = -1;
-        float bestArea = -1.0f;
+// BVH2 -> BVH4 after k_fit: thread i collapses node i, reading the child boxes straight from the finished BVH2 wide nodes.
+__global__ void __launch_bounds__(kThreads) k_collapse4(const rt_wide_node *wide, uint32_t n_internal, rt_wide4_node *wide4) {
+    // the block's kThreads x 128-byte nodes leave through shared memory as one contiguous run of 16-byte stores; slot
+    // k of thread t sits at t * 8 + (k ^ (t & 7)) so that neither side has bank conflicts
+    __shared__ float4 s_out[kThreads * 8];
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n_internal) {
+        const float4 *w = reinterpret_cast<const float4 *>(wide + i);
+        const float4 w0 = w[0], w1 = w[1], w2 = w[2], w3 = w[3];
+        WideChildren::Slot s[4];
+        s[0].c = w0, s[0].h = w1;
+        s[1].c = make_float4(w2.x, w2.y, w2.z, w1.w), s[1].h = w3;
+        const int cnt = collapse4(WideChildren{wide}, s);
+        float4 *o = s_out + threadIdx.x * 8;
+        const int sw = threadIdx.x & 7;
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
-            if (k < cnt && !(__float_as_uint(c[k].w) & RT_NODE_LEAF_FLAG)) {
-                const float a = h[k].x * h[k].y + h[k].y * h[k].z + h[k].z * h[k].x;
-                if (a > bestArea) bestArea = a, best = k;
-            }
+            o[(2 * k) ^ sw] = k < cnt ? s[k].c : wide4_empty(false);
+            o[(2 * k + 1) ^ sw] = k < cnt ? make_float4(s[k].h.x, s[k].h.y, s[k].h.z, 0.0f) : wide4_empty(true);
         }
-        if (best < 0) break;
-        float4 bc = c[0];
-#pragma unroll
-        for (int k = 1; k < 4; ++k)
-            if (k == best) bc = c[k];
-        const float4 *w = reinterpret_cast<const float4 *>(wide + __float_as_uint(bc.w));
-        const float4 w0 = __ldcg(w), w1 = __ldcg(w + 1), w2 = __ldcg(w + 2), w3 = __ldcg(w + 3);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            if (k == best) c[k] = w0, h[k] = w1;
-            if (k == cnt) c[k] = make_float4(w2.x, w2.y, w2.z, w1.w), h[k] = w3;
-        }
-        cnt++;
     }
-    float4 *o = reinterpret_cast<float4 *>(wide4 + parent);
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        if (k < cnt) {
-            o[2 * k] = c[k];
-            o[2 * k + 1] = make_float4(h[k].x, h[k].y, h[k].z, 0.0f);
-        } else {
-            o[2 * k] = make_float4(0.0f, 0.0f, 0.0f, __uint_as_float(RT_WIDE4_EMPTY));
-            o[2 * k + 1] = make_float4(-1.0f, -1.0f, -1.0f, 0.0f);
-        }
+    __syncthreads();
+    const uint32_t b0 = blockIdx.x * blockDim.x;
+    const uint32_t valid = 8 * min(uint32_t(kThreads), n_internal - b0);
+    float4 *dst = reinterpret_cast<float4 *>(wide4 + b0);
+    for (uint32_t g = threadIdx.x; g < valid; g += kThreads) {
+        const uint32_t t = g >> 3, e = g & 7;
+        dst[g] = s_out[t * 8 + (e ^ (t & 7))];
     }
 }
 
-template <bool WIDE4 = false>
-__device__ __forceinline__ void fit_merge_store(uint32_t parent, uint32_t l, uint32_t r, uint32_t lc, uint32_t rc, Box bl, Box br,
-                                                uint32_t nInternal, rt_aabb_node *nodes, rt_wide_node *wide, rt_ext_header *ext, Box &box,
-                                                rt_wide4_node *wide4 = nullptr) {
-    if (rc < lc) {  // smaller subtree on the left; ties keep the Karras order
-        uint32_t t = l; l = r; r = t;
-        Box tb = bl; bl = br; br = tb;
-    }
-    float mn[3], mx[3];
-#pragma unroll
-    for (int k = 0; k < 3; ++k) {  // GetBoxFromChildBoxes: FL/RayTracingHelper.hlsli:297-307
-        mn[k] = fminf(bl.c[k] - bl.h[k], br.c[k] - br.h[k]);
-        mx[k] = fmaxf(bl.c[k] + bl.h[k], br.c[k] + br.h[k]);
-    }
-    box = aabb_to_box(mn, mx);
-    store_node(nodes, parent, box, l & 0x00ffffffu, r);
-    const uint32_t lref = l >= nInternal ? (RT_NODE_LEAF_FLAG | (l - nInternal)) : l;
-    const uint32_t rref = r >= nInternal ? (RT_NODE_LEAF_FLAG | (r - nInternal)) : r;
-    float4 *w = reinterpret_cast<float4 *>(wide + parent);
-    w[0] = make_float4(bl.c[0], bl.c[1], bl.c[2], __uint_as_float(lref));
-    w[1] = make_float4(bl.h[0], bl.h[1], bl.h[2], __uint_as_float(rref));
-    w[2] = make_float4(br.c[0], br.c[1], br.c[2], 0.0f);
-    w[3] = make_float4(br.h[0], br.h[1], br.h[2], 0.0f);
-    if (WIDE4) collapse4_store(parent, bl, lref, br, rref, wide, wide4);
-    if (parent == 0) {
-        ext->root_center[0] = box.c[0], ext->root_center[1] = box.c[1], ext->root_center[2] = box.c[2];
-        ext->root_half[0] = box.h[0], ext->root_half[1] = box.h[1], ext->root_half[2] = box.h[2];
-    }
-}
-
+// ------------------------------------------------------------------------------------------ block fit
+// A full bottom-level build fits the lower levels of the tree inside the thread block.  A block owns kFitBlock
+// consecutive sorted slots and works in rounds over a shared-memory ready queue: a node enters the queue when its second
+// child has been fitted, and the nodes of a round are handed to consecutive threads, so the warps stay dense where the
+// one-thread-per-leaf climb runs at 6-7 of 32 lanes (ncu) and pays a global atomic plus two device-wide fences per
+// level.  Child boxes and subtree sizes are exchanged through shared memory.  Nodes whose parent lies outside the block
+// leave through an exit list and finish with a global climb.  Results (reference nodes, wide nodes, 4-wide nodes, child
+// order) are those of the global climb, bit for bit: the child order depends only on the subtree sizes and the Karras
+// order, never on who arrives first.  Two kernels share this structure and differ in where the topology comes from:
+// k_fit_local reads the hierarchy array, k_lbvh_fit grows the Karras hierarchy from the Morton codes as it goes.
+//
+// Shared index of a node: leaf -> slot - b0 in [0, B); internal node i -> B + i - b0 in [B, 2B).
 constexpr size_t kFitLocalDynSmem = sizeof(float) * 6 * 2 * kFitBlock + sizeof(uint32_t) * 4 * kFitBlock;
+__device__ __forceinline__ uint32_t shared_index(uint32_t node, uint32_t nInternal, uint32_t b0) {
+    return node >= nInternal ? node - nInternal - b0 : kFitBlock + node - b0;
+}
+__device__ __forceinline__ Box shared_box(const float (*s_box)[6], uint32_t si) {
+    Box b;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) b.c[k] = s_box[si][k], b.h[k] = s_box[si][3 + k];
+    return b;
+}
+__device__ __forceinline__ void put_shared_box(float (*s_box)[6], uint32_t si, const Box &b) {
+#pragma unroll
+    for (int k = 0; k < 3; ++k) s_box[si][k] = b.c[k], s_box[si][3 + k] = b.h[k];
+}
+
+// This thread's leaf into shared memory: the box from the 48-byte packed record k_rearrange_tris wrote next to the
+// reference-format Primitive (same nine floats through three aligned 16-byte loads instead of ten 4-byte loads at
+// stride 40), and whether it is procedural.  Returns the box.
+__device__ __forceinline__ Box stage_leaf(float4 q0, float4 q1, float4 q2, float (*s_box)[6], uint8_t *s_proc) {
+    const float v[9] = {q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, q1.z, q1.w, q2.x};
+    const bool procedural = (__float_as_uint(q2.w) & RT_PACKED_PROCEDURAL) != 0;
+    const Box box = leaf_box(v, procedural);
+    put_shared_box(s_box, threadIdx.x, box);
+    s_proc[threadIdx.x] = procedural ? 1 : 0;
+    return box;
+}
+
+// Rounds.  fit_ready(entry, next) fits one ready entry of s_queue[cur] and queues what it readies in s_queue[next].  The
+// number of ready nodes never grows (a node fitted in one round readies at most its one parent), so once a round fits in
+// a warp the rest of the chain is run by warp 0 alone with warp barriers ...
+template <class Entry, class FitReady>
+__device__ __forceinline__ void block_fit_rounds(uint32_t *s_qn, Entry (*s_queue)[kFitBlock], const FitReady &fit_ready, const float (*s_box)[6],
+                                                 const uint8_t *s_proc, uint32_t b0, uint32_t nInternal, uint32_t cntLeaf, rt_aabb_node *nodes) {
+    int cur = 0;
+    for (; s_qn[cur] > 32; cur ^= 1) {  // block-uniform: s_qn[cur] is stable between the two barriers
+        if (threadIdx.x < s_qn[cur]) fit_ready(s_queue[cur][threadIdx.x], cur ^ 1);
+        __syncthreads();
+        if (threadIdx.x == 0) s_qn[cur] = 0;
+        __syncthreads();
+    }
+    __syncthreads();  // every warp has read the exit condition before warp 0 starts rewriting the queue counters
+    if (threadIdx.x < 32) {
+        for (;; cur ^= 1) {
+            const uint32_t q = s_qn[cur];
+            if (q == 0) break;
+            if (threadIdx.x < q) fit_ready(s_queue[cur][threadIdx.x], cur ^ 1);
+            __syncwarp();
+            if (threadIdx.x == 0) s_qn[cur] = 0;
+            __syncwarp();
+        }
+    } else {
+        // ... while the other warps write the leaf nodes {center, slot | flags}, {halfDim, 1}, which no round touches
+        // (a third of k_fit_local's stall samples were warps waiting at the barrier below for warp 0's tail)
+        float4 *dst = reinterpret_cast<float4 *>(nodes + nInternal + b0);
+        for (uint32_t g = threadIdx.x - 32; g < 2 * cntLeaf; g += kFitBlock - 32) {
+            const uint32_t e = g >> 1;
+            const float *bx = s_box[e];
+            if (g & 1) dst[g] = make_float4(bx[3], bx[4], bx[5], __uint_as_float(1u));
+            else dst[g] = make_float4(bx[0], bx[1], bx[2], __uint_as_float((b0 + e) | RT_NODE_LEAF_FLAG | (s_proc[e] ? RT_NODE_PROCEDURAL_FLAG : 0u)));
+        }
+    }
+    __syncthreads();
+}
+
+// collapse4's children from the block's shared memory: the boxes in s_box, the children of a node the block fitted
+// from `children` (see block_write_out).
+template <class Children>
+struct SharedChildren {
+    struct Slot {
+        uint32_t ref, si;  // traversal-section reference, shared index
+    };
+    const float (*s_box)[6];
+    Children children;
+    uint32_t nInternal, b0;
+    __device__ __forceinline__ uint32_t ref(const Slot &s) const { return s.ref; }
+    __device__ __forceinline__ float3 half(const Slot &s) const { return make_float3(s_box[s.si][3], s_box[s.si][4], s_box[s.si][5]); }
+    __device__ __forceinline__ Slot slot(uint32_t node) const { return {node_ref(node, nInternal), shared_index(node, nInternal, b0)}; }
+    __device__ __forceinline__ void open(const Slot &s, Slot &l, Slot &r) const {
+        uint32_t a, b;
+        children(s.ref - b0, a, b);
+        l = slot(a), r = slot(b);
+    }
+};
+
+// Write-out.  Everything the block fitted is described by shared memory (boxes, children), so the reference nodes, the
+// wide nodes and the 4-wide nodes leave as contiguous runs of 16-byte stores — the rounds issued none.  (One thread
+// storing its own node's 32 + 64 bytes touched 32 sectors per warp instruction.)  fitted(e): the block fitted internal
+// node b0 + e; children(e, l, r): that node's children, in their final order.  s_w4 receives the 4-wide child lists.
+template <class Fitted, class Children>
+__device__ __forceinline__ void block_write_out(uint32_t b0, uint32_t nInternal, uint32_t cntInt, const float (*s_box)[6], uint32_t (*s_w4)[4],
+                                                const Fitted &fitted, const Children &children, rt_aabb_node *nodes, rt_wide_node *wide,
+                                                rt_wide4_node *wide4, rt_ext_header *ext) {
+    {   // internal reference nodes: {center, left}, {halfDim, right}
+        float4 *dst = reinterpret_cast<float4 *>(nodes + b0);
+        for (uint32_t g = threadIdx.x; g < 2 * cntInt; g += kFitBlock) {
+            const uint32_t e = g >> 1;
+            if (!fitted(e)) continue;
+            uint32_t l, r;
+            children(e, l, r);
+            const float *bx = s_box[kFitBlock + e];
+            if (g & 1) dst[g] = make_float4(bx[3], bx[4], bx[5], __uint_as_float(r));
+            else dst[g] = make_float4(bx[0], bx[1], bx[2], __uint_as_float(l & 0x00ffffffu));
+        }
+    }
+    {   // wide nodes: both child boxes and child references
+        float4 *dst = reinterpret_cast<float4 *>(wide + b0);
+        for (uint32_t g = threadIdx.x; g < 4 * cntInt; g += kFitBlock) {
+            const uint32_t e = g >> 2, part = g & 3;
+            if (!fitted(e)) continue;
+            uint32_t l, r;
+            children(e, l, r);
+            const float *bx = s_box[shared_index(part < 2 ? l : r, nInternal, b0)];
+            const uint32_t w = part == 0 ? node_ref(l, nInternal) : (part == 1 ? node_ref(r, nInternal) : 0u);
+            if (part & 1) dst[g] = make_float4(bx[3], bx[4], bx[5], __uint_as_float(w));
+            else dst[g] = make_float4(bx[0], bx[1], bx[2], __uint_as_float(w));
+        }
+    }
+    // 4-wide nodes, straight from shared memory: the child lists first ...
+    if (threadIdx.x < cntInt && fitted(threadIdx.x)) {
+        const SharedChildren<Children> src{s_box, children, nInternal, b0};
+        typename SharedChildren<Children>::Slot s[4];
+        uint32_t l, r;
+        children(threadIdx.x, l, r);
+        s[0] = src.slot(l), s[1] = src.slot(r);
+        const int cnt = collapse4(src, s);
+#pragma unroll
+        for (int k = 0; k < 4; ++k) s_w4[threadIdx.x][k] = k < cnt ? s[k].ref : RT_WIDE4_EMPTY;
+    }
+    __syncthreads();
+    {   // ... then the 128-byte nodes as one contiguous run
+        float4 *dst = reinterpret_cast<float4 *>(wide4 + b0);
+        for (uint32_t g = threadIdx.x; g < 8 * cntInt; g += kFitBlock) {
+            const uint32_t e = g >> 3, part = g & 7;
+            if (!fitted(e)) continue;
+            const uint32_t ref = s_w4[e][part >> 1];
+            if (ref == RT_WIDE4_EMPTY) {
+                dst[g] = wide4_empty(part & 1);
+            } else {
+                const float *bx = s_box[(ref & RT_NODE_LEAF_FLAG) ? (ref & 0x00ffffffu) - b0 : kFitBlock + ref - b0];
+                dst[g] = (part & 1) ? make_float4(bx[3], bx[4], bx[5], 0.0f) : make_float4(bx[0], bx[1], bx[2], __uint_as_float(ref));
+            }
+        }
+    }
+    if (b0 == 0 && nInternal > 0 && threadIdx.x == 0 && fitted(0)) store_root(ext, shared_box(s_box, kFitBlock));  // the whole tree was local
+}
+
+// The block fit driven by the hierarchy array: a parent flagged `local` (k_hierarchy; kept valid by k_treelet_reorder)
+// has its whole subtree among the block's slots.  Full BLAS builds with treelet passes or ALLOW_UPDATE.
 __global__ void __launch_bounds__(kFitBlock) k_fit_local(uint32_t n, const rt_hierarchy_node *hier, uint32_t *counters, rt_aabb_node *nodes,
                                                          const rt_packed_tri *packed, rt_wide_node *wide, rt_wide4_node *wide4,
                                                          rt_ext_header *ext, const uint8_t *local, uint32_t *exit_nodes,
                                                          uint16_t *exit_sizes) {
-    // shared index of a node: leaf -> slot - b0 in [0, B); internal -> B + index - b0 in [B, 2B)
     extern __shared__ __align__(16) uint8_t s_dyn[];  // kFitLocalDynSmem bytes: the boxes and the 4-wide child lists
     float(*s_box)[6] = reinterpret_cast<float(*)[6]>(s_dyn);
     uint32_t(*s_w4)[4] = reinterpret_cast<uint32_t(*)[4]>(s_dyn + sizeof(float) * 6 * 2 * kFitBlock);
@@ -731,8 +937,6 @@ __global__ void __launch_bounds__(kFitBlock) k_fit_local(uint32_t n, const rt_hi
     float4 q0 = make_float4(0, 0, 0, 0), q1 = q0, q2 = q0;
     uint32_t leafParent = 0;
     if (slot < n) {
-        // the 48-byte packed record k_rearrange_tris wrote next to the reference-format Primitive: same nine floats
-        // through three aligned 16-byte loads instead of ten 4-byte loads at stride 40
         const float4 *q = reinterpret_cast<const float4 *>(packed + slot);
         q0 = q[0], q1 = q[1], q2 = q[2];
         if (n > 1) leafParent = __ldg(hw + 3 * size_t(nInternal + slot)) & ~treelet::kCollapseBit;
@@ -748,234 +952,58 @@ __global__ void __launch_bounds__(kFitBlock) k_fit_local(uint32_t n, const rt_hi
             s_exit[atomicAdd(&s_en, 1u)] = node;
         }
     };
-    auto shared_index = [&](uint32_t node) { return node >= nInternal ? node - nInternal - b0 : kFitBlock + node - b0; };
-    auto load_box = [&](uint32_t si) {
-        Box b;
-#pragma unroll
-        for (int k = 0; k < 3; ++k) b.c[k] = s_box[si][k], b.h[k] = s_box[si][3 + k];
-        return b;
-    };
     if (slot < n) {
-        const float v[9] = {q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, q1.z, q1.w, q2.x};
-        float mn[3], mx[3];
-        const bool procedural = (__float_as_uint(q2.w) & RT_PACKED_PROCEDURAL) != 0;
-        if (procedural) {
-#pragma unroll
-            for (int k = 0; k < 3; ++k) mn[k] = v[k], mx[k] = v[3 + k];
-        } else {
-#pragma unroll
-            for (int k = 0; k < 3; ++k) {
-                mn[k] = fminf(fminf(v[k], v[3 + k]), v[6 + k]);
-                mx[k] = fmaxf(fmaxf(v[k], v[3 + k]), v[6 + k]);
-                mn[k] = fminf(mn[k], mx[k] - 0.001f);  // AABB_Min_Padding
-            }
-        }
-        const Box box = aabb_to_box(mn, mx);
-#pragma unroll
-        for (int k = 0; k < 3; ++k) s_box[threadIdx.x][k] = box.c[k], s_box[threadIdx.x][3 + k] = box.h[k];
+        const Box box = stage_leaf(q0, q1, q2, s_box, s_proc);
         s_size[threadIdx.x] = 1;
-        s_proc[threadIdx.x] = procedural ? 1 : 0;
-        if (n == 1) {
-            ext->root_center[0] = box.c[0], ext->root_center[1] = box.c[1], ext->root_center[2] = box.c[2];
-            ext->root_half[0] = box.h[0], ext->root_half[1] = box.h[1], ext->root_half[2] = box.h[2];
-        } else {
-            report(nInternal + slot, leafParent, 0);
-        }
+        if (n == 1) store_root(ext, box);
+        else report(nInternal + slot, leafParent, 0);
     }
     __syncthreads();
-    // One ready node: its box from its children's shared boxes (GetBoxFromChildBoxes, FL/RayTracingHelper.hlsli:297-307),
-    // published in shared memory; nothing is stored to global memory here.
+    // One ready node: its box from its children's shared boxes, published in shared memory; nothing is stored to
+    // global memory here.
     auto fit_ready = [&](uint32_t p, int next) {
         const uint32_t *rec = s_hier + 3 * (p - b0);
         const uint32_t up = rec[0] & ~treelet::kCollapseBit;
-        uint32_t li = shared_index(rec[1]), ri = shared_index(rec[2]);
-        if (s_size[ri] < s_size[li]) {  // operand order of the reference's min/max: smaller subtree first
+        uint32_t li = shared_index(rec[1], nInternal, b0), ri = shared_index(rec[2], nInternal, b0);
+        if (s_size[ri] < s_size[li]) {  // smaller subtree on the left; ties keep the Karras order
             const uint32_t t = li; li = ri; ri = t;
         }
-        const Box bl = load_box(li), br = load_box(ri);
-        float mn[3], mx[3];
-#pragma unroll
-        for (int k = 0; k < 3; ++k) {
-            mn[k] = fminf(bl.c[k] - bl.h[k], br.c[k] - br.h[k]);
-            mx[k] = fmaxf(bl.c[k] + bl.h[k], br.c[k] + br.h[k]);
-        }
-        const Box box = aabb_to_box(mn, mx);
         const uint32_t pi = kFitBlock + p - b0;
-#pragma unroll
-        for (int k = 0; k < 3; ++k) s_box[pi][k] = box.c[k], s_box[pi][3 + k] = box.h[k];
+        put_shared_box(s_box, pi, merge_boxes(shared_box(s_box, li), shared_box(s_box, ri)));
         s_size[pi] = s_size[li] + s_size[ri];
         if (p != 0) report(p, up, next);
     };
-    // Rounds.  The number of ready nodes never grows (a node fitted in one round readies at most its one parent), so
-    // once a round fits in a warp the rest of the chain is run by warp 0 alone with warp barriers.
-    int cur = 0;
-    for (; s_qn[cur] > 32; cur ^= 1) {  // block-uniform: s_qn[cur] is stable between the two barriers
-        if (threadIdx.x < s_qn[cur]) fit_ready(s_queue[cur][threadIdx.x], cur ^ 1);
-        __syncthreads();
-        if (threadIdx.x == 0) s_qn[cur] = 0;
-        __syncthreads();
-    }
-    __syncthreads();  // every warp has read the exit condition before warp 0 starts rewriting the queue counters
-    if (threadIdx.x < 32) {
-        for (;; cur ^= 1) {
-            const uint32_t q = s_qn[cur];
-            if (q == 0) break;
-            if (threadIdx.x < q) fit_ready(s_queue[cur][threadIdx.x], cur ^ 1);
-            __syncwarp();
-            if (threadIdx.x == 0) s_qn[cur] = 0;
-            __syncwarp();
-        }
-    } else {
-        // ... while the other warps write the leaf nodes {center, slot | flags}, {halfDim, 1}, which no round touches
-        // (a third of this kernel's stall samples were warps waiting at the barrier below for warp 0's tail)
-        float4 *dst = reinterpret_cast<float4 *>(nodes + nInternal + b0);
-        for (uint32_t g = threadIdx.x - 32; g < 2 * cntLeaf; g += kFitBlock - 32) {
-            const uint32_t e = g >> 1;
-            const float *bx = s_box[e];
-            if (g & 1) dst[g] = make_float4(bx[3], bx[4], bx[5], __uint_as_float(1u));
-            else dst[g] = make_float4(bx[0], bx[1], bx[2], __uint_as_float((b0 + e) | RT_NODE_LEAF_FLAG | (s_proc[e] ? RT_NODE_PROCEDURAL_FLAG : 0u)));
-        }
-    }
-    __syncthreads();
-    // Write-out.  Everything this block fitted is described by shared memory (boxes, subtree sizes, hierarchy records),
-    // so the reference nodes and the wide nodes leave as contiguous runs of 16-byte stores — the rounds above issued
-    // none.  (One thread storing its own node's 32 + 64 bytes touched 32 sectors per warp instruction.)
+    block_fit_rounds(s_qn, s_queue, fit_ready, s_box, s_proc, b0, nInternal, cntLeaf, nodes);
     const uint32_t en = s_en;
     if (threadIdx.x == 0 && en) s_base = atomicAdd(&counters[nInternal], en);  // counters[n-1] is no node's counter
-    // Child order of a fitted node: smaller subtree on the left; ties keep the Karras order.  Applied once, in place, to
-    // the shared copy of the hierarchy records, so that the write-out loops below (which visit a node once per 16-byte
-    // store) just read {left, right}.
+    // The child order of a fitted node is applied once, in place, to the shared copy of the hierarchy records, so that
+    // the write-out (which visits a node once per 16-byte store) just reads {left, right}.
     if (threadIdx.x < cntInt && s_arrive[threadIdx.x] == 2) {
         const uint32_t l = s_hier[3 * threadIdx.x + 1], r = s_hier[3 * threadIdx.x + 2];
-        if (s_size[shared_index(r)] < s_size[shared_index(l)]) s_hier[3 * threadIdx.x + 1] = r, s_hier[3 * threadIdx.x + 2] = l;
+        if (s_size[shared_index(r, nInternal, b0)] < s_size[shared_index(l, nInternal, b0)]) s_hier[3 * threadIdx.x + 1] = r, s_hier[3 * threadIdx.x + 2] = l;
     }
     __syncthreads();
-    auto children = [&](uint32_t e, uint32_t &l, uint32_t &r, uint32_t &li, uint32_t &ri) {
-        l = s_hier[3 * e + 1], r = s_hier[3 * e + 2];
-        li = shared_index(l), ri = shared_index(r);
-    };
-    {   // internal reference nodes: {center, left}, {halfDim, right}
-        float4 *dst = reinterpret_cast<float4 *>(nodes + b0);
-        for (uint32_t g = threadIdx.x; g < 2 * cntInt; g += kFitBlock) {
-            const uint32_t e = g >> 1;
-            if (s_arrive[e] != 2) continue;
-            uint32_t l, r, li, ri;
-            children(e, l, r, li, ri);
-            const float *bx = s_box[kFitBlock + e];
-            if (g & 1) dst[g] = make_float4(bx[3], bx[4], bx[5], __uint_as_float(r));
-            else dst[g] = make_float4(bx[0], bx[1], bx[2], __uint_as_float(l & 0x00ffffffu));
-        }
-    }
-    {   // wide nodes: both child boxes and child references
-        float4 *dst = reinterpret_cast<float4 *>(wide + b0);
-        for (uint32_t g = threadIdx.x; g < 4 * cntInt; g += kFitBlock) {
-            const uint32_t e = g >> 2, part = g & 3;
-            if (s_arrive[e] != 2) continue;
-            uint32_t l, r, li, ri;
-            children(e, l, r, li, ri);
-            const float *bx = s_box[part < 2 ? li : ri];
-            const uint32_t lref = l >= nInternal ? (RT_NODE_LEAF_FLAG | (l - nInternal)) : l;
-            const uint32_t rref = r >= nInternal ? (RT_NODE_LEAF_FLAG | (r - nInternal)) : r;
-            const uint32_t w = part == 0 ? lref : (part == 1 ? rref : 0u);
-            if (part & 1) dst[g] = make_float4(bx[3], bx[4], bx[5], __uint_as_float(w));
-            else dst[g] = make_float4(bx[0], bx[1], bx[2], __uint_as_float(w));
-        }
-    }
-    // 4-wide traversal nodes of the fitted nodes (what k_collapse4 derives from the wide nodes, here straight from
-    // shared memory): open, twice, the internal child with the largest surface area; the child lists first ...
-    if (threadIdx.x < cntInt && s_arrive[threadIdx.x] == 2) {
-        uint32_t ref[4] = {RT_WIDE4_EMPTY, RT_WIDE4_EMPTY, RT_WIDE4_EMPTY, RT_WIDE4_EMPTY}, si[4] = {0, 0, 0, 0};
-        int cnt = 2;
-        auto to_ref = [&](uint32_t node) { return node >= nInternal ? (RT_NODE_LEAF_FLAG | (node - nInternal)) : node; };
-        {
-            uint32_t l, r, li, ri;
-            children(threadIdx.x, l, r, li, ri);
-            ref[0] = to_ref(l), ref[1] = to_ref(r), si[0] = li, si[1] = ri;
-        }
-#pragma unroll
-        for (int it = 0; it < 2; ++it) {
-            int best = -1;
-            float bestArea = -1.0f;
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                if (k < cnt && !(ref[k] & RT_NODE_LEAF_FLAG)) {
-                    const float *h = s_box[si[k]] + 3;
-                    const float a = h[0] * h[1] + h[1] * h[2] + h[2] * h[0];
-                    if (a > bestArea) bestArea = a, best = k;
-                }
-            }
-            if (best < 0) break;
-            uint32_t opened = ref[0];
-#pragma unroll
-            for (int k = 1; k < 4; ++k)
-                if (k == best) opened = ref[k];
-            uint32_t l, r, li, ri;
-            children(opened - b0, l, r, li, ri);
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                if (k == best) ref[k] = to_ref(l), si[k] = li;
-                if (k == cnt) ref[k] = to_ref(r), si[k] = ri;
-            }
-            cnt++;
-        }
-#pragma unroll
-        for (int k = 0; k < 4; ++k) s_w4[threadIdx.x][k] = ref[k];
-    }
-    __syncthreads();
-    {   // ... then the 128-byte nodes as one contiguous run
-        float4 *dst = reinterpret_cast<float4 *>(wide4 + b0);
-        for (uint32_t g = threadIdx.x; g < 8 * cntInt; g += kFitBlock) {
-            const uint32_t e = g >> 3, part = g & 7;
-            if (s_arrive[e] != 2) continue;
-            const uint32_t ref = s_w4[e][part >> 1];
-            if (ref == RT_WIDE4_EMPTY) {
-                dst[g] = (part & 1) ? make_float4(-1.0f, -1.0f, -1.0f, 0.0f) : make_float4(0.0f, 0.0f, 0.0f, __uint_as_float(RT_WIDE4_EMPTY));
-            } else {
-                const float *bx = s_box[(ref & RT_NODE_LEAF_FLAG) ? (ref & 0x00ffffffu) - b0 : kFitBlock + ref - b0];
-                dst[g] = (part & 1) ? make_float4(bx[3], bx[4], bx[5], 0.0f) : make_float4(bx[0], bx[1], bx[2], __uint_as_float(ref));
-            }
-        }
-    }
-    if (b0 == 0 && nInternal > 0 && threadIdx.x == 0 && s_arrive[0] == 2) {  // the whole tree was local
-        const float *bx = s_box[kFitBlock];
-        ext->root_center[0] = bx[0], ext->root_center[1] = bx[1], ext->root_center[2] = bx[2];
-        ext->root_half[0] = bx[3], ext->root_half[1] = bx[4], ext->root_half[2] = bx[5];
-    }
+    block_write_out(
+        b0, nInternal, cntInt, s_box, s_w4, [&](uint32_t e) { return s_arrive[e] == 2; },
+        [&](uint32_t e, uint32_t &l, uint32_t &r) { l = s_hier[3 * e + 1], r = s_hier[3 * e + 2]; }, nodes, wide, wide4, ext);
     __syncthreads();
     // the nodes whose parent's subtree crosses the block boundary continue in k_fit_exits
     if (threadIdx.x < en) {
         const uint32_t node = s_exit[threadIdx.x];
         exit_nodes[s_base + threadIdx.x] = node;
-        exit_sizes[s_base + threadIdx.x] = uint16_t(s_size[shared_index(node)]);
+        exit_sizes[s_base + threadIdx.x] = uint16_t(s_size[shared_index(node, nInternal, b0)]);
     }
 }
 
-// Second half of k_fit_local: one thread per exit-list entry climbs through global memory exactly as k_fit does.
+// Second half of k_fit_local: one thread per exit-list entry climbs through global memory.
 __global__ void __launch_bounds__(kThreads) k_fit_exits(uint32_t n, const rt_hierarchy_node *hier, uint32_t *counters, rt_aabb_node *nodes,
                                                         rt_wide_node *wide, rt_wide4_node *wide4, rt_ext_header *ext,
                                                         const uint32_t *exit_nodes, const uint16_t *exit_sizes) {
     const uint32_t nInternal = n - 1;
     const uint32_t entries = __ldcg(&counters[nInternal]);
-    const uint32_t *hw = reinterpret_cast<const uint32_t *>(hier);
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < entries; i += gridDim.x * blockDim.x) {  // grid: see k_lbvh_exits
-    uint32_t node = exit_nodes[i];
-    uint32_t count = exit_sizes[i];
-    Box box = load_node_box(nodes, node);
-    while (true) {
-        const uint32_t parent = __ldg(hw + 3 * size_t(node)) & ~treelet::kCollapseBit;
-        const uint32_t l = __ldg(hw + 3 * size_t(parent) + 1), r = __ldg(hw + 3 * size_t(parent) + 2);
-        __threadfence();
-        const uint32_t other = atomicAdd(&counters[parent], count);
-        if (other == 0) break;  // first to arrive: the sibling will fit the parent
-        __threadfence();
-        const bool isLeft = (l == node);
-        const Box sb = load_node_box(nodes, isLeft ? r : l);
-        fit_merge_store<true>(parent, l, r, isLeft ? count : other, isLeft ? other : count, isLeft ? box : sb, isLeft ? sb : box, nInternal,
-                              nodes, wide, ext, box, wide4);
-        if (parent == 0) break;
-        count += other;
-        node = parent;
-    }
+        const uint32_t node = exit_nodes[i];
+        climb<false, true>(node, exit_sizes[i], load_node_box(nodes, node), nInternal, hier, nullptr, counters, nodes, wide, wide4, ext);
     }
 }
 
@@ -1005,7 +1033,6 @@ __global__ void __launch_bounds__(kFitBlock) k_lbvh_fit(uint32_t n, const uint32
                                                         rt_ext_header *ext, uint32_t *exit_count, uint32_t *exit_nodes, uint32_t *exit_lo,
                                                         uint32_t *exit_hi) {
     constexpr int B = kFitBlock;
-    // shared index of a node: leaf -> slot - b0 in [0, B); internal -> B + id - b0 in [B, 2B)
     extern __shared__ __align__(16) uint8_t s_dyn[];  // kFitLocalDynSmem bytes: the boxes and the 4-wide child lists
     float(*s_box)[6] = reinterpret_cast<float(*)[6]>(s_dyn);
     uint32_t(*s_w4)[4] = reinterpret_cast<uint32_t(*)[4]>(s_dyn + sizeof(float) * 6 * 2 * B);
@@ -1036,13 +1063,6 @@ __global__ void __launch_bounds__(kFitBlock) k_lbvh_fit(uint32_t n, const uint32
         s_delta[threadIdx.x + 1] = int8_t(lbvh_delta(codes, n, slot));
         if (threadIdx.x == 0) s_delta[0] = int8_t(lbvh_delta(codes, n, slot - 1));  // slot 0: index "-1"
     }
-    auto shared_index = [&](uint32_t node) { return node >= nInternal ? node - nInternal - b0 : B + node - b0; };
-    auto load_box = [&](uint32_t si) {
-        Box b;
-#pragma unroll
-        for (int k = 0; k < 3; ++k) b.c[k] = s_box[si][k], b.h[k] = s_box[si][3 + k];
-        return b;
-    };
     // a finished node [lo, hi] (global slots, inside this block) reports to the split it hangs on
     auto report = [&](uint32_t node, uint32_t lo, uint32_t hi, int next) {
         const bool goRight = s_delta[hi - b0 + 1] > s_delta[lo - b0];
@@ -1057,175 +1077,40 @@ __global__ void __launch_bounds__(kFitBlock) k_lbvh_fit(uint32_t n, const uint32
         }
     };
     if (slot < n) {
-        const float v[9] = {q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, q1.z, q1.w, q2.x};
-        float mn[3], mx[3];
-        const bool procedural = (__float_as_uint(q2.w) & RT_PACKED_PROCEDURAL) != 0;
-        if (procedural) {
-#pragma unroll
-            for (int k = 0; k < 3; ++k) mn[k] = v[k], mx[k] = v[3 + k];
-        } else {
-#pragma unroll
-            for (int k = 0; k < 3; ++k) {
-                mn[k] = fminf(fminf(v[k], v[3 + k]), v[6 + k]);
-                mx[k] = fmaxf(fmaxf(v[k], v[3 + k]), v[6 + k]);
-                mn[k] = fminf(mn[k], mx[k] - 0.001f);  // AABB_Min_Padding
-            }
-        }
-        const Box box = aabb_to_box(mn, mx);
-#pragma unroll
-        for (int k = 0; k < 3; ++k) s_box[threadIdx.x][k] = box.c[k], s_box[threadIdx.x][3 + k] = box.h[k];
-        s_proc[threadIdx.x] = procedural ? 1 : 0;
-        if (n == 1) {
-            ext->root_center[0] = box.c[0], ext->root_center[1] = box.c[1], ext->root_center[2] = box.c[2];
-            ext->root_half[0] = box.h[0], ext->root_half[1] = box.h[1], ext->root_half[2] = box.h[2];
-        }
+        const Box box = stage_leaf(q0, q1, q2, s_box, s_proc);
+        if (n == 1) store_root(ext, box);
     }
     __syncthreads();  // s_delta, the cleared slots
     if (slot < n && n > 1) report(nInternal + slot, slot, slot, 0);
     __syncthreads();
-    // One ready split: both children are in shared memory (GetBoxFromChildBoxes, FL/RayTracingHelper.hlsli:297-307).
+    // One ready split: both children are in shared memory.
     auto fit_ready = [&](uint32_t g, int next) {
         const uint32_t lo = b0 + s_bound[0][g], hi = b0 + s_bound[1][g], split = b0 + g;
         uint32_t a = s_kid[0][g], b = s_kid[1][g];
         if (hi - split < split - lo + 1) {  // smaller subtree on the left; ties keep the Karras order
             const uint32_t t = a; a = b; b = t;
         }
-        const Box bl = load_box(shared_index(a)), br = load_box(shared_index(b));
-        float mn[3], mx[3];
-#pragma unroll
-        for (int k = 0; k < 3; ++k) {
-            mn[k] = fminf(bl.c[k] - bl.h[k], br.c[k] - br.h[k]);
-            mx[k] = fmaxf(bl.c[k] + bl.h[k], br.c[k] + br.h[k]);
-        }
-        const Box box = aabb_to_box(mn, mx);
+        const Box box = merge_boxes(shared_box(s_box, shared_index(a, nInternal, b0)), shared_box(s_box, shared_index(b, nInternal, b0)));
         const bool root = lo == 0 && hi == n - 1;
         const uint32_t id = root ? 0u : (s_delta[hi - b0 + 1] > s_delta[lo - b0] ? hi : lo);
         const uint32_t e = id - b0;
-#pragma unroll
-        for (int k = 0; k < 3; ++k) s_box[B + e][k] = box.c[k], s_box[B + e][3 + k] = box.h[k];
+        put_shared_box(s_box, B + e, box);
         s_left[e] = a, s_right[e] = b;
         s_range[e] = (lo - b0) | ((hi - b0) << 16);
         s_fitted[e] = 1;
         if (!root) report(id, lo, hi, next);
     };
-    // Rounds.  The number of ready splits never grows, so once a round fits in a warp the rest is run by warp 0 alone.
-    int cur = 0;
-    for (; s_qn[cur] > 32; cur ^= 1) {  // block-uniform: s_qn[cur] is stable between the two barriers
-        if (threadIdx.x < s_qn[cur]) fit_ready(s_queue[cur][threadIdx.x], cur ^ 1);
-        __syncthreads();
-        if (threadIdx.x == 0) s_qn[cur] = 0;
-        __syncthreads();
-    }
-    __syncthreads();  // every warp has read the exit condition before warp 0 starts rewriting the queue counters
-    if (threadIdx.x < 32) {
-        for (;; cur ^= 1) {
-            const uint32_t q = s_qn[cur];
-            if (q == 0) break;
-            if (threadIdx.x < q) fit_ready(s_queue[cur][threadIdx.x], cur ^ 1);
-            __syncwarp();
-            if (threadIdx.x == 0) s_qn[cur] = 0;
-            __syncwarp();
-        }
-    } else {
-        // ... while the other warps write the leaf nodes {center, slot | flags}, {halfDim, 1}, which no round touches
-        // (in k_fit_local a third of the stall samples are warps waiting at the barrier below for this tail)
-        float4 *dst = reinterpret_cast<float4 *>(nodes + nInternal + b0);
-        for (uint32_t g = threadIdx.x - 32; g < 2 * cntLeaf; g += B - 32) {
-            const uint32_t e = g >> 1;
-            const float *bx = s_box[e];
-            if (g & 1) dst[g] = make_float4(bx[3], bx[4], bx[5], __uint_as_float(1u));
-            else dst[g] = make_float4(bx[0], bx[1], bx[2], __uint_as_float((b0 + e) | RT_NODE_LEAF_FLAG | (s_proc[e] ? RT_NODE_PROCEDURAL_FLAG : 0u)));
-        }
-    }
-    __syncthreads();
+    block_fit_rounds(s_qn, s_queue, fit_ready, s_box, s_proc, b0, nInternal, cntLeaf, nodes);
     // a node still waiting at a split is one whose sibling reaches out of the block
     if (s_arrive[threadIdx.x] == 1u) {
         const uint32_t l = s_kid[0][threadIdx.x];
         s_exit[atomicAdd(&s_en, 1u)] = l != kNoKid ? l : s_kid[1][threadIdx.x];
     }
     __syncthreads();
-    // Write-out: everything this block fitted leaves as contiguous runs of 16-byte stores.
     const uint32_t en = s_en;
-    auto to_ref = [&](uint32_t node) { return node >= nInternal ? (RT_NODE_LEAF_FLAG | (node - nInternal)) : node; };
-    {   // internal reference nodes: {center, left}, {halfDim, right}
-        float4 *dst = reinterpret_cast<float4 *>(nodes + b0);
-        for (uint32_t g = threadIdx.x; g < 2 * cntInt; g += B) {
-            const uint32_t e = g >> 1;
-            if (!s_fitted[e]) continue;
-            const float *bx = s_box[B + e];
-            if (g & 1) dst[g] = make_float4(bx[3], bx[4], bx[5], __uint_as_float(s_right[e]));
-            else dst[g] = make_float4(bx[0], bx[1], bx[2], __uint_as_float(s_left[e] & 0x00ffffffu));
-        }
-    }
-    {   // wide nodes: both child boxes and child references
-        float4 *dst = reinterpret_cast<float4 *>(wide + b0);
-        for (uint32_t g = threadIdx.x; g < 4 * cntInt; g += B) {
-            const uint32_t e = g >> 2, part = g & 3;
-            if (!s_fitted[e]) continue;
-            const uint32_t l = s_left[e], r = s_right[e];
-            const float *bx = s_box[shared_index(part < 2 ? l : r)];
-            const uint32_t w = part == 0 ? to_ref(l) : (part == 1 ? to_ref(r) : 0u);
-            if (part & 1) dst[g] = make_float4(bx[3], bx[4], bx[5], __uint_as_float(w));
-            else dst[g] = make_float4(bx[0], bx[1], bx[2], __uint_as_float(w));
-        }
-    }
-    // 4-wide traversal nodes (k_collapse4's rule: open, twice, the internal child with the largest surface area): the
-    // child lists first ...
-    if (threadIdx.x < cntInt && s_fitted[threadIdx.x]) {
-        uint32_t ref[4] = {RT_WIDE4_EMPTY, RT_WIDE4_EMPTY, RT_WIDE4_EMPTY, RT_WIDE4_EMPTY}, si[4] = {0, 0, 0, 0};
-        int cnt = 2;
-        {
-            const uint32_t l = s_left[threadIdx.x], r = s_right[threadIdx.x];
-            ref[0] = to_ref(l), ref[1] = to_ref(r), si[0] = shared_index(l), si[1] = shared_index(r);
-        }
-#pragma unroll
-        for (int it = 0; it < 2; ++it) {
-            int best = -1;
-            float bestArea = -1.0f;
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                if (k < cnt && !(ref[k] & RT_NODE_LEAF_FLAG)) {
-                    const float *h = s_box[si[k]] + 3;
-                    const float a = h[0] * h[1] + h[1] * h[2] + h[2] * h[0];
-                    if (a > bestArea) bestArea = a, best = k;
-                }
-            }
-            if (best < 0) break;
-            uint32_t opened = ref[0];
-#pragma unroll
-            for (int k = 1; k < 4; ++k)
-                if (k == best) opened = ref[k];
-            const uint32_t l = s_left[opened - b0], r = s_right[opened - b0];
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                if (k == best) ref[k] = to_ref(l), si[k] = shared_index(l);
-                if (k == cnt) ref[k] = to_ref(r), si[k] = shared_index(r);
-            }
-            cnt++;
-        }
-#pragma unroll
-        for (int k = 0; k < 4; ++k) s_w4[threadIdx.x][k] = ref[k];
-    }
-    __syncthreads();
-    {   // ... then the 128-byte nodes as one contiguous run
-        float4 *dst = reinterpret_cast<float4 *>(wide4 + b0);
-        for (uint32_t g = threadIdx.x; g < 8 * cntInt; g += B) {
-            const uint32_t e = g >> 3, part = g & 7;
-            if (!s_fitted[e]) continue;
-            const uint32_t ref = s_w4[e][part >> 1];
-            if (ref == RT_WIDE4_EMPTY) {
-                dst[g] = (part & 1) ? make_float4(-1.0f, -1.0f, -1.0f, 0.0f) : make_float4(0.0f, 0.0f, 0.0f, __uint_as_float(RT_WIDE4_EMPTY));
-            } else {
-                const float *bx = s_box[(ref & RT_NODE_LEAF_FLAG) ? (ref & 0x00ffffffu) - b0 : B + ref - b0];
-                dst[g] = (part & 1) ? make_float4(bx[3], bx[4], bx[5], 0.0f) : make_float4(bx[0], bx[1], bx[2], __uint_as_float(ref));
-            }
-        }
-    }
-    if (b0 == 0 && nInternal > 0 && threadIdx.x == 0 && s_fitted[0]) {  // node 0 is the root: the whole tree was local
-        const float *bx = s_box[B];
-        ext->root_center[0] = bx[0], ext->root_center[1] = bx[1], ext->root_center[2] = bx[2];
-        ext->root_half[0] = bx[3], ext->root_half[1] = bx[4], ext->root_half[2] = bx[5];
-    }
+    block_write_out(
+        b0, nInternal, cntInt, s_box, s_w4, [&](uint32_t e) { return s_fitted[e] != 0; },
+        [&](uint32_t e, uint32_t &l, uint32_t &r) { l = s_left[e], r = s_right[e]; }, nodes, wide, wide4, ext);
     // the nodes that leave the block continue in k_lbvh_exits: {node, lo, hi}
     if (threadIdx.x == 0 && en) s_base = atomicAdd(exit_count, en);
     __syncthreads();
@@ -1279,76 +1164,12 @@ __global__ void __launch_bounds__(kThreads) k_lbvh_exits(uint32_t n, const uint3
             up = lbvh_delta(codes, n, nhi) > lbvh_delta(codes, n, nlo - 1);
             id = up ? nhi : nlo;
         }
-        // Karras order: the child on the lower slots is "left"; fit_merge_store applies the size rule
-        fit_merge_store<true>(id, goRight ? node : sib, goRight ? sib : node, split - nlo + 1, nhi - split, goRight ? box : sb,
-                              goRight ? sb : box, nInternal, nodes, wide, ext, box, wide4);
+        // Karras order: the child on the lower slots is "left"; fit_parent applies the size rule
+        box = fit_parent<true, true>(id, goRight ? node : sib, goRight ? sib : node, split - nlo + 1, nhi - split, goRight ? box : sb,
+                                     goRight ? sb : box, nInternal, nodes, wide, wide4, ext);
         if (root) break;
         node = id, lo = nlo, hi = nhi, goRight = up;
     }
-    }
-}
-
-// BVH2 -> BVH4 for the traversal kernels.  Thread i opens node i's two children and then, twice, the internal slot
-// with the largest surface area (half-extent product sum), reading the child boxes straight from the BVH2 wide nodes.
-__global__ void __launch_bounds__(kThreads) k_collapse4(const rt_wide_node *wide, uint32_t n_internal, rt_wide4_node *wide4) {
-    // the block's kThreads x 128-byte nodes leave through shared memory as one contiguous run of 16-byte stores; slot
-    // k of thread t sits at t * 8 + (k ^ (t & 7)) so that neither side has bank conflicts
-    __shared__ float4 s_out[kThreads * 8];
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    float4 c[4], h[4];  // {center, ref}, {half, -}
-    int cnt = 2;
-    if (i < n_internal) {
-    {
-        const float4 *w = reinterpret_cast<const float4 *>(wide + i);
-        const float4 w0 = w[0], w1 = w[1], w2 = w[2], w3 = w[3];
-        c[0] = w0, h[0] = w1;
-        c[1] = make_float4(w2.x, w2.y, w2.z, w1.w), h[1] = w3;
-    }
-#pragma unroll
-    for (int it = 0; it < 2; ++it) {
-        int best = -1;
-        float bestArea = -1.0f;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            if (k < cnt && !(__float_as_uint(c[k].w) & RT_NODE_LEAF_FLAG)) {
-                const float a = h[k].x * h[k].y + h[k].y * h[k].z + h[k].z * h[k].x;
-                if (a > bestArea) bestArea = a, best = k;
-            }
-        }
-        if (best < 0) break;
-        float4 bc = c[0];
-#pragma unroll
-        for (int k = 1; k < 4; ++k)
-            if (k == best) bc = c[k];
-        const float4 *w = reinterpret_cast<const float4 *>(wide + __float_as_uint(bc.w));
-        const float4 w0 = w[0], w1 = w[1], w2 = w[2], w3 = w[3];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            if (k == best) c[k] = w0, h[k] = w1;
-            if (k == cnt) c[k] = make_float4(w2.x, w2.y, w2.z, w1.w), h[k] = w3;
-        }
-        cnt++;
-    }
-    float4 *o = s_out + threadIdx.x * 8;
-    const int sw = threadIdx.x & 7;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        if (k < cnt) {
-            o[(2 * k) ^ sw] = c[k];
-            o[(2 * k + 1) ^ sw] = make_float4(h[k].x, h[k].y, h[k].z, 0.0f);
-        } else {
-            o[(2 * k) ^ sw] = make_float4(0.0f, 0.0f, 0.0f, __uint_as_float(RT_WIDE4_EMPTY));
-            o[(2 * k + 1) ^ sw] = make_float4(-1.0f, -1.0f, -1.0f, 0.0f);
-        }
-    }
-    }
-    __syncthreads();
-    const uint32_t b0 = blockIdx.x * blockDim.x;
-    const uint32_t valid = 8 * min(uint32_t(kThreads), n_internal - b0);
-    float4 *dst = reinterpret_cast<float4 *>(wide4 + b0);
-    for (uint32_t g = threadIdx.x; g < valid; g += kThreads) {
-        const uint32_t t = g >> 3, e = g & 7;
-        dst[g] = s_out[t * 8 + (e ^ (t & 7))];
     }
 }
 
@@ -1790,7 +1611,7 @@ static int build_common(rt_context *ctx, uint32_t n, bool top, uint32_t flags, u
         }
     }
     if (!fused) RT_CUDA(cudaMemsetAsync(counters, 0, 4ull * n, st));
-    bool fitted_locally = false;
+    rt_wide4_node *wide4 = reinterpret_cast<rt_wide4_node *>(result + R.wide4);
     if (fused) {
         RT_CUDA(cudaFuncSetAttribute(k_lbvh_fit, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kFitLocalDynSmem)));  // per device
         // exit list {node, lo, hi} in buffers this path leaves unused (the sort's ping-pong pair, the arrival counters);
@@ -1799,14 +1620,12 @@ static int build_common(rt_context *ctx, uint32_t n, bool top, uint32_t flags, u
         uint32_t *exit_nodes = reinterpret_cast<uint32_t *>(scratch + L.valsB), *exit_lo = reinterpret_cast<uint32_t *>(scratch + L.keysB);
         const uint32_t *codes_sorted = reinterpret_cast<uint32_t *>(scratch + L.keysC);
         unsigned long long *g_slot = reinterpret_cast<unsigned long long *>(hier);
-        rt_wide4_node *wide4 = reinterpret_cast<rt_wide4_node *>(result + R.wide4);
         k_lbvh_fit<<<rt_div_up(n, kFitBlock), kFitBlock, kFitLocalDynSmem, st>>>(n, codes_sorted, nodes, packed, wide, wide4, ext,
                                                                                  exit_count, exit_nodes, exit_lo, counters);
         if (n > kFitBlock) {  // a build of one block leaves no exits
             k_lbvh_exits<<<std::max(1, rt_div_up(n / 8, kThreads)), kThreads, 0, st>>>(n, codes_sorted, g_slot, nodes, wide, wide4, ext, exit_count, exit_nodes, exit_lo, counters);
             ctx->launches++;
         }
-        fitted_locally = true;
     } else if (top) {
         if (update)
             k_fit<true, true><<<grid, kThreads, 0, st>>>(n, hier, counters, nodes, nullptr, boxes, perm, wide, ext, parents);
@@ -1822,21 +1641,19 @@ static int build_common(rt_context *ctx, uint32_t n, bool top, uint32_t flags, u
             uint32_t *exit_nodes = reinterpret_cast<uint32_t *>(scratch + L.valsB);
             uint16_t *exit_sizes = reinterpret_cast<uint16_t *>(scratch + L.keysB + align_up(n, 256));
             RT_CUDA(cudaFuncSetAttribute(k_fit_local, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kFitLocalDynSmem)));  // per device
-            k_fit_local<<<rt_div_up(n, kFitBlock), kFitBlock, kFitLocalDynSmem, st>>>(n, hier, counters, nodes, packed, wide,
-                                                                                      reinterpret_cast<rt_wide4_node *>(result + R.wide4), ext,
+            k_fit_local<<<rt_div_up(n, kFitBlock), kFitBlock, kFitLocalDynSmem, st>>>(n, hier, counters, nodes, packed, wide, wide4, ext,
                                                                                       fit_local, exit_nodes, exit_sizes);
-            fitted_locally = true;
             if (n > 1) {
                 // every block leaves at least one and on average ~log2(kFitBlock) entries; n bounds it
-                k_fit_exits<<<std::max(1, rt_div_up(n / 4, kThreads)), kThreads, 0, st>>>(n, hier, counters, nodes, wide, reinterpret_cast<rt_wide4_node *>(result + R.wide4), ext,
-                                                       exit_nodes, exit_sizes);
+                k_fit_exits<<<std::max(1, rt_div_up(n / 4, kThreads)), kThreads, 0, st>>>(n, hier, counters, nodes, wide, wide4, ext,
+                                                                                            exit_nodes, exit_sizes);
                 ctx->launches++;
             }
         }
     }
     ctx->launches++;
-    if (n > 1 && !fitted_locally) {  // k_fit_local / k_fit_exits write the 4-wide nodes themselves
-        k_collapse4<<<rt_div_up(n - 1, kThreads), kThreads, 0, st>>>(wide, n - 1, reinterpret_cast<rt_wide4_node *>(result + R.wide4));
+    if (n > 1 && (top || update)) {  // k_fit leaves the 4-wide nodes to k_collapse4
+        k_collapse4<<<rt_div_up(n - 1, kThreads), kThreads, 0, st>>>(wide, n - 1, wide4);
         ctx->launches++;
     }
     RT_LAUNCH_CHECK();

@@ -484,11 +484,15 @@ class Accel:
         nbytes = int(lib.rt_blob_bytes(self.n, 1 if self.top else 0))
         return self.result.download(np.uint8, nbytes)
 
+    def ext_header(self) -> np.ndarray:
+        """The 128-byte rt_ext_header behind the blob (csrc/common.cuh) as 32 little-endian 32-bit words."""
+        ext = (int(lib.rt_blob_bytes(self.n, 1 if self.top else 0)) + 63) // 64 * 64
+        return self.result.download(np.uint32, 32, offset=ext)
+
     def traversal_section(self) -> dict:
         """The arrays the trace kernels read — BVH2 wide nodes (64 B), packed leaves (48 B triangles / 96 B instances),
-        4-wide nodes (128 B) — located through the 128-byte rt_ext_header behind the blob (csrc/common.cuh)."""
-        ext = (int(lib.rt_blob_bytes(self.n, 1 if self.top else 0)) + 63) // 64 * 64
-        hdr = self.result.download(np.uint64, 16, offset=ext)
+        4-wide nodes (128 B) — located through the rt_ext_header behind the blob."""
+        hdr = self.ext_header().view(np.uint64)
         off_wide, off_leaf, off_wide4 = int(hdr[2]), int(hdr[3]), int(hdr[8])
         n_int = max(self.n - 1, 0)
         return {"wide": self.result.download(np.uint32, 16 * n_int, offset=off_wide).reshape(-1, 16),
