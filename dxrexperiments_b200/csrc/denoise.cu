@@ -17,6 +17,7 @@
 // Out-of-image texels read as 0 for both the input and the joint image (D3D out-of-bounds load).
 #include <cuda_fp16.h>
 
+#include <initializer_list>
 #include <type_traits>
 
 #include "common.cuh"
@@ -80,6 +81,10 @@ __device__ __forceinline__ f32x2 fma2(f32x2 a, f32x2 b, f32x2 c) {
     asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
     return r;
 }
+
+// Rec. 601 luma: reinhardToneMap's luminance (DenoiseCommon.hlsli:33-38) and the edge-stopping luminance of
+// rt_denoise_progressive.
+__device__ __forceinline__ float luminance(float r, float g, float b) { return (r * 0.299f + g * 0.587f) + b * 0.114f; }
 
 // PASS 0 = horizontal (DenoiseCompositorH.hlsl), PASS 1 = vertical + composite (DenoiseCompositorV.hlsl).
 template <int PASS>
@@ -235,7 +240,7 @@ __global__ void __launch_bounds__(kThreadsDn, 3) k_denoise(const __grid_constant
         else if (A.prm.debugVisualize == 3) cr = cjx[r], cg = cjy[r], cb = cjz[r];
         cr *= A.prm.exposure, cg *= A.prm.exposure, cb *= A.prm.exposure;
         if (A.prm.tonemap) {  // reinhardToneMap :33-38
-            const float lum = (cr * 0.299f + cg * 0.587f) + cb * 0.114f;
+            const float lum = luminance(cr, cg, cb);
             const float reinhard = lum / (lum + 1);
             const float s = reinhard / lum;
             cr = fmaxf(cr * s, 0.0f), cg = fmaxf(cg * s, 0.0f), cb = fmaxf(cb * s, 0.0f);
@@ -249,7 +254,183 @@ __global__ void __launch_bounds__(kThreadsDn, 3) k_denoise(const __grid_constant
     }
 }
 
+// ---- rt_denoise_progressive (include/rt_core.h states the filter): one thread per pixel, taps read through L1.  Every
+// tap's weight and sum are formed in the order the header and tests/progressive_denoise_reference.py give.
+constexpr int PD_TX = 32, PD_TY = 8;
+
+struct ProgDenoiseArgs {
+    const float4 *beauty, *albedo, *normal;
+    const float4 *src;  // (C, var) of the previous step (iterations)
+    float4 *dst;        // (C, var), or (C, 1) rounded as a render target when `last`
+    int w, h, step, last, half, nexp;
+    float sigma_l, inv_a;
+};
+
+__device__ __forceinline__ float normal_weight(float4 np, float4 nq, int nexp) {
+    float d = fmaxf(0.0f, (np.x * nq.x + np.y * nq.y) + np.z * nq.z);
+    for (int i = 0; i < nexp; ++i) d = d * d;
+    return d;
+}
+
+__device__ __forceinline__ void pd_store(const ProgDenoiseArgs &A, size_t i, float r, float g, float b, float var) {
+    if (!A.last) {
+        A.dst[i] = make_float4(r, g, b, var);
+        return;
+    }
+    if (A.half) r = __half2float(__float2half_rn(r)), g = __half2float(__float2half_rn(g)), b = __half2float(__float2half_rn(b));
+    A.dst[i] = make_float4(r, g, b, 1.0f);
+}
+
+// (C, var0): var0 = max(0, m2 - m1^2) of L over the wN-weighted 7 x 7 window
+__global__ void __launch_bounds__(PD_TX * PD_TY) k_pd_variance(const __grid_constant__ ProgDenoiseArgs A) {
+    const int x = blockIdx.x * PD_TX + threadIdx.x, y = blockIdx.y * PD_TY + threadIdx.y;
+    if (x >= A.w || y >= A.h) return;
+    const size_t i = size_t(y) * A.w + x;
+    const float4 c = __ldg(A.beauty + i), np = __ldg(A.normal + i);
+    float var = 0.0f;
+    if (np.w != 0.0f) {
+        float sw = 0.0f, s1 = 0.0f, s2 = 0.0f;
+        for (int dy = -3; dy <= 3; ++dy) {
+            const int qy = y + dy;
+            if (qy < 0 || qy >= A.h) continue;
+#pragma unroll
+            for (int dx = -3; dx <= 3; ++dx) {
+                const int qx = x + dx;
+                if (qx < 0 || qx >= A.w) continue;
+                const size_t j = size_t(qy) * A.w + qx;
+                float wn = 1.0f;
+                float4 cq = c;
+                if (dx != 0 || dy != 0) {
+                    wn = normal_weight(np, __ldg(A.normal + j), A.nexp);
+                    if (wn == 0.0f) continue;
+                    cq = __ldg(A.beauty + j);
+                }
+                const float l = luminance(cq.x, cq.y, cq.z);
+                s1 = s1 + wn * l, s2 = s2 + wn * (l * l), sw = sw + wn;
+            }
+        }
+        const float m1 = s1 / sw, m2 = s2 / sw;
+        var = fmaxf(0.0f, m2 - m1 * m1);
+    }
+    pd_store(A, i, c.x, c.y, c.z, var);
+}
+
+// one a-trous iteration at step A.step: (C, var) from A.src -> A.dst
+__global__ void __launch_bounds__(PD_TX * PD_TY) k_pd_atrous(const __grid_constant__ ProgDenoiseArgs A) {
+    const int x = blockIdx.x * PD_TX + threadIdx.x, y = blockIdx.y * PD_TY + threadIdx.y;
+    if (x >= A.w || y >= A.h) return;
+    const size_t i = size_t(y) * A.w + x;
+    const float4 cp = __ldg(A.src + i), np = __ldg(A.normal + i);
+    if (np.w == 0.0f) {  // sky: copied
+        pd_store(A, i, cp.x, cp.y, cp.z, cp.w);
+        return;
+    }
+    const float kH[3] = {0.25f, 0.5f, 0.25f};
+    const float kB[5] = {0.0625f, 0.25f, 0.375f, 0.25f, 0.0625f};
+    // g(p): the 3 x 3 wN-weighted prefilter of var
+    float gs = 0.0f, gw = 0.0f;
+#pragma unroll
+    for (int dy = -1; dy <= 1; ++dy) {
+        const int qy = y + dy;
+        if (qy < 0 || qy >= A.h) continue;
+#pragma unroll
+        for (int dx = -1; dx <= 1; ++dx) {
+            const int qx = x + dx;
+            if (qx < 0 || qx >= A.w) continue;
+            const size_t j = size_t(qy) * A.w + qx;
+            float wn = 1.0f, v = cp.w;
+            if (dx != 0 || dy != 0) {
+                wn = normal_weight(np, __ldg(A.normal + j), A.nexp);
+                if (wn == 0.0f) continue;
+                v = __ldg(A.src + j).w;
+            }
+            const float wg = (kH[dx + 1] * kH[dy + 1]) * wn;
+            if (wg == 0.0f) continue;
+            gs = gs + wg * v, gw = gw + wg;
+        }
+    }
+    const float g = gs / gw;
+    const float inv_l = 1.0f / (A.sigma_l * sqrtf(g) + 1e-10f);
+    const float lp = luminance(cp.x, cp.y, cp.z);
+    const float4 ap = __ldg(A.albedo + i);
+    float sr = 0.0f, sg = 0.0f, sb = 0.0f, sv = 0.0f, sw = 0.0f;
+#pragma unroll
+    for (int dy = -2; dy <= 2; ++dy) {
+        const int qy = y + A.step * dy;
+        if (qy < 0 || qy >= A.h) continue;
+#pragma unroll
+        for (int dx = -2; dx <= 2; ++dx) {
+            const int qx = x + A.step * dx;
+            if (qx < 0 || qx >= A.w) continue;
+            const size_t j = size_t(qy) * A.w + qx;
+            float w = kB[2] * kB[2];
+            float4 cq = cp;
+            if (dx != 0 || dy != 0) {
+                const float wn = normal_weight(np, __ldg(A.normal + j), A.nexp);
+                if (wn == 0.0f) continue;
+                cq = __ldg(A.src + j);
+                const float4 aq = __ldg(A.albedo + j);
+                const float dl = fabsf(lp - luminance(cq.x, cq.y, cq.z));
+                const float da = (fabsf(ap.x - aq.x) + fabsf(ap.y - aq.y)) + fabsf(ap.z - aq.z);
+                w = ((kB[dx + 2] * kB[dy + 2]) * wn) * expf(-(dl * inv_l + da * A.inv_a));
+                if (w == 0.0f) continue;
+            }
+            sr = sr + w * cq.x, sg = sg + w * cq.y, sb = sb + w * cq.z;
+            sv = sv + (w * w) * cq.w, sw = sw + w;
+        }
+    }
+    pd_store(A, i, sr / sw, sg / sw, sb / sw, sv / (sw * sw));
+}
+
 }  // namespace
+
+extern "C" int rt_denoise_progressive(rt_context *ctx, const float *beauty, const float *albedo, const float *normal, float *tmp,
+                                      float *out, uint32_t width, uint32_t height, const rt_progressive_denoise_params *prm) {
+    RT_REQUIRE(ctx && beauty && albedo && normal && tmp && out && prm, "null argument");
+    RT_REQUIRE(((uintptr_t(beauty) | uintptr_t(albedo) | uintptr_t(normal) | uintptr_t(tmp) | uintptr_t(out)) & 15) == 0,
+               "images must be 16-byte aligned");
+    RT_REQUIRE(width > 0 && height > 0, "empty image");
+    RT_REQUIRE(width <= 0x7FFFFFFFu && height <= 65535u * PD_TY, "image too large for one launch");
+    RT_REQUIRE(prm->iterations <= 5 && prm->normal_exponent_log2 <= 8, "iterations 0..5, normal_exponent_log2 0..8");
+    RT_REQUIRE(prm->sigma_luminance > 0.0f && prm->sigma_luminance <= 3.4e38f, "sigma_luminance must be finite and > 0");
+    RT_REQUIRE(prm->sigma_albedo >= 0.0f && prm->sigma_albedo <= 3.4e38f, "sigma_albedo must be finite and >= 0");
+    // byte ranges [p, p + n): out and tmp are written, so neither may share a byte with any other argument
+    const uint64_t img = uint64_t(width) * height * 16;
+    auto overlap = [](const void *a, uint64_t na, const void *b, uint64_t nb) {
+        return uintptr_t(a) < uintptr_t(b) + nb && uintptr_t(b) < uintptr_t(a) + na;
+    };
+    for (const float *in : {beauty, albedo, normal}) {
+        RT_REQUIRE(!overlap(out, img, in, img), "out overlaps an input");
+        RT_REQUIRE(!overlap(tmp, 2 * img, in, img), "tmp overlaps an input");
+    }
+    RT_REQUIRE(!overlap(out, img, tmp, 2 * img), "out overlaps tmp");
+    RT_CUDA(cudaSetDevice(ctx->device));
+    ProgDenoiseArgs A{};
+    A.beauty = reinterpret_cast<const float4 *>(beauty);
+    A.albedo = reinterpret_cast<const float4 *>(albedo);
+    A.normal = reinterpret_cast<const float4 *>(normal);
+    A.w = int(width), A.h = int(height);
+    A.half = int(ctx->render_options.half_render_targets);
+    A.nexp = int(prm->normal_exponent_log2);
+    A.sigma_l = prm->sigma_luminance;
+    A.inv_a = prm->sigma_albedo > 0.0f ? 1.0f / prm->sigma_albedo : 0.0f;
+    const int n = int(prm->iterations);
+    const dim3 grid(rt_div_up(width, PD_TX), rt_div_up(height, PD_TY)), block(PD_TX, PD_TY);
+    float4 *ping[2] = {reinterpret_cast<float4 *>(tmp), reinterpret_cast<float4 *>(tmp) + size_t(width) * height};
+    A.dst = n == 0 ? reinterpret_cast<float4 *>(out) : ping[0];
+    A.last = n == 0;
+    k_pd_variance<<<grid, block, 0, ctx->stream>>>(A);
+    for (int it = 0; it < n; ++it) {
+        A.src = ping[it & 1];
+        A.step = 1 << it;
+        A.last = it == n - 1;
+        A.dst = A.last ? reinterpret_cast<float4 *>(out) : ping[(it + 1) & 1];
+        k_pd_atrous<<<grid, block, 0, ctx->stream>>>(A);
+    }
+    ctx->launches += 1 + n;
+    RT_LAUNCH_CHECK();
+    return RT_OK;
+}
 
 extern "C" int rt_denoise(rt_context *ctx, const float *direct, const float *indirect_specular, float *tmp, float *out, uint32_t width,
                           uint32_t height, const rt_denoiser_params *prm) {

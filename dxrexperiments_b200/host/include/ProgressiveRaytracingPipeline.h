@@ -69,6 +69,7 @@ protected:
     std::array<bool, RT_AOV_COUNT> mAovEnabled{};
     std::array<DXRFramework::RtBuffer::SharedPtr, RT_AOV_COUNT> mAovResource;
     UINT mNumOutputs;
+    UINT mOutputWidth = 0, mOutputHeight = 0;  // of the last createOutputResource
     PerFrameConstants mConstantBuffer{};
     DXRFramework::RtTexture::SharedPtr mEnvCube;
     bool mActive = true;
@@ -91,10 +92,16 @@ public:
     bool mFrameAccumulationEnabled = true;
     UINT getAccumCount() const { return mAccumCount; }
     void restartAccumulation() { mHasLastCamera = false; }  // what a UI change does (mLastCameraVPMatrix = Matrix4())
+    // The beauty output filtered by rt_denoise_progressive, with the albedo and normal AOVs as guides (both must be enabled
+    // with enableAov).  Stream-ordered after the last render(); the filter's scratch and the returned output are allocated on
+    // first use and reused by later calls, so the result is valid until the next denoise().
+    DXRFramework::RtBuffer::SharedPtr denoise(const rt_progressive_denoise_params &params);
 
 private:
     explicit ProgressiveRaytracingPipeline(DXRFramework::RtContext::SharedPtr context);
     UINT mAccumCount = 0;
     float mLastCameraVP[16] = {};
     bool mHasLastCamera = false;
+    DXRFramework::RtBuffer::SharedPtr mDenoiseTmp, mDenoiseOut;
+    uint64_t mDenoiseBytes = 0;
 };

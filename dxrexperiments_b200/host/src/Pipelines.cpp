@@ -86,6 +86,7 @@ bool RaytracingPipelineBase::loadEnvironmentDDS(const std::string &path) {
 
 void RaytracingPipelineBase::createOutputResource(DXGI_FORMAT /*format*/, UINT width, UINT height) {
     mOutputResource.clear();
+    mOutputWidth = width, mOutputHeight = height;
     for (UINT i = 0; i < mNumOutputs; ++i) {
         auto b = mRtContext->createBuffer(uint64_t(width) * height * 16);
         b->clear();
@@ -192,6 +193,23 @@ void ProgressiveRaytracingPipeline::update(float elapsedTime, UINT elapsedFrames
     fillCommonConstants(elapsedTime, elapsedFrames, width, height);
     mConstantBuffer.cameraParams.accumCount = mAccumCount++;
     mConstantBuffer.options = mShaderDebugOptions;
+}
+
+RtBuffer::SharedPtr ProgressiveRaytracingPipeline::denoise(const rt_progressive_denoise_params &params) {
+    const auto albedo = mAovResource[RT_AOV_ALBEDO], normal = mAovResource[RT_AOV_NORMAL];
+    ThrowIfFalse(albedo && normal, "ProgressiveRaytracingPipeline::denoise needs the albedo and normal AOVs enabled");
+    const uint64_t bytes = uint64_t(mOutputWidth) * mOutputHeight * 16;
+    if (!mDenoiseOut || mDenoiseBytes != bytes) {
+        mDenoiseTmp = mRtContext->createBuffer(2 * bytes);
+        mDenoiseOut = mRtContext->createBuffer(bytes);
+        mDenoiseBytes = bytes;
+    }
+    ThrowIfFailed(rt_denoise_progressive(mRtContext->getNative(), static_cast<const float *>(mOutputResource.at(0)->ptr()),
+                                         static_cast<const float *>(albedo->ptr()), static_cast<const float *>(normal->ptr()),
+                                         static_cast<float *>(mDenoiseTmp->ptr()), static_cast<float *>(mDenoiseOut->ptr()), mOutputWidth,
+                                         mOutputHeight, &params),
+                  "rt_denoise_progressive");
+    return mDenoiseOut;
 }
 
 // ------------------------------------------------------------------------------------------------ realtime

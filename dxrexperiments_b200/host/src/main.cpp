@@ -7,6 +7,8 @@
 //   dxr_headless ... --exr frame.exr [--exr-half]        OpenEXR output (fp32, or HALF = the reference's R16G16B16A16_FLOAT)
 //   dxr_headless --pipeline progressive ... --aov albedo albedo.pfm --aov normal normal.exr   AOV outputs, accumulated from the
 //     same rays as --out (direct, indirect-diffuse, indirect-specular, albedo, fresnel, normal; EXR when the path ends in .exr)
+//   dxr_headless --pipeline progressive ... --denoise-progressive clean.pfm   the beauty output filtered with the albedo and
+//     normal AOVs as guides (rt_denoise_progressive; the flag enables both AOVs; EXR when the path ends in .exr)
 // Multi-GPU (one process per GPU, replicated scene; the frame's samples and strips are sharded, one NCCL reduce at the end):
 //   for r in 0 1; do dxr_headless ... --spp 64 --world 2 --rank $r --comm-file /tmp/id [--strip-groups 2] --out frame.pfm & done
 #include <chrono>
@@ -74,6 +76,7 @@ static int usage() {
               "             [--out file.pfm] [--out2 file.pfm] [--denoise file.pfm] [--exr file.exr [--exr-half]] [--dump-frames file.bin] [--device N]\n"
               "             [--radiance-depth 1|2] [--fp16-targets] [--denoise-mock direct.pfm specular.pfm --denoise out.pfm [--kernel-size K]]\n"
               "             [--aov direct|indirect-diffuse|indirect-specular|albedo|fresnel|normal file.pfm|file.exr]...   (progressive only)\n"
+              "             [--denoise-progressive file.pfm|file.exr]   (progressive only: the beauty output filtered with the albedo and normal AOVs)\n"
               "             [--world N --rank R --comm-file path [--strip-groups G] [--strip-rows 32] [--band-shard]]   (one process per GPU)");
     return 0;
 }
@@ -94,6 +97,9 @@ int main(int argc, char **argv) {
     const int world = int(a.num("world", 1)), rank = int(a.num("rank", 0));
     try {
         if (world < 1 || rank < 0 || rank >= world) throw std::runtime_error("--world / --rank");
+        const bool denoiseProgressive = a.has("denoise-progressive");
+        if (denoiseProgressive && (pipelineName == "realtime" || a.str("denoise-progressive", "").empty()))
+            throw std::runtime_error("--denoise-progressive takes a path and needs --pipeline progressive (--denoise filters the realtime pipeline)");
         auto context = RtContext::create(int(a.num("device", rank)));
         if (a.has("denoise-mock")) {
             // DenoiseCompositor with mock inputs (src/DenoiseCompositor.cpp:52-60 loads DirectLighting.png / IndirectSpecular.png and
@@ -196,6 +202,7 @@ int main(int argc, char **argv) {
                 aovFiles.emplace_back(id, v[i + 1]);
             }
         }
+        if (denoiseProgressive) pipeline->enableAov(RT_AOV_ALBEDO), pipeline->enableAov(RT_AOV_NORMAL);
         pipeline->loadResources(3);
         pipeline->createOutputResource(DXGI_FORMAT_R16G16B16A16_FLOAT, width, height);
         pipeline->setRenderOptions(UINT(a.num("radiance-depth", 1)), a.has("fp16-targets"));
@@ -237,9 +244,6 @@ int main(int argc, char **argv) {
         // ---- the path's one collective: every output is summed onto rank 0, weighted by the rank's share of the samples
         std::vector<RtBuffer::SharedPtr> finalOut;
         for (int i = 0; i < pipeline->getNumOutputs(); ++i) finalOut.push_back(pipeline->getOutputResource(i));
-        // the AOVs are running means like the beauty output, so they reduce with the same weights
-        const size_t numBeauty = finalOut.size();
-        for (const auto &f : aovFiles) finalOut.push_back(pipeline->getAovResource(rt_aov(f.first)));
         std::shared_ptr<DenoiseCompositor> bandDenoiser;
         RtBuffer::SharedPtr bandFrame;
         if (bandShard) {
@@ -251,12 +255,13 @@ int main(int argc, char **argv) {
             bandFrame = rank == 0 ? context->createBuffer(floats * 4) : nullptr;
             context->reduceAccumulation(bandDenoiser->getOutputResource(), bandFrame, floats, 1.0f, 0);
         } else if (world > 1) {
+            // in place: on the root the pipeline's own buffers then hold the frame, which is what denoise() filters.  The
+            // enabled AOVs are running means like the beauty output, so they reduce with the same weights.
             const uint64_t floats = uint64_t(width) * height * 4;
-            for (size_t i = 0; i < finalOut.size(); ++i) {
-                RtBuffer::SharedPtr recv = rank == 0 ? context->createBuffer(floats * 4) : nullptr;
-                context->reduceAccumulation(finalOut[i], recv, floats, float(mySamples) / float(spp), 0);
-                if (rank == 0) finalOut[i] = recv;
-            }
+            std::vector<RtBuffer::SharedPtr> reduced = finalOut;
+            for (int k = 0; k < RT_AOV_COUNT; ++k)
+                if (auto b = pipeline->getAovResource(rt_aov(k))) reduced.push_back(b);
+            for (const auto &b : reduced) context->reduceAccumulation(b, rank == 0 ? b : nullptr, floats, float(mySamples) / float(spp), 0);
         }
         context->waitForGpu();
         context->checkDeviceStatus();
@@ -272,8 +277,14 @@ int main(int argc, char **argv) {
         };
         if (a.has("out")) save(finalOut[0], a.str("out", ""));
         if (a.has("exr")) save(finalOut[0], a.str("exr", ""));
-        if (a.has("out2") && numBeauty > 1) save(finalOut[1], a.str("out2", ""));
-        for (size_t i = 0; i < aovFiles.size(); ++i) save(finalOut[numBeauty + i], aovFiles[i].second);
+        if (a.has("out2") && finalOut.size() > 1) save(finalOut[1], a.str("out2", ""));
+        for (const auto &f : aovFiles) save(pipeline->getAovResource(rt_aov(f.first)), f.second);
+        if (denoiseProgressive && rank == 0) {
+            const rt_progressive_denoise_params params = RT_PROGRESSIVE_DENOISE_DEFAULTS;
+            auto clean = std::static_pointer_cast<ProgressiveRaytracingPipeline>(pipeline)->denoise(params);
+            context->waitForGpu();
+            save(clean, a.str("denoise-progressive", ""));
+        }
         if (bandShard) {
             save(bandFrame, a.str("denoise", ""));
         } else if (a.has("denoise") && rank == 0) {

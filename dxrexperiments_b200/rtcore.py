@@ -87,6 +87,7 @@ def _load():
         "rt_enable_stage_timing": (i32, [vp, i32]),
         "rt_get_stage_timing": (i32, [vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double), i32]),
         "rt_denoise": (i32, [vp, vp, vp, vp, vp, u32, u32, vp]),
+        "rt_denoise_progressive": (i32, [vp, vp, vp, vp, vp, vp, u32, u32, vp]),
         "rt_trace_rays": (i32, [vp, vp, vp, u64, u32, u32, vp]),
         "rt_trace_rays_stats": (i32, [vp, vp, vp, u64, u32, u32, vp, vp]),
         "rt_trace_rays_hit_groups": (i32, [vp, vp, vp, u64, u32, u32, u32, u32, vp, u32, vp]),
@@ -352,6 +353,17 @@ class Context:
         out = d_out.download(np.float32).reshape(h, w, 4)
         tmp = d_tmp.download(np.float32).reshape(h, w, 4)
         return out, tmp
+
+    def denoise_progressive(self, beauty: np.ndarray, albedo: np.ndarray, normal: np.ndarray,
+                            params: T.ProgressiveDenoiseParams = None) -> np.ndarray:
+        """rt_denoise_progressive on host images: (h, w, 4) float32 beauty, albedo and normal AOVs -> (h, w, 4) float32."""
+        h, w = beauty.shape[:2]
+        d_in = [self.upload(np.ascontiguousarray(a, np.float32).reshape(-1)) for a in (beauty, albedo, normal)]
+        d_tmp = self.alloc(32 * w * h)
+        d_out = self.alloc(16 * w * h)
+        params = T.progressive_denoise_defaults() if params is None else params
+        check(lib.rt_denoise_progressive(self.handle, *(d.ptr for d in d_in), d_tmp.ptr, d_out.ptr, w, h, C.byref(params)))
+        return d_out.download(np.float32).reshape(h, w, 4)
 
     def ray_counts(self, reset=False) -> T.RayCounts:
         c = T.RayCounts()
@@ -640,6 +652,7 @@ class Renderer:
         if unknown:
             raise ValueError(f"unknown AOV names {unknown}; known: {T.AOV_NAMES}")
         self.aovs = {a: ctx.alloc(16 * width * height).zero() for a in aovs}
+        self._denoise_bufs = None  # (tmp, out) of denoise(), allocated on first use
 
     def dispatch(self, frame: T.PerFrameConstants, region=None, strips=None):
         """region: (x0, y0, x1, y1) pixel rectangle; strips: (strip_rows, groups, group) strip-interleaved shard."""
@@ -679,3 +692,16 @@ class Renderer:
     def aov(self, name: str) -> np.ndarray:
         """The accumulated AOV `name` (one of the names passed as aovs=) as (height, width, 4) float32."""
         return self.aovs[name].download(np.float32).reshape(self.height, self.width, 4)
+
+    def denoise(self, params: T.ProgressiveDenoiseParams = None) -> np.ndarray:
+        """The beauty output filtered by rt_denoise_progressive with the albedo and normal AOVs as guides, as (height, width,
+        4) float32.  Filters the device buffers in place of a host round trip; needs aovs= to include "albedo" and "normal"."""
+        if self.kind != PROGRESSIVE or "albedo" not in self.aovs or "normal" not in self.aovs:
+            raise ValueError('denoise() needs a progressive Renderer with the "albedo" and "normal" AOVs')
+        if self._denoise_bufs is None:
+            self._denoise_bufs = (self.ctx.alloc(32 * self.width * self.height), self.ctx.alloc(16 * self.width * self.height))
+        tmp, out = self._denoise_bufs
+        params = T.progressive_denoise_defaults() if params is None else params
+        check(lib.rt_denoise_progressive(self.ctx.handle, self.out[0].ptr, self.aovs["albedo"].ptr, self.aovs["normal"].ptr, tmp.ptr,
+                                         out.ptr, self.width, self.height, C.byref(params)))
+        return out.download(np.float32).reshape(self.height, self.width, 4)

@@ -47,6 +47,17 @@ class DenoiserParams(C.Structure):  # include/DenoiseCompositor.h:41-49
                 ("gammaCorrect", C.c_uint32), ("maxKernelSize", C.c_int32), ("debugVisualize", C.c_uint32)]
 
 
+class ProgressiveDenoiseParams(C.Structure):  # rt_progressive_denoise_params (include/rt_types.h)
+    _fields_ = [("iterations", C.c_uint32), ("normal_exponent_log2", C.c_uint32), ("sigma_luminance", C.c_float),
+                ("sigma_albedo", C.c_float)]
+
+
+def progressive_denoise_defaults() -> ProgressiveDenoiseParams:
+    """RT_PROGRESSIVE_DENOISE_DEFAULTS (include/rt_types.h): the parameters rt_denoise_progressive is used with unless told
+    otherwise (DESIGN.md 4.4 records how they were chosen)."""
+    return ProgressiveDenoiseParams(5, 7, 4.0, 0.1)
+
+
 class GeometryDesc(C.Structure):
     _fields_ = [("vertex_buffer", C.c_void_p), ("vertex_count", C.c_uint32), ("vertex_stride_bytes", C.c_uint32),
                 ("index_buffer", C.c_void_p), ("index_count", C.c_uint32), ("index_format", C.c_uint32),
@@ -87,6 +98,7 @@ class AsInfo(C.Structure):  # rt_as_info
 assert C.sizeof(PerFrameConstants) == 188
 assert C.sizeof(MaterialParams) == 64
 assert C.sizeof(DenoiserParams) == 24
+assert C.sizeof(ProgressiveDenoiseParams) == 16
 assert C.sizeof(InstanceDesc) == 64
 assert C.sizeof(HitRecord) == 80
 assert C.sizeof(GeometryDesc) == 48

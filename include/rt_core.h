@@ -280,6 +280,28 @@ int rt_debug_download(rt_context *ctx, int array, uint32_t plane, void *host, ui
  * indirect specular -> tmp) then pass V (-> out, + direct, exposure, Reinhard, gamma).  RGBA fp32, tightly packed. */
 int rt_denoise(rt_context *ctx, const float *direct, const float *indirect_specular, float *tmp, float *out,
                uint32_t width, uint32_t height, const rt_denoiser_params *params);
+/* Denoiser for the accumulated frame of the progressive program (new work: the reference has no counterpart; its nearest
+ * relative is DenoiseCompositor::dispatch, which filters indirect specular only).  Spatial SVGF without its temporal part
+ * (Schied et al. 2017): an edge-avoiding a-trous wavelet filter (Dammertz et al. 2010) guided by the AOVs.  Inputs are
+ * RGBA fp32 images, tightly packed, width x height: beauty = gOutput, albedo = RT_AOV_ALBEDO, normal = RT_AOV_NORMAL
+ * (N = .xyz, coverage c = .w).  Per pixel p, with L = (r*0.299f + g*0.587f) + b*0.114f:
+ *   wN(p,q) = max(0, (Np.x*Nq.x + Np.y*Nq.y) + Np.z*Nq.z), squared normal_exponent_log2 times.  For the centre tap q = p
+ *     every edge-stopping factor is 1.  Taps outside the image or with weight 0 contribute nothing.
+ *   A pixel with c == 0 (sky) is copied unchanged; its N = 0 gives wN = 0, so it never contributes to a neighbour.
+ *   var0 = max(0, m2 - m1*m1), m1 / m2 the wN-weighted means of L / L*L over the 7 x 7 window.
+ *   Iteration i = 0 .. iterations-1, step s = 2^i, kernel b = (1/16, 1/4, 3/8, 1/4, 1/16) over the 5 x 5 taps
+ *   q = p + s*(dx, dy), summed dy outer, dx inner:
+ *     g(p) = sum (h(dy)*h(dx))*wN * var / sum (h(dy)*h(dx))*wN over the 3 x 3 neighbours, h = (1/4, 1/2, 1/4);
+ *     w = ((b(dx)*b(dy))*wN) * expf(-(|Lp-Lq|*invL + |dA|_1*invA)), |dA|_1 = (|dr| + |dg|) + |db| of the albedo;
+ *     invL = 1/(sigma_luminance*sqrtf(g(p)) + 1e-10f), invA = 1/sigma_albedo or 0 when sigma_albedo = 0;
+ *     C' = sum w*C / sum w, var' = sum (w*w)*var / (sum w)^2; L is recomputed from C every iteration.
+ *   out = (C, 1) after the last iteration; under half_render_targets the store rounds through fp16 (intermediates fp32).
+ * tmp holds 2 * width * height RGBA fp32 (C, var) ping-pong images.  1 + iterations launches on the context's stream, no
+ * host synchronisation.  RT_ERR_INVALID_ARG: a null pointer, a buffer not 16-byte aligned, an empty image, parameters out
+ * of range, or out / tmp overlapping an input or each other.  The inputs are only read. */
+int rt_denoise_progressive(rt_context *ctx, const float *beauty, const float *albedo, const float *normal,
+                           float *tmp /* 2 * width * height RGBA fp32 */, float *out,
+                           uint32_t width, uint32_t height, const rt_progressive_denoise_params *params);
 
 /* ---- wavefront primitives exposed for parity tests and benchmarks */
 /* Fallback_TraceRay without shader call-outs (FL/TraverseShader.hlsli:21-73): n rays -> n hits. */

@@ -90,6 +90,16 @@ typedef struct rt_denoiser_params {
     uint32_t debugVisualize; /* 0 composite, 1 denoised, 2 input, 3 joint */
 } rt_denoiser_params; /* 24 B */
 
+/* rt_denoise_progressive (rt_core.h); new work, no reference counterpart. */
+typedef struct rt_progressive_denoise_params {
+    uint32_t iterations;           /* 0..5: a-trous steps 1, 2, 4, 8, 16 */
+    uint32_t normal_exponent_log2; /* 0..8: the normal weight is max(0, Np.Nq)^(2^this) */
+    float sigma_luminance;         /* > 0 */
+    float sigma_albedo;            /* >= 0, 0 = no albedo term */
+} rt_progressive_denoise_params; /* 16 B */
+/* Defaults, chosen on the CPU restatement of the filter (DESIGN.md 4.4). */
+#define RT_PROGRESSIVE_DENOISE_DEFAULTS {5u, 7u, 4.0f, 0.1f}
+
 /* Interleaved vertex the hit shaders read: libs/DXRFramework/RtModel.cpp:13-17 (stride 24). */
 typedef struct rt_vertex {
     float position[3];
