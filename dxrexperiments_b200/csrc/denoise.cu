@@ -281,12 +281,9 @@ __device__ __forceinline__ void pd_store(const ProgDenoiseArgs &A, size_t i, flo
     A.dst[i] = make_float4(r, g, b, 1.0f);
 }
 
-// (C, var0): var0 = max(0, m2 - m1^2) of L over the wN-weighted 7 x 7 window
-__global__ void __launch_bounds__(PD_TX * PD_TY) k_pd_variance(const __grid_constant__ ProgDenoiseArgs A) {
-    const int x = blockIdx.x * PD_TX + threadIdx.x, y = blockIdx.y * PD_TY + threadIdx.y;
-    if (x >= A.w || y >= A.h) return;
-    const size_t i = size_t(y) * A.w + x;
-    const float4 c = __ldg(A.beauty + i), np = __ldg(A.normal + i);
+// var0 of pixel (x, y), colour c, normal np: max(0, m2 - m1^2) of L over the wN-weighted 7 x 7 window of the colour image
+// A.beauty, 0 for sky
+__device__ __forceinline__ float window_variance(const ProgDenoiseArgs &A, int x, int y, float4 c, float4 np) {
     float var = 0.0f;
     if (np.w != 0.0f) {
         float sw = 0.0f, s1 = 0.0f, s2 = 0.0f;
@@ -312,7 +309,16 @@ __global__ void __launch_bounds__(PD_TX * PD_TY) k_pd_variance(const __grid_cons
         const float m1 = s1 / sw, m2 = s2 / sw;
         var = fmaxf(0.0f, m2 - m1 * m1);
     }
-    pd_store(A, i, c.x, c.y, c.z, var);
+    return var;
+}
+
+// (C, var0): var0 = max(0, m2 - m1^2) of L over the wN-weighted 7 x 7 window
+__global__ void __launch_bounds__(PD_TX * PD_TY) k_pd_variance(const __grid_constant__ ProgDenoiseArgs A) {
+    const int x = blockIdx.x * PD_TX + threadIdx.x, y = blockIdx.y * PD_TY + threadIdx.y;
+    if (x >= A.w || y >= A.h) return;
+    const size_t i = size_t(y) * A.w + x;
+    const float4 c = __ldg(A.beauty + i), np = __ldg(A.normal + i);
+    pd_store(A, i, c.x, c.y, c.z, window_variance(A, x, y, c, np));
 }
 
 // one a-trous iteration at step A.step: (C, var) from A.src -> A.dst
@@ -382,44 +388,112 @@ __global__ void __launch_bounds__(PD_TX * PD_TY) k_pd_atrous(const __grid_consta
     pd_store(A, i, sr / sw, sg / sw, sb / sw, sv / (sw * sw));
 }
 
-}  // namespace
+// ---- rt_denoise_temporal (include/rt_core.h states the temporal pass): reproject and blend into the history, then the
+// variance of the integrated colour, then the a-trous iterations above.  tests/temporal_denoise_reference.py restates it.
+struct TemporalArgs {
+    const float4 *beauty, *normal, *position;
+    const float4 *prev;  // prev_history (4 planes), nullptr: no history
+    float4 *hist;        // history (4 planes)
+    int w, h;
+    float eye[3], jitter[2], U[3], V[3], W[3];  // the previous frame's camera
+    float alpha_c, alpha_m, normal_cos, pos_tol;
+};
 
-extern "C" int rt_denoise_progressive(rt_context *ctx, const float *beauty, const float *albedo, const float *normal, float *tmp,
-                                      float *out, uint32_t width, uint32_t height, const rt_progressive_denoise_params *prm) {
-    RT_REQUIRE(ctx && beauty && albedo && normal && tmp && out && prm, "null argument");
-    RT_REQUIRE(((uintptr_t(beauty) | uintptr_t(albedo) | uintptr_t(normal) | uintptr_t(tmp) | uintptr_t(out)) & 15) == 0,
-               "images must be 16-byte aligned");
+__device__ __forceinline__ float dot3(float ax, float ay, float az, const float b[3]) { return (ax * b[0] + ay * b[1]) + az * b[2]; }
+
+__global__ void __launch_bounds__(PD_TX * PD_TY) k_td_reproject(const __grid_constant__ TemporalArgs A) {
+    const int x = blockIdx.x * PD_TX + threadIdx.x, y = blockIdx.y * PD_TY + threadIdx.y;
+    if (x >= A.w || y >= A.h) return;
+    const size_t plane = size_t(A.w) * A.h, i = size_t(y) * A.w + x;
+    const float4 c = __ldg(A.beauty + i), np = __ldg(A.normal + i), pp = __ldg(A.position + i);
+    float hr = 0.0f, hg = 0.0f, hb = 0.0f, hn = 0.0f, h1 = 0.0f, h2 = 0.0f;
+    if (A.prev && np.w == 1.0f) {
+        // o' is the progressive primary ray's origin (primary_ray in shade.cuh, jitterScale 30)
+        const float rx = pp.x - (A.eye[0] + A.jitter[0] * 30.0f), ry = pp.y - (A.eye[1] + A.jitter[1] * 30.0f), rz = pp.z - (A.eye[2] + 0.0f);
+        const float zc = dot3(rx, ry, rz, A.W) / dot3(A.W[0], A.W[1], A.W[2], A.W);
+        const float sx = (dot3(rx, ry, rz, A.U) / dot3(A.U[0], A.U[1], A.U[2], A.U)) / zc;
+        const float sy = -((dot3(rx, ry, rz, A.V) / dot3(A.V[0], A.V[1], A.V[2], A.V)) / zc);
+        const float fx = ((sx + 1.0f) * 0.5f) * float(A.w) - 0.5f, fy = ((sy + 1.0f) * 0.5f) * float(A.h) - 0.5f;
+        // outside (-1, w) x (-1, h) every tap is outside the image or has weight 0 (and NaN fails the test)
+        if (zc > 0.0f && fx > -1.0f && fx < float(A.w) && fy > -1.0f && fy < float(A.h)) {
+            const float x0f = floorf(fx), y0f = floorf(fy);
+            const float ax = fx - x0f, ay = fy - y0f;
+            const int x0 = int(x0f), y0 = int(y0f);
+            const float lim = A.pos_tol * sqrtf((rx * rx + ry * ry) + rz * rz);
+            float sw = 0.0f;
+#pragma unroll
+            for (int dy = 0; dy < 2; ++dy) {
+#pragma unroll
+                for (int dx = 0; dx < 2; ++dx) {
+                    const int qx = x0 + dx, qy = y0 + dy;
+                    if (qx < 0 || qy < 0 || qx >= A.w || qy >= A.h) continue;
+                    const float wt = (dx ? ax : 1.0f - ax) * (dy ? ay : 1.0f - ay);
+                    if (wt == 0.0f) continue;
+                    const size_t j = size_t(qy) * A.w + qx;
+                    const float4 nq = __ldg(A.prev + 2 * plane + j);
+                    if (nq.w != 1.0f || (np.x * nq.x + np.y * nq.y) + np.z * nq.z < A.normal_cos) continue;
+                    const float4 pq = __ldg(A.prev + 3 * plane + j);
+                    const float ex = pq.x - pp.x, ey = pq.y - pp.y, ez = pq.z - pp.z;
+                    if (sqrtf((ex * ex + ey * ey) + ez * ez) > lim) continue;
+                    const float4 cq = __ldg(A.prev + j), mq = __ldg(A.prev + plane + j);
+                    hr = hr + wt * cq.x, hg = hg + wt * cq.y, hb = hb + wt * cq.z, hn = hn + wt * cq.w;
+                    h1 = h1 + wt * mq.x, h2 = h2 + wt * mq.y, sw = sw + wt;
+                }
+            }
+            if (sw > 0.0f) hr = hr / sw, hg = hg / sw, hb = hb / sw, hn = hn / sw, h1 = h1 / sw, h2 = h2 / sw;
+        }
+    }
+    const float n = fminf(hn + 1.0f, 32.0f);
+    const float a = fmaxf(1.0f / n, A.alpha_c), am = fmaxf(1.0f / n, A.alpha_m);
+    const float l = luminance(c.x, c.y, c.z);
+    A.hist[i] = make_float4((1.0f - a) * hr + a * c.x, (1.0f - a) * hg + a * c.y, (1.0f - a) * hb + a * c.z, n);
+    A.hist[plane + i] = make_float4((1.0f - am) * h1 + am * l, (1.0f - am) * h2 + am * (l * l), 0.0f, 0.0f);
+    A.hist[2 * plane + i] = np;
+    A.hist[3 * plane + i] = pp;
+}
+
+// (C, var0) of the integrated colour: A.beauty = history plane 0 (C, n), A.src = history plane 1 (m1, m2)
+__global__ void __launch_bounds__(PD_TX * PD_TY) k_td_variance(const __grid_constant__ ProgDenoiseArgs A) {
+    const int x = blockIdx.x * PD_TX + threadIdx.x, y = blockIdx.y * PD_TY + threadIdx.y;
+    if (x >= A.w || y >= A.h) return;
+    const size_t i = size_t(y) * A.w + x;
+    const float4 c = __ldg(A.beauty + i), np = __ldg(A.normal + i);
+    float var;
+    if (c.w >= 4.0f) {
+        const float4 m = __ldg(A.src + i);
+        var = fmaxf(0.0f, m.y - m.x * m.x);
+    } else {
+        var = window_variance(A, x, y, c, np);
+    }
+    pd_store(A, i, c.x, c.y, c.z, var);
+}
+
+bool overlap(const void *a, uint64_t na, const void *b, uint64_t nb) { return uintptr_t(a) < uintptr_t(b) + nb && uintptr_t(b) < uintptr_t(a) + na; }
+
+// The a-trous stage's parameters and the image size, as both progressive denoisers check them and pass them to the kernels.
+int pd_args(rt_context *ctx, const rt_progressive_denoise_params *prm, uint32_t width, uint32_t height, ProgDenoiseArgs &A) {
     RT_REQUIRE(width > 0 && height > 0, "empty image");
     RT_REQUIRE(width <= 0x7FFFFFFFu && height <= 65535u * PD_TY, "image too large for one launch");
     RT_REQUIRE(prm->iterations <= 5 && prm->normal_exponent_log2 <= 8, "iterations 0..5, normal_exponent_log2 0..8");
     RT_REQUIRE(prm->sigma_luminance > 0.0f && prm->sigma_luminance <= 3.4e38f, "sigma_luminance must be finite and > 0");
     RT_REQUIRE(prm->sigma_albedo >= 0.0f && prm->sigma_albedo <= 3.4e38f, "sigma_albedo must be finite and >= 0");
-    // byte ranges [p, p + n): out and tmp are written, so neither may share a byte with any other argument
-    const uint64_t img = uint64_t(width) * height * 16;
-    auto overlap = [](const void *a, uint64_t na, const void *b, uint64_t nb) {
-        return uintptr_t(a) < uintptr_t(b) + nb && uintptr_t(b) < uintptr_t(a) + na;
-    };
-    for (const float *in : {beauty, albedo, normal}) {
-        RT_REQUIRE(!overlap(out, img, in, img), "out overlaps an input");
-        RT_REQUIRE(!overlap(tmp, 2 * img, in, img), "tmp overlaps an input");
-    }
-    RT_REQUIRE(!overlap(out, img, tmp, 2 * img), "out overlaps tmp");
-    RT_CUDA(cudaSetDevice(ctx->device));
-    ProgDenoiseArgs A{};
-    A.beauty = reinterpret_cast<const float4 *>(beauty);
-    A.albedo = reinterpret_cast<const float4 *>(albedo);
-    A.normal = reinterpret_cast<const float4 *>(normal);
+    A = ProgDenoiseArgs{};
     A.w = int(width), A.h = int(height);
     A.half = int(ctx->render_options.half_render_targets);
     A.nexp = int(prm->normal_exponent_log2);
     A.sigma_l = prm->sigma_luminance;
     A.inv_a = prm->sigma_albedo > 0.0f ? 1.0f / prm->sigma_albedo : 0.0f;
-    const int n = int(prm->iterations);
-    const dim3 grid(rt_div_up(width, PD_TX), rt_div_up(height, PD_TY)), block(PD_TX, PD_TY);
-    float4 *ping[2] = {reinterpret_cast<float4 *>(tmp), reinterpret_cast<float4 *>(tmp) + size_t(width) * height};
+    return RT_OK;
+}
+
+// `first` writes (C, var0) to tmp[0] (or out when there are no iterations), then one k_pd_atrous per iteration ping-pongs
+// through tmp and the last one writes out
+void pd_launch(rt_context *ctx, void (*first)(ProgDenoiseArgs), ProgDenoiseArgs A, int n, float *tmp, float *out) {
+    const dim3 grid(rt_div_up(uint32_t(A.w), PD_TX), rt_div_up(uint32_t(A.h), PD_TY)), block(PD_TX, PD_TY);
+    float4 *ping[2] = {reinterpret_cast<float4 *>(tmp), reinterpret_cast<float4 *>(tmp) + size_t(A.w) * A.h};
     A.dst = n == 0 ? reinterpret_cast<float4 *>(out) : ping[0];
     A.last = n == 0;
-    k_pd_variance<<<grid, block, 0, ctx->stream>>>(A);
+    first<<<grid, block, 0, ctx->stream>>>(A);
     for (int it = 0; it < n; ++it) {
         A.src = ping[it & 1];
         A.step = 1 << it;
@@ -428,6 +502,81 @@ extern "C" int rt_denoise_progressive(rt_context *ctx, const float *beauty, cons
         k_pd_atrous<<<grid, block, 0, ctx->stream>>>(A);
     }
     ctx->launches += 1 + n;
+}
+
+}  // namespace
+
+extern "C" int rt_denoise_progressive(rt_context *ctx, const float *beauty, const float *albedo, const float *normal, float *tmp,
+                                      float *out, uint32_t width, uint32_t height, const rt_progressive_denoise_params *prm) {
+    RT_REQUIRE(ctx && beauty && albedo && normal && tmp && out && prm, "null argument");
+    RT_REQUIRE(((uintptr_t(beauty) | uintptr_t(albedo) | uintptr_t(normal) | uintptr_t(tmp) | uintptr_t(out)) & 15) == 0,
+               "images must be 16-byte aligned");
+    ProgDenoiseArgs A;
+    if (const int e = pd_args(ctx, prm, width, height, A)) return e;
+    // byte ranges [p, p + n): out and tmp are written, so neither may share a byte with any other argument
+    const uint64_t img = uint64_t(width) * height * 16;
+    for (const float *in : {beauty, albedo, normal}) {
+        RT_REQUIRE(!overlap(out, img, in, img), "out overlaps an input");
+        RT_REQUIRE(!overlap(tmp, 2 * img, in, img), "tmp overlaps an input");
+    }
+    RT_REQUIRE(!overlap(out, img, tmp, 2 * img), "out overlaps tmp");
+    RT_CUDA(cudaSetDevice(ctx->device));
+    A.beauty = reinterpret_cast<const float4 *>(beauty);
+    A.albedo = reinterpret_cast<const float4 *>(albedo);
+    A.normal = reinterpret_cast<const float4 *>(normal);
+    pd_launch(ctx, k_pd_variance, A, int(prm->iterations), tmp, out);
+    RT_LAUNCH_CHECK();
+    return RT_OK;
+}
+
+extern "C" int rt_denoise_temporal(rt_context *ctx, const float *beauty, const float *albedo, const float *normal, const float *position,
+                                   const rt_camera_params *prev_camera, const float *prev_history, float *history, float *tmp, float *out,
+                                   uint32_t width, uint32_t height, const rt_temporal_denoise_params *prm) {
+    RT_REQUIRE(ctx && beauty && albedo && normal && position && history && tmp && out && prm, "null argument");
+    RT_REQUIRE((prev_camera == nullptr) == (prev_history == nullptr), "prev_camera and prev_history are both given or both NULL");
+    RT_REQUIRE(((uintptr_t(beauty) | uintptr_t(albedo) | uintptr_t(normal) | uintptr_t(position) | uintptr_t(prev_history) |
+                 uintptr_t(history) | uintptr_t(tmp) | uintptr_t(out)) & 15) == 0,
+               "images must be 16-byte aligned");
+    ProgDenoiseArgs A;
+    if (const int e = pd_args(ctx, &prm->spatial, width, height, A)) return e;
+    RT_REQUIRE(prm->alpha_color > 0.0f && prm->alpha_color <= 1.0f, "alpha_color in (0, 1]");
+    RT_REQUIRE(prm->alpha_moments > 0.0f && prm->alpha_moments <= 1.0f, "alpha_moments in (0, 1]");
+    RT_REQUIRE(prm->normal_cos >= -1.0f && prm->normal_cos <= 1.0f, "normal_cos in [-1, 1]");
+    RT_REQUIRE(prm->position_tolerance >= 0.0f && prm->position_tolerance <= 3.4e38f, "position_tolerance must be finite and >= 0");
+    // byte ranges [p, p + n): history, tmp and out are written, so none may share a byte with any other argument
+    const uint64_t img = uint64_t(width) * height * 16;
+    for (const float *in : {beauty, albedo, normal, position, prev_history}) {
+        const uint64_t n = in == prev_history ? 4 * img : img;
+        if (!in) continue;
+        RT_REQUIRE(!overlap(history, 4 * img, in, n), "history overlaps an input or prev_history");
+        RT_REQUIRE(!overlap(tmp, 2 * img, in, n), "tmp overlaps an input or prev_history");
+        RT_REQUIRE(!overlap(out, img, in, n), "out overlaps an input or prev_history");
+    }
+    RT_REQUIRE(!overlap(history, 4 * img, tmp, 2 * img) && !overlap(history, 4 * img, out, img) && !overlap(out, img, tmp, 2 * img),
+               "history, tmp and out overlap");
+    RT_CUDA(cudaSetDevice(ctx->device));
+    TemporalArgs T{};
+    T.beauty = reinterpret_cast<const float4 *>(beauty);
+    T.normal = reinterpret_cast<const float4 *>(normal);
+    T.position = reinterpret_cast<const float4 *>(position);
+    T.prev = reinterpret_cast<const float4 *>(prev_history);
+    T.hist = reinterpret_cast<float4 *>(history);
+    T.w = int(width), T.h = int(height);
+    if (prev_camera) {
+        for (int k = 0; k < 3; ++k)
+            T.eye[k] = prev_camera->worldEyePos[k], T.U[k] = prev_camera->U[k], T.V[k] = prev_camera->V[k], T.W[k] = prev_camera->W[k];
+        T.jitter[0] = prev_camera->jitters[0], T.jitter[1] = prev_camera->jitters[1];
+    }
+    T.alpha_c = prm->alpha_color, T.alpha_m = prm->alpha_moments;
+    T.normal_cos = prm->normal_cos, T.pos_tol = prm->position_tolerance;
+    k_td_reproject<<<dim3(rt_div_up(width, PD_TX), rt_div_up(height, PD_TY)), dim3(PD_TX, PD_TY), 0, ctx->stream>>>(T);
+    ctx->launches += 1;
+    const size_t plane = size_t(width) * height;
+    A.beauty = T.hist;  // (C, n): the integrated colour is what the variance and the a-trous stage filter
+    A.src = T.hist + plane;
+    A.albedo = reinterpret_cast<const float4 *>(albedo);
+    A.normal = T.normal;
+    pd_launch(ctx, k_td_variance, A, int(prm->spatial.iterations), tmp, out);
     RT_LAUNCH_CHECK();
     return RT_OK;
 }

@@ -226,11 +226,11 @@ __device__ __forceinline__ void write_aov(const Launch &L, const AovOut &a, int 
     if (a.mask & (1u << k)) write_pixel(L, a.ptr[k], a.pitch[k], x, y, c, true);
 }
 
-// The normal AOV: the running mean of (N, coverage) without write_pixel's clamp at 0, so that negative components
-// survive and `w` is the fraction of samples that hit.
-__device__ __forceinline__ void write_normal_aov(const Launch &L, const AovOut &a, uint32_t x, uint32_t y, f3 n, float coverage) {
-    if (!(a.mask & (1u << RT_AOV_NORMAL))) return;
-    float4 *px = reinterpret_cast<float4 *>(reinterpret_cast<uint8_t *>(a.ptr[RT_AOV_NORMAL]) + size_t(y) * a.pitch[RT_AOV_NORMAL]) + x;
+// The normal and position AOVs: the running mean of (N or P, coverage) without write_pixel's clamp at 0, so that negative
+// components survive and `w` is the fraction of samples that hit.
+__device__ __forceinline__ void write_geometry_aov(const Launch &L, const AovOut &a, int k, uint32_t x, uint32_t y, f3 n, float coverage) {
+    if (!(a.mask & (1u << k))) return;
+    float4 *px = reinterpret_cast<float4 *>(reinterpret_cast<uint8_t *>(a.ptr[k]) + size_t(y) * a.pitch[k]) + x;
     const uint32_t cnt = L.f.cameraParams.accumCount;
     const float4 prev = *px;
     const float fn = float(cnt), fn1 = float(cnt + 1);
@@ -269,7 +269,8 @@ __device__ __forceinline__ uint32_t octant_of(f3 d) {
 #ifndef RT_RESOLVE_MIN_BLOCKS
 #define RT_RESOLVE_MIN_BLOCKS 12
 #endif
-// AOV: write the AOV outputs of the primary misses and the normal AOV of every pixel (progressive program only).
+// AOV: write the AOV outputs of the primary misses and the normal and position AOVs of every pixel (progressive program
+// only).
 template <bool AOV>
 __global__ void __launch_bounds__(kShadeThreads) k_shade_primary(const __grid_constant__ Launch L, WS ws, const rt_hit_record_dev *recs,
                                                                  uint32_t n_recs, const float *env, uint32_t envSize, float *out0,
@@ -304,7 +305,8 @@ __global__ void __launch_bounds__(kShadeThreads) k_shade_primary(const __grid_co
                     write_aov(L, aov, RT_AOV_INDIRECT_SPECULAR, x, y, c);
                     write_aov(L, aov, RT_AOV_ALBEDO, x, y, c);
                     write_aov(L, aov, RT_AOV_FRESNEL, x, y, c);
-                    write_normal_aov(L, aov, x, y, mk3(0, 0, 0), 0.0f);
+                    write_geometry_aov(L, aov, RT_AOV_NORMAL, x, y, mk3(0, 0, 0), 0.0f);
+                    write_geometry_aov(L, aov, RT_AOV_POSITION, x, y, mk3(0, 0, 0), 0.0f);
                 }
             }
         }
@@ -322,8 +324,9 @@ __global__ void __launch_bounds__(kShadeThreads) k_shade_primary(const __grid_co
         const rt_hit_record_dev &R = recs[rec];
         const uint32_t prim = __float_as_uint(hA.w);
         const f3 N = normalize3(interpolate_normal(R, prim, hA.y, hA.z));
-        if (AOV) write_normal_aov(L, aov, x, y, N, 1.0f);
+        if (AOV) write_geometry_aov(L, aov, RT_AOV_NORMAL, x, y, N, 1.0f);
         pos = o + hA.x * d;  // HitWorldPosition
+        if (AOV) write_geometry_aov(L, aov, RT_AOV_POSITION, x, y, pos, 1.0f);
         const rt_debug_options &opt = L.f.options;
         if (!L.realtime && opt.showAmbientOcclusionOnly) {
             // evaluateAO: S/RaytracingCommon.hlsli:98-124 — 4 shadow rays, tMax 10

@@ -96,6 +96,12 @@ public:
     // with enableAov).  Stream-ordered after the last render(); the filter's scratch and the returned output are allocated on
     // first use and reused by later calls, so the result is valid until the next denoise().
     DXRFramework::RtBuffer::SharedPtr denoise(const rt_progressive_denoise_params &params);
+    // The beauty output filtered by rt_denoise_temporal: the frames filtered since the last resetTemporal() are the history,
+    // reprojected through the position AOV into the camera of the last render().  Needs the albedo, normal and position
+    // AOVs enabled and mFrameAccumulationEnabled false (one sample per frame).  Call once after every render(); the result
+    // is valid until the next call.
+    DXRFramework::RtBuffer::SharedPtr denoiseTemporal(const rt_temporal_denoise_params &params);
+    void resetTemporal() { mHasTemporalHistory = false; }
 
 private:
     explicit ProgressiveRaytracingPipeline(DXRFramework::RtContext::SharedPtr context);
@@ -104,4 +110,10 @@ private:
     bool mHasLastCamera = false;
     DXRFramework::RtBuffer::SharedPtr mDenoiseTmp, mDenoiseOut;
     uint64_t mDenoiseBytes = 0;
+    // rt_denoise_temporal: the history pair (mTemporalHistory[0] = the last call's), its scratch and output, and the camera
+    // of the frame the last call filtered
+    DXRFramework::RtBuffer::SharedPtr mTemporalHistory[2], mTemporalTmp, mTemporalOut;
+    uint64_t mTemporalBytes = 0;
+    CameraParams mPrevCamera{};
+    bool mHasTemporalHistory = false;
 };

@@ -212,6 +212,32 @@ RtBuffer::SharedPtr ProgressiveRaytracingPipeline::denoise(const rt_progressive_
     return mDenoiseOut;
 }
 
+RtBuffer::SharedPtr ProgressiveRaytracingPipeline::denoiseTemporal(const rt_temporal_denoise_params &params) {
+    const auto albedo = mAovResource[RT_AOV_ALBEDO], normal = mAovResource[RT_AOV_NORMAL], position = mAovResource[RT_AOV_POSITION];
+    ThrowIfFalse(albedo && normal && position, "ProgressiveRaytracingPipeline::denoiseTemporal needs the albedo, normal and position AOVs enabled");
+    ThrowIfFalse(!mFrameAccumulationEnabled, "ProgressiveRaytracingPipeline::denoiseTemporal needs mFrameAccumulationEnabled = false");
+    const uint64_t bytes = uint64_t(mOutputWidth) * mOutputHeight * 16;
+    if (!mTemporalOut || mTemporalBytes != bytes) {
+        mTemporalHistory[0] = mRtContext->createBuffer(4 * bytes);
+        mTemporalHistory[1] = mRtContext->createBuffer(4 * bytes);
+        mTemporalTmp = mRtContext->createBuffer(2 * bytes);
+        mTemporalOut = mRtContext->createBuffer(bytes);
+        mTemporalBytes = bytes;
+        mHasTemporalHistory = false;
+    }
+    std::swap(mTemporalHistory[0], mTemporalHistory[1]);  // [1] = the last call's history, [0] = this call's
+    ThrowIfFailed(rt_denoise_temporal(mRtContext->getNative(), static_cast<const float *>(mOutputResource.at(0)->ptr()),
+                                      static_cast<const float *>(albedo->ptr()), static_cast<const float *>(normal->ptr()),
+                                      static_cast<const float *>(position->ptr()), mHasTemporalHistory ? &mPrevCamera : nullptr,
+                                      mHasTemporalHistory ? static_cast<const float *>(mTemporalHistory[1]->ptr()) : nullptr,
+                                      static_cast<float *>(mTemporalHistory[0]->ptr()), static_cast<float *>(mTemporalTmp->ptr()),
+                                      static_cast<float *>(mTemporalOut->ptr()), mOutputWidth, mOutputHeight, &params),
+                  "rt_denoise_temporal");
+    mPrevCamera = mConstantBuffer.cameraParams;
+    mHasTemporalHistory = true;
+    return mTemporalOut;
+}
+
 // ------------------------------------------------------------------------------------------------ realtime
 RealtimeRaytracingPipeline::RealtimeRaytracingPipeline(RtContext::SharedPtr context)
     : RaytracingPipelineBase(context, kRealtimeRaytracingLibrary, kRealtimeRaytracingLibrarySize, 60, 2) {}

@@ -9,6 +9,8 @@
 //     same rays as --out (direct, indirect-diffuse, indirect-specular, albedo, fresnel, normal; EXR when the path ends in .exr)
 //   dxr_headless --pipeline progressive ... --denoise-progressive clean.pfm   the beauty output filtered with the albedo and
 //     normal AOVs as guides (rt_denoise_progressive; the flag enables both AOVs; EXR when the path ends in .exr)
+//   dxr_headless --pipeline progressive ... --orbit 0.5 --spp 16 --denoise-temporal clean.pfm   one sample per frame from a
+//     camera orbiting --at by 0.5 degrees per frame, every frame filtered by rt_denoise_temporal; writes the last frame's output
 // Multi-GPU (one process per GPU, replicated scene; the frame's samples and strips are sharded, one NCCL reduce at the end):
 //   for r in 0 1; do dxr_headless ... --spp 64 --world 2 --rank $r --comm-file /tmp/id [--strip-groups 2] --out frame.pfm & done
 #include <chrono>
@@ -75,8 +77,10 @@ static int usage() {
               "             [--spp N] [--seed S] [--no-jitter] [--eye x y z] [--at x y z] [--light-pos x y z] [--env-dds file | --env-raw file size]\n"
               "             [--out file.pfm] [--out2 file.pfm] [--denoise file.pfm] [--exr file.exr [--exr-half]] [--dump-frames file.bin] [--device N]\n"
               "             [--radiance-depth 1|2] [--fp16-targets] [--denoise-mock direct.pfm specular.pfm --denoise out.pfm [--kernel-size K]]\n"
-              "             [--aov direct|indirect-diffuse|indirect-specular|albedo|fresnel|normal file.pfm|file.exr]...   (progressive only)\n"
+              "             [--aov direct|indirect-diffuse|indirect-specular|albedo|fresnel|normal|position file.pfm|file.exr]...   (progressive only)\n"
               "             [--denoise-progressive file.pfm|file.exr]   (progressive only: the beauty output filtered with the albedo and normal AOVs)\n"
+              "             [--orbit DEGREES]   (frame f: the eye rotated about --at around +y by f * DEGREES)\n"
+              "             [--denoise-temporal file.pfm|file.exr]   (progressive, one GPU: accumulation off, every frame filtered by rt_denoise_temporal)\n"
               "             [--world N --rank R --comm-file path [--strip-groups G] [--strip-rows 32] [--band-shard]]   (one process per GPU)");
     return 0;
 }
@@ -100,6 +104,9 @@ int main(int argc, char **argv) {
         const bool denoiseProgressive = a.has("denoise-progressive");
         if (denoiseProgressive && (pipelineName == "realtime" || a.str("denoise-progressive", "").empty()))
             throw std::runtime_error("--denoise-progressive takes a path and needs --pipeline progressive (--denoise filters the realtime pipeline)");
+        const bool denoiseTemporal = a.has("denoise-temporal");
+        if (denoiseTemporal && (pipelineName == "realtime" || world > 1 || a.str("denoise-temporal", "").empty()))
+            throw std::runtime_error("--denoise-temporal takes a path and needs --pipeline progressive on one GPU (no --world > 1)");
         auto context = RtContext::create(int(a.num("device", rank)));
         if (a.has("denoise-mock")) {
             // DenoiseCompositor with mock inputs (src/DenoiseCompositor.cpp:52-60 loads DirectLighting.png / IndirectSpecular.png and
@@ -187,7 +194,8 @@ int main(int argc, char **argv) {
             pipeline->setEnvironment(tex);
         }
         // --aov NAME PATH, repeatable: names in rt_aov id order
-        static const char *const kAovNames[RT_AOV_COUNT] = {"direct", "indirect-diffuse", "indirect-specular", "albedo", "fresnel", "normal"};
+        static const char *const kAovNames[RT_AOV_COUNT] = {"direct", "indirect-diffuse", "indirect-specular", "albedo", "fresnel", "normal",
+                                                                   "position"};
         std::vector<std::pair<int, std::string>> aovFiles;
         if (a.has("aov")) {
             const auto &v = a.kv.at("aov");
@@ -203,6 +211,11 @@ int main(int argc, char **argv) {
             }
         }
         if (denoiseProgressive) pipeline->enableAov(RT_AOV_ALBEDO), pipeline->enableAov(RT_AOV_NORMAL);
+        const auto progressive = std::dynamic_pointer_cast<ProgressiveRaytracingPipeline>(pipeline);
+        if (denoiseTemporal) {
+            pipeline->enableAov(RT_AOV_ALBEDO), pipeline->enableAov(RT_AOV_NORMAL), pipeline->enableAov(RT_AOV_POSITION);
+            progressive->mFrameAccumulationEnabled = false;
+        }
         pipeline->loadResources(3);
         pipeline->createOutputResource(DXGI_FORMAT_R16G16B16A16_FLOAT, width, height);
         pipeline->setRenderOptions(UINT(a.num("radiance-depth", 1)), a.has("fp16-targets"));
@@ -227,7 +240,14 @@ int main(int argc, char **argv) {
         std::ofstream frames;
         if (a.has("dump-frames")) frames.open(a.str("dump-frames", ""), std::ios::binary);
         UINT mySamples = 0;
+        const rt_temporal_denoise_params temporalParams = RT_TEMPORAL_DENOISE_DEFAULTS;
+        RtBuffer::SharedPtr temporalOut;
         for (UINT f = 0; f < spp; ++f) {
+            if (a.has("orbit")) {  // the eye rotated about `at` around +y (scenes.orbit)
+                const double ang = double(f) * a.num("orbit", 0.0) * 3.14159265358979323846 / 180.0, c = std::cos(ang), s = std::sin(ang);
+                const double dx = double(eye.x) - at.x, dz = double(eye.z) - at.z;
+                camera->SetEyeAtUp({float(at.x + c * dx + s * dz), eye.y, float(at.z - s * dx + c * dz)}, at, {0, 1, 0});
+            }
             if (!bandShard && f % sampleGroups != sampleGroup) {  // another sample group's frame: keep the jitter sequence in step
                 pipeline->skipFrame();
                 continue;
@@ -240,6 +260,7 @@ int main(int argc, char **argv) {
             }
             if (frames) frames.write(reinterpret_cast<const char *>(&pipeline->getFrameConstants()), sizeof(PerFrameConstants));
             pipeline->render(f % 3, width, height);
+            if (denoiseTemporal) temporalOut = progressive->denoiseTemporal(temporalParams);
         }
         // ---- the path's one collective: every output is summed onto rank 0, weighted by the rank's share of the samples
         std::vector<RtBuffer::SharedPtr> finalOut;
@@ -285,6 +306,7 @@ int main(int argc, char **argv) {
             context->waitForGpu();
             save(clean, a.str("denoise-progressive", ""));
         }
+        if (denoiseTemporal && temporalOut) save(temporalOut, a.str("denoise-temporal", ""));
         if (bandShard) {
             save(bandFrame, a.str("denoise", ""));
         } else if (a.has("denoise") && rank == 0) {

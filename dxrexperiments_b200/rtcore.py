@@ -88,6 +88,7 @@ def _load():
         "rt_get_stage_timing": (i32, [vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double), i32]),
         "rt_denoise": (i32, [vp, vp, vp, vp, vp, u32, u32, vp]),
         "rt_denoise_progressive": (i32, [vp, vp, vp, vp, vp, vp, u32, u32, vp]),
+        "rt_denoise_temporal": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, u32, u32, vp]),
         "rt_trace_rays": (i32, [vp, vp, vp, u64, u32, u32, vp]),
         "rt_trace_rays_stats": (i32, [vp, vp, vp, u64, u32, u32, vp, vp]),
         "rt_trace_rays_hit_groups": (i32, [vp, vp, vp, u64, u32, u32, u32, u32, vp, u32, vp]),
@@ -365,6 +366,22 @@ class Context:
         check(lib.rt_denoise_progressive(self.handle, *(d.ptr for d in d_in), d_tmp.ptr, d_out.ptr, w, h, C.byref(params)))
         return d_out.download(np.float32).reshape(h, w, 4)
 
+    def denoise_temporal(self, beauty: np.ndarray, albedo: np.ndarray, normal: np.ndarray, position: np.ndarray,
+                         prev_camera: T.CameraParams = None, prev_history: np.ndarray = None,
+                         params: T.TemporalDenoiseParams = None):
+        """rt_denoise_temporal on host images: (h, w, 4) float32 beauty and albedo, normal and position AOVs, the previous
+        frame's camera and the history it returned (both None for a first frame) -> (out (h, w, 4), history (4, h, w, 4)),
+        both float32.  The history planes are (C, n), (m1, m2, 0, 0), normal, position (include/rt_core.h)."""
+        h, w = beauty.shape[:2]
+        d_in = [self.upload(np.ascontiguousarray(a, np.float32).reshape(-1)) for a in (beauty, albedo, normal, position)]
+        d_prev = None if prev_history is None else self.upload(np.ascontiguousarray(prev_history, np.float32).reshape(-1))
+        d_hist, d_tmp, d_out = self.alloc(64 * w * h), self.alloc(32 * w * h), self.alloc(16 * w * h)
+        params = T.temporal_denoise_defaults() if params is None else params
+        check(lib.rt_denoise_temporal(self.handle, *(d.ptr for d in d_in), C.byref(prev_camera) if prev_camera is not None else None,
+                                      d_prev.ptr if d_prev is not None else None, d_hist.ptr, d_tmp.ptr, d_out.ptr, w, h,
+                                      C.byref(params)))
+        return d_out.download(np.float32).reshape(h, w, 4), d_hist.download(np.float32).reshape(4, h, w, 4)
+
     def ray_counts(self, reset=False) -> T.RayCounts:
         c = T.RayCounts()
         check(lib.rt_get_ray_counts(self.handle, C.byref(c), 1 if reset else 0))
@@ -568,6 +585,8 @@ class Program:
 
 
 PROGRESSIVE, REALTIME = 0, 1
+_AOV_IDS = {**{name: k for k, name in enumerate(T.AOV_NAMES)}, T.AOV_POSITION_NAME: T.AOV_POSITION}
+assert sorted(_AOV_IDS.values()) == list(range(T.AOV_COUNT))
 
 
 class Comm:
@@ -632,8 +651,9 @@ class Renderer:
         of width*height RGBA fp32, one per output slot; allocated here when omitted.
         instance_mesh: optional list, one mesh index per transform (instancing: many instances of few BLASes);
         by default instance i is mesh i.
-        aovs: names from types.AOV_NAMES (progressive program only): each gets a zeroed width*height RGBA fp32 buffer
-        that every dispatch accumulates next to the beauty output (rt_set_aov_output); read it back with aov(name)."""
+        aovs: names from types.AOV_NAMES or types.AOV_POSITION_NAME (progressive program only): each gets a zeroed
+        width*height RGBA fp32 buffer that every dispatch accumulates next to the beauty output (rt_set_aov_output); read it
+        back with aov(name)."""
         self.ctx, self.width, self.height, self.kind = ctx, width, height, kind
         self.blases = [ctx.build_blas_from_mesh(m, build_flags=build_flags) for m in meshes]  # 0 = the application's flags (RtModel.cpp:86-118)
         if instance_mesh is None:
@@ -648,18 +668,20 @@ class Renderer:
         n_out = 2 if kind == REALTIME else 1
         self.out = list(outputs) if outputs is not None else [ctx.alloc(16 * width * height).zero() for _ in range(n_out)]
         assert len(self.out) == n_out
-        unknown = [a for a in aovs if a not in T.AOV_NAMES]
+        unknown = [a for a in aovs if a not in _AOV_IDS]
         if unknown:
-            raise ValueError(f"unknown AOV names {unknown}; known: {T.AOV_NAMES}")
+            raise ValueError(f"unknown AOV names {unknown}; known: {tuple(_AOV_IDS)}")
         self.aovs = {a: ctx.alloc(16 * width * height).zero() for a in aovs}
         self._denoise_bufs = None  # (tmp, out) of denoise(), allocated on first use
+        self._last_camera = None   # cameraParams of the last dispatch
+        self.reset_temporal()
 
     def dispatch(self, frame: T.PerFrameConstants, region=None, strips=None):
         """region: (x0, y0, x1, y1) pixel rectangle; strips: (strip_rows, groups, group) strip-interleaved shard."""
         # global root arguments are (re)bound per dispatch, as render() does (ProgressiveRaytracingPipeline.cpp:236-242)
         for slot, o in enumerate(self.out):
             check(lib.rt_set_output(self.ctx.handle, slot, o.ptr, 16 * self.width))
-        for k, name in enumerate(T.AOV_NAMES):  # all six, so that AOVs another Renderer bound on this context are unbound
+        for name, k in _AOV_IDS.items():  # all of them, so that AOVs another Renderer bound on this context are unbound
             buf = self.aovs.get(name)
             check(lib.rt_set_aov_output(self.ctx.handle, k, buf.ptr if buf is not None else None, 16 * self.width if buf is not None else 0))
         check(lib.rt_set_tlas(self.ctx.handle, self.tlas.result.ptr))
@@ -671,6 +693,7 @@ class Renderer:
         else:
             x0, y0, x1, y1 = region
             check(lib.rt_dispatch_rays_region(self.ctx.handle, self.program.handle, self.width, self.height, x0, y0, x1, y1))
+        self._last_camera = T.CameraParams.from_buffer_copy(bytes(frame.cameraParams))
 
     def realtime_band(self, frame: T.PerFrameConstants, band, params: T.DenoiserParams, tmp: "Buffer", final: "Buffer"):
         """One rank's share of a realtime frame sharded by row bands (sharding.band_plan): render rows [r0, r1) of the two
@@ -705,3 +728,34 @@ class Renderer:
         check(lib.rt_denoise_progressive(self.ctx.handle, self.out[0].ptr, self.aovs["albedo"].ptr, self.aovs["normal"].ptr, tmp.ptr,
                                          out.ptr, self.width, self.height, C.byref(params)))
         return out.download(np.float32).reshape(self.height, self.width, 4)
+
+    def denoise_temporal(self, params: T.TemporalDenoiseParams = None) -> np.ndarray:
+        """The last dispatch's beauty output filtered by rt_denoise_temporal, as (height, width, 4) float32: the frames
+        filtered since the last reset_temporal() are the history, reprojected through the position AOV.  Needs aovs= to
+        include "albedo", "normal" and "position", and a last dispatch of one sample with accumulation off (accumCount 0)."""
+        if self.kind != PROGRESSIVE or any(a not in self.aovs for a in ("albedo", "normal", T.AOV_POSITION_NAME)):
+            raise ValueError('denoise_temporal() needs a progressive Renderer with the "albedo", "normal" and "position" AOVs')
+        if self._last_camera is None or self._last_camera.accumCount != 0:
+            raise ValueError("denoise_temporal() filters frames of one sample: the last dispatch must have accumCount 0")
+        if self._temporal is None:
+            px = self.width * self.height
+            self._temporal = [self.ctx.alloc(64 * px), self.ctx.alloc(64 * px), self.ctx.alloc(32 * px), self.ctx.alloc(16 * px)]
+        prev, hist, tmp, out = self._temporal
+        params = T.temporal_denoise_defaults() if params is None else params
+        prev_cam = self._prev_camera
+        check(lib.rt_denoise_temporal(self.ctx.handle, self.out[0].ptr, self.aovs["albedo"].ptr, self.aovs["normal"].ptr,
+                                      self.aovs[T.AOV_POSITION_NAME].ptr, C.byref(prev_cam) if prev_cam is not None else None,
+                                      prev.ptr if prev_cam is not None else None, hist.ptr, tmp.ptr, out.ptr, self.width,
+                                      self.height, C.byref(params)))
+        self._temporal[0], self._temporal[1] = hist, prev  # this frame's history is the next call's prev_history
+        self._prev_camera = T.CameraParams.from_buffer_copy(bytes(self._last_camera))
+        return out.download(np.float32).reshape(self.height, self.width, 4)
+
+    def temporal_history(self) -> np.ndarray:
+        """The history the last denoise_temporal() wrote, as (4, height, width, 4) float32 (planes as in include/rt_core.h)."""
+        return self._temporal[0].download(np.float32).reshape(4, self.height, self.width, 4)
+
+    def reset_temporal(self):
+        """Drop the history: the next denoise_temporal() filters its frame as a first frame."""
+        self._temporal = None
+        self._prev_camera = None

@@ -261,6 +261,15 @@ class Camera:
         return (u * ulen).astype(f32), (v * vlen).astype(f32), w.astype(f32)
 
 
+def orbit(camera: Camera, degrees: float) -> Camera:
+    """`camera` with its eye rotated by `degrees` about its `at` point around +y (right-handed: +x turns towards -z)."""
+    a = np.radians(float(degrees))
+    c, s = float(np.cos(a)), float(np.sin(a))
+    dx, dz = camera.eye[0] - camera.at[0], camera.eye[2] - camera.at[2]
+    eye = (camera.at[0] + c * dx + s * dz, camera.eye[1], camera.at[2] - s * dx + c * dz)
+    return Camera(eye=eye, at=camera.at, up=camera.up, fov_y=camera.fov_y)
+
+
 @dataclass
 class FrameSetup:
     """Deterministic replacement of the wall-clock driven parts of update() (SURVEY.md A6)."""

@@ -58,6 +58,17 @@ def progressive_denoise_defaults() -> ProgressiveDenoiseParams:
     return ProgressiveDenoiseParams(5, 7, 4.0, 0.1)
 
 
+class TemporalDenoiseParams(C.Structure):  # rt_temporal_denoise_params (include/rt_types.h)
+    _fields_ = [("spatial", ProgressiveDenoiseParams), ("alpha_color", C.c_float), ("alpha_moments", C.c_float),
+                ("normal_cos", C.c_float), ("position_tolerance", C.c_float)]
+
+
+def temporal_denoise_defaults() -> TemporalDenoiseParams:
+    """RT_TEMPORAL_DENOISE_DEFAULTS (include/rt_types.h): the parameters rt_denoise_temporal is used with unless told
+    otherwise (DESIGN.md 4.4.2 records how they were chosen)."""
+    return TemporalDenoiseParams(progressive_denoise_defaults(), 0.2, 0.2, 0.9, 0.02)
+
+
 class GeometryDesc(C.Structure):
     _fields_ = [("vertex_buffer", C.c_void_p), ("vertex_count", C.c_uint32), ("vertex_stride_bytes", C.c_uint32),
                 ("index_buffer", C.c_void_p), ("index_count", C.c_uint32), ("index_format", C.c_uint32),
@@ -99,6 +110,7 @@ assert C.sizeof(PerFrameConstants) == 188
 assert C.sizeof(MaterialParams) == 64
 assert C.sizeof(DenoiserParams) == 24
 assert C.sizeof(ProgressiveDenoiseParams) == 16
+assert C.sizeof(TemporalDenoiseParams) == 32
 assert C.sizeof(InstanceDesc) == 64
 assert C.sizeof(HitRecord) == 80
 assert C.sizeof(GeometryDesc) == 48
@@ -153,8 +165,11 @@ ANYHIT_NONE, ANYHIT_ACCEPT, ANYHIT_IGNORE, ANYHIT_END_SEARCH, ANYHIT_CUTOUT = 0,
 INTERSECTION_NONE, INTERSECTION_BOX, INTERSECTION_SPHERE = 0, 1, 2
 HIT_KIND_TRIANGLE_FRONT_FACE = 0xFE
 # rt_aov (include/rt_core.h): AOV outputs of the progressive program, in id order
-AOV_DIRECT, AOV_INDIRECT_DIFFUSE, AOV_INDIRECT_SPECULAR, AOV_ALBEDO, AOV_FRESNEL, AOV_NORMAL, AOV_COUNT = range(7)
+AOV_DIRECT, AOV_INDIRECT_DIFFUSE, AOV_INDIRECT_SPECULAR, AOV_ALBEDO, AOV_FRESNEL, AOV_NORMAL, AOV_POSITION, AOV_COUNT = range(8)
+# the names of AOVs 0-5: the five debug-view terms and the normal
 AOV_NAMES = ("direct", "indirect-diffuse", "indirect-specular", "albedo", "fresnel", "normal")
+# the world-position AOV (what rt_denoise_temporal reprojects through), kept out of AOV_NAMES, which names AOVs 0-5 only
+AOV_POSITION_NAME = "position"
 
 
 def parse_blas_blob(blob: np.ndarray):

@@ -195,7 +195,9 @@ int rt_set_output(rt_context *ctx, uint32_t slot, float *rgba, uint64_t pitch_by
  * and for a primary miss the environment times environmentStrength; they are clamped at 0 with alpha 1 like gOutput.
  * NORMAL holds (N, 1) for a hit and (0, 0, 0, 0) for a miss, without the clamp, so its w is the fraction of samples that
  * hit.  N is the normalised interpolated vertex normal exactly as shade() receives it: the OBJECT-space normal, which
- * the reference does not transform by the instance.  Debug views change gOutput only; the AOVs keep these definitions. */
+ * the reference does not transform by the instance.  POSITION is stored like NORMAL (no clamp, w = coverage) with P the
+ * world-space primary hit point o + t*d (HitWorldPosition, o including the RayGen's jitter) in place of N: it is what
+ * rt_denoise_temporal reprojects through.  Debug views change gOutput only; the AOVs keep these definitions. */
 typedef enum rt_aov {
     RT_AOV_DIRECT = 0,
     RT_AOV_INDIRECT_DIFFUSE = 1,
@@ -203,7 +205,8 @@ typedef enum rt_aov {
     RT_AOV_ALBEDO = 3,
     RT_AOV_FRESNEL = 4,
     RT_AOV_NORMAL = 5,
-    RT_AOV_COUNT = 6
+    RT_AOV_POSITION = 6,
+    RT_AOV_COUNT = 7
 } rt_aov;
 /* Binds AOV `aov` (an rt_aov id; others are RT_ERR_INVALID_ARG) to a caller-owned RGBA fp32 image; NULL unbinds.  A
  * dispatch checks pitch_bytes >= width*16 for every bound AOV.  A dispatch with any AOV bound is RT_ERR_INVALID_ARG for
@@ -302,6 +305,37 @@ int rt_denoise(rt_context *ctx, const float *direct, const float *indirect_specu
 int rt_denoise_progressive(rt_context *ctx, const float *beauty, const float *albedo, const float *normal,
                            float *tmp /* 2 * width * height RGBA fp32 */, float *out,
                            uint32_t width, uint32_t height, const rt_progressive_denoise_params *params);
+/* The same filter with SVGF's temporal pass in front of it (Schied et al. 2017), for frames of one sample each
+ * (accumulation off) from a moving camera.  Inputs as rt_denoise_progressive plus position = RT_AOV_POSITION (P = .xyz);
+ * prev_camera (host memory) is the camera of the previous frame, as rt_set_frame_constants received it.  A history image
+ * is 4 planes of width x height RGBA fp32: 0 = (integrated C.rgb, history length n), 1 = (m1, m2, 0, 0) the integrated
+ * luminance moments, 2 = this frame's normal AOV, 3 = this frame's position AOV.  The call reads prev_history and writes
+ * history; the caller swaps them every frame.  prev_camera and prev_history are both NULL for a first frame (or after a
+ * reset).  Per pixel p, with L, wN and the window as above and c the coverage of the normal AOV:
+ *   Reproject (only if c == 1 and prev_history != NULL): o' = prev eye + (jitters[0]*30, jitters[1]*30, 0), the origin of
+ *     the progressive primary ray; r = Pp - o'; zc = dot(r, W')/dot(W', W'), no history if !(zc > 0);
+ *     sx = (dot(r, U')/dot(U', U'))/zc, sy = -((dot(r, V')/dot(V', V'))/zc) (the inverse of the primary ray: U', V', W'
+ *     are orthogonal); fx = ((sx + 1)*0.5)*width - 0.5, fy likewise; dot(a, b) = (a.x*b.x + a.y*b.y) + a.z*b.z.
+ *   Bilinear fetch: x0 = floor(fx), y0 = floor(fy), ax = fx - x0, ay = fy - y0; taps (x0, y0), (x0+1, y0), (x0, y0+1),
+ *     (x0+1, y0+1) in that order with weights (1-ax)*(1-ay), ax*(1-ay), (1-ax)*ay, ax*ay.  A tap is dropped when it lies
+ *     outside the image, its weight is 0, its coverage (plane 2 .w) is not 1, dot(Nq, Np) < normal_cos, or
+ *     |Pq - Pp| > position_tolerance*|Pp - o'| (|v| = sqrtf(dot(v, v))).  C_h, n_h, m1_h, m2_h are the weighted sums over
+ *     the remaining taps divided by the sum of their weights; with none left (or no fx, fy inside (-1, width) x
+ *     (-1, height)) they are 0.
+ *   Blend: n = min(n_h + 1, 32); a = max(1/n, alpha_color), am = max(1/n, alpha_moments); C = (1 - a)*C_h + a*C_cur;
+ *     m1 = (1 - am)*m1_h + am*L(C_cur), m2 = (1 - am)*m2_h + am*(L*L).
+ *   Variance: var0 = max(0, m2 - m1*m1) if n >= 4, else the 7 x 7 window estimate over the integrated C.
+ *   Then the a-trous iterations of rt_denoise_progressive run unchanged on (C, var0) and write out.
+ * Without history every pixel has n = 1 and C = C_cur, so out equals rt_denoise_progressive's bit for bit.  The history
+ * is fp32 always; only out is rounded through fp16 under half_render_targets.  tmp holds 2 * width * height RGBA fp32.
+ * 2 + iterations launches on the context's stream, no host synchronisation.  RT_ERR_INVALID_ARG: a null pointer (other
+ * than the prev_camera / prev_history pair), exactly one of that pair NULL, a buffer not 16-byte aligned, an empty image,
+ * parameters out of range, or history / tmp / out overlapping an input, prev_history or each other.  The inputs and
+ * prev_history are only read. */
+int rt_denoise_temporal(rt_context *ctx, const float *beauty, const float *albedo, const float *normal, const float *position,
+                        const rt_camera_params *prev_camera, const float *prev_history,
+                        float *history /* 4 * width * height RGBA fp32 */, float *tmp /* 2 * width * height RGBA fp32 */,
+                        float *out, uint32_t width, uint32_t height, const rt_temporal_denoise_params *params);
 
 /* ---- wavefront primitives exposed for parity tests and benchmarks */
 /* Fallback_TraceRay without shader call-outs (FL/TraverseShader.hlsli:21-73): n rays -> n hits. */

@@ -100,6 +100,17 @@ typedef struct rt_progressive_denoise_params {
 /* Defaults, chosen on the CPU restatement of the filter (DESIGN.md 4.4). */
 #define RT_PROGRESSIVE_DENOISE_DEFAULTS {5u, 7u, 4.0f, 0.1f}
 
+/* rt_denoise_temporal (rt_core.h); new work, no reference counterpart. */
+typedef struct rt_temporal_denoise_params {
+    rt_progressive_denoise_params spatial; /* the a-trous stage, exactly as rt_denoise_progressive */
+    float alpha_color;                     /* (0, 1]: floor of the current frame's blend weight (SVGF: 0.2) */
+    float alpha_moments;                   /* (0, 1]: the same for the luminance moments (SVGF: 0.2) */
+    float normal_cos;                      /* [-1, 1]: a history tap is rejected when dot(Nq, Np) < this */
+    float position_tolerance;              /* >= 0: ... or when |Pq - Pp| > this * |Pp - o_prev| */
+} rt_temporal_denoise_params; /* 32 B */
+/* Defaults, chosen on the CPU restatement of the filter (DESIGN.md 4.4.2). */
+#define RT_TEMPORAL_DENOISE_DEFAULTS {RT_PROGRESSIVE_DENOISE_DEFAULTS, 0.2f, 0.2f, 0.9f, 0.02f}
+
 /* Interleaved vertex the hit shaders read: libs/DXRFramework/RtModel.cpp:13-17 (stride 24). */
 typedef struct rt_vertex {
     float position[3];
