@@ -261,6 +261,15 @@ int rt_set_aov_output(rt_context *ctx, uint32_t aov, float *rgba, uint64_t pitch
     ctx->aov_pitch[aov] = pitch;
     return RT_OK;
 }
+int rt_set_instance_motion(rt_context *ctx, const float *world_to_previous_world, uint32_t n) {
+    RT_REQUIRE(ctx != nullptr, "ctx");
+    RT_REQUIRE((world_to_previous_world == nullptr) == (n == 0), "motion matrices: NULL with n = 0, or a pointer with n > 0");
+    RT_REQUIRE((uintptr_t(world_to_previous_world) & 15) == 0, "motion matrices must be 16-byte aligned");
+    RT_REQUIRE(n <= 0xFFFFFFu, "more than 2^24 - 1 motion matrices (InstanceIndex is 24 bits)");
+    ctx->motion = world_to_previous_world;
+    ctx->n_motion = n;
+    return RT_OK;
+}
 int rt_set_render_options(rt_context *ctx, const rt_render_options *o) {
     RT_REQUIRE(ctx && o, "null argument");
     RT_REQUIRE(o->max_radiance_ray_depth == 1 || o->max_radiance_ray_depth == 2, "max_radiance_ray_depth must be 1 or 2");

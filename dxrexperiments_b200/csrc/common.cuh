@@ -61,6 +61,8 @@ struct rt_context {
     uint64_t pitch[2] = {0, 0};
     float *aov[RT_AOV_COUNT] = {};  // rt_set_aov_output: progressive AOV images, nullptr = unbound
     uint64_t aov_pitch[RT_AOV_COUNT] = {};
+    const float *motion = nullptr;  // rt_set_instance_motion: n_motion row-major 3x4 world -> previous-world matrices (device)
+    uint32_t n_motion = 0;
     const void *tlas = nullptr;
     rt_render_options render_options{1u, 0u};
 

@@ -401,15 +401,19 @@ struct TemporalArgs {
 
 __device__ __forceinline__ float dot3(float ax, float ay, float az, const float b[3]) { return (ax * b[0] + ay * b[1]) + az * b[2]; }
 
-__global__ void __launch_bounds__(PD_TX * PD_TY) k_td_reproject(const __grid_constant__ TemporalArgs A) {
+// One pixel of the reprojection and blend.  MOTION (rt_denoise_temporal_motion): the point projected into the previous
+// frame and compared with the history's positions is Q = prev_pos[i] instead of this frame's P.
+template <bool MOTION>
+__device__ __forceinline__ void td_reproject(const TemporalArgs &A, const float4 *prev_pos) {
     const int x = blockIdx.x * PD_TX + threadIdx.x, y = blockIdx.y * PD_TY + threadIdx.y;
     if (x >= A.w || y >= A.h) return;
     const size_t plane = size_t(A.w) * A.h, i = size_t(y) * A.w + x;
     const float4 c = __ldg(A.beauty + i), np = __ldg(A.normal + i), pp = __ldg(A.position + i);
     float hr = 0.0f, hg = 0.0f, hb = 0.0f, hn = 0.0f, h1 = 0.0f, h2 = 0.0f;
     if (A.prev && np.w == 1.0f) {
+        const float4 q = MOTION ? __ldg(prev_pos + i) : pp;
         // o' is the progressive primary ray's origin (primary_ray in shade.cuh, jitterScale 30)
-        const float rx = pp.x - (A.eye[0] + A.jitter[0] * 30.0f), ry = pp.y - (A.eye[1] + A.jitter[1] * 30.0f), rz = pp.z - (A.eye[2] + 0.0f);
+        const float rx = q.x - (A.eye[0] + A.jitter[0] * 30.0f), ry = q.y - (A.eye[1] + A.jitter[1] * 30.0f), rz = q.z - (A.eye[2] + 0.0f);
         const float zc = dot3(rx, ry, rz, A.W) / dot3(A.W[0], A.W[1], A.W[2], A.W);
         const float sx = (dot3(rx, ry, rz, A.U) / dot3(A.U[0], A.U[1], A.U[2], A.U)) / zc;
         const float sy = -((dot3(rx, ry, rz, A.V) / dot3(A.V[0], A.V[1], A.V[2], A.V)) / zc);
@@ -433,7 +437,7 @@ __global__ void __launch_bounds__(PD_TX * PD_TY) k_td_reproject(const __grid_con
                     const float4 nq = __ldg(A.prev + 2 * plane + j);
                     if (nq.w != 1.0f || (np.x * nq.x + np.y * nq.y) + np.z * nq.z < A.normal_cos) continue;
                     const float4 pq = __ldg(A.prev + 3 * plane + j);
-                    const float ex = pq.x - pp.x, ey = pq.y - pp.y, ez = pq.z - pp.z;
+                    const float ex = pq.x - q.x, ey = pq.y - q.y, ez = pq.z - q.z;
                     if (sqrtf((ex * ex + ey * ey) + ez * ez) > lim) continue;
                     const float4 cq = __ldg(A.prev + j), mq = __ldg(A.prev + plane + j);
                     hr = hr + wt * cq.x, hg = hg + wt * cq.y, hb = hb + wt * cq.z, hn = hn + wt * cq.w;
@@ -450,6 +454,12 @@ __global__ void __launch_bounds__(PD_TX * PD_TY) k_td_reproject(const __grid_con
     A.hist[plane + i] = make_float4((1.0f - am) * h1 + am * l, (1.0f - am) * h2 + am * (l * l), 0.0f, 0.0f);
     A.hist[2 * plane + i] = np;
     A.hist[3 * plane + i] = pp;
+}
+
+__global__ void __launch_bounds__(PD_TX * PD_TY) k_td_reproject(const __grid_constant__ TemporalArgs A) { td_reproject<false>(A, nullptr); }
+
+__global__ void __launch_bounds__(PD_TX * PD_TY) k_td_reproject_motion(const __grid_constant__ TemporalArgs A, const float4 *prev_pos) {
+    td_reproject<true>(A, prev_pos);
 }
 
 // (C, var0) of the integrated colour: A.beauty = history plane 0 (C, n), A.src = history plane 1 (m1, m2)
@@ -529,13 +539,15 @@ extern "C" int rt_denoise_progressive(rt_context *ctx, const float *beauty, cons
     return RT_OK;
 }
 
-extern "C" int rt_denoise_temporal(rt_context *ctx, const float *beauty, const float *albedo, const float *normal, const float *position,
-                                   const rt_camera_params *prev_camera, const float *prev_history, float *history, float *tmp, float *out,
-                                   uint32_t width, uint32_t height, const rt_temporal_denoise_params *prm) {
-    RT_REQUIRE(ctx && beauty && albedo && normal && position && history && tmp && out && prm, "null argument");
+// rt_denoise_temporal (motion == false) and rt_denoise_temporal_motion (motion == true: previous_position is Q)
+static int denoise_temporal(rt_context *ctx, const float *beauty, const float *albedo, const float *normal, const float *position,
+                            const float *previous_position, bool motion, const rt_camera_params *prev_camera, const float *prev_history,
+                            float *history, float *tmp, float *out, uint32_t width, uint32_t height, const rt_temporal_denoise_params *prm) {
+    RT_REQUIRE(ctx && beauty && albedo && normal && position && (previous_position || !motion) && history && tmp && out && prm,
+               "null argument");
     RT_REQUIRE((prev_camera == nullptr) == (prev_history == nullptr), "prev_camera and prev_history are both given or both NULL");
-    RT_REQUIRE(((uintptr_t(beauty) | uintptr_t(albedo) | uintptr_t(normal) | uintptr_t(position) | uintptr_t(prev_history) |
-                 uintptr_t(history) | uintptr_t(tmp) | uintptr_t(out)) & 15) == 0,
+    RT_REQUIRE(((uintptr_t(beauty) | uintptr_t(albedo) | uintptr_t(normal) | uintptr_t(position) | uintptr_t(previous_position) |
+                 uintptr_t(prev_history) | uintptr_t(history) | uintptr_t(tmp) | uintptr_t(out)) & 15) == 0,
                "images must be 16-byte aligned");
     ProgDenoiseArgs A;
     if (const int e = pd_args(ctx, &prm->spatial, width, height, A)) return e;
@@ -545,7 +557,7 @@ extern "C" int rt_denoise_temporal(rt_context *ctx, const float *beauty, const f
     RT_REQUIRE(prm->position_tolerance >= 0.0f && prm->position_tolerance <= 3.4e38f, "position_tolerance must be finite and >= 0");
     // byte ranges [p, p + n): history, tmp and out are written, so none may share a byte with any other argument
     const uint64_t img = uint64_t(width) * height * 16;
-    for (const float *in : {beauty, albedo, normal, position, prev_history}) {
+    for (const float *in : {beauty, albedo, normal, position, previous_position, prev_history}) {
         const uint64_t n = in == prev_history ? 4 * img : img;
         if (!in) continue;
         RT_REQUIRE(!overlap(history, 4 * img, in, n), "history overlaps an input or prev_history");
@@ -569,7 +581,9 @@ extern "C" int rt_denoise_temporal(rt_context *ctx, const float *beauty, const f
     }
     T.alpha_c = prm->alpha_color, T.alpha_m = prm->alpha_moments;
     T.normal_cos = prm->normal_cos, T.pos_tol = prm->position_tolerance;
-    k_td_reproject<<<dim3(rt_div_up(width, PD_TX), rt_div_up(height, PD_TY)), dim3(PD_TX, PD_TY), 0, ctx->stream>>>(T);
+    const dim3 grid(rt_div_up(width, PD_TX), rt_div_up(height, PD_TY)), block(PD_TX, PD_TY);
+    if (motion) k_td_reproject_motion<<<grid, block, 0, ctx->stream>>>(T, reinterpret_cast<const float4 *>(previous_position));
+    else k_td_reproject<<<grid, block, 0, ctx->stream>>>(T);
     ctx->launches += 1;
     const size_t plane = size_t(width) * height;
     A.beauty = T.hist;  // (C, n): the integrated colour is what the variance and the a-trous stage filter
@@ -579,6 +593,21 @@ extern "C" int rt_denoise_temporal(rt_context *ctx, const float *beauty, const f
     pd_launch(ctx, k_td_variance, A, int(prm->spatial.iterations), tmp, out);
     RT_LAUNCH_CHECK();
     return RT_OK;
+}
+
+extern "C" int rt_denoise_temporal(rt_context *ctx, const float *beauty, const float *albedo, const float *normal, const float *position,
+                                   const rt_camera_params *prev_camera, const float *prev_history, float *history, float *tmp, float *out,
+                                   uint32_t width, uint32_t height, const rt_temporal_denoise_params *prm) {
+    return denoise_temporal(ctx, beauty, albedo, normal, position, nullptr, false, prev_camera, prev_history, history, tmp, out, width,
+                            height, prm);
+}
+
+extern "C" int rt_denoise_temporal_motion(rt_context *ctx, const float *beauty, const float *albedo, const float *normal,
+                                          const float *position, const float *previous_position, const rt_camera_params *prev_camera,
+                                          const float *prev_history, float *history, float *tmp, float *out, uint32_t width,
+                                          uint32_t height, const rt_temporal_denoise_params *prm) {
+    return denoise_temporal(ctx, beauty, albedo, normal, position, previous_position, true, prev_camera, prev_history, history, tmp, out,
+                            width, height, prm);
 }
 
 extern "C" int rt_denoise(rt_context *ctx, const float *direct, const float *indirect_specular, float *tmp, float *out, uint32_t width,

@@ -144,9 +144,11 @@ __device__ __forceinline__ void flush_stats(const TraceCtr &c, uint32_t rays, un
 #define RT_PRIMARY_MIN_BLOCKS 7  // 72 registers: the kernel is latency-bound (26 % of the warp slots active at 6 blocks); A/B round 2: 5 / 6 / 7 / 8
                                  // blocks per SM = 5363 / 5767 / 6103 / 5802 Mrays/s on C2, 3053 / 3160 / 3329 / 3035 on 1.31 M triangles
 #endif
-template <bool STATS>
-__global__ void __launch_bounds__(kBlock, RT_PRIMARY_MIN_BLOCKS) k_primary(const __grid_constant__ Launch L, const void *tlas, WS ws, uint32_t *status,
-                                                    unsigned long long *stats) {
+// INST: also store each pixel's InstanceIndex() to inst[p], which the previous-position AOV looks its motion up by (the
+// hit-group record does not determine the instance: it is RayContribution + InstanceContributionToHitGroupIndex).
+template <bool STATS, bool INST>
+__device__ __forceinline__ void primary_tile(const Launch &L, const void *tlas, const WS &ws, uint32_t *status, unsigned long long *stats,
+                                             uint32_t *inst) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const uint32_t tilesX = (L.rw + 7) / 8;
     const uint32_t tile = blockIdx.x * (kBlock / 32) + warp;
@@ -167,8 +169,22 @@ __global__ void __launch_bounds__(kBlock, RT_PRIMARY_MIN_BLOCKS) k_primary(const
         const uint32_t p = ly * L.rw + lx;
         ws.hitA[p] = make_float4(h.t, h.u, h.v, __uint_as_float(h.prim));
         ws.hitRec[p] = h.record;
+        if (INST) inst[p] = h.inst_index;
     }
     if (STATS) flush_stats(ctr, inside ? 1u : 0u, stats);
+}
+
+template <bool STATS>
+__global__ void __launch_bounds__(kBlock, RT_PRIMARY_MIN_BLOCKS) k_primary(const __grid_constant__ Launch L, const void *tlas, WS ws, uint32_t *status,
+                                                    unsigned long long *stats) {
+    primary_tile<STATS, false>(L, tlas, ws, status, stats, nullptr);
+}
+
+// k_primary for a dispatch with the previous-position AOV bound
+template <bool STATS>
+__global__ void __launch_bounds__(kBlock, RT_PRIMARY_MIN_BLOCKS) k_primary_inst(const __grid_constant__ Launch L, const void *tlas, WS ws,
+                                                                                uint32_t *status, unsigned long long *stats, uint32_t *inst) {
+    primary_tile<STATS, true>(L, tlas, ws, status, stats, inst);
 }
 
 // ------------------------------------------------------------------------------------------------ light helpers
@@ -219,7 +235,20 @@ struct AovOut {
     float *ptr[RT_AOV_COUNT];
     uint64_t pitch[RT_AOV_COUNT];
     uint32_t mask;
+    uint32_t n_motion;      // rt_set_instance_motion: matrices bound (0: none)
+    const float4 *motion;   // 3 rows of (m0, m1, m2, m3) per instance
+    const uint32_t *inst;   // [P] InstanceIndex() of each pixel's primary hit (k_primary_inst), previous-position AOV only
 };
+
+// P' of the previous-position AOV for the primary hit P of workspace pixel p (include/rt_core.h states the rule).
+__device__ __forceinline__ f3 previous_position(const AovOut &a, uint32_t p, f3 P) {
+    const uint32_t i = a.inst[p];
+    if (i >= a.n_motion) return P;
+    const float4 *m = a.motion + 3 * size_t(i);
+    const float4 r0 = __ldg(m), r1 = __ldg(m + 1), r2 = __ldg(m + 2);
+    return mk3(((r0.x * P.x + r0.y * P.y) + r0.z * P.z) + r0.w, ((r1.x * P.x + r1.y * P.y) + r1.z * P.z) + r1.w,
+               ((r2.x * P.x + r2.y * P.y) + r2.z * P.z) + r2.w);
+}
 
 // AOVs 0-4 accumulate exactly as the beauty frame does, so each one equals the matching debug view bit for bit.
 __device__ __forceinline__ void write_aov(const Launch &L, const AovOut &a, int k, uint32_t x, uint32_t y, f3 c) {
@@ -269,8 +298,8 @@ __device__ __forceinline__ uint32_t octant_of(f3 d) {
 #ifndef RT_RESOLVE_MIN_BLOCKS
 #define RT_RESOLVE_MIN_BLOCKS 12
 #endif
-// AOV: write the AOV outputs of the primary misses and the normal and position AOVs of every pixel (progressive program
-// only).
+// AOV: write the AOV outputs of the primary misses and the normal, position and previous-position AOVs of every pixel
+// (progressive program only).
 template <bool AOV>
 __global__ void __launch_bounds__(kShadeThreads) k_shade_primary(const __grid_constant__ Launch L, WS ws, const rt_hit_record_dev *recs,
                                                                  uint32_t n_recs, const float *env, uint32_t envSize, float *out0,
@@ -307,6 +336,7 @@ __global__ void __launch_bounds__(kShadeThreads) k_shade_primary(const __grid_co
                     write_aov(L, aov, RT_AOV_FRESNEL, x, y, c);
                     write_geometry_aov(L, aov, RT_AOV_NORMAL, x, y, mk3(0, 0, 0), 0.0f);
                     write_geometry_aov(L, aov, RT_AOV_POSITION, x, y, mk3(0, 0, 0), 0.0f);
+                    write_geometry_aov(L, aov, RT_AOV_PREVIOUS_POSITION, x, y, mk3(0, 0, 0), 0.0f);
                 }
             }
         }
@@ -327,6 +357,8 @@ __global__ void __launch_bounds__(kShadeThreads) k_shade_primary(const __grid_co
         if (AOV) write_geometry_aov(L, aov, RT_AOV_NORMAL, x, y, N, 1.0f);
         pos = o + hA.x * d;  // HitWorldPosition
         if (AOV) write_geometry_aov(L, aov, RT_AOV_POSITION, x, y, pos, 1.0f);
+        if (AOV && (aov.mask & (1u << RT_AOV_PREVIOUS_POSITION)))
+            write_geometry_aov(L, aov, RT_AOV_PREVIOUS_POSITION, x, y, previous_position(aov, p, pos), 1.0f);
         const rt_debug_options &opt = L.f.options;
         if (!L.realtime && opt.showAmbientOcclusionOnly) {
             // evaluateAO: S/RaytracingCommon.hlsli:98-124 — 4 shadow rays, tMax 10
@@ -795,7 +827,8 @@ __global__ void k_scale(float *buf, uint64_t n, float s) {
 
 // ------------------------------------------------------------------------------------------------ host
 // `part` of `parts`: the dispatch may run as several independent pixel bands, each with its own workspace of P pixels.
-int ensure_workspace(rt_context *ctx, uint64_t P, WS &ws, uint32_t part = 0, uint32_t parts = 1) {
+// inst: the pixels' InstanceIndex() array, which exists only while the previous-position AOV is bound (nullptr otherwise).
+int ensure_workspace(rt_context *ctx, uint64_t P, WS &ws, uint32_t part = 0, uint32_t parts = 1, uint32_t **inst = nullptr) {
     uint64_t o = 0;
     auto take = [&](uint64_t bytes) {
         uint64_t r = o;
@@ -810,6 +843,8 @@ int ensure_workspace(rt_context *ctx, uint64_t P, WS &ws, uint32_t part = 0, uin
     const bool depth2 = ctx->render_options.max_radiance_ray_depth >= 2;
     const uint64_t oTerQ = take(depth2 ? 32 * 2 * P : 0), oTerH = take(depth2 ? 16 * 2 * P : 0), oTerR = take(depth2 ? 4 * 2 * P : 0),
                    oTerRad = take(depth2 ? 16 * 2 * P : 0), oT3 = take(depth2 ? 8 * 2 * P : 0);
+    const bool prevPos = ctx->aov[RT_AOV_PREVIOUS_POSITION] != nullptr;
+    const uint64_t oInst = take(prevPos ? 4 * P : 0);
     const uint64_t one = align_up(o, 256);
     if (ctx->ws.bytes < one * parts) {
         if (ctx->ws.base) {
@@ -831,6 +866,7 @@ int ensure_workspace(rt_context *ctx, uint64_t P, WS &ws, uint32_t part = 0, uin
     ws.vis1 = b + oV1;
     ws.terQ = (rt_ray *)(b + oTerQ), ws.terHitA = (float4 *)(b + oTerH), ws.terRec = (uint32_t *)(b + oTerR);
     ws.terRad = (float4 *)(b + oTerRad), ws.T3 = (float2 *)(b + oT3);
+    if (inst) *inst = prevPos ? (uint32_t *)(b + oInst) : nullptr;
     return RT_OK;
 }
 
@@ -865,8 +901,8 @@ int upload_records(rt_program *prog) {
 
 extern "C" {
 
-static int dispatch_band(rt_context *ctx, rt_program *prog, const Launch &L, const WS &ws, cudaStream_t st, cudaStream_t side,
-                         cudaEvent_t ev_fork, cudaEvent_t ev_join);
+static int dispatch_band(rt_context *ctx, rt_program *prog, const Launch &L, const WS &ws, uint32_t *inst, cudaStream_t st,
+                         cudaStream_t side, cudaEvent_t ev_fork, cudaEvent_t ev_join);
 
 static int dispatch_impl(rt_context *ctx, rt_program *prog, uint32_t width, uint32_t height, uint32_t x0, uint32_t y0, uint32_t x1,
                          uint32_t y1, uint32_t stripShift, uint32_t stripGroups, uint32_t stripGroup) {
@@ -941,13 +977,15 @@ static int dispatch_impl(rt_context *ctx, rt_program *prog, uint32_t width, uint
             Launch Lk = L;
             Lk.v0 = y[k], Lk.rh = y[k + 1] - y[k];
             WS wk;
-            rc = ensure_workspace(ctx, Pmax, wk, k, bands);
+            uint32_t *inst;
+            rc = ensure_workspace(ctx, Pmax, wk, k, bands, &inst);
             if (rc) return rc;
             if (k == 0) {
-                rc = dispatch_band(ctx, prog, Lk, wk, ctx->stream, ctx->side_stream, ctx->ev_fork, ctx->ev_join);
+                rc = dispatch_band(ctx, prog, Lk, wk, inst, ctx->stream, ctx->side_stream, ctx->ev_fork, ctx->ev_join);
             } else {
                 RT_CUDA(cudaStreamWaitEvent(ctx->band_streams[k][0], ctx->ev_band_fork, 0));
-                rc = dispatch_band(ctx, prog, Lk, wk, ctx->band_streams[k][0], ctx->band_streams[k][1], ctx->band_events[k][0], ctx->band_events[k][1]);
+                rc = dispatch_band(ctx, prog, Lk, wk, inst, ctx->band_streams[k][0], ctx->band_streams[k][1], ctx->band_events[k][0],
+                                   ctx->band_events[k][1]);
                 if (rc == RT_OK) RT_CUDA(cudaEventRecord(ctx->band_events[k][2], ctx->band_streams[k][0]));
             }
             if (rc) return rc;
@@ -957,7 +995,8 @@ static int dispatch_impl(rt_context *ctx, rt_program *prog, uint32_t width, uint
     }
     const uint64_t P = uint64_t(L.rw) * L.rh;
     WS ws;
-    rc = ensure_workspace(ctx, P, ws);
+    uint32_t *inst;
+    rc = ensure_workspace(ctx, P, ws, 0, 1, &inst);
     if (rc) return rc;
     if (ctx->capture) ctx->dbg_pixels = P;
     if (!timing && !ctx->collect_stats && !ctx->side_stream) {
@@ -965,12 +1004,13 @@ static int dispatch_impl(rt_context *ctx, rt_program *prog, uint32_t width, uint
         RT_CUDA(cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming));
         RT_CUDA(cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming));
     }
-    return dispatch_band(ctx, prog, L, ws, ctx->stream, ctx->side_stream, ctx->ev_fork, ctx->ev_join);
+    return dispatch_band(ctx, prog, L, ws, inst, ctx->stream, ctx->side_stream, ctx->ev_fork, ctx->ev_join);
 }
 
-// One band of a dispatch: the seven wavefront stages on `st`, the depth-0 shadow wave on `side`.
-static int dispatch_band(rt_context *ctx, rt_program *prog, const Launch &L, const WS &ws, cudaStream_t st, cudaStream_t side,
-                         cudaEvent_t ev_fork, cudaEvent_t ev_join) {
+// One band of a dispatch: the seven wavefront stages on `st`, the depth-0 shadow wave on `side`.  inst: the band's
+// InstanceIndex() array when the previous-position AOV is bound, else nullptr.
+static int dispatch_band(rt_context *ctx, rt_program *prog, const Launch &L, const WS &ws, uint32_t *inst, cudaStream_t st,
+                         cudaStream_t side, cudaEvent_t ev_fork, cudaEvent_t ev_join) {
     const bool timing = ctx->timing;
     RT_CUDA(cudaMemsetAsync(ws.counters, 0, 256, st));
     const uint32_t tiles = ((L.rw + 7) / 8) * ((L.rh + 3) / 4);
@@ -978,8 +1018,14 @@ static int dispatch_band(rt_context *ctx, rt_program *prog, const Launch &L, con
     if (timing) RT_CUDA(cudaEventRecord(ctx->ev[0], st));
     unsigned long long *sPrim = ctx->ray_counts + 8, *sSec = ctx->ray_counts + 16, *sShadow = ctx->ray_counts + 24;
     const bool stats = ctx->collect_stats;
-    if (stats) k_primary<true><<<rt_div_up(tiles, kBlock / 32), kBlock, 0, st>>>(L, ctx->tlas, ws, ctx->status, sPrim);
-    else k_primary<false><<<rt_div_up(tiles, kBlock / 32), kBlock, 0, st>>>(L, ctx->tlas, ws, ctx->status, sPrim);
+    const uint32_t primBlocks = rt_div_up(tiles, kBlock / 32);
+    if (inst) {
+        if (stats) k_primary_inst<true><<<primBlocks, kBlock, 0, st>>>(L, ctx->tlas, ws, ctx->status, sPrim, inst);
+        else k_primary_inst<false><<<primBlocks, kBlock, 0, st>>>(L, ctx->tlas, ws, ctx->status, sPrim, inst);
+    } else {
+        if (stats) k_primary<true><<<primBlocks, kBlock, 0, st>>>(L, ctx->tlas, ws, ctx->status, sPrim);
+        else k_primary<false><<<primBlocks, kBlock, 0, st>>>(L, ctx->tlas, ws, ctx->status, sPrim);
+    }
     if (timing) RT_CUDA(cudaEventRecord(ctx->ev[1], st));
     const uint32_t shadeTiles = ((L.rw + kShadeTile - 1) / kShadeTile) * ((L.rh + kShadeTile - 1) / kShadeTile);
     AovOut aov{};
@@ -987,6 +1033,9 @@ static int dispatch_band(rt_context *ctx, rt_program *prog, const Launch &L, con
         aov.ptr[k] = ctx->aov[k], aov.pitch[k] = ctx->aov_pitch[k];
         if (ctx->aov[k]) aov.mask |= 1u << k;
     }
+    aov.n_motion = ctx->n_motion;
+    aov.motion = reinterpret_cast<const float4 *>(ctx->motion);
+    aov.inst = inst;
     if (aov.mask)
         k_shade_primary<true><<<shadeTiles, kShadeThreads, 0, st>>>(L, ws, prog->dev_recs, prog->n_recs, prog->env_texels, prog->env_size,
                                                                     ctx->output[0], ctx->pitch[0], ctx->output[1], ctx->pitch[1], ctx->ray_counts, ctx->status, aov);

@@ -1,6 +1,7 @@
 // DXRFramework.cpp — implementation of the headless DXRFramework layer over the rt_core C ABI.
 // Mirrors the behaviour of libs/DXRFramework/Rt{Context,Model,Scene,Program,Params,Bindings}.cpp of the reference.
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <fstream>
 #include <map>
@@ -272,6 +273,48 @@ void RtModel::build(RtContext::SharedPtr context) {
 
 // ============================================================================================ RtScene
 void RtScene::build(RtContext::SharedPtr context, UINT hitGroupCount) {
+    mHitGroupCount = hitGroupCount;
+    buildTlas(context, false);
+}
+
+// the instance desc's row-major 3x4 (the transpose of the row-vector XMMATRIX, TopLevelASGenerator.cpp:353-355) in double
+static void affine3x4(const XMMATRIX &transform, double out[12]) {
+    float m[16];
+    const XMMATRIX t = XMMatrixTranspose(transform);
+    std::memcpy(m, &t, sizeof(m));
+    for (int k = 0; k < 12; ++k) out[k] = m[k];
+}
+
+void RtScene::update(RtContext::SharedPtr context) {
+    const size_t n = mInstances.size();
+    std::vector<float> motion(12 * std::max<size_t>(n, 1));
+    for (size_t i = 0; i < n; ++i) {
+        double p[12], c[12], inv[12], r[12];
+        affine3x4(mBuiltTransforms[i], p);
+        affine3x4(mInstances[i].transform, c);
+        // inverse of [A t]: [A^-1, -A^-1 t], A^-1 = adj(A) / det(A)
+        const double a00 = c[0], a01 = c[1], a02 = c[2], a10 = c[4], a11 = c[5], a12 = c[6], a20 = c[8], a21 = c[9], a22 = c[10];
+        const double det = a00 * (a11 * a22 - a12 * a21) - a01 * (a10 * a22 - a12 * a20) + a02 * (a10 * a21 - a11 * a20);
+        ThrowIfFalse(det != 0.0 && std::isfinite(det), "RtScene::update: an instance transform is not invertible");
+        const double adj[9] = {a11 * a22 - a12 * a21, a02 * a21 - a01 * a22, a01 * a12 - a02 * a11,
+                               a12 * a20 - a10 * a22, a00 * a22 - a02 * a20, a02 * a10 - a00 * a12,
+                               a10 * a21 - a11 * a20, a01 * a20 - a00 * a21, a00 * a11 - a01 * a10};
+        for (int row = 0; row < 3; ++row) {
+            for (int col = 0; col < 3; ++col) inv[4 * row + col] = adj[3 * row + col] / det;
+            inv[4 * row + 3] = -(inv[4 * row] * c[3] + inv[4 * row + 1] * c[7] + inv[4 * row + 2] * c[11]);
+        }
+        for (int row = 0; row < 3; ++row) {
+            for (int col = 0; col < 4; ++col)
+                r[4 * row + col] = p[4 * row] * inv[col] + p[4 * row + 1] * inv[4 + col] + p[4 * row + 2] * inv[8 + col] + (col == 3 ? p[4 * row + 3] : 0.0);
+        }
+        for (int k = 0; k < 12; ++k) motion[12 * i + k] = float(r[k]);
+    }
+    if (!mMotionBuffer) mMotionBuffer = context->createBuffer(motion.data(), motion.size() * sizeof(float));
+    else mMotionBuffer->upload(motion.data(), motion.size() * sizeof(float));
+    buildTlas(context, true);
+}
+
+void RtScene::buildTlas(RtContext::SharedPtr context, bool performUpdate) {
     std::vector<rt_instance_desc> descs(mInstances.size());
     for (size_t i = 0; i < mInstances.size(); ++i) {
         if (!mInstances[i].model->mBlasBuffer) mInstances[i].model->build(context);
@@ -281,18 +324,21 @@ void RtScene::build(RtContext::SharedPtr context, UINT hitGroupCount) {
         XMMATRIX m = XMMatrixTranspose(mInstances[i].transform);
         std::memcpy(d.transform, &m, sizeof(d.transform));
         d.instance_id_and_mask = (uint32_t(i) & 0xFFFFFFu) | (0xFFu << 24);
-        d.hit_group_and_flags = (uint32_t(i * hitGroupCount) & 0xFFFFFFu) | (uint32_t(RT_INSTANCE_FLAG_NONE) << 24);
+        d.hit_group_and_flags = (uint32_t(i * mHitGroupCount) & 0xFFFFFFu) | (uint32_t(RT_INSTANCE_FLAG_NONE) << 24);
         d.blas = reinterpret_cast<uint64_t>(mInstances[i].model->mBlasBuffer->ptr());
     }
     const uint32_t n = static_cast<uint32_t>(descs.size());
     rt_prebuild_info info{};
     ThrowIfFailed(rt_tlas_prebuild(context->getNative(), n, RT_BUILD_FLAG_ALLOW_UPDATE, &info), "rt_tlas_prebuild");
-    auto scratch = context->createBuffer(info.scratch_bytes);
-    mTlasBuffer = context->createBuffer(info.result_bytes);
+    auto scratch = context->createBuffer(std::max<uint64_t>(performUpdate && info.update_scratch_bytes ? info.update_scratch_bytes : info.scratch_bytes, 16));
+    if (!performUpdate) mTlasBuffer = context->createBuffer(info.result_bytes);
     auto instanceDesc = context->createBuffer(descs.data(), std::max<uint64_t>(sizeof(rt_instance_desc) * n, 64));
-    ThrowIfFailed(rt_tlas_build(context->getNative(), static_cast<const rt_instance_desc *>(instanceDesc->ptr()), n, RT_BUILD_FLAG_ALLOW_UPDATE,
-                                scratch->ptr(), scratch->size(), mTlasBuffer->ptr(), mTlasBuffer->size()), "rt_tlas_build");
+    const uint32_t flags = uint32_t(RT_BUILD_FLAG_ALLOW_UPDATE) | (performUpdate ? uint32_t(RT_BUILD_FLAG_PERFORM_UPDATE) : 0u);
+    ThrowIfFailed(rt_tlas_build(context->getNative(), static_cast<const rt_instance_desc *>(instanceDesc->ptr()), n, flags, scratch->ptr(),
+                                scratch->size(), mTlasBuffer->ptr(), mTlasBuffer->size()), "rt_tlas_build");
     context->waitForGpu();
+    mBuiltTransforms.clear();
+    for (const Node &node : mInstances) mBuiltTransforms.push_back(node.transform);
 }
 
 // ============================================================================================ RtProgram

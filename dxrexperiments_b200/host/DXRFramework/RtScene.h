@@ -22,6 +22,15 @@ public:
     // i * hitGroupCount, mask 0xFF, flags NONE (RtScene.cpp:27-30, Helpers/TopLevelASGenerator.cpp:343-362).
     void build(RtContext::SharedPtr context, UINT hitGroupCount);
 
+    // Moving instances (new work: the reference's scene is static).  setTransform changes an instance's object->world
+    // transform; update refits the TLAS in place (PERFORM_UPDATE) and makes the motion the change from the transforms of
+    // the previous build or update to these: one row-major 3x4 world -> previous-world matrix per instance,
+    // prevObjectToWorld * inverse(objectToWorld) in double and rounded to float, for rt_set_instance_motion.
+    void setTransform(UINT index, DirectX::XMMATRIX transform) { mInstances.at(index).transform = transform; }
+    void update(RtContext::SharedPtr context);
+    // the device array of the motion matrices, nullptr before the first update
+    const float *getMotionPtr() const { return mMotionBuffer ? static_cast<const float *>(mMotionBuffer->ptr()) : nullptr; }
+
 private:
     RtScene() = default;
     struct Node {
@@ -29,7 +38,10 @@ private:
         DirectX::XMMATRIX transform;
     };
     std::vector<Node> mInstances;
-    RtBuffer::SharedPtr mTlasBuffer;
+    std::vector<DirectX::XMMATRIX> mBuiltTransforms;  // the transforms of the last build or update
+    UINT mHitGroupCount = 0;
+    RtBuffer::SharedPtr mTlasBuffer, mMotionBuffer;
+    void buildTlas(RtContext::SharedPtr context, bool performUpdate);
 };
 
 }  // namespace DXRFramework

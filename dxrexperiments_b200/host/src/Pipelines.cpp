@@ -167,6 +167,9 @@ void RaytracingPipelineBase::render(UINT /*frameIndex*/, UINT width, UINT height
         ThrowIfFailed(rt_set_aov_output(ctx, k, mAovResource[k] ? static_cast<float *>(mAovResource[k]->ptr()) : nullptr, uint64_t(width) * 16),
                       "rt_set_aov_output");
     ThrowIfFailed(rt_set_tlas(ctx, mRtScene->getTlasWrappedPtr()), "rt_set_tlas");
+    // the scene's instance motion for the previous-position AOV; NULL otherwise, so that no earlier binding is inherited
+    const float *motion = mAovResource[RT_AOV_PREVIOUS_POSITION] ? mRtScene->getMotionPtr() : nullptr;
+    ThrowIfFailed(rt_set_instance_motion(ctx, motion, motion ? mRtScene->getNumInstances() : 0), "rt_set_instance_motion");
     ThrowIfFailed(rt_set_render_options(ctx, &mRenderOptions), "rt_set_render_options");
 
     if (mBandRow1 > mBandRow0) mRtContext->raytraceRegion(mRtBindings, mRtState, width, height, 0, mBandRow0, width, std::min(mBandRow1, height));
@@ -226,13 +229,23 @@ RtBuffer::SharedPtr ProgressiveRaytracingPipeline::denoiseTemporal(const rt_temp
         mHasTemporalHistory = false;
     }
     std::swap(mTemporalHistory[0], mTemporalHistory[1]);  // [1] = the last call's history, [0] = this call's
-    ThrowIfFailed(rt_denoise_temporal(mRtContext->getNative(), static_cast<const float *>(mOutputResource.at(0)->ptr()),
-                                      static_cast<const float *>(albedo->ptr()), static_cast<const float *>(normal->ptr()),
-                                      static_cast<const float *>(position->ptr()), mHasTemporalHistory ? &mPrevCamera : nullptr,
-                                      mHasTemporalHistory ? static_cast<const float *>(mTemporalHistory[1]->ptr()) : nullptr,
-                                      static_cast<float *>(mTemporalHistory[0]->ptr()), static_cast<float *>(mTemporalTmp->ptr()),
-                                      static_cast<float *>(mTemporalOut->ptr()), mOutputWidth, mOutputHeight, &params),
-                  "rt_denoise_temporal");
+    const rt_camera_params *prevCamera = mHasTemporalHistory ? &mPrevCamera : nullptr;
+    const float *prevHistory = mHasTemporalHistory ? static_cast<const float *>(mTemporalHistory[1]->ptr()) : nullptr;
+    if (const auto previous = mAovResource[RT_AOV_PREVIOUS_POSITION])  // moving instances: reproject through their motion
+        ThrowIfFailed(rt_denoise_temporal_motion(mRtContext->getNative(), static_cast<const float *>(mOutputResource.at(0)->ptr()),
+                                                 static_cast<const float *>(albedo->ptr()), static_cast<const float *>(normal->ptr()),
+                                                 static_cast<const float *>(position->ptr()), static_cast<const float *>(previous->ptr()),
+                                                 prevCamera, prevHistory, static_cast<float *>(mTemporalHistory[0]->ptr()),
+                                                 static_cast<float *>(mTemporalTmp->ptr()), static_cast<float *>(mTemporalOut->ptr()),
+                                                 mOutputWidth, mOutputHeight, &params),
+                      "rt_denoise_temporal_motion");
+    else
+        ThrowIfFailed(rt_denoise_temporal(mRtContext->getNative(), static_cast<const float *>(mOutputResource.at(0)->ptr()),
+                                          static_cast<const float *>(albedo->ptr()), static_cast<const float *>(normal->ptr()),
+                                          static_cast<const float *>(position->ptr()), prevCamera, prevHistory,
+                                          static_cast<float *>(mTemporalHistory[0]->ptr()), static_cast<float *>(mTemporalTmp->ptr()),
+                                          static_cast<float *>(mTemporalOut->ptr()), mOutputWidth, mOutputHeight, &params),
+                      "rt_denoise_temporal");
     mPrevCamera = mConstantBuffer.cameraParams;
     mHasTemporalHistory = true;
     return mTemporalOut;

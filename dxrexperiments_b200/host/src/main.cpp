@@ -77,9 +77,11 @@ static int usage() {
               "             [--spp N] [--seed S] [--no-jitter] [--eye x y z] [--at x y z] [--light-pos x y z] [--env-dds file | --env-raw file size]\n"
               "             [--out file.pfm] [--out2 file.pfm] [--denoise file.pfm] [--exr file.exr [--exr-half]] [--dump-frames file.bin] [--device N]\n"
               "             [--radiance-depth 1|2] [--fp16-targets] [--denoise-mock direct.pfm specular.pfm --denoise out.pfm [--kernel-size K]]\n"
-              "             [--aov direct|indirect-diffuse|indirect-specular|albedo|fresnel|normal|position file.pfm|file.exr]...   (progressive only)\n"
+              "             [--aov direct|indirect-diffuse|indirect-specular|albedo|fresnel|normal|position|previous-position file.pfm|file.exr]...\n"
+              "                                                                    (progressive only)\n"
               "             [--denoise-progressive file.pfm|file.exr]   (progressive only: the beauty output filtered with the albedo and normal AOVs)\n"
               "             [--orbit DEGREES]   (frame f: the eye rotated about --at around +y by f * DEGREES)\n"
+              "             [--move DX DY DZ]   (frame f: instance 0 translated by f * (DX, DY, DZ); the camera stays unless --orbit)\n"
               "             [--denoise-temporal file.pfm|file.exr]   (progressive, one GPU: accumulation off, every frame filtered by rt_denoise_temporal)\n"
               "             [--world N --rank R --comm-file path [--strip-groups G] [--strip-rows 32] [--band-shard]]   (one process per GPU)");
     return 0;
@@ -195,7 +197,7 @@ int main(int argc, char **argv) {
         }
         // --aov NAME PATH, repeatable: names in rt_aov id order
         static const char *const kAovNames[RT_AOV_COUNT] = {"direct", "indirect-diffuse", "indirect-specular", "albedo", "fresnel", "normal",
-                                                                   "position"};
+                                                                   "position", "previous-position"};
         std::vector<std::pair<int, std::string>> aovFiles;
         if (a.has("aov")) {
             const auto &v = a.kv.at("aov");
@@ -214,6 +216,7 @@ int main(int argc, char **argv) {
         const auto progressive = std::dynamic_pointer_cast<ProgressiveRaytracingPipeline>(pipeline);
         if (denoiseTemporal) {
             pipeline->enableAov(RT_AOV_ALBEDO), pipeline->enableAov(RT_AOV_NORMAL), pipeline->enableAov(RT_AOV_POSITION);
+            if (a.has("move")) pipeline->enableAov(RT_AOV_PREVIOUS_POSITION);  // moving instances: the motion variant
             progressive->mFrameAccumulationEnabled = false;
         }
         pipeline->loadResources(3);
@@ -247,6 +250,11 @@ int main(int argc, char **argv) {
                 const double ang = double(f) * a.num("orbit", 0.0) * 3.14159265358979323846 / 180.0, c = std::cos(ang), s = std::sin(ang);
                 const double dx = double(eye.x) - at.x, dz = double(eye.z) - at.z;
                 camera->SetEyeAtUp({float(at.x + c * dx + s * dz), eye.y, float(at.z - s * dx + c * dz)}, at, {0, 1, 0});
+            }
+            if (a.has("move") && f > 0) {  // instance 0 at f * (DX, DY, DZ): a TLAS refit, and the motion since frame f - 1
+                scene->setTransform(0, DirectX::XMMatrixTranslation(float(f * a.num("move", 0.0, 0)), float(f * a.num("move", 0.0, 1)),
+                                                                    float(f * a.num("move", 0.0, 2))));
+                scene->update(context);
             }
             if (!bandShard && f % sampleGroups != sampleGroup) {  // another sample group's frame: keep the jitter sequence in step
                 pipeline->skipFrame();

@@ -78,6 +78,7 @@ def _load():
         "rt_set_output": (i32, [vp, u32, vp, u64]),
         "rt_set_aov_output": (i32, [vp, u32, vp, u64]),
         "rt_set_tlas": (i32, [vp, vp]),
+        "rt_set_instance_motion": (i32, [vp, vp, u32]),
         "rt_set_render_options": (i32, [vp, vp]),
         "rt_dispatch_rays": (i32, [vp, vp, u32, u32, u32]),
         "rt_dispatch_rays_region": (i32, [vp, vp, u32, u32, u32, u32, u32, u32]),
@@ -89,6 +90,7 @@ def _load():
         "rt_denoise": (i32, [vp, vp, vp, vp, vp, u32, u32, vp]),
         "rt_denoise_progressive": (i32, [vp, vp, vp, vp, vp, vp, u32, u32, vp]),
         "rt_denoise_temporal": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, u32, u32, vp]),
+        "rt_denoise_temporal_motion": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, u32, u32, vp]),
         "rt_trace_rays": (i32, [vp, vp, vp, u64, u32, u32, vp]),
         "rt_trace_rays_stats": (i32, [vp, vp, vp, u64, u32, u32, vp, vp]),
         "rt_trace_rays_hit_groups": (i32, [vp, vp, vp, u64, u32, u32, u32, u32, vp, u32, vp]),
@@ -382,6 +384,27 @@ class Context:
                                       C.byref(params)))
         return d_out.download(np.float32).reshape(h, w, 4), d_hist.download(np.float32).reshape(4, h, w, 4)
 
+    def denoise_temporal_motion(self, beauty: np.ndarray, albedo: np.ndarray, normal: np.ndarray, position: np.ndarray,
+                                previous_position: np.ndarray, prev_camera: T.CameraParams = None, prev_history: np.ndarray = None,
+                                params: T.TemporalDenoiseParams = None):
+        """rt_denoise_temporal_motion on host images: denoise_temporal with the previous-position AOV, which the
+        reprojection and the position test use in place of the position AOV."""
+        h, w = beauty.shape[:2]
+        d_in = [self.upload(np.ascontiguousarray(a, np.float32).reshape(-1)) for a in (beauty, albedo, normal, position, previous_position)]
+        d_prev = None if prev_history is None else self.upload(np.ascontiguousarray(prev_history, np.float32).reshape(-1))
+        d_hist, d_tmp, d_out = self.alloc(64 * w * h), self.alloc(32 * w * h), self.alloc(16 * w * h)
+        params = T.temporal_denoise_defaults() if params is None else params
+        check(lib.rt_denoise_temporal_motion(self.handle, *(d.ptr for d in d_in),
+                                             C.byref(prev_camera) if prev_camera is not None else None,
+                                             d_prev.ptr if d_prev is not None else None, d_hist.ptr, d_tmp.ptr, d_out.ptr, w, h,
+                                             C.byref(params)))
+        return d_out.download(np.float32).reshape(h, w, 4), d_hist.download(np.float32).reshape(4, h, w, 4)
+
+    def set_instance_motion(self, matrices=None, n: int = 0):
+        """rt_set_instance_motion: `matrices` is a device Buffer (or address) of n row-major 3x4 float32 world ->
+        previous-world matrices, one per InstanceIndex(); None with n = 0 unbinds."""
+        check(lib.rt_set_instance_motion(self.handle, _ptr(matrices), n))
+
     def ray_counts(self, reset=False) -> T.RayCounts:
         c = T.RayCounts()
         check(lib.rt_get_ray_counts(self.handle, C.byref(c), 1 if reset else 0))
@@ -585,7 +608,8 @@ class Program:
 
 
 PROGRESSIVE, REALTIME = 0, 1
-_AOV_IDS = {**{name: k for k, name in enumerate(T.AOV_NAMES)}, T.AOV_POSITION_NAME: T.AOV_POSITION}
+_AOV_IDS = {**{name: k for k, name in enumerate(T.AOV_NAMES)}, T.AOV_POSITION_NAME: T.AOV_POSITION,
+            T.AOV_PREVIOUS_POSITION_NAME: T.AOV_PREVIOUS_POSITION}
 assert sorted(_AOV_IDS.values()) == list(range(T.AOV_COUNT))
 
 
@@ -651,7 +675,8 @@ class Renderer:
         of width*height RGBA fp32, one per output slot; allocated here when omitted.
         instance_mesh: optional list, one mesh index per transform (instancing: many instances of few BLASes);
         by default instance i is mesh i.
-        aovs: names from types.AOV_NAMES or types.AOV_POSITION_NAME (progressive program only): each gets a zeroed
+        aovs: names from types.AOV_NAMES, types.AOV_POSITION_NAME or types.AOV_PREVIOUS_POSITION_NAME (progressive program
+        only): each gets a zeroed
         width*height RGBA fp32 buffer that every dispatch accumulates next to the beauty output (rt_set_aov_output); read it
         back with aov(name)."""
         self.ctx, self.width, self.height, self.kind = ctx, width, height, kind
@@ -659,7 +684,11 @@ class Renderer:
         if instance_mesh is None:
             instance_mesh = list(range(len(meshes)))
         assert len(instance_mesh) == len(transforms)
-        self.tlas = ctx.build_tlas([self.blases[k] for k in instance_mesh], transforms)
+        self.instance_mesh = list(instance_mesh)
+        self.transforms = np.asarray(transforms, np.float32).reshape(len(self.instance_mesh), 12).copy()
+        self.tlas = ctx.build_tlas([self.blases[k] for k in instance_mesh], self.transforms)
+        self.motion = None   # (n, 12) float32 world -> previous-world matrices of the last set_transforms(), None before it
+        self._motion_buf = None
         self.program = Program(ctx, kind)
         for i, k in enumerate(instance_mesh):
             for ray_type in range(2):
@@ -684,6 +713,8 @@ class Renderer:
         for name, k in _AOV_IDS.items():  # all of them, so that AOVs another Renderer bound on this context are unbound
             buf = self.aovs.get(name)
             check(lib.rt_set_aov_output(self.ctx.handle, k, buf.ptr if buf is not None else None, 16 * self.width if buf is not None else 0))
+        # every call, so that motion another Renderer bound on this context is never inherited
+        self.ctx.set_instance_motion(self._motion_buf, len(self.instance_mesh) if self._motion_buf is not None else 0)
         check(lib.rt_set_tlas(self.ctx.handle, self.tlas.result.ptr))
         check(lib.rt_set_frame_constants(self.ctx.handle, C.byref(frame)))
         if strips is not None:
@@ -694,6 +725,32 @@ class Renderer:
             x0, y0, x1, y1 = region
             check(lib.rt_dispatch_rays_region(self.ctx.handle, self.program.handle, self.width, self.height, x0, y0, x1, y1))
         self._last_camera = T.CameraParams.from_buffer_copy(bytes(frame.cameraParams))
+
+    def set_transforms(self, transforms):
+        """Move the instances: rebuild the TLAS with `transforms` (one object->world 3x4 per instance, as the constructor
+        took them) and make the instance motion, which the previous-position AOV applies, the change from the transforms
+        before this call to these: matrix i = prevObjectToWorld_i * inverse(objectToWorld_i), computed in float64 and
+        rounded to float32.  Call it once per frame of a moving sequence (with unchanged transforms for a frame where
+        nothing moves): the motion is always that of the last two calls, and none (identity) before the first."""
+        new = np.asarray(transforms, np.float32)
+        if new.size != 12 * len(self.instance_mesh):
+            raise ValueError(f"set_transforms() needs {len(self.instance_mesh)} 3x4 transforms, got an array of {new.size} values")
+        new = new.reshape(len(self.instance_mesh), 12)
+
+        def four(t):
+            m = np.zeros((t.shape[0], 4, 4))
+            m[:, :3, :] = t.astype(np.float64).reshape(-1, 3, 4)
+            m[:, 3, 3] = 1.0
+            return m
+        cur = four(new)
+        if np.any(~np.isfinite(new)) or np.any(np.abs(np.linalg.det(cur)) < 1e-30):
+            raise ValueError("set_transforms() needs finite, invertible transforms")
+        motion = (four(self.transforms) @ np.linalg.inv(cur))[:, :3, :].reshape(-1, 12).astype(np.float32)
+        self.tlas = self.ctx.build_tlas([self.blases[k] for k in self.instance_mesh], new)
+        self.transforms, self.motion = new.copy(), motion
+        if self._motion_buf is None:
+            self._motion_buf = self.ctx.alloc(48 * max(len(self.instance_mesh), 1))
+        self._motion_buf.upload(motion.reshape(-1))
 
     def realtime_band(self, frame: T.PerFrameConstants, band, params: T.DenoiserParams, tmp: "Buffer", final: "Buffer"):
         """One rank's share of a realtime frame sharded by row bands (sharding.band_plan): render rows [r0, r1) of the two
@@ -732,7 +789,9 @@ class Renderer:
     def denoise_temporal(self, params: T.TemporalDenoiseParams = None) -> np.ndarray:
         """The last dispatch's beauty output filtered by rt_denoise_temporal, as (height, width, 4) float32: the frames
         filtered since the last reset_temporal() are the history, reprojected through the position AOV.  Needs aovs= to
-        include "albedo", "normal" and "position", and a last dispatch of one sample with accumulation off (accumCount 0)."""
+        include "albedo", "normal" and "position", and a last dispatch of one sample with accumulation off (accumCount 0).
+        With the "previous-position" AOV also bound it runs rt_denoise_temporal_motion, which reprojects through that AOV,
+        so that instances moved by set_transforms() keep their history."""
         if self.kind != PROGRESSIVE or any(a not in self.aovs for a in ("albedo", "normal", T.AOV_POSITION_NAME)):
             raise ValueError('denoise_temporal() needs a progressive Renderer with the "albedo", "normal" and "position" AOVs')
         if self._last_camera is None or self._last_camera.accumCount != 0:
@@ -743,10 +802,13 @@ class Renderer:
         prev, hist, tmp, out = self._temporal
         params = T.temporal_denoise_defaults() if params is None else params
         prev_cam = self._prev_camera
-        check(lib.rt_denoise_temporal(self.ctx.handle, self.out[0].ptr, self.aovs["albedo"].ptr, self.aovs["normal"].ptr,
-                                      self.aovs[T.AOV_POSITION_NAME].ptr, C.byref(prev_cam) if prev_cam is not None else None,
-                                      prev.ptr if prev_cam is not None else None, hist.ptr, tmp.ptr, out.ptr, self.width,
-                                      self.height, C.byref(params)))
+        guides = (self.out[0].ptr, self.aovs["albedo"].ptr, self.aovs["normal"].ptr, self.aovs[T.AOV_POSITION_NAME].ptr)
+        history = (C.byref(prev_cam) if prev_cam is not None else None, prev.ptr if prev_cam is not None else None, hist.ptr,
+                   tmp.ptr, out.ptr, self.width, self.height, C.byref(params))
+        if T.AOV_PREVIOUS_POSITION_NAME in self.aovs:
+            check(lib.rt_denoise_temporal_motion(self.ctx.handle, *guides, self.aovs[T.AOV_PREVIOUS_POSITION_NAME].ptr, *history))
+        else:
+            check(lib.rt_denoise_temporal(self.ctx.handle, *guides, *history))
         self._temporal[0], self._temporal[1] = hist, prev  # this frame's history is the next call's prev_history
         self._prev_camera = T.CameraParams.from_buffer_copy(bytes(self._last_camera))
         return out.download(np.float32).reshape(self.height, self.width, 4)

@@ -270,6 +270,17 @@ def orbit(camera: Camera, degrees: float) -> Camera:
     return Camera(eye=eye, at=camera.at, up=camera.up, fov_y=camera.fov_y)
 
 
+SLIDING_BOX_START = (-0.6, -0.999, 0.7)  # the box's translation at frame 0: on the floor, in front of the two Cornell boxes
+
+
+def sliding_box(frame: int, step=(0.08, 0.0, 0.0)):
+    """A moving-instance scene: (meshes, transforms) of a small box (instance 0, 0.3 wide) sliding across the floor of the
+    Cornell room (instance 1, fixed).  At `frame` the box is translated by SLIDING_BOX_START + frame * step."""
+    t = np.array(IDENTITY_3X4, np.float64)
+    t[[3, 7, 11]] = np.array(SLIDING_BOX_START, np.float64) + frame * np.array(step, np.float64)
+    return [box((-0.15, 0.0, -0.15), (0.15, 0.3, 0.15)), cornell_box()], [t.astype(np.float32), IDENTITY_3X4.copy()]
+
+
 @dataclass
 class FrameSetup:
     """Deterministic replacement of the wall-clock driven parts of update() (SURVEY.md A6)."""

@@ -165,11 +165,15 @@ ANYHIT_NONE, ANYHIT_ACCEPT, ANYHIT_IGNORE, ANYHIT_END_SEARCH, ANYHIT_CUTOUT = 0,
 INTERSECTION_NONE, INTERSECTION_BOX, INTERSECTION_SPHERE = 0, 1, 2
 HIT_KIND_TRIANGLE_FRONT_FACE = 0xFE
 # rt_aov (include/rt_core.h): AOV outputs of the progressive program, in id order
-AOV_DIRECT, AOV_INDIRECT_DIFFUSE, AOV_INDIRECT_SPECULAR, AOV_ALBEDO, AOV_FRESNEL, AOV_NORMAL, AOV_POSITION, AOV_COUNT = range(8)
+(AOV_DIRECT, AOV_INDIRECT_DIFFUSE, AOV_INDIRECT_SPECULAR, AOV_ALBEDO, AOV_FRESNEL, AOV_NORMAL, AOV_POSITION, AOV_PREVIOUS_POSITION,
+ AOV_COUNT) = range(9)
 # the names of AOVs 0-5: the five debug-view terms and the normal
 AOV_NAMES = ("direct", "indirect-diffuse", "indirect-specular", "albedo", "fresnel", "normal")
 # the world-position AOV (what rt_denoise_temporal reprojects through), kept out of AOV_NAMES, which names AOVs 0-5 only
 AOV_POSITION_NAME = "position"
+# the same hit point carried into the previous frame by its instance's motion (what rt_denoise_temporal_motion reprojects
+# through), also kept out of AOV_NAMES
+AOV_PREVIOUS_POSITION_NAME = "previous-position"
 
 
 def parse_blas_blob(blob: np.ndarray):

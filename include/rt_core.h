@@ -197,7 +197,13 @@ int rt_set_output(rt_context *ctx, uint32_t slot, float *rgba, uint64_t pitch_by
  * hit.  N is the normalised interpolated vertex normal exactly as shade() receives it: the OBJECT-space normal, which
  * the reference does not transform by the instance.  POSITION is stored like NORMAL (no clamp, w = coverage) with P the
  * world-space primary hit point o + t*d (HitWorldPosition, o including the RayGen's jitter) in place of N: it is what
- * rt_denoise_temporal reprojects through.  Debug views change gOutput only; the AOVs keep these definitions. */
+ * rt_denoise_temporal reprojects through.  PREVIOUS_POSITION is stored exactly like POSITION with P' in place of P: the
+ * same hit point carried into the previous frame's world by the motion of the instance it lies on
+ * (rt_set_instance_motion).  With M the bound matrix of InstanceIndex() = i, P' = M * (P, 1), each row evaluated as
+ * ((m0*Px + m1*Py) + m2*Pz) + m3; P' = P (a copy, no arithmetic) when no motion is bound or i >= n.  No binding
+ * therefore gives a PREVIOUS_POSITION equal to POSITION bit for bit, and so does an identity matrix (x*1 and adding +0
+ * are exact; the one exception is a coordinate of -0, which comes out +0).  It is what
+ * rt_denoise_temporal_motion reprojects through.  Debug views change gOutput only; the AOVs keep these definitions. */
 typedef enum rt_aov {
     RT_AOV_DIRECT = 0,
     RT_AOV_INDIRECT_DIFFUSE = 1,
@@ -206,13 +212,22 @@ typedef enum rt_aov {
     RT_AOV_FRESNEL = 4,
     RT_AOV_NORMAL = 5,
     RT_AOV_POSITION = 6,
-    RT_AOV_COUNT = 7
+    RT_AOV_PREVIOUS_POSITION = 7,
+    RT_AOV_COUNT = 8
 } rt_aov;
 /* Binds AOV `aov` (an rt_aov id; others are RT_ERR_INVALID_ARG) to a caller-owned RGBA fp32 image; NULL unbinds.  A
  * dispatch checks pitch_bytes >= width*16 for every bound AOV.  A dispatch with any AOV bound is RT_ERR_INVALID_ARG for
  * a realtime program (its outputs already are AOVs) and in the showAmbientOcclusionOnly view (which traces AO rays
  * instead of lighting).  The maxIterations early-out leaves the AOVs untouched, as it leaves gOutput. */
 int rt_set_aov_output(rt_context *ctx, uint32_t aov, float *rgba, uint64_t pitch_bytes);
+/* Per-instance motion for RT_AOV_PREVIOUS_POSITION (new work: the reference has no counterpart).  world_to_previous_world
+ * is a DEVICE array of n row-major 3x4 fp32 matrices; matrix i maps this frame's world space to the previous frame's for
+ * the instance with InstanceIndex() == i.  A host computes it as prevObjectToWorld_i * inverse(objectToWorld_i).  It is
+ * context state like rt_set_tlas, read by the dispatches that write PREVIOUS_POSITION; the caller keeps the array alive
+ * and unchanged until they are done.  NULL with n = 0 unbinds.  RT_ERR_INVALID_ARG: NULL with n > 0 or a pointer with
+ * n = 0, a pointer not 16-byte aligned, n > 2^24 - 1.  Only rigid (per-instance) motion is described: a deforming mesh's
+ * moved vertices are not, and such pixels lose their history through the position test. */
+int rt_set_instance_motion(rt_context *ctx, const float *world_to_previous_world, uint32_t n);
 int rt_set_tlas(rt_context *ctx, const void *tlas_result);
 /* Two things that are constants of the reference and options here (defaults = the reference's shaders / this library's
  * declared fp32 deviation):
@@ -336,6 +351,22 @@ int rt_denoise_temporal(rt_context *ctx, const float *beauty, const float *albed
                         const rt_camera_params *prev_camera, const float *prev_history,
                         float *history /* 4 * width * height RGBA fp32 */, float *tmp /* 2 * width * height RGBA fp32 */,
                         float *out, uint32_t width, uint32_t height, const rt_temporal_denoise_params *params);
+/* rt_denoise_temporal for scenes whose instances move between frames.  previous_position = RT_AOV_PREVIOUS_POSITION
+ * (Q = .xyz: where this frame's primary hit point was in the previous frame's world, rt_set_instance_motion).  Q takes
+ * the place of Pp in exactly two places of the rule above:
+ *   the reprojection: r = Q - o';
+ *   the position test: a tap is dropped when |Pq - Q| > position_tolerance*|Q - o'|.
+ * Everything else is unchanged: the normal test compares this frame's normal AOV with the history's (the normal AOV is
+ * object-space, so a rigid instance motion leaves it unchanged), and history plane 3 stores this frame's P, which the
+ * next frame's Pq is.  previous_position == position therefore gives rt_denoise_temporal's out and history bit for bit.
+ * A deforming mesh (a BLAS refit with moved vertices) has no motion here: its pixels fail the position test as under
+ * rt_denoise_temporal.  previous_position is required; its alignment and overlap rules are those of the other inputs,
+ * and it is only read.  Launches and RT_ERR_INVALID_ARG cases otherwise as rt_denoise_temporal. */
+int rt_denoise_temporal_motion(rt_context *ctx, const float *beauty, const float *albedo, const float *normal,
+                               const float *position, const float *previous_position, const rt_camera_params *prev_camera,
+                               const float *prev_history, float *history /* 4 * width * height RGBA fp32 */,
+                               float *tmp /* 2 * width * height RGBA fp32 */, float *out, uint32_t width, uint32_t height,
+                               const rt_temporal_denoise_params *params);
 
 /* ---- wavefront primitives exposed for parity tests and benchmarks */
 /* Fallback_TraceRay without shader call-outs (FL/TraverseShader.hlsli:21-73): n rays -> n hits. */
