@@ -270,6 +270,14 @@ int rt_set_instance_motion(rt_context *ctx, const float *world_to_previous_world
     ctx->n_motion = n;
     return RT_OK;
 }
+int rt_set_adaptive_sampling(rt_context *ctx, uint32_t *counts, float *moments) {
+    RT_REQUIRE(ctx != nullptr, "ctx");
+    RT_REQUIRE((counts == nullptr) == (moments == nullptr), "counts and moments are both given or both NULL");
+    RT_REQUIRE((uintptr_t(counts) & 3) == 0 && (uintptr_t(moments) & 7) == 0, "counts must be 4-byte and moments 8-byte aligned");
+    ctx->adaptive_counts = counts;
+    ctx->adaptive_moments = moments;
+    return RT_OK;
+}
 int rt_set_render_options(rt_context *ctx, const rt_render_options *o) {
     RT_REQUIRE(ctx && o, "null argument");
     RT_REQUIRE(o->max_radiance_ray_depth == 1 || o->max_radiance_ray_depth == 2, "max_radiance_ray_depth must be 1 or 2");

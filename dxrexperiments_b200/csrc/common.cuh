@@ -63,6 +63,8 @@ struct rt_context {
     uint64_t aov_pitch[RT_AOV_COUNT] = {};
     const float *motion = nullptr;  // rt_set_instance_motion: n_motion row-major 3x4 world -> previous-world matrices (device)
     uint32_t n_motion = 0;
+    uint32_t *adaptive_counts = nullptr;  // rt_set_adaptive_sampling: width x height n_p | converged << 31 (device), nullptr = unbound
+    float *adaptive_moments = nullptr;    // width x height (m1, m2) fp32 (device)
     const void *tlas = nullptr;
     rt_render_options render_options{1u, 0u};
 
@@ -207,6 +209,10 @@ __device__ __forceinline__ float mul_(float a, float b) { return __fmul_rn(a, b)
 __device__ __forceinline__ float add_(float a, float b) { return __fadd_rn(a, b); }
 __device__ __forceinline__ float sub_(float a, float b) { return __fsub_rn(a, b); }
 __device__ __forceinline__ float div_(float a, float b) { return __fdiv_rn(a, b); }
+
+// Rec. 601 luma: reinhardToneMap's luminance (DenoiseCommon.hlsli:33-38), the edge-stopping luminance of
+// rt_denoise_progressive and the luminance whose moments adaptive sampling (rt_set_adaptive_sampling) accumulates.
+__device__ __forceinline__ float luminance(float r, float g, float b) { return (r * 0.299f + g * 0.587f) + b * 0.114f; }
 
 __device__ __forceinline__ f3 xform_point(const float *m, f3 v) {
     return mk3(add_(add_(add_(mul_(m[0], v.x), mul_(m[1], v.y)), mul_(m[2], v.z)), m[3]),

@@ -82,10 +82,6 @@ __device__ __forceinline__ f32x2 fma2(f32x2 a, f32x2 b, f32x2 c) {
     return r;
 }
 
-// Rec. 601 luma: reinhardToneMap's luminance (DenoiseCommon.hlsli:33-38) and the edge-stopping luminance of
-// rt_denoise_progressive.
-__device__ __forceinline__ float luminance(float r, float g, float b) { return (r * 0.299f + g * 0.587f) + b * 0.114f; }
-
 // PASS 0 = horizontal (DenoiseCompositorH.hlsl), PASS 1 = vertical + composite (DenoiseCompositorV.hlsl).
 template <int PASS>
 __global__ void __launch_bounds__(kThreadsDn, 3) k_denoise(const __grid_constant__ DenoiseArgs A) {
@@ -643,6 +639,87 @@ extern "C" int rt_denoise(rt_context *ctx, const float *direct, const float *ind
     const size_t v_smem = (6 * size_t(V_TH + 2 * A.k + 8) * V_TW + 64) * sizeof(float);
     k_denoise<1><<<dim3(rt_div_up(width, V_TW), rt_div_up(height, V_TH)), kThreadsDn, v_smem, ctx->stream>>>(A);
     ctx->launches += 2;
+    RT_LAUNCH_CHECK();
+    return RT_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ adaptive sampling
+// rt_adaptive_update: one thread per pixel over 16 x 16 tiles; the 18 x 18 window of "error at most threshold" flags the
+// tile's one-pixel dilation reads is computed once per block into shared memory.
+namespace {
+
+constexpr int AU_T = 16;
+
+struct AdaptiveArgs {
+    const float2 *moments;
+    uint32_t *counts;
+    uint32_t *active;
+    int w, h;
+    float threshold, floor;
+    uint32_t min_samples, max_samples;
+};
+
+// e_q <= threshold for pixel (x, y); true outside the image, which the dilation ignores
+__device__ __forceinline__ bool adaptive_error_ok(const AdaptiveArgs &A, int x, int y) {
+    if (x < 0 || y < 0 || x >= A.w || y >= A.h) return true;
+    const size_t i = size_t(y) * A.w + x;
+    const uint32_t n = A.counts[i] & ~RT_ADAPTIVE_CONVERGED;
+    if (n < 2) return false;  // sigma = +inf
+    const float2 m = __ldg(A.moments + i);
+    const float sigma = sqrtf(fmaxf(0.0f, m.y - m.x * m.x) / float(n - 1));
+    return sigma / (m.x + A.floor) <= A.threshold;  // NaN fails
+}
+
+__global__ void __launch_bounds__(AU_T * AU_T) k_adaptive_update(const __grid_constant__ AdaptiveArgs A) {
+    __shared__ uint8_t ok[AU_T + 2][AU_T + 2];
+    const int bx = blockIdx.x * AU_T, by = blockIdx.y * AU_T;
+    for (int k = threadIdx.y * AU_T + threadIdx.x; k < (AU_T + 2) * (AU_T + 2); k += AU_T * AU_T)
+        ok[k / (AU_T + 2)][k % (AU_T + 2)] = adaptive_error_ok(A, bx + k % (AU_T + 2) - 1, by + k / (AU_T + 2) - 1) ? 1 : 0;
+    __syncthreads();
+    const int x = bx + threadIdx.x, y = by + threadIdx.y;
+    bool active = false;
+    if (x < A.w && y < A.h) {
+        const size_t i = size_t(y) * A.w + x;
+        const uint32_t c = A.counts[i], n = c & ~RT_ADAPTIVE_CONVERGED;
+        bool conv = (c & RT_ADAPTIVE_CONVERGED) || n >= A.max_samples;
+        if (!conv && n >= A.min_samples) {
+            conv = true;
+#pragma unroll
+            for (int dy = 0; dy < 3; ++dy)
+#pragma unroll
+                for (int dx = 0; dx < 3; ++dx) conv = conv && ok[threadIdx.y + dy][threadIdx.x + dx];
+        }
+        // only bit 31 of a neighbour's word changes, which adaptive_error_ok masks off
+        if (conv && !(c & RT_ADAPTIVE_CONVERGED)) A.counts[i] = c | RT_ADAPTIVE_CONVERGED;
+        active = !conv;
+    }
+    const unsigned b = __ballot_sync(0xffffffffu, active);
+    if (A.active && ((threadIdx.y * AU_T + threadIdx.x) & 31) == 0 && b) atomicAdd(A.active, uint32_t(__popc(b)));  // one lane per warp
+}
+
+}  // namespace
+
+extern "C" int rt_adaptive_update(rt_context *ctx, const float *moments, uint32_t *counts, uint32_t width, uint32_t height,
+                                  const rt_adaptive_params *prm, uint32_t *active_count) {
+    RT_REQUIRE(ctx && moments && counts && prm, "null argument");
+    RT_REQUIRE(((uintptr_t(counts) | uintptr_t(active_count)) & 3) == 0 && (uintptr_t(moments) & 7) == 0,
+               "counts and active_count must be 4-byte and moments 8-byte aligned");
+    RT_REQUIRE(width > 0 && height > 0, "empty image");
+    RT_REQUIRE(width <= 0x7FFFFFFFu && height <= 65535u * AU_T, "image too large for one launch");
+    RT_REQUIRE(prm->threshold >= 0.0f && prm->threshold <= 3.4e38f, "threshold must be finite and >= 0");
+    RT_REQUIRE(prm->floor > 0.0f && prm->floor <= 3.4e38f, "floor must be finite and > 0");
+    RT_REQUIRE(prm->min_samples >= 1 && prm->min_samples <= prm->max_samples && prm->max_samples <= 0x7FFFFFFFu,
+               "1 <= min_samples <= max_samples <= 2^31 - 1");
+    const uint64_t px = uint64_t(width) * height;
+    RT_REQUIRE(!overlap(counts, 4 * px, moments, 8 * px), "counts overlaps moments");
+    RT_REQUIRE(!active_count || (!overlap(active_count, 4, moments, 8 * px) && !overlap(active_count, 4, counts, 4 * px)),
+               "active_count overlaps moments or counts");
+    RT_CUDA(cudaSetDevice(ctx->device));
+    if (active_count) RT_CUDA(cudaMemsetAsync(active_count, 0, 4, ctx->stream));
+    const AdaptiveArgs A{reinterpret_cast<const float2 *>(moments), counts, active_count, int(width), int(height), prm->threshold, prm->floor,
+                         prm->min_samples, prm->max_samples};
+    k_adaptive_update<<<dim3(rt_div_up(width, AU_T), rt_div_up(height, AU_T)), dim3(AU_T, AU_T), 0, ctx->stream>>>(A);
+    ctx->launches++;
     RT_LAUNCH_CHECK();
     return RT_OK;
 }

@@ -144,16 +144,27 @@ __device__ __forceinline__ void flush_stats(const TraceCtr &c, uint32_t rays, un
 #define RT_PRIMARY_MIN_BLOCKS 7  // 72 registers: the kernel is latency-bound (26 % of the warp slots active at 6 blocks); A/B round 2: 5 / 6 / 7 / 8
                                  // blocks per SM = 5363 / 5767 / 6103 / 5802 Mrays/s on C2, 3053 / 3160 / 3329 / 3035 on 1.31 M triangles
 #endif
+// Adaptive sampling (rt_set_adaptive_sampling): the per-pixel sample counts (bit 31: converged) and luminance moments, in
+// image order.  Only the ADAPTIVE instantiations of k_primary, k_primary_inst, k_shade_primary and k_resolve read them.
+struct Adaptive {
+    uint32_t *counts;
+    float2 *moments;
+};
+
+__device__ __forceinline__ size_t image_index(const Launch &L, uint32_t x, uint32_t y) { return size_t(y) * L.width + x; }
+
 // INST: also store each pixel's InstanceIndex() to inst[p], which the previous-position AOV looks its motion up by (the
 // hit-group record does not determine the instance: it is RayContribution + InstanceContributionToHitGroupIndex).
-template <bool STATS, bool INST>
+// ADAPTIVE: a converged pixel traces nothing and is not counted.
+template <bool STATS, bool INST, bool ADAPTIVE>
 __device__ __forceinline__ void primary_tile(const Launch &L, const void *tlas, const WS &ws, uint32_t *status, unsigned long long *stats,
-                                             uint32_t *inst) {
+                                             uint32_t *inst, const uint32_t *counts) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const uint32_t tilesX = (L.rw + 7) / 8;
     const uint32_t tile = blockIdx.x * (kBlock / 32) + warp;
     const uint32_t lx = (tile % tilesX) * 8 + (lane & 7), ly = (tile / tilesX) * 4 + (lane >> 3);
-    const bool inside = lx < L.rw && ly < L.rh;
+    const bool inside = lx < L.rw && ly < L.rh &&
+                        (!ADAPTIVE || !(counts[image_index(L, L.x0 + lx, image_row(L, ly))] & RT_ADAPTIVE_CONVERGED));
     TraceCtr ctr{0, 0, 0, 0};
     if (inside) {
         const uint32_t x = L.x0 + lx, y = image_row(L, ly);
@@ -174,17 +185,18 @@ __device__ __forceinline__ void primary_tile(const Launch &L, const void *tlas, 
     if (STATS) flush_stats(ctr, inside ? 1u : 0u, stats);
 }
 
-template <bool STATS>
+template <bool STATS, bool ADAPTIVE>
 __global__ void __launch_bounds__(kBlock, RT_PRIMARY_MIN_BLOCKS) k_primary(const __grid_constant__ Launch L, const void *tlas, WS ws, uint32_t *status,
-                                                    unsigned long long *stats) {
-    primary_tile<STATS, false>(L, tlas, ws, status, stats, nullptr);
+                                                    unsigned long long *stats, const uint32_t *counts) {
+    primary_tile<STATS, false, ADAPTIVE>(L, tlas, ws, status, stats, nullptr, counts);
 }
 
 // k_primary for a dispatch with the previous-position AOV bound
-template <bool STATS>
+template <bool STATS, bool ADAPTIVE>
 __global__ void __launch_bounds__(kBlock, RT_PRIMARY_MIN_BLOCKS) k_primary_inst(const __grid_constant__ Launch L, const void *tlas, WS ws,
-                                                                                uint32_t *status, unsigned long long *stats, uint32_t *inst) {
-    primary_tile<STATS, true>(L, tlas, ws, status, stats, inst);
+                                                                                uint32_t *status, unsigned long long *stats, uint32_t *inst,
+                                                                                const uint32_t *counts) {
+    primary_tile<STATS, true, ADAPTIVE>(L, tlas, ws, status, stats, inst, counts);
 }
 
 // ------------------------------------------------------------------------------------------------ light helpers
@@ -213,11 +225,12 @@ __device__ __forceinline__ LightEval eval_lights(const rt_per_frame_constants &f
     return e;
 }
 
-__device__ __forceinline__ void write_pixel(const Launch &L, float *out, uint64_t pitch, uint32_t x, uint32_t y, f3 c, bool accumulate) {
+// n: the samples already in the running mean (accumCount, or the pixel's count under adaptive sampling)
+__device__ __forceinline__ void write_pixel(const Launch &L, float *out, uint64_t pitch, uint32_t x, uint32_t y, f3 c, bool accumulate,
+                                            uint32_t n) {
     float4 *px = reinterpret_cast<float4 *>(reinterpret_cast<uint8_t *>(out) + size_t(y) * pitch) + x;
     float4 cur = make_float4(fmaxf(c.x, 0.0f), fmaxf(c.y, 0.0f), fmaxf(c.z, 0.0f), 1.0f);
     if (accumulate) {  // RayGen: S/ProgressiveRaytracing.hlsl:36-38
-        const uint32_t n = L.f.cameraParams.accumCount;
         float4 prev = *px;
         const float fn = float(n), fn1 = float(n + 1);
         cur = make_float4((fn * prev.x + cur.x) / fn1, (fn * prev.y + cur.y) / fn1, (fn * prev.z + cur.z) / fn1,
@@ -251,16 +264,16 @@ __device__ __forceinline__ f3 previous_position(const AovOut &a, uint32_t p, f3 
 }
 
 // AOVs 0-4 accumulate exactly as the beauty frame does, so each one equals the matching debug view bit for bit.
-__device__ __forceinline__ void write_aov(const Launch &L, const AovOut &a, int k, uint32_t x, uint32_t y, f3 c) {
-    if (a.mask & (1u << k)) write_pixel(L, a.ptr[k], a.pitch[k], x, y, c, true);
+__device__ __forceinline__ void write_aov(const Launch &L, const AovOut &a, int k, uint32_t x, uint32_t y, f3 c, uint32_t n) {
+    if (a.mask & (1u << k)) write_pixel(L, a.ptr[k], a.pitch[k], x, y, c, true, n);
 }
 
 // The normal and position AOVs: the running mean of (N or P, coverage) without write_pixel's clamp at 0, so that negative
 // components survive and `w` is the fraction of samples that hit.
-__device__ __forceinline__ void write_geometry_aov(const Launch &L, const AovOut &a, int k, uint32_t x, uint32_t y, f3 n, float coverage) {
+__device__ __forceinline__ void write_geometry_aov(const Launch &L, const AovOut &a, int k, uint32_t x, uint32_t y, f3 n, float coverage,
+                                                   uint32_t cnt) {
     if (!(a.mask & (1u << k))) return;
     float4 *px = reinterpret_cast<float4 *>(reinterpret_cast<uint8_t *>(a.ptr[k]) + size_t(y) * a.pitch[k]) + x;
-    const uint32_t cnt = L.f.cameraParams.accumCount;
     const float4 prev = *px;
     const float fn = float(cnt), fn1 = float(cnt + 1);
     float4 cur = make_float4((fn * prev.x + n.x) / fn1, (fn * prev.y + n.y) / fn1, (fn * prev.z + n.z) / fn1, (fn * prev.w + coverage) / fn1);
@@ -268,6 +281,15 @@ __device__ __forceinline__ void write_geometry_aov(const Launch &L, const AovOut
         cur = make_float4(__half2float(__float2half_rn(cur.x)), __half2float(__float2half_rn(cur.y)), __half2float(__float2half_rn(cur.z)),
                           __half2float(__float2half_rn(cur.w)));
     *px = cur;
+}
+
+// Adaptive sampling: fold the sample c (clamped as write_pixel clamps it) into pixel i's luminance moments and count it.
+__device__ __forceinline__ void write_moments(const Adaptive &ad, size_t i, f3 c, uint32_t n) {
+    const float l = luminance(fmaxf(c.x, 0.0f), fmaxf(c.y, 0.0f), fmaxf(c.z, 0.0f));
+    const float2 m = ad.moments[i];
+    const float fn = float(n), fn1 = float(n + 1);
+    ad.moments[i] = make_float2((fn * m.x + l) / fn1, (fn * m.y + l * l) / fn1);
+    ad.counts[i] = n + 1;
 }
 
 // ------------------------------------------------------------------------------------------------ K2
@@ -299,18 +321,25 @@ __device__ __forceinline__ uint32_t octant_of(f3 d) {
 #define RT_RESOLVE_MIN_BLOCKS 12
 #endif
 // AOV: write the AOV outputs of the primary misses and the normal, position and previous-position AOVs of every pixel
-// (progressive program only).
-template <bool AOV>
+// (progressive program only).  ADAPTIVE: a converged pixel is treated as outside the launch, the running means use the
+// pixel's count, and a miss folds its sample into the moments here (a hit does so in k_resolve).
+template <bool AOV, bool ADAPTIVE>
 __global__ void __launch_bounds__(kShadeThreads) k_shade_primary(const __grid_constant__ Launch L, WS ws, const rt_hit_record_dev *recs,
                                                                  uint32_t n_recs, const float *env, uint32_t envSize, float *out0,
                                                                  uint64_t pitch0, float *out1, uint64_t pitch1,
-                                                                 unsigned long long *rayCounts, uint32_t *status, const AovOut aov) {
+                                                                 unsigned long long *rayCounts, uint32_t *status, const AovOut aov,
+                                                                 const Adaptive ad) {
     __shared__ uint32_t s_count[kBins], s_offset[kBins], s_base;
     const uint32_t tilesX = (L.rw + kShadeTile - 1) / kShadeTile;
     const uint32_t lx = (blockIdx.x % tilesX) * kShadeTile + (threadIdx.x % kShadeTile);
     const uint32_t ly = (blockIdx.x / tilesX) * kShadeTile + (threadIdx.x / kShadeTile);
     const uint32_t p = ly * L.rw + lx;
-    const bool inRange = lx < L.rw && ly < L.rh;
+    bool inRange = lx < L.rw && ly < L.rh;
+    uint32_t n = L.f.cameraParams.accumCount;
+    if (ADAPTIVE && inRange) {
+        n = ad.counts[image_index(L, L.x0 + lx, image_row(L, ly))];
+        if (n & RT_ADAPTIVE_CONVERGED) inRange = false;
+    }
     if (threadIdx.x < kBins) s_count[threadIdx.x] = 0;
     bool isHit = false;
     float4 hA = make_float4(0, 0, 0, 0);
@@ -324,20 +353,21 @@ __global__ void __launch_bounds__(kShadeThreads) k_shade_primary(const __grid_co
         if (!isHit) {  // PrimaryMiss
             f3 c = sample_env(env, envSize, d) * L.f.options.environmentStrength;
             if (L.realtime) {
-                write_pixel(L, out0, pitch0, x, y, c, false);
-                write_pixel(L, out1, pitch1, x, y, mk3(0, 0, 0), false);
+                write_pixel(L, out0, pitch0, x, y, c, false, n);
+                write_pixel(L, out1, pitch1, x, y, mk3(0, 0, 0), false, n);
             } else {
-                write_pixel(L, out0, pitch0, x, y, c, true);
+                write_pixel(L, out0, pitch0, x, y, c, true, n);
                 if (AOV) {  // every debug view shows the environment for a miss
-                    write_aov(L, aov, RT_AOV_DIRECT, x, y, c);
-                    write_aov(L, aov, RT_AOV_INDIRECT_DIFFUSE, x, y, c);
-                    write_aov(L, aov, RT_AOV_INDIRECT_SPECULAR, x, y, c);
-                    write_aov(L, aov, RT_AOV_ALBEDO, x, y, c);
-                    write_aov(L, aov, RT_AOV_FRESNEL, x, y, c);
-                    write_geometry_aov(L, aov, RT_AOV_NORMAL, x, y, mk3(0, 0, 0), 0.0f);
-                    write_geometry_aov(L, aov, RT_AOV_POSITION, x, y, mk3(0, 0, 0), 0.0f);
-                    write_geometry_aov(L, aov, RT_AOV_PREVIOUS_POSITION, x, y, mk3(0, 0, 0), 0.0f);
+                    write_aov(L, aov, RT_AOV_DIRECT, x, y, c, n);
+                    write_aov(L, aov, RT_AOV_INDIRECT_DIFFUSE, x, y, c, n);
+                    write_aov(L, aov, RT_AOV_INDIRECT_SPECULAR, x, y, c, n);
+                    write_aov(L, aov, RT_AOV_ALBEDO, x, y, c, n);
+                    write_aov(L, aov, RT_AOV_FRESNEL, x, y, c, n);
+                    write_geometry_aov(L, aov, RT_AOV_NORMAL, x, y, mk3(0, 0, 0), 0.0f, n);
+                    write_geometry_aov(L, aov, RT_AOV_POSITION, x, y, mk3(0, 0, 0), 0.0f, n);
+                    write_geometry_aov(L, aov, RT_AOV_PREVIOUS_POSITION, x, y, mk3(0, 0, 0), 0.0f, n);
                 }
+                if (ADAPTIVE) write_moments(ad, image_index(L, x, y), c, n);
             }
         }
     }
@@ -354,11 +384,11 @@ __global__ void __launch_bounds__(kShadeThreads) k_shade_primary(const __grid_co
         const rt_hit_record_dev &R = recs[rec];
         const uint32_t prim = __float_as_uint(hA.w);
         const f3 N = normalize3(interpolate_normal(R, prim, hA.y, hA.z));
-        if (AOV) write_geometry_aov(L, aov, RT_AOV_NORMAL, x, y, N, 1.0f);
+        if (AOV) write_geometry_aov(L, aov, RT_AOV_NORMAL, x, y, N, 1.0f, n);
         pos = o + hA.x * d;  // HitWorldPosition
-        if (AOV) write_geometry_aov(L, aov, RT_AOV_POSITION, x, y, pos, 1.0f);
+        if (AOV) write_geometry_aov(L, aov, RT_AOV_POSITION, x, y, pos, 1.0f, n);
         if (AOV && (aov.mask & (1u << RT_AOV_PREVIOUS_POSITION)))
-            write_geometry_aov(L, aov, RT_AOV_PREVIOUS_POSITION, x, y, previous_position(aov, p, pos), 1.0f);
+            write_geometry_aov(L, aov, RT_AOV_PREVIOUS_POSITION, x, y, previous_position(aov, p, pos), 1.0f, n);
         const rt_debug_options &opt = L.f.options;
         if (!L.realtime && opt.showAmbientOcclusionOnly) {
             // evaluateAO: S/RaytracingCommon.hlsli:98-124 — 4 shadow rays, tMax 10
@@ -687,14 +717,16 @@ __device__ __forceinline__ f3 secondary_radiance(const Launch &L, const WS &ws, 
     return (mk3(m.emissive[0], m.emissive[1], m.emissive[2]) * m.emissive[3] + albedo * diffuseComponent) + specTerm;
 }
 
-// AOV: also write AOVs 0-4 of every hit slot (progressive program only).
-template <bool AOV>
+// AOV: also write AOVs 0-4 of every hit slot (progressive program only).  ADAPTIVE: the running means use the pixel's
+// count, and every slot folds its sample into the moments and counts it.
+template <bool AOV, bool ADAPTIVE>
 __global__ void __launch_bounds__(kBlock, RT_RESOLVE_MIN_BLOCKS) k_resolve(const __grid_constant__ Launch L, WS ws, const rt_hit_record_dev *recs, float *out0,
-                                                    uint64_t pitch0, float *out1, uint64_t pitch1, const AovOut aov) {
+                                                    uint64_t pitch0, float *out1, uint64_t pitch1, const AovOut aov, const Adaptive ad) {
     const uint32_t n = ws.counters[0];
     for (uint32_t s = blockIdx.x * blockDim.x + threadIdx.x; s < n; s += gridDim.x * blockDim.x) {
         const uint4 info = ws.slotInfo[s];
         const uint32_t x = L.x0 + info.x % L.rw, y = image_row(L, info.x / L.rw);
+        const uint32_t np = ADAPTIVE ? ad.counts[image_index(L, x, y)] : L.f.cameraParams.accumCount;
         const rt_material_params &m = recs[info.y].mat;
         const uint32_t flags = info.z;
         f3 color;
@@ -708,7 +740,8 @@ __global__ void __launch_bounds__(kBlock, RT_RESOLVE_MIN_BLOCKS) k_resolve(const
             vis += float(v[2 * pl]) * nol.z / pdf.z;
             vis += float(v[3 * pl]) * nol.w / pdf.w;
             const float ao = vis / 4.0f;
-            write_pixel(L, out0, pitch0, x, y, mk3(ao, ao, ao), true);
+            write_pixel(L, out0, pitch0, x, y, mk3(ao, ao, ao), true, np);
+            if (ADAPTIVE) write_moments(ad, image_index(L, x, y), mk3(ao, ao, ao), np);
             continue;
         }
         const float4 s0 = ws.S0[s], s1 = ws.S1[s], s2 = ws.S2[s];
@@ -743,16 +776,16 @@ __global__ void __launch_bounds__(kBlock, RT_RESOLVE_MIN_BLOCKS) k_resolve(const
         const f3 albedo = mk3(m.albedo[0], m.albedo[1], m.albedo[2]);
         if (L.realtime) {
             // aov.directLighting / aov.indirectSpecular: S/RealtimeRaytracing.hlsl:95-100
-            write_pixel(L, out0, pitch0, x, y, albedo * direct / RT_M_PI, false);
-            write_pixel(L, out1, pitch1, x, y, m.reflectivity * spec * fres, false);
+            write_pixel(L, out0, pitch0, x, y, albedo * direct / RT_M_PI, false, np);
+            write_pixel(L, out1, pitch1, x, y, m.reflectivity * spec * fres, false, np);
             continue;
         }
         if (AOV) {  // the expressions of the debug views below, so that each AOV equals its view bit for bit
-            write_aov(L, aov, RT_AOV_DIRECT, x, y, albedo * direct / RT_M_PI);
-            write_aov(L, aov, RT_AOV_INDIRECT_DIFFUSE, x, y, albedo * indirect / RT_M_PI);
-            write_aov(L, aov, RT_AOV_INDIRECT_SPECULAR, x, y, m.reflectivity * spec * fres);
-            write_aov(L, aov, RT_AOV_ALBEDO, x, y, albedo);
-            write_aov(L, aov, RT_AOV_FRESNEL, x, y, fres);
+            write_aov(L, aov, RT_AOV_DIRECT, x, y, albedo * direct / RT_M_PI, np);
+            write_aov(L, aov, RT_AOV_INDIRECT_DIFFUSE, x, y, albedo * indirect / RT_M_PI, np);
+            write_aov(L, aov, RT_AOV_INDIRECT_SPECULAR, x, y, m.reflectivity * spec * fres, np);
+            write_aov(L, aov, RT_AOV_ALBEDO, x, y, albedo, np);
+            write_aov(L, aov, RT_AOV_FRESNEL, x, y, fres, np);
         }
         const rt_debug_options &opt = L.f.options;
         const f3 diffuseComponent = (direct + indirect) / RT_M_PI;
@@ -762,7 +795,8 @@ __global__ void __launch_bounds__(kBlock, RT_RESOLVE_MIN_BLOCKS) k_resolve(const
         else if (opt.showGBufferAlbedoOnly) color = albedo;
         else if (opt.showDirectLightingOnly) color = albedo * direct / RT_M_PI;
         else color = (mk3(m.emissive[0], m.emissive[1], m.emissive[2]) * m.emissive[3] + albedo * diffuseComponent) + m.reflectivity * spec * fres;
-        write_pixel(L, out0, pitch0, x, y, color, true);
+        write_pixel(L, out0, pitch0, x, y, color, true, np);
+        if (ADAPTIVE) write_moments(ad, image_index(L, x, y), color, np);
     }
 }
 
@@ -922,6 +956,7 @@ static int dispatch_impl(rt_context *ctx, rt_program *prog, uint32_t width, uint
     }
     RT_REQUIRE(!anyAov || prog->kind != RT_PROGRAM_REALTIME, "AOV outputs bound for a realtime program (its outputs already are AOVs)");
     RT_REQUIRE(!anyAov || !ctx->frame.options.showAmbientOcclusionOnly, "AOV outputs bound in the ambient-occlusion debug view");
+    RT_REQUIRE(!ctx->adaptive_counts || prog->kind != RT_PROGRAM_REALTIME, "adaptive sampling bound for a realtime program");
     RT_CUDA(cudaSetDevice(ctx->device));
     const bool realtime = prog->kind == RT_PROGRAM_REALTIME;
     // RayGen early-out: S/ProgressiveRaytracing.hlsl:13-15
@@ -1019,13 +1054,15 @@ static int dispatch_band(rt_context *ctx, rt_program *prog, const Launch &L, con
     unsigned long long *sPrim = ctx->ray_counts + 8, *sSec = ctx->ray_counts + 16, *sShadow = ctx->ray_counts + 24;
     const bool stats = ctx->collect_stats;
     const uint32_t primBlocks = rt_div_up(tiles, kBlock / 32);
-    if (inst) {
-        if (stats) k_primary_inst<true><<<primBlocks, kBlock, 0, st>>>(L, ctx->tlas, ws, ctx->status, sPrim, inst);
-        else k_primary_inst<false><<<primBlocks, kBlock, 0, st>>>(L, ctx->tlas, ws, ctx->status, sPrim, inst);
-    } else {
-        if (stats) k_primary<true><<<primBlocks, kBlock, 0, st>>>(L, ctx->tlas, ws, ctx->status, sPrim);
-        else k_primary<false><<<primBlocks, kBlock, 0, st>>>(L, ctx->tlas, ws, ctx->status, sPrim);
-    }
+    const Adaptive ad{ctx->adaptive_counts, reinterpret_cast<float2 *>(ctx->adaptive_moments)};
+    const bool adaptive = ad.counts != nullptr;
+    // one kernel of each family per (stats, inst, adaptive) combination: pick it once, launch it with the same arguments
+    void (*prim)(Launch, const void *, WS, uint32_t *, unsigned long long *, const uint32_t *) = k_primary<false, false>;
+    void (*primInst)(Launch, const void *, WS, uint32_t *, unsigned long long *, uint32_t *, const uint32_t *) = k_primary_inst<false, false>;
+    if (adaptive) prim = stats ? k_primary<true, true> : k_primary<false, true>, primInst = stats ? k_primary_inst<true, true> : k_primary_inst<false, true>;
+    else if (stats) prim = k_primary<true, false>, primInst = k_primary_inst<true, false>;
+    if (inst) primInst<<<primBlocks, kBlock, 0, st>>>(L, ctx->tlas, ws, ctx->status, sPrim, inst, ad.counts);
+    else prim<<<primBlocks, kBlock, 0, st>>>(L, ctx->tlas, ws, ctx->status, sPrim, ad.counts);
     if (timing) RT_CUDA(cudaEventRecord(ctx->ev[1], st));
     const uint32_t shadeTiles = ((L.rw + kShadeTile - 1) / kShadeTile) * ((L.rh + kShadeTile - 1) / kShadeTile);
     AovOut aov{};
@@ -1036,12 +1073,10 @@ static int dispatch_band(rt_context *ctx, rt_program *prog, const Launch &L, con
     aov.n_motion = ctx->n_motion;
     aov.motion = reinterpret_cast<const float4 *>(ctx->motion);
     aov.inst = inst;
-    if (aov.mask)
-        k_shade_primary<true><<<shadeTiles, kShadeThreads, 0, st>>>(L, ws, prog->dev_recs, prog->n_recs, prog->env_texels, prog->env_size,
-                                                                    ctx->output[0], ctx->pitch[0], ctx->output[1], ctx->pitch[1], ctx->ray_counts, ctx->status, aov);
-    else
-        k_shade_primary<false><<<shadeTiles, kShadeThreads, 0, st>>>(L, ws, prog->dev_recs, prog->n_recs, prog->env_texels, prog->env_size,
-                                                                     ctx->output[0], ctx->pitch[0], ctx->output[1], ctx->pitch[1], ctx->ray_counts, ctx->status, aov);
+    auto shade0 = aov.mask ? (adaptive ? k_shade_primary<true, true> : k_shade_primary<true, false>)
+                           : (adaptive ? k_shade_primary<false, true> : k_shade_primary<false, false>);
+    shade0<<<shadeTiles, kShadeThreads, 0, st>>>(L, ws, prog->dev_recs, prog->n_recs, prog->env_texels, prog->env_size, ctx->output[0], ctx->pitch[0],
+                                                 ctx->output[1], ctx->pitch[1], ctx->ray_counts, ctx->status, aov, ad);
     if (timing) RT_CUDA(cudaEventRecord(ctx->ev[2], st));
     // The depth-0 shadow wave and the secondary-ray chain (trace -> shade -> depth-1 shadow wave) both depend only on
     // k_shade_primary and meet again in k_resolve.  Outside the instrumented / per-stage-timed modes the shadow wave
@@ -1076,8 +1111,8 @@ static int dispatch_band(rt_context *ctx, rt_program *prog, const Launch &L, con
         ctx->launches += 2;
     }
     if (overlap) RT_CUDA(cudaStreamWaitEvent(st, ev_join, 0));
-    if (aov.mask) k_resolve<true><<<qgrid, kBlock, 0, st>>>(L, ws, prog->dev_recs, ctx->output[0], ctx->pitch[0], ctx->output[1], ctx->pitch[1], aov);
-    else k_resolve<false><<<qgrid, kBlock, 0, st>>>(L, ws, prog->dev_recs, ctx->output[0], ctx->pitch[0], ctx->output[1], ctx->pitch[1], aov);
+    auto resolve = aov.mask ? (adaptive ? k_resolve<true, true> : k_resolve<true, false>) : (adaptive ? k_resolve<false, true> : k_resolve<false, false>);
+    resolve<<<qgrid, kBlock, 0, st>>>(L, ws, prog->dev_recs, ctx->output[0], ctx->pitch[0], ctx->output[1], ctx->pitch[1], aov, ad);
     ctx->launches += 7;
     RT_LAUNCH_CHECK();
     if (timing) {

@@ -68,6 +68,9 @@ protected:
     std::vector<DXRFramework::RtBuffer::SharedPtr> mOutputResource;
     std::array<bool, RT_AOV_COUNT> mAovEnabled{};
     std::array<DXRFramework::RtBuffer::SharedPtr, RT_AOV_COUNT> mAovResource;
+    // adaptive sampling (ProgressiveRaytracingPipeline::setAdaptiveSampling): per-pixel counts and moments, null when off;
+    // render() binds them (or unbinds) on every call
+    DXRFramework::RtBuffer::SharedPtr mAdaptiveCounts, mAdaptiveMoments;
     UINT mNumOutputs;
     UINT mOutputWidth = 0, mOutputHeight = 0;  // of the last createOutputResource
     PerFrameConstants mConstantBuffer{};
@@ -102,6 +105,15 @@ public:
     // is valid until the next call.
     DXRFramework::RtBuffer::SharedPtr denoiseTemporal(const rt_temporal_denoise_params &params);
     void resetTemporal() { mHasTemporalHistory = false; }
+    // Adaptive sampling (rt_set_adaptive_sampling): call after createOutputResource.  Allocates zeroed per-pixel sample counts
+    // and luminance moments, which every later render() binds; converged pixels are skipped.  A restart of the accumulation
+    // (a camera move, restartAccumulation, accumulation off) zeroes them, so every pixel is active again.
+    void setAdaptiveSampling(const rt_adaptive_params &params);
+    // rt_adaptive_update with the parameters of setAdaptiveSampling: marks converged pixels and returns how many pixels are
+    // still active (synchronises).
+    UINT adaptiveUpdate();
+    // width x height uint32: n_p in bits 0-30, converged in bit 31 (null unless setAdaptiveSampling was called)
+    DXRFramework::RtBuffer::SharedPtr getSampleCountResource() const { return mAdaptiveCounts; }
 
 private:
     explicit ProgressiveRaytracingPipeline(DXRFramework::RtContext::SharedPtr context);
@@ -116,4 +128,6 @@ private:
     uint64_t mTemporalBytes = 0;
     CameraParams mPrevCamera{};
     bool mHasTemporalHistory = false;
+    rt_adaptive_params mAdaptiveParams = RT_ADAPTIVE_DEFAULTS;
+    DXRFramework::RtBuffer::SharedPtr mAdaptiveActive;  // one uint32: rt_adaptive_update's active count
 };

@@ -170,6 +170,9 @@ void RaytracingPipelineBase::render(UINT /*frameIndex*/, UINT width, UINT height
     // the scene's instance motion for the previous-position AOV; NULL otherwise, so that no earlier binding is inherited
     const float *motion = mAovResource[RT_AOV_PREVIOUS_POSITION] ? mRtScene->getMotionPtr() : nullptr;
     ThrowIfFailed(rt_set_instance_motion(ctx, motion, motion ? mRtScene->getNumInstances() : 0), "rt_set_instance_motion");
+    ThrowIfFailed(rt_set_adaptive_sampling(ctx, mAdaptiveCounts ? static_cast<uint32_t *>(mAdaptiveCounts->ptr()) : nullptr,
+                                           mAdaptiveMoments ? static_cast<float *>(mAdaptiveMoments->ptr()) : nullptr),
+                  "rt_set_adaptive_sampling");
     ThrowIfFailed(rt_set_render_options(ctx, &mRenderOptions), "rt_set_render_options");
 
     if (mBandRow1 > mBandRow0) mRtContext->raytraceRegion(mRtBindings, mRtState, width, height, 0, mBandRow0, width, std::min(mBandRow1, height));
@@ -192,10 +195,32 @@ void ProgressiveRaytracingPipeline::update(float elapsedTime, UINT elapsedFrames
         mAccumCount = 0;
         std::memcpy(mLastCameraVP, vp, sizeof(vp));
         mHasLastCamera = true;
+        if (mAdaptiveCounts) mAdaptiveCounts->clear(), mAdaptiveMoments->clear();  // the running means restart with n_p = 0
     }
     fillCommonConstants(elapsedTime, elapsedFrames, width, height);
     mConstantBuffer.cameraParams.accumCount = mAccumCount++;
     mConstantBuffer.options = mShaderDebugOptions;
+}
+
+void ProgressiveRaytracingPipeline::setAdaptiveSampling(const rt_adaptive_params &params) {
+    ThrowIfFalse(mOutputWidth > 0 && mOutputHeight > 0, "ProgressiveRaytracingPipeline::setAdaptiveSampling needs createOutputResource first");
+    const uint64_t pixels = uint64_t(mOutputWidth) * mOutputHeight;
+    mAdaptiveCounts = mRtContext->createBuffer(4 * pixels);
+    mAdaptiveMoments = mRtContext->createBuffer(8 * pixels);
+    mAdaptiveActive = mRtContext->createBuffer(4);
+    mAdaptiveCounts->clear(), mAdaptiveMoments->clear();
+    mAdaptiveParams = params;
+}
+
+UINT ProgressiveRaytracingPipeline::adaptiveUpdate() {
+    ThrowIfFalse(mAdaptiveCounts != nullptr, "ProgressiveRaytracingPipeline::adaptiveUpdate needs setAdaptiveSampling first");
+    ThrowIfFailed(rt_adaptive_update(mRtContext->getNative(), static_cast<const float *>(mAdaptiveMoments->ptr()),
+                                     static_cast<uint32_t *>(mAdaptiveCounts->ptr()), mOutputWidth, mOutputHeight, &mAdaptiveParams,
+                                     static_cast<uint32_t *>(mAdaptiveActive->ptr())),
+                  "rt_adaptive_update");
+    uint32_t active = 0;
+    mAdaptiveActive->download(&active, sizeof(active));  // synchronises
+    return active;
 }
 
 RtBuffer::SharedPtr ProgressiveRaytracingPipeline::denoise(const rt_progressive_denoise_params &params) {

@@ -11,6 +11,9 @@
 //     normal AOVs as guides (rt_denoise_progressive; the flag enables both AOVs; EXR when the path ends in .exr)
 //   dxr_headless --pipeline progressive ... --orbit 0.5 --spp 16 --denoise-temporal clean.pfm   one sample per frame from a
 //     camera orbiting --at by 0.5 degrees per frame, every frame filtered by rt_denoise_temporal; writes the last frame's output
+//   dxr_headless --pipeline progressive ... --spp 256 --adaptive 0.1 [--adaptive-min 8] [--adaptive-every 4] --sample-counts n.pfm
+//     adaptive sampling: --spp is the per-pixel sample cap; rt_adaptive_update runs every 4 dispatches and the run stops when
+//     no pixel is active; --sample-counts writes each pixel's sample count as a grey heat map
 // Multi-GPU (one process per GPU, replicated scene; the frame's samples and strips are sharded, one NCCL reduce at the end):
 //   for r in 0 1; do dxr_headless ... --spp 64 --world 2 --rank $r --comm-file /tmp/id [--strip-groups 2] --out frame.pfm & done
 #include <chrono>
@@ -83,6 +86,8 @@ static int usage() {
               "             [--orbit DEGREES]   (frame f: the eye rotated about --at around +y by f * DEGREES)\n"
               "             [--move DX DY DZ]   (frame f: instance 0 translated by f * (DX, DY, DZ); the camera stays unless --orbit)\n"
               "             [--denoise-temporal file.pfm|file.exr]   (progressive, one GPU: accumulation off, every frame filtered by rt_denoise_temporal)\n"
+              "             [--adaptive THRESHOLD [--adaptive-min N] [--adaptive-every K] [--sample-counts file.pfm|file.exr]]\n"
+              "                                                                    (progressive, one GPU: --spp is the sample cap)\n"
               "             [--world N --rank R --comm-file path [--strip-groups G] [--strip-rows 32] [--band-shard]]   (one process per GPU)");
     return 0;
 }
@@ -109,6 +114,13 @@ int main(int argc, char **argv) {
         const bool denoiseTemporal = a.has("denoise-temporal");
         if (denoiseTemporal && (pipelineName == "realtime" || world > 1 || a.str("denoise-temporal", "").empty()))
             throw std::runtime_error("--denoise-temporal takes a path and needs --pipeline progressive on one GPU (no --world > 1)");
+        const bool adaptive = a.has("adaptive");
+        if (adaptive && (pipelineName == "realtime" || world > 1 || denoiseTemporal || a.str("adaptive", "").empty()))
+            throw std::runtime_error("--adaptive takes a threshold and needs --pipeline progressive on one GPU, without --denoise-temporal");
+        if (a.has("sample-counts") && (!adaptive || a.str("sample-counts", "").empty()))
+            throw std::runtime_error("--sample-counts takes a path and needs --adaptive");
+        const UINT adaptiveEvery = UINT(a.num("adaptive-every", 4));
+        if (adaptive && (adaptiveEvery < 1 || spp < 1)) throw std::runtime_error("--adaptive-every and --spp must be at least 1");
         auto context = RtContext::create(int(a.num("device", rank)));
         if (a.has("denoise-mock")) {
             // DenoiseCompositor with mock inputs (src/DenoiseCompositor.cpp:52-60 loads DirectLighting.png / IndirectSpecular.png and
@@ -222,6 +234,13 @@ int main(int argc, char **argv) {
         pipeline->loadResources(3);
         pipeline->createOutputResource(DXGI_FORMAT_R16G16B16A16_FLOAT, width, height);
         pipeline->setRenderOptions(UINT(a.num("radiance-depth", 1)), a.has("fp16-targets"));
+        if (adaptive) {  // threshold, floor, min_samples (capped at --spp), max_samples = --spp
+            rt_adaptive_params ap = RT_ADAPTIVE_DEFAULTS;
+            ap.threshold = float(a.num("adaptive", 0.0));
+            ap.min_samples = std::min<uint32_t>(uint32_t(a.num("adaptive-min", ap.min_samples)), spp);
+            ap.max_samples = spp;
+            progressive->setAdaptiveSampling(ap);
+        }
         // --band-shard (realtime pipeline + --denoise, one frame): rank r renders AND filters its row band plus the filter's reach;
         // the reduce composites the filtered bands instead of the AOVs (dxrexperiments_b200/sharding.py band_plan)
         const bool bandShard = a.has("band-shard") && world > 1;
@@ -245,6 +264,7 @@ int main(int argc, char **argv) {
         UINT mySamples = 0;
         const rt_temporal_denoise_params temporalParams = RT_TEMPORAL_DENOISE_DEFAULTS;
         RtBuffer::SharedPtr temporalOut;
+        UINT dispatches = 0;
         for (UINT f = 0; f < spp; ++f) {
             if (a.has("orbit")) {  // the eye rotated about `at` around +y (scenes.orbit)
                 const double ang = double(f) * a.num("orbit", 0.0) * 3.14159265358979323846 / 180.0, c = std::cos(ang), s = std::sin(ang);
@@ -268,7 +288,9 @@ int main(int argc, char **argv) {
             }
             if (frames) frames.write(reinterpret_cast<const char *>(&pipeline->getFrameConstants()), sizeof(PerFrameConstants));
             pipeline->render(f % 3, width, height);
+            ++dispatches;
             if (denoiseTemporal) temporalOut = progressive->denoiseTemporal(temporalParams);
+            if (adaptive && (f + 1) % adaptiveEvery == 0 && progressive->adaptiveUpdate() == 0) break;  // every pixel converged
         }
         // ---- the path's one collective: every output is summed onto rank 0, weighted by the rank's share of the samples
         std::vector<RtBuffer::SharedPtr> finalOut;
@@ -315,6 +337,18 @@ int main(int argc, char **argv) {
             save(clean, a.str("denoise-progressive", ""));
         }
         if (denoiseTemporal && temporalOut) save(temporalOut, a.str("denoise-temporal", ""));
+        if (a.has("sample-counts")) {  // n_p as a grey heat map (the converged bit masked off)
+            std::vector<uint32_t> counts(size_t(width) * height);
+            progressive->getSampleCountResource()->download(counts.data(), counts.size() * sizeof(uint32_t));
+            for (size_t i = 0; i < counts.size(); ++i) {
+                const float n = float(counts[i] & ~RT_ADAPTIVE_CONVERGED);
+                img[4 * i] = img[4 * i + 1] = img[4 * i + 2] = n, img[4 * i + 3] = 1.0f;
+            }
+            const std::string path = a.str("sample-counts", "");
+            const bool exr = path.size() > 4 && path.substr(path.size() - 4) == ".exr";
+            if (!(exr ? ImageIO::writeEXR(path, img.data(), width, height, false) : ImageIO::writePFM(path, img.data(), width, height)))
+                throw std::runtime_error("cannot write " + path);
+        }
         if (bandShard) {
             save(bandFrame, a.str("denoise", ""));
         } else if (a.has("denoise") && rank == 0) {
@@ -332,9 +366,10 @@ int main(int argc, char **argv) {
         const double rays = double(rc.primary + rc.secondary + rc.shadow);
         std::printf("{\"pipeline\": \"%s\", \"triangles\": %u, \"width\": %u, \"height\": %u, \"frames\": %u, \"build_ms\": %.3f, \"render_ms\": %.3f, "
                     "\"rays\": %.0f, \"mrays_per_s\": %.1f, \"kernel_launches\": %llu, \"world\": %d, \"rank\": %d, \"strip_groups\": %u, "
-                    "\"samples_on_rank\": %u, \"core\": \"%s\"}\n",
+                    "\"samples_on_rank\": %u, \"dispatches\": %u, \"primary_rays\": %llu, \"core\": \"%s\"}\n",
                     pipeline->getName(), model->getNumTriangles(), width, height, spp, buildMs, renderMs, rays, rays / (renderMs * 1e3),
-                    (unsigned long long)context->launchCount(), world, rank, stripGroups, mySamples, rt_version());
+                    (unsigned long long)context->launchCount(), world, rank, stripGroups, mySamples, dispatches, (unsigned long long)rc.primary,
+                    rt_version());
     } catch (const std::exception &e) {
         std::fprintf(stderr, "dxr_headless: %s\n", e.what());
         return 1;

@@ -80,6 +80,8 @@ def _load():
         "rt_set_tlas": (i32, [vp, vp]),
         "rt_set_instance_motion": (i32, [vp, vp, u32]),
         "rt_set_render_options": (i32, [vp, vp]),
+        "rt_set_adaptive_sampling": (i32, [vp, vp, vp]),
+        "rt_adaptive_update": (i32, [vp, vp, vp, u32, u32, vp, vp]),
         "rt_dispatch_rays": (i32, [vp, vp, u32, u32, u32]),
         "rt_dispatch_rays_region": (i32, [vp, vp, u32, u32, u32, u32, u32, u32]),
         "rt_get_ray_counts": (i32, [vp, vp, i32]),
@@ -405,6 +407,17 @@ class Context:
         previous-world matrices, one per InstanceIndex(); None with n = 0 unbinds."""
         check(lib.rt_set_instance_motion(self.handle, _ptr(matrices), n))
 
+    def set_adaptive_sampling(self, counts=None, moments=None):
+        """rt_set_adaptive_sampling: `counts` (width*height uint32) and `moments` (width*height*2 float32) are device Buffers
+        (or addresses) that the following progressive dispatches sample adaptively with; None, None unbinds."""
+        check(lib.rt_set_adaptive_sampling(self.handle, _ptr(counts), _ptr(moments)))
+
+    def adaptive_update(self, moments, counts, width: int, height: int, params: T.AdaptiveParams = None, active_count=None):
+        """rt_adaptive_update on device buffers: marks converged pixels in `counts`; `active_count` (a device Buffer or
+        address of one uint32, or None) receives the number of pixels still active.  Stream-ordered, no synchronisation."""
+        params = T.adaptive_defaults() if params is None else params
+        check(lib.rt_adaptive_update(self.handle, _ptr(moments), _ptr(counts), width, height, C.byref(params), _ptr(active_count)))
+
     def ray_counts(self, reset=False) -> T.RayCounts:
         c = T.RayCounts()
         check(lib.rt_get_ray_counts(self.handle, C.byref(c), 1 if reset else 0))
@@ -670,7 +683,7 @@ class Renderer:
     """Convenience host for tests/bench: one scene (instances of meshes), one program, fp32 outputs on the device."""
 
     def __init__(self, ctx: Context, meshes, transforms, materials, env_texels, kind=PROGRESSIVE, width=256, height=256,
-                 outputs=None, instance_mesh=None, build_flags: int = 0, aovs=()):
+                 outputs=None, instance_mesh=None, build_flags: int = 0, aovs=(), adaptive: bool = False):
         """outputs: optional list of caller-owned device buffers (anything with .ptr, e.g. a wrapped torch tensor)
         of width*height RGBA fp32, one per output slot; allocated here when omitted.
         instance_mesh: optional list, one mesh index per transform (instancing: many instances of few BLASes);
@@ -678,7 +691,9 @@ class Renderer:
         aovs: names from types.AOV_NAMES, types.AOV_POSITION_NAME or types.AOV_PREVIOUS_POSITION_NAME (progressive program
         only): each gets a zeroed
         width*height RGBA fp32 buffer that every dispatch accumulates next to the beauty output (rt_set_aov_output); read it
-        back with aov(name)."""
+        back with aov(name).
+        adaptive: sample adaptively (rt_set_adaptive_sampling, progressive program only): zeroed per-pixel sample counts and
+        luminance moments that every dispatch binds; adaptive_update() marks converged pixels, which later dispatches skip."""
         self.ctx, self.width, self.height, self.kind = ctx, width, height, kind
         self.blases = [ctx.build_blas_from_mesh(m, build_flags=build_flags) for m in meshes]  # 0 = the application's flags (RtModel.cpp:86-118)
         if instance_mesh is None:
@@ -701,6 +716,11 @@ class Renderer:
         if unknown:
             raise ValueError(f"unknown AOV names {unknown}; known: {tuple(_AOV_IDS)}")
         self.aovs = {a: ctx.alloc(16 * width * height).zero() for a in aovs}
+        if adaptive and kind != PROGRESSIVE:
+            raise ValueError("adaptive sampling needs the progressive program")
+        self.adaptive = None  # (counts, moments, active count) device buffers
+        if adaptive:
+            self.adaptive = (ctx.alloc(4 * width * height).zero(), ctx.alloc(8 * width * height).zero(), ctx.alloc(4))
         self._denoise_bufs = None  # (tmp, out) of denoise(), allocated on first use
         self._last_camera = None   # cameraParams of the last dispatch
         self.reset_temporal()
@@ -715,6 +735,8 @@ class Renderer:
             check(lib.rt_set_aov_output(self.ctx.handle, k, buf.ptr if buf is not None else None, 16 * self.width if buf is not None else 0))
         # every call, so that motion another Renderer bound on this context is never inherited
         self.ctx.set_instance_motion(self._motion_buf, len(self.instance_mesh) if self._motion_buf is not None else 0)
+        # likewise the adaptive sampling buffers
+        self.ctx.set_adaptive_sampling(*(self.adaptive[:2] if self.adaptive is not None else (None, None)))
         check(lib.rt_set_tlas(self.ctx.handle, self.tlas.result.ptr))
         check(lib.rt_set_frame_constants(self.ctx.handle, C.byref(frame)))
         if strips is not None:
@@ -725,6 +747,36 @@ class Renderer:
             x0, y0, x1, y1 = region
             check(lib.rt_dispatch_rays_region(self.ctx.handle, self.program.handle, self.width, self.height, x0, y0, x1, y1))
         self._last_camera = T.CameraParams.from_buffer_copy(bytes(frame.cameraParams))
+
+    def _need_adaptive(self, what):
+        if self.adaptive is None:
+            raise ValueError(f"{what} needs a Renderer constructed with adaptive=True")
+
+    def adaptive_update(self, params: T.AdaptiveParams = None) -> int:
+        """rt_adaptive_update over the whole image: mark the pixels that have converged under `params` (default
+        types.adaptive_defaults()) and return how many pixels are still active (synchronises)."""
+        self._need_adaptive("adaptive_update()")
+        counts, moments, active = self.adaptive
+        self.ctx.adaptive_update(moments, counts, self.width, self.height, params, active)
+        return int(active.download(np.uint32, 1)[0])
+
+    def sample_counts(self):
+        """(n, converged): the samples accumulated into each pixel as (height, width) uint32 and the converged mask as
+        (height, width) bool."""
+        self._need_adaptive("sample_counts()")
+        c = self.adaptive[0].download(np.uint32).reshape(self.height, self.width)
+        return c & np.uint32(~T.ADAPTIVE_CONVERGED & 0xFFFFFFFF), (c & np.uint32(T.ADAPTIVE_CONVERGED)) != 0
+
+    def moments(self) -> np.ndarray:
+        """The running luminance moments (m1, m2) of every pixel as (height, width, 2) float32."""
+        self._need_adaptive("moments()")
+        return self.adaptive[1].download(np.float32).reshape(self.height, self.width, 2)
+
+    def reset_adaptive(self):
+        """Start over: zero the sample counts (every pixel active again), the moments, the outputs and the AOVs."""
+        self._need_adaptive("reset_adaptive()")
+        for b in (*self.adaptive[:2], *self.out, *self.aovs.values()):
+            b.zero()
 
     def set_transforms(self, transforms):
         """Move the instances: rebuild the TLAS with `transforms` (one object->world 3x4 per instance, as the constructor
@@ -794,6 +846,8 @@ class Renderer:
         so that instances moved by set_transforms() keep their history."""
         if self.kind != PROGRESSIVE or any(a not in self.aovs for a in ("albedo", "normal", T.AOV_POSITION_NAME)):
             raise ValueError('denoise_temporal() needs a progressive Renderer with the "albedo", "normal" and "position" AOVs')
+        if self.adaptive is not None:
+            raise ValueError("denoise_temporal() filters frames of one sample, which adaptive sampling does not make")
         if self._last_camera is None or self._last_camera.accumCount != 0:
             raise ValueError("denoise_temporal() filters frames of one sample: the last dispatch must have accumCount 0")
         if self._temporal is None:

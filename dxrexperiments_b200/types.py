@@ -69,6 +69,20 @@ def temporal_denoise_defaults() -> TemporalDenoiseParams:
     return TemporalDenoiseParams(progressive_denoise_defaults(), 0.2, 0.2, 0.9, 0.02)
 
 
+class AdaptiveParams(C.Structure):  # rt_adaptive_params (include/rt_types.h)
+    _fields_ = [("threshold", C.c_float), ("floor", C.c_float), ("min_samples", C.c_uint32), ("max_samples", C.c_uint32)]
+
+
+def adaptive_defaults() -> AdaptiveParams:
+    """RT_ADAPTIVE_DEFAULTS (include/rt_types.h): the parameters rt_adaptive_update is used with unless told otherwise
+    (DESIGN.md 4.6 records how they were chosen)."""
+    return AdaptiveParams(0.1, 0.1, 8, 1024)
+
+
+# bit 31 of an adaptive sample count (RT_ADAPTIVE_CONVERGED): the pixel has converged and dispatches skip it
+ADAPTIVE_CONVERGED = 0x80000000
+
+
 class GeometryDesc(C.Structure):
     _fields_ = [("vertex_buffer", C.c_void_p), ("vertex_count", C.c_uint32), ("vertex_stride_bytes", C.c_uint32),
                 ("index_buffer", C.c_void_p), ("index_count", C.c_uint32), ("index_format", C.c_uint32),
@@ -111,6 +125,7 @@ assert C.sizeof(MaterialParams) == 64
 assert C.sizeof(DenoiserParams) == 24
 assert C.sizeof(ProgressiveDenoiseParams) == 16
 assert C.sizeof(TemporalDenoiseParams) == 32
+assert C.sizeof(AdaptiveParams) == 16
 assert C.sizeof(InstanceDesc) == 64
 assert C.sizeof(HitRecord) == 80
 assert C.sizeof(GeometryDesc) == 48

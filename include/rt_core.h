@@ -228,6 +228,36 @@ int rt_set_aov_output(rt_context *ctx, uint32_t aov, float *rgba, uint64_t pitch
  * n = 0, a pointer not 16-byte aligned, n > 2^24 - 1.  Only rigid (per-instance) motion is described: a deforming mesh's
  * moved vertices are not, and such pixels lose their history through the position test. */
 int rt_set_instance_motion(rt_context *ctx, const float *world_to_previous_world, uint32_t n);
+/* Adaptive sampling of the progressive program (new work: the reference has no counterpart; it accumulates every pixel
+ * with the one global accumCount).  counts is a DEVICE array of width x height uint32 in image order (y * width + x):
+ * bits 0-30 hold n_p, the samples accumulated into pixel p, and bit 31 (RT_ADAPTIVE_CONVERGED) marks p converged.
+ * moments is a DEVICE array of width x height (m1, m2) fp32 pairs: the running means of L and L*L, with
+ * L = (r*0.299f + g*0.587f) + b*0.114f of the sample written to gOutput after its clamp at 0 (whatever gOutput shows:
+ * the beauty frame, a debug view or the ambient-occlusion view).  moments stays fp32 under half_render_targets (L*L
+ * overflows fp16 beyond L = 256).  Context state like rt_set_instance_motion: the caller keeps both arrays alive until
+ * the dispatches that use them are done.  NULL, NULL unbinds.  RT_ERR_INVALID_ARG: exactly one of the two NULL, counts
+ * not 4-byte or moments not 8-byte aligned, and (at dispatch) a realtime program dispatched while they are bound.
+ * While bound, every progressive dispatch (region, interleaved, multi-band, instrumented, debug capture) does this:
+ *   a pixel of the launch with bit 31 set is skipped: it traces no ray, is not counted by rt_get_ray_counts, takes no
+ *     hit slot, and writes nothing to gOutput, an AOV, counts or moments;
+ *   every other pixel is sampled exactly as without the binding, except that every running mean (gOutput, the AOVs and
+ *     the moments) uses n_p in place of accumCount: v' = (n_p*v + s) / (n_p + 1); the pixel then stores n_p + 1.
+ * accumCount keeps its other two roles: the maxIterations early-out and (on the host) the jitter sequence.  So with
+ * counts starting at 0 and no rt_adaptive_update, dispatch k writes exactly what the unbound pipeline writes with
+ * accumCount = k, bit for bit, in every output and AOV. */
+int rt_set_adaptive_sampling(rt_context *ctx, uint32_t *counts, float *moments);
+/* Marks converged pixels: sets bit 31 of counts[p] (never clears it, so the active set only shrinks) when
+ *   n_p >= max_samples, or
+ *   n_p >= min_samples and e_q <= threshold for every q of p's 3 x 3 window inside the image (Cycles' one-pixel
+ *   dilation: an unconverged neighbour keeps p active),
+ * with n = counts & 0x7FFFFFFF, sigma_p = sqrtf(fmaxf(0, m2 - m1*m1) / float(n_p - 1)) for n_p >= 2 (+inf below),
+ * e_p = sigma_p / (m1 + floor).  A NaN error never passes.  active_count (DEVICE, may be NULL) receives the number of
+ * pixels without bit 31 after the update.  At most two operations (a memset and a kernel) on the context's stream, no
+ * host synchronisation.  A host may also set or clear bit 31 itself, e.g. to freeze or reopen a region.
+ * RT_ERR_INVALID_ARG: a null moments / counts / params, an empty image, counts or active_count not 4-byte or moments not
+ * 8-byte aligned, parameters out of range (rt_types.h), or counts / active_count overlapping moments or each other. */
+int rt_adaptive_update(rt_context *ctx, const float *moments, uint32_t *counts, uint32_t width, uint32_t height,
+                       const rt_adaptive_params *params, uint32_t *active_count);
 int rt_set_tlas(rt_context *ctx, const void *tlas_result);
 /* Two things that are constants of the reference and options here (defaults = the reference's shaders / this library's
  * declared fp32 deviation):
@@ -279,7 +309,9 @@ int rt_get_stage_timing(rt_context *ctx, double *primary_ms, double *secondary_m
  * 2-3 ambient-occlusion debug view).  There is no reference counterpart (the Fallback Layer keeps this state in
  * registers of its uber shader, FL/TraverseShader.hlsli:21-73); the oracle re-traces the downloaded rays. */
 typedef enum rt_debug_array {
-    RT_DEBUG_PRIMARY_HITS = 0,       /* pixels x {float t, u, v; uint32 PrimitiveIndex (0xFFFFFFFF = miss)}, pixel order of the dispatch */
+    RT_DEBUG_PRIMARY_HITS = 0,       /* pixels x {float t, u, v; uint32 PrimitiveIndex (0xFFFFFFFF = miss)}, pixel order of the dispatch;
+                                        under adaptive sampling a skipped (converged) pixel traces nothing and its entry here and
+                                        in RT_DEBUG_PRIMARY_RECORDS keeps whatever an earlier dispatch left */
     RT_DEBUG_PRIMARY_RECORDS = 1,    /* pixels x uint32 hit-group record index (InstanceContribution + ray type) */
     RT_DEBUG_SLOT_INFO = 2,          /* hit_slots x {uint32 pixel, record, flags, 0} */
     RT_DEBUG_SECONDARY_RAYS = 3,     /* hit_slots x rt_ray per plane; tmax < 0 marks an inactive slot */

@@ -111,6 +111,18 @@ typedef struct rt_temporal_denoise_params {
 /* Defaults, chosen on the CPU restatement of the filter (DESIGN.md 4.4.2). */
 #define RT_TEMPORAL_DENOISE_DEFAULTS {RT_PROGRESSIVE_DENOISE_DEFAULTS, 0.2f, 0.2f, 0.9f, 0.02f}
 
+/* rt_adaptive_update (rt_core.h); new work, no reference counterpart. */
+typedef struct rt_adaptive_params {
+    float threshold;      /* >= 0, finite: a pixel may converge once its relative standard error is at most this */
+    float floor;          /* > 0, finite: added to the mean luminance in the relative error's denominator */
+    uint32_t min_samples; /* >= 1: no pixel converges on its error with fewer samples */
+    uint32_t max_samples; /* min_samples .. 2^31 - 1: every pixel converges at this many samples */
+} rt_adaptive_params; /* 16 B */
+/* Defaults, chosen on the CPU restatement of the rule (DESIGN.md 4.6). */
+#define RT_ADAPTIVE_DEFAULTS {0.1f, 0.1f, 8u, 1024u}
+/* Bit 31 of a sample count: the pixel has converged and dispatches skip it. */
+#define RT_ADAPTIVE_CONVERGED 0x80000000u
+
 /* Interleaved vertex the hit shaders read: libs/DXRFramework/RtModel.cpp:13-17 (stride 24). */
 typedef struct rt_vertex {
     float position[3];
