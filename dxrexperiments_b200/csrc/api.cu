@@ -270,6 +270,15 @@ int rt_set_instance_motion(rt_context *ctx, const float *world_to_previous_world
     ctx->n_motion = n;
     return RT_OK;
 }
+int rt_set_instance_deformation(rt_context *ctx, const rt_deformation_desc *descs, uint32_t n) {
+    RT_REQUIRE(ctx != nullptr, "ctx");
+    RT_REQUIRE((descs == nullptr) == (n == 0), "deformation descriptors: NULL with n = 0, or a pointer with n > 0");
+    RT_REQUIRE((uintptr_t(descs) & 15) == 0, "deformation descriptors must be 16-byte aligned");
+    RT_REQUIRE(n <= 0xFFFFFFu, "more than 2^24 - 1 deformation descriptors (InstanceIndex is 24 bits)");
+    ctx->deform = descs;
+    ctx->n_deform = n;
+    return RT_OK;
+}
 int rt_set_adaptive_sampling(rt_context *ctx, uint32_t *counts, float *moments) {
     RT_REQUIRE(ctx != nullptr, "ctx");
     RT_REQUIRE((counts == nullptr) == (moments == nullptr), "counts and moments are both given or both NULL");

@@ -63,6 +63,8 @@ struct rt_context {
     uint64_t aov_pitch[RT_AOV_COUNT] = {};
     const float *motion = nullptr;  // rt_set_instance_motion: n_motion row-major 3x4 world -> previous-world matrices (device)
     uint32_t n_motion = 0;
+    const rt_deformation_desc *deform = nullptr;  // rt_set_instance_deformation: n_deform descriptors (device)
+    uint32_t n_deform = 0;
     uint32_t *adaptive_counts = nullptr;  // rt_set_adaptive_sampling: width x height n_p | converged << 31 (device), nullptr = unbound
     float *adaptive_moments = nullptr;    // width x height (m1, m2) fp32 (device)
     const void *tlas = nullptr;
@@ -88,6 +90,8 @@ struct rt_context {
     double t_primary = 0, t_secondary = 0, t_shadow = 0;
     uint64_t n_secondary_timed = 0;
 };
+
+static_assert(sizeof(rt_deformation_desc) == 64, "rt_deformation_desc is four 16-byte loads");
 
 struct rt_hit_record_dev {  // device copy of rt_hit_record
     const float *vb;        // rt_vertex[] viewed as floats (stride 6)

@@ -251,16 +251,45 @@ struct AovOut {
     uint32_t n_motion;      // rt_set_instance_motion: matrices bound (0: none)
     const float4 *motion;   // 3 rows of (m0, m1, m2, m3) per instance
     const uint32_t *inst;   // [P] InstanceIndex() of each pixel's primary hit (k_primary_inst), previous-position AOV only
+    const rt_deformation_desc *deform;  // rt_set_instance_deformation: n_deform descriptors (0: none)
+    uint32_t n_deform;
 };
 
-// P' of the previous-position AOV for the primary hit P of workspace pixel p (include/rt_core.h states the rule).
-__device__ __forceinline__ f3 previous_position(const AovOut &a, uint32_t p, f3 P) {
+// P' of the previous-position AOV for the primary hit P of workspace pixel p on primitive prim of record R at
+// barycentrics (bu, bv) (include/rt_core.h states the rule).
+__device__ __forceinline__ f3 previous_position(const AovOut &a, uint32_t p, f3 P, const rt_hit_record_dev &R, uint32_t prim, float bu,
+                                                float bv, uint32_t *status) {
     const uint32_t i = a.inst[p];
-    if (i >= a.n_motion) return P;
-    const float4 *m = a.motion + 3 * size_t(i);
+    if (i < a.n_motion) {
+        const float4 *m = a.motion + 3 * size_t(i);
+        const float4 r0 = __ldg(m), r1 = __ldg(m + 1), r2 = __ldg(m + 2);
+        P = mk3(((r0.x * P.x + r0.y * P.y) + r0.z * P.z) + r0.w, ((r1.x * P.x + r1.y * P.y) + r1.z * P.z) + r1.w,
+                ((r2.x * P.x + r2.y * P.y) + r2.z * P.z) + r2.w);
+    }
+    if (i >= a.n_deform) return P;
+    // the descriptor as four 16-byte loads: {pointer, stride_bytes, vertex_count}, then the three rows of the 3x4
+    const uint4 *q = reinterpret_cast<const uint4 *>(a.deform + i);
+    const uint4 h = __ldg(q);
+    const float *prev = reinterpret_cast<const float *>(uint64_t(h.x) | (uint64_t(h.y) << 32));
+    if (prev == nullptr) return P;
+    const uint32_t *idx = R.ib + size_t(prim) * 3;
+    const uint32_t i0 = __ldg(idx), i1 = __ldg(idx + 1), i2 = __ldg(idx + 2);
+    if (h.z < 12u || (h.z & 3u) || i0 >= h.w || i1 >= h.w || i2 >= h.w) {
+        atomicOr(status, 8u);  // rt_get_status -> RT_ERR_INVALID_ARG, as for a missing hit record
+        return P;
+    }
+    const size_t s = h.z / 4u;
+    const float *q0 = prev + i0 * s, *q1 = prev + i1 * s, *q2 = prev + i2 * s;
+    const float *v0 = R.vb + size_t(i0) * 6, *v1 = R.vb + size_t(i1) * 6, *v2 = R.vb + size_t(i2) * 6;
+    const f3 d0 = mk3(__ldg(q0) - __ldg(v0), __ldg(q0 + 1) - __ldg(v0 + 1), __ldg(q0 + 2) - __ldg(v0 + 2));
+    const f3 d1 = mk3(__ldg(q1) - __ldg(v1), __ldg(q1 + 1) - __ldg(v1 + 1), __ldg(q1 + 2) - __ldg(v1 + 2));
+    const f3 d2 = mk3(__ldg(q2) - __ldg(v2), __ldg(q2 + 1) - __ldg(v2 + 1), __ldg(q2 + 2) - __ldg(v2 + 2));
+    const float b0 = 1.f - bu - bv, b1 = bu, b2 = bv;
+    const f3 D = (d0 * b0 + d1 * b1) + d2 * b2;
+    const float4 *m = reinterpret_cast<const float4 *>(q + 1);
     const float4 r0 = __ldg(m), r1 = __ldg(m + 1), r2 = __ldg(m + 2);
-    return mk3(((r0.x * P.x + r0.y * P.y) + r0.z * P.z) + r0.w, ((r1.x * P.x + r1.y * P.y) + r1.z * P.z) + r1.w,
-               ((r2.x * P.x + r2.y * P.y) + r2.z * P.z) + r2.w);
+    return mk3(P.x + ((r0.x * D.x + r0.y * D.y) + r0.z * D.z), P.y + ((r1.x * D.x + r1.y * D.y) + r1.z * D.z),
+               P.z + ((r2.x * D.x + r2.y * D.y) + r2.z * D.z));
 }
 
 // AOVs 0-4 accumulate exactly as the beauty frame does, so each one equals the matching debug view bit for bit.
@@ -388,7 +417,7 @@ __global__ void __launch_bounds__(kShadeThreads) k_shade_primary(const __grid_co
         pos = o + hA.x * d;  // HitWorldPosition
         if (AOV) write_geometry_aov(L, aov, RT_AOV_POSITION, x, y, pos, 1.0f, n);
         if (AOV && (aov.mask & (1u << RT_AOV_PREVIOUS_POSITION)))
-            write_geometry_aov(L, aov, RT_AOV_PREVIOUS_POSITION, x, y, previous_position(aov, p, pos), 1.0f, n);
+            write_geometry_aov(L, aov, RT_AOV_PREVIOUS_POSITION, x, y, previous_position(aov, p, pos, R, prim, hA.y, hA.z, status), 1.0f, n);
         const rt_debug_options &opt = L.f.options;
         if (!L.realtime && opt.showAmbientOcclusionOnly) {
             // evaluateAO: S/RaytracingCommon.hlsli:98-124 — 4 shadow rays, tMax 10
@@ -1073,6 +1102,8 @@ static int dispatch_band(rt_context *ctx, rt_program *prog, const Launch &L, con
     aov.n_motion = ctx->n_motion;
     aov.motion = reinterpret_cast<const float4 *>(ctx->motion);
     aov.inst = inst;
+    aov.deform = ctx->deform;
+    aov.n_deform = ctx->n_deform;
     auto shade0 = aov.mask ? (adaptive ? k_shade_primary<true, true> : k_shade_primary<true, false>)
                            : (adaptive ? k_shade_primary<false, true> : k_shade_primary<false, false>);
     shade0<<<shadeTiles, kShadeThreads, 0, st>>>(L, ws, prog->dev_recs, prog->n_recs, prog->env_texels, prog->env_size, ctx->output[0], ctx->pitch[0],

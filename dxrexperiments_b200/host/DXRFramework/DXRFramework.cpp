@@ -221,6 +221,7 @@ RtModel::RtModel(RtContext::SharedPtr context, std::vector<Vertex> vertices, std
     mHasIndexBuffer = !indices.empty();
     ThrowIfFalse(mNumVertices > 0, "RtModel: empty vertex buffer");
     mVertexBuffer = context->createBuffer(vertices.data(), vertices.size() * sizeof(Vertex));
+    mVertices = std::move(vertices);
     if (mHasIndexBuffer) mIndexBuffer = context->createBuffer(indices.data(), indices.size() * sizeof(uint32_t));
     else {  // the hit shaders always read an index buffer (Load3x32BitIndices): synthesise 0,1,2,...
         std::vector<uint32_t> iota(mNumVertices);
@@ -245,8 +246,8 @@ RtModel::SharedPtr RtModel::createProcedural(RtContext::SharedPtr context, const
     return m;
 }
 
-void RtModel::build(RtContext::SharedPtr context) {
-    // blasGenerator.AddVertexBuffer(VB, 0, nVerts, sizeof(Vertex), IB, 0, nTris*3, R32_UINT, nullptr, 0), opaque, no update
+rt_geometry_desc RtModel::geometryDesc() const {
+    // blasGenerator.AddVertexBuffer(VB, 0, nVerts, sizeof(Vertex), IB, 0, nTris*3, R32_UINT, nullptr, 0), opaque
     rt_geometry_desc g{};
     g.vertex_buffer = mVertexBuffer->ptr();
     g.vertex_count = mNumVertices;
@@ -260,15 +261,38 @@ void RtModel::build(RtContext::SharedPtr context) {
     }
     g.transform3x4 = nullptr;
     g.flags = mOpaque ? RT_GEOMETRY_FLAG_OPAQUE : RT_GEOMETRY_FLAG_NONE;
+    return g;
+}
+
+void RtModel::build(RtContext::SharedPtr context) {
+    const rt_geometry_desc g = geometryDesc();
+    const uint32_t flags = mDynamic ? RT_BUILD_FLAG_ALLOW_UPDATE : RT_BUILD_FLAG_NONE;  // the reference: no update
     rt_prebuild_info info{};
-    ThrowIfFailed(rt_blas_prebuild(context->getNative(), &g, 1, RT_BUILD_FLAG_NONE, &info), "rt_blas_prebuild");
+    ThrowIfFailed(rt_blas_prebuild(context->getNative(), &g, 1, flags, &info), "rt_blas_prebuild");
     auto scratch = context->createBuffer(info.scratch_bytes);
     mBlasBuffer = context->createBuffer(info.result_bytes);
-    ThrowIfFailed(rt_blas_build(context->getNative(), &g, 1, RT_BUILD_FLAG_NONE, scratch->ptr(), scratch->size(), mBlasBuffer->ptr(),
+    ThrowIfFailed(rt_blas_build(context->getNative(), &g, 1, flags, scratch->ptr(), scratch->size(), mBlasBuffer->ptr(),
                                 mBlasBuffer->size()), "rt_blas_build");
     context->waitForGpu();  // scratch goes out of scope, as after WaitForGpu in the reference
     mVertexBufferSrvHandle = context->createBufferSRVHandle(mVertexBuffer);
     mIndexBufferSrvHandle = context->createBufferSRVHandle(mIndexBuffer);
+}
+
+void RtModel::setVertices(RtContext::SharedPtr context, const std::vector<Vertex> &vertices) {
+    ThrowIfFalse(mDynamic && !mProcedural && mBlasBuffer, "RtModel::setVertices needs a triangle model built after setDynamic(true)");
+    ThrowIfFalse(vertices.size() == mVertices.size(), "RtModel::setVertices: the vertex count must not change");
+    const uint64_t bytes = mVertices.size() * sizeof(Vertex);
+    if (!mPrevPositions) mPrevPositions = context->createBuffer(bytes);
+    mPrevPositions->upload(mVertices.data(), bytes);
+    mVertexBuffer->upload(vertices.data(), bytes);
+    mVertices = vertices;
+    const rt_geometry_desc g = geometryDesc();
+    rt_prebuild_info info{};
+    ThrowIfFailed(rt_blas_prebuild(context->getNative(), &g, 1, RT_BUILD_FLAG_ALLOW_UPDATE, &info), "rt_blas_prebuild");
+    auto scratch = context->createBuffer(std::max<uint64_t>(info.update_scratch_bytes ? info.update_scratch_bytes : info.scratch_bytes, 16));
+    ThrowIfFailed(rt_blas_build(context->getNative(), &g, 1, RT_BUILD_FLAG_ALLOW_UPDATE | RT_BUILD_FLAG_PERFORM_UPDATE, scratch->ptr(),
+                                scratch->size(), mBlasBuffer->ptr(), mBlasBuffer->size()), "rt_blas_build (update)");
+    context->waitForGpu();
 }
 
 // ============================================================================================ RtScene
@@ -311,6 +335,24 @@ void RtScene::update(RtContext::SharedPtr context) {
     }
     if (!mMotionBuffer) mMotionBuffer = context->createBuffer(motion.data(), motion.size() * sizeof(float));
     else mMotionBuffer->upload(motion.data(), motion.size() * sizeof(float));
+    // deforming models: their previous positions and the transforms before this update (rt_set_instance_deformation)
+    std::vector<rt_deformation_desc> deform(std::max<size_t>(n, 1));
+    bool deforming = false;
+    for (size_t i = 0; i < n; ++i) {
+        const RtModel &m = *mInstances[i].model;
+        rt_deformation_desc &d = deform[i];
+        std::memset(&d, 0, sizeof(d));
+        d.previous_positions = m.getPreviousPositionsPtr();
+        d.stride_bytes = sizeof(Vertex);
+        d.vertex_count = m.mNumVertices;
+        double p[12];
+        affine3x4(mBuiltTransforms[i], p);
+        for (int k = 0; k < 12; ++k) d.object_to_previous_world[k] = float(p[k]);
+        deforming = deforming || d.previous_positions;
+    }
+    if (!deforming) mDeformBuffer.reset();
+    else if (!mDeformBuffer) mDeformBuffer = context->createBuffer(deform.data(), deform.size() * sizeof(rt_deformation_desc));
+    else mDeformBuffer->upload(deform.data(), deform.size() * sizeof(rt_deformation_desc));
     buildTlas(context, true);
 }
 

@@ -39,6 +39,17 @@ public:
     UINT getNumTriangles() const { return mNumTriangles; }
     RtBuffer::SharedPtr getBlasBuffer() const { return mBlasBuffer; }
 
+    // Deforming meshes (new work: the reference's models are static).  setDynamic(true) before the scene is built selects
+    // RT_BUILD_FLAG_ALLOW_UPDATE for the BLAS (the default stays RT_BUILD_FLAG_NONE).  setVertices replaces every vertex
+    // (same count and order) in the vertex buffer the hit records point to, refits the BLAS in place (PERFORM_UPDATE) and
+    // makes the vertices from before the call the previous positions that RtScene::update describes for
+    // rt_set_instance_deformation.  Call it once per frame, then RtScene::update, which refits the TLAS.
+    void setDynamic(bool dynamic) { mDynamic = dynamic; }
+    void setVertices(RtContext::SharedPtr context, const std::vector<Vertex> &vertices);
+    const std::vector<Vertex> &getVertices() const { return mVertices; }  // the host copy of the current vertices
+    // the device copy of the vertices before the last setVertices (stride sizeof(Vertex)), nullptr before the first
+    const float *getPreviousPositionsPtr() const { return mPrevPositions ? static_cast<const float *>(mPrevPositions->ptr()) : nullptr; }
+
     // Parses an OBJ file into the interleaved layout; returns false if the file cannot be read.
     static bool loadObj(const std::string &path, std::vector<Vertex> &vertices, std::vector<uint32_t> &indices);
     // The reference's loader (RtModel.cpp:26-58): Assimp import with Triangulate | GenSmoothNormals | FlipUVs |
@@ -52,10 +63,12 @@ private:
     void build(RtContext::SharedPtr context);  // RtModel.cpp:86-118
 
     bool mHasIndexBuffer = false;
-    bool mProcedural = false, mOpaque = true;
+    bool mProcedural = false, mOpaque = true, mDynamic = false;
+    std::vector<Vertex> mVertices;
     UINT mNumVertices = 0;
     UINT mNumTriangles = 0;
-    RtBuffer::SharedPtr mVertexBuffer, mIndexBuffer, mBlasBuffer;
+    RtBuffer::SharedPtr mVertexBuffer, mIndexBuffer, mBlasBuffer, mPrevPositions;
+    rt_geometry_desc geometryDesc() const;
     uint64_t mVertexBufferSrvHandle = 0, mIndexBufferSrvHandle = 0;
 };
 

@@ -30,6 +30,12 @@ public:
     void update(RtContext::SharedPtr context);
     // the device array of the motion matrices, nullptr before the first update
     const float *getMotionPtr() const { return mMotionBuffer ? static_cast<const float *>(mMotionBuffer->ptr()) : nullptr; }
+    // update also describes deforming models (RtModel::setVertices): one rt_deformation_desc per instance with its model's
+    // previous positions (NULL for a model that has none) and the row-major 3x4 of the instance's transform before this
+    // update.  The device array, nullptr while no instance has previous positions.
+    const rt_deformation_desc *getDeformationPtr() const {
+        return mDeformBuffer ? static_cast<const rt_deformation_desc *>(mDeformBuffer->ptr()) : nullptr;
+    }
 
 private:
     RtScene() = default;
@@ -40,7 +46,7 @@ private:
     std::vector<Node> mInstances;
     std::vector<DirectX::XMMATRIX> mBuiltTransforms;  // the transforms of the last build or update
     UINT mHitGroupCount = 0;
-    RtBuffer::SharedPtr mTlasBuffer, mMotionBuffer;
+    RtBuffer::SharedPtr mTlasBuffer, mMotionBuffer, mDeformBuffer;
     void buildTlas(RtContext::SharedPtr context, bool performUpdate);
 };
 

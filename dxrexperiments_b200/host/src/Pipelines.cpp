@@ -170,6 +170,9 @@ void RaytracingPipelineBase::render(UINT /*frameIndex*/, UINT width, UINT height
     // the scene's instance motion for the previous-position AOV; NULL otherwise, so that no earlier binding is inherited
     const float *motion = mAovResource[RT_AOV_PREVIOUS_POSITION] ? mRtScene->getMotionPtr() : nullptr;
     ThrowIfFailed(rt_set_instance_motion(ctx, motion, motion ? mRtScene->getNumInstances() : 0), "rt_set_instance_motion");
+    // likewise its deforming models' previous positions (RtScene::update)
+    const rt_deformation_desc *deform = mAovResource[RT_AOV_PREVIOUS_POSITION] ? mRtScene->getDeformationPtr() : nullptr;
+    ThrowIfFailed(rt_set_instance_deformation(ctx, deform, deform ? mRtScene->getNumInstances() : 0), "rt_set_instance_deformation");
     ThrowIfFailed(rt_set_adaptive_sampling(ctx, mAdaptiveCounts ? static_cast<uint32_t *>(mAdaptiveCounts->ptr()) : nullptr,
                                            mAdaptiveMoments ? static_cast<float *>(mAdaptiveMoments->ptr()) : nullptr),
                   "rt_set_adaptive_sampling");

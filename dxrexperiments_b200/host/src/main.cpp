@@ -85,6 +85,8 @@ static int usage() {
               "             [--denoise-progressive file.pfm|file.exr]   (progressive only: the beauty output filtered with the albedo and normal AOVs)\n"
               "             [--orbit DEGREES]   (frame f: the eye rotated about --at around +y by f * DEGREES)\n"
               "             [--move DX DY DZ]   (frame f: instance 0 translated by f * (DX, DY, DZ); the camera stays unless --orbit)\n"
+              "             [--deform DX DY DZ] (frame f: every vertex of model 0 at its rest position + f * (DX, DY, DZ) * h, h its rest\n"
+              "                                  height normalised to [0, 1]: a shear, refitted per frame; progressive pipeline only)\n"
               "             [--denoise-temporal file.pfm|file.exr]   (progressive, one GPU: accumulation off, every frame filtered by rt_denoise_temporal)\n"
               "             [--adaptive THRESHOLD [--adaptive-min N] [--adaptive-every K] [--sample-counts file.pfm|file.exr]]\n"
               "                                                                    (progressive, one GPU: --spp is the sample cap)\n"
@@ -119,6 +121,9 @@ int main(int argc, char **argv) {
             throw std::runtime_error("--adaptive takes a threshold and needs --pipeline progressive on one GPU, without --denoise-temporal");
         if (a.has("sample-counts") && (!adaptive || a.str("sample-counts", "").empty()))
             throw std::runtime_error("--sample-counts takes a path and needs --adaptive");
+        const bool deform = a.has("deform");
+        if (deform && (pipelineName == "realtime" || a.kv.at("deform").size() != 3))
+            throw std::runtime_error("--deform takes DX DY DZ and needs --pipeline progressive (the realtime program has no previous-position AOV)");
         const UINT adaptiveEvery = UINT(a.num("adaptive-every", 4));
         if (adaptive && (adaptiveEvery < 1 || spp < 1)) throw std::runtime_error("--adaptive-every and --spp must be at least 1");
         auto context = RtContext::create(int(a.num("device", rank)));
@@ -168,6 +173,8 @@ int main(int argc, char **argv) {
             model = RtModel::create(context, v, idx);
         } else model = RtModel::create(context, std::string("<none>"));  // the reference's fallback triangle
         scene->addModel(model, DirectX::XMMatrixIdentity());
+        if (deform) model->setDynamic(true);
+        const std::vector<Vertex> restVertices = deform ? model->getVertices() : std::vector<Vertex>();
 
         RaytracingPipeline::Material material{};
         material.params.albedo[0] = 0.95f, material.params.albedo[1] = 0.05f, material.params.albedo[2] = 0.0f, material.params.albedo[3] = 1.0f;
@@ -228,7 +235,7 @@ int main(int argc, char **argv) {
         const auto progressive = std::dynamic_pointer_cast<ProgressiveRaytracingPipeline>(pipeline);
         if (denoiseTemporal) {
             pipeline->enableAov(RT_AOV_ALBEDO), pipeline->enableAov(RT_AOV_NORMAL), pipeline->enableAov(RT_AOV_POSITION);
-            if (a.has("move")) pipeline->enableAov(RT_AOV_PREVIOUS_POSITION);  // moving instances: the motion variant
+            if (a.has("move") || deform) pipeline->enableAov(RT_AOV_PREVIOUS_POSITION);  // moving instances or a deforming model: the motion variant
             progressive->mFrameAccumulationEnabled = false;
         }
         pipeline->loadResources(3);
@@ -271,11 +278,21 @@ int main(int argc, char **argv) {
                 const double dx = double(eye.x) - at.x, dz = double(eye.z) - at.z;
                 camera->SetEyeAtUp({float(at.x + c * dx + s * dz), eye.y, float(at.z - s * dx + c * dz)}, at, {0, 1, 0});
             }
-            if (a.has("move") && f > 0) {  // instance 0 at f * (DX, DY, DZ): a TLAS refit, and the motion since frame f - 1
+            if (deform && f > 0) {  // model 0 sheared by f * (DX, DY, DZ) (scenes.sheared_positions): a BLAS refit
+                float lo = restVertices[0].position.y, hi = lo;
+                for (const Vertex &v : restVertices) lo = std::min(lo, v.position.y), hi = std::max(hi, v.position.y);
+                const double off[3] = {double(f) * a.num("deform", 0.0, 0), double(f) * a.num("deform", 0.0, 1), double(f) * a.num("deform", 0.0, 2)};
+                std::vector<Vertex> v = restVertices;
+                for (Vertex &x : v) {
+                    const double h = hi > lo ? (double(x.position.y) - lo) / (double(hi) - lo) : 0.0;
+                    x.position = {float(x.position.x + h * off[0]), float(x.position.y + h * off[1]), float(x.position.z + h * off[2])};
+                }
+                model->setVertices(context, v);
+            }
+            if (a.has("move") && f > 0)  // instance 0 at f * (DX, DY, DZ)
                 scene->setTransform(0, DirectX::XMMatrixTranslation(float(f * a.num("move", 0.0, 0)), float(f * a.num("move", 0.0, 1)),
                                                                     float(f * a.num("move", 0.0, 2))));
-                scene->update(context);
-            }
+            if ((a.has("move") || deform) && f > 0) scene->update(context);  // a TLAS refit, and the motion since frame f - 1
             if (!bandShard && f % sampleGroups != sampleGroup) {  // another sample group's frame: keep the jitter sequence in step
                 pipeline->skipFrame();
                 continue;

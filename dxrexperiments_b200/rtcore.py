@@ -79,6 +79,7 @@ def _load():
         "rt_set_aov_output": (i32, [vp, u32, vp, u64]),
         "rt_set_tlas": (i32, [vp, vp]),
         "rt_set_instance_motion": (i32, [vp, vp, u32]),
+        "rt_set_instance_deformation": (i32, [vp, vp, u32]),
         "rt_set_render_options": (i32, [vp, vp]),
         "rt_set_adaptive_sampling": (i32, [vp, vp, vp]),
         "rt_adaptive_update": (i32, [vp, vp, vp, u32, u32, vp, vp]),
@@ -407,6 +408,11 @@ class Context:
         previous-world matrices, one per InstanceIndex(); None with n = 0 unbinds."""
         check(lib.rt_set_instance_motion(self.handle, _ptr(matrices), n))
 
+    def set_instance_deformation(self, descs=None, n: int = 0):
+        """rt_set_instance_deformation: `descs` is a device Buffer (or address) of n types.DeformationDesc, one per
+        InstanceIndex(); None with n = 0 unbinds."""
+        check(lib.rt_set_instance_deformation(self.handle, _ptr(descs), n))
+
     def set_adaptive_sampling(self, counts=None, moments=None):
         """rt_set_adaptive_sampling: `counts` (width*height uint32) and `moments` (width*height*2 float32) are device Buffers
         (or addresses) that the following progressive dispatches sample adaptively with; None, None unbinds."""
@@ -683,7 +689,7 @@ class Renderer:
     """Convenience host for tests/bench: one scene (instances of meshes), one program, fp32 outputs on the device."""
 
     def __init__(self, ctx: Context, meshes, transforms, materials, env_texels, kind=PROGRESSIVE, width=256, height=256,
-                 outputs=None, instance_mesh=None, build_flags: int = 0, aovs=(), adaptive: bool = False):
+                 outputs=None, instance_mesh=None, build_flags: int = 0, aovs=(), adaptive: bool = False, deforming=()):
         """outputs: optional list of caller-owned device buffers (anything with .ptr, e.g. a wrapped torch tensor)
         of width*height RGBA fp32, one per output slot; allocated here when omitted.
         instance_mesh: optional list, one mesh index per transform (instancing: many instances of few BLASes);
@@ -693,9 +699,16 @@ class Renderer:
         width*height RGBA fp32 buffer that every dispatch accumulates next to the beauty output (rt_set_aov_output); read it
         back with aov(name).
         adaptive: sample adaptively (rt_set_adaptive_sampling, progressive program only): zeroed per-pixel sample counts and
-        luminance moments that every dispatch binds; adaptive_update() marks converged pixels, which later dispatches skip."""
+        luminance moments that every dispatch binds; adaptive_update() marks converged pixels, which later dispatches skip.
+        deforming: indices of the meshes whose vertices set_vertices() may change; their BLASes are built with
+        BUILD_FLAG_ALLOW_UPDATE so that it can refit them."""
         self.ctx, self.width, self.height, self.kind = ctx, width, height, kind
-        self.blases = [ctx.build_blas_from_mesh(m, build_flags=build_flags) for m in meshes]  # 0 = the application's flags (RtModel.cpp:86-118)
+        self.deforming = frozenset(int(k) for k in deforming)
+        if any(not 0 <= k < len(meshes) for k in self.deforming):
+            raise ValueError(f"deforming names meshes {sorted(self.deforming)}, but there are {len(meshes)}")
+        # 0 = the application's flags (RtModel.cpp:86-118)
+        self.blases = [ctx.build_blas_from_mesh(m, build_flags=build_flags | (T.BUILD_FLAG_ALLOW_UPDATE if k in self.deforming else 0))
+                       for k, m in enumerate(meshes)]
         if instance_mesh is None:
             instance_mesh = list(range(len(meshes)))
         assert len(instance_mesh) == len(transforms)
@@ -704,6 +717,10 @@ class Renderer:
         self.tlas = ctx.build_tlas([self.blases[k] for k in instance_mesh], self.transforms)
         self.motion = None   # (n, 12) float32 world -> previous-world matrices of the last set_transforms(), None before it
         self._motion_buf = None
+        self.prev_transforms = self.transforms.copy()  # the transforms before the last set_transforms()
+        self._vertices = {k: np.ascontiguousarray(meshes[k].vertices).copy() for k in self.deforming}  # host copy of each VB
+        self._prev_vb = {}        # mesh -> device previous positions (a VERTEX_DTYPE array), from its first set_vertices()
+        self._deform_buf = None   # one DeformationDesc per instance, from the first set_vertices()
         self.program = Program(ctx, kind)
         for i, k in enumerate(instance_mesh):
             for ray_type in range(2):
@@ -735,6 +752,7 @@ class Renderer:
             check(lib.rt_set_aov_output(self.ctx.handle, k, buf.ptr if buf is not None else None, 16 * self.width if buf is not None else 0))
         # every call, so that motion another Renderer bound on this context is never inherited
         self.ctx.set_instance_motion(self._motion_buf, len(self.instance_mesh) if self._motion_buf is not None else 0)
+        self.ctx.set_instance_deformation(self._deform_buf, len(self.instance_mesh) if self._deform_buf is not None else 0)
         # likewise the adaptive sampling buffers
         self.ctx.set_adaptive_sampling(*(self.adaptive[:2] if self.adaptive is not None else (None, None)))
         check(lib.rt_set_tlas(self.ctx.handle, self.tlas.result.ptr))
@@ -799,10 +817,55 @@ class Renderer:
             raise ValueError("set_transforms() needs finite, invertible transforms")
         motion = (four(self.transforms) @ np.linalg.inv(cur))[:, :3, :].reshape(-1, 12).astype(np.float32)
         self.tlas = self.ctx.build_tlas([self.blases[k] for k in self.instance_mesh], new)
-        self.transforms, self.motion = new.copy(), motion
+        self.prev_transforms, self.transforms, self.motion = self.transforms, new.copy(), motion
         if self._motion_buf is None:
             self._motion_buf = self.ctx.alloc(48 * max(len(self.instance_mesh), 1))
         self._motion_buf.upload(motion.reshape(-1))
+        if self._deform_buf is not None:
+            self._upload_deformation()
+
+    def set_vertices(self, mesh: int, positions, normals):
+        """Deform mesh `mesh` (one of the constructor's deforming=): upload (V, 3) positions and normals in place of its
+        vertices (same count and order; the hit records keep their buffers), refit its BLAS (PERFORM_UPDATE) and rebuild
+        the TLAS.  The vertices from before this call become the mesh's previous positions, which the previous-position
+        AOV carries its hit points back through (rt_set_instance_deformation), together with the transforms from before
+        the last set_transforms().  Call it once per frame for each deforming mesh, as set_transforms() is called, with
+        unchanged positions for a frame where the mesh rests."""
+        if mesh not in self.deforming:
+            raise ValueError(f"set_vertices() needs a mesh listed in deforming= ({sorted(self.deforming)}), got {mesh}")
+        old = self._vertices[mesh]
+        pos, nrm = np.asarray(positions, np.float32), np.asarray(normals, np.float32)
+        if pos.shape != (old.shape[0], 3) or nrm.shape != (old.shape[0], 3):
+            raise ValueError(f"set_vertices() needs ({old.shape[0]}, 3) positions and normals, got {pos.shape} and {nrm.shape}")
+        if not (np.isfinite(pos).all() and np.isfinite(nrm).all()):
+            raise ValueError("set_vertices() needs finite positions and normals")
+        new = np.zeros(old.shape[0], T.VERTEX_DTYPE)
+        new["position"], new["normal"] = pos, nrm
+        if mesh not in self._prev_vb:
+            self._prev_vb[mesh] = self.ctx.alloc(old.nbytes)
+        self._prev_vb[mesh].upload(old)
+        acc = self.blases[mesh]
+        acc.vb.upload(new)
+        self.ctx.update_blas(acc, acc._keep)
+        self._vertices[mesh] = new
+        self.tlas = self.ctx.build_tlas([self.blases[k] for k in self.instance_mesh], self.transforms)
+        self._upload_deformation()
+
+    def _upload_deformation(self):
+        """One DeformationDesc per instance: the previous positions of its mesh (NULL while it has none) and the
+        transform from before the last set_transforms()."""
+        n = len(self.instance_mesh)
+        descs = (T.DeformationDesc * n)()
+        for i, k in enumerate(self.instance_mesh):
+            prev = self._prev_vb.get(k)
+            if prev is not None:
+                descs[i].previous_positions = prev.ptr
+                descs[i].stride_bytes = T.VERTEX_DTYPE.itemsize
+                descs[i].vertex_count = self._vertices[k].shape[0]
+            descs[i].object_to_previous_world[:] = self.prev_transforms[i].tolist()
+        if self._deform_buf is None:
+            self._deform_buf = self.ctx.alloc(C.sizeof(descs))
+        self._deform_buf.upload(np.frombuffer(descs, np.uint8))
 
     def realtime_band(self, frame: T.PerFrameConstants, band, params: T.DenoiserParams, tmp: "Buffer", final: "Buffer"):
         """One rank's share of a realtime frame sharded by row bands (sharding.band_plan): render rows [r0, r1) of the two
@@ -843,7 +906,7 @@ class Renderer:
         filtered since the last reset_temporal() are the history, reprojected through the position AOV.  Needs aovs= to
         include "albedo", "normal" and "position", and a last dispatch of one sample with accumulation off (accumCount 0).
         With the "previous-position" AOV also bound it runs rt_denoise_temporal_motion, which reprojects through that AOV,
-        so that instances moved by set_transforms() keep their history."""
+        so that instances moved by set_transforms() and meshes deformed by set_vertices() keep their history."""
         if self.kind != PROGRESSIVE or any(a not in self.aovs for a in ("albedo", "normal", T.AOV_POSITION_NAME)):
             raise ValueError('denoise_temporal() needs a progressive Renderer with the "albedo", "normal" and "position" AOVs')
         if self.adaptive is not None:

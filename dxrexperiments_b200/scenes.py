@@ -281,6 +281,46 @@ def sliding_box(frame: int, step=(0.08, 0.0, 0.0)):
     return [box((-0.15, 0.0, -0.15), (0.15, 0.3, 0.15)), cornell_box()], [t.astype(np.float32), IDENTITY_3X4.copy()]
 
 
+def sheared_positions(positions, offset) -> np.ndarray:
+    """(V, 3) float32: every vertex moved by offset * h, h its height normalised to [0, 1] over the mesh (a shear that
+    keeps the lowest vertices fixed), in float64 and rounded once.  dxr_headless --deform computes the same."""
+    p = np.asarray(positions, np.float32).astype(np.float64)
+    lo, hi = p[:, 1].min(), p[:, 1].max()
+    h = (p[:, 1] - lo) / (hi - lo) if hi > lo else np.zeros(p.shape[0])
+    return (p + h[:, None] * np.asarray(offset, np.float64)).astype(np.float32)
+
+
+def sheared_box(frame: int, step=(0.08, 0.0, 0.0)):
+    """A deforming-mesh scene: sliding_box(0)'s (meshes, transforms) with the box's top vertices moved by frame * step
+    and its bottom vertices fixed (normals unchanged).  The deformation is affine, so an instance transform can express
+    it too: sliding_box(0)'s transform times the shear x += (frame * step) * y / 0.3."""
+    meshes, transforms = sliding_box(0)
+    v = meshes[0].vertices.copy()
+    v["position"] = sheared_positions(v["position"], frame * np.asarray(step, np.float64))
+    return [Mesh(v, meshes[0].indices), meshes[1]], transforms
+
+
+def waving_sheet(frame: float, amplitude: float = 0.15, wavelength: float = 1.6, speed: float = 0.5, cells=(48, 24)):
+    """A deforming-mesh scene: (meshes, transforms) of an upright sheet (instance 0, x in [-0.7, 0.7], y in [-0.95, 0.45],
+    facing the camera at z = 0.8) in the open front of the Cornell room (instance 1), with a travelling wave
+    z = 0.8 + amplitude * sin(k x - speed * frame), k = 2 pi / wavelength, on a grid of cells[0] x cells[1] quads.  The
+    defaults turn a normal by at most amplitude * k * speed = 0.29 rad (17 degrees) per frame, under the temporal
+    denoiser's arccos(normal_cos = 0.9) = 26 degrees, and move a point by up to 0.075 along z per frame, more than
+    position_tolerance * distance (0.02 * ~2.8), so without its vertex motion the sheet loses history."""
+    nx, ny = cells
+    k = 2.0 * np.pi / wavelength
+    xs, ys = np.linspace(-0.7, 0.7, nx + 1), np.linspace(-0.95, 0.45, ny + 1)
+    x, y = np.meshgrid(xs, ys)
+    ph = k * x - speed * frame
+    p = np.stack([x, y, 0.8 + amplitude * np.sin(ph)], -1).reshape(-1, 3)
+    n = np.stack([-amplitude * k * np.cos(ph), np.zeros_like(x), np.ones_like(x)], -1).reshape(-1, 3)
+    n /= np.linalg.norm(n, axis=1, keepdims=True)
+    i = np.arange((ny + 1) * (nx + 1)).reshape(ny + 1, nx + 1)
+    a, b, c, d = i[:-1, :-1], i[:-1, 1:], i[1:, 1:], i[1:, :-1]  # counter-clockwise seen from +z: front faces the camera
+    idx = np.stack([a, b, c, a, c, d], -1).reshape(-1)
+    return [_pack(p, n, idx), cornell_box()], [IDENTITY_3X4.copy(), IDENTITY_3X4.copy()]
+
+
 @dataclass
 class FrameSetup:
     """Deterministic replacement of the wall-clock driven parts of update() (SURVEY.md A6)."""

@@ -83,6 +83,11 @@ def adaptive_defaults() -> AdaptiveParams:
 ADAPTIVE_CONVERGED = 0x80000000
 
 
+class DeformationDesc(C.Structure):  # rt_deformation_desc (include/rt_types.h), one per InstanceIndex()
+    _fields_ = [("previous_positions", C.c_void_p), ("stride_bytes", C.c_uint32), ("vertex_count", C.c_uint32),
+                ("object_to_previous_world", C.c_float * 12)]
+
+
 class GeometryDesc(C.Structure):
     _fields_ = [("vertex_buffer", C.c_void_p), ("vertex_count", C.c_uint32), ("vertex_stride_bytes", C.c_uint32),
                 ("index_buffer", C.c_void_p), ("index_count", C.c_uint32), ("index_format", C.c_uint32),
@@ -126,6 +131,7 @@ assert C.sizeof(DenoiserParams) == 24
 assert C.sizeof(ProgressiveDenoiseParams) == 16
 assert C.sizeof(TemporalDenoiseParams) == 32
 assert C.sizeof(AdaptiveParams) == 16
+assert C.sizeof(DeformationDesc) == 64
 assert C.sizeof(InstanceDesc) == 64
 assert C.sizeof(HitRecord) == 80
 assert C.sizeof(GeometryDesc) == 48

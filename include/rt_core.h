@@ -199,7 +199,8 @@ int rt_set_output(rt_context *ctx, uint32_t slot, float *rgba, uint64_t pitch_by
  * world-space primary hit point o + t*d (HitWorldPosition, o including the RayGen's jitter) in place of N: it is what
  * rt_denoise_temporal reprojects through.  PREVIOUS_POSITION is stored exactly like POSITION with P' in place of P: the
  * same hit point carried into the previous frame's world by the motion of the instance it lies on
- * (rt_set_instance_motion).  With M the bound matrix of InstanceIndex() = i, P' = M * (P, 1), each row evaluated as
+ * (rt_set_instance_motion) and, on a deforming mesh, by the motion of its vertices (rt_set_instance_deformation, which
+ * adds a term Dw to the P' below).  With M the bound matrix of InstanceIndex() = i, P' = M * (P, 1), each row evaluated as
  * ((m0*Px + m1*Py) + m2*Pz) + m3; P' = P (a copy, no arithmetic) when no motion is bound or i >= n.  No binding
  * therefore gives a PREVIOUS_POSITION equal to POSITION bit for bit, and so does an identity matrix (x*1 and adding +0
  * are exact; the one exception is a coordinate of -0, which comes out +0).  It is what
@@ -225,9 +226,34 @@ int rt_set_aov_output(rt_context *ctx, uint32_t aov, float *rgba, uint64_t pitch
  * the instance with InstanceIndex() == i.  A host computes it as prevObjectToWorld_i * inverse(objectToWorld_i).  It is
  * context state like rt_set_tlas, read by the dispatches that write PREVIOUS_POSITION; the caller keeps the array alive
  * and unchanged until they are done.  NULL with n = 0 unbinds.  RT_ERR_INVALID_ARG: NULL with n > 0 or a pointer with
- * n = 0, a pointer not 16-byte aligned, n > 2^24 - 1.  Only rigid (per-instance) motion is described: a deforming mesh's
- * moved vertices are not, and such pixels lose their history through the position test. */
+ * n = 0, a pointer not 16-byte aligned, n > 2^24 - 1.  Only rigid (per-instance) motion is described here; a deforming
+ * mesh's moved vertices are described by rt_set_instance_deformation. */
 int rt_set_instance_motion(rt_context *ctx, const float *world_to_previous_world, uint32_t n);
+/* Per-vertex motion of deforming meshes for RT_AOV_PREVIOUS_POSITION (new work: the reference has no counterpart).
+ * descs is a DEVICE array of n rt_deformation_desc (rt_types.h); entry i describes the instance with InstanceIndex() == i:
+ *   previous_positions holds last frame's position of every vertex, indexed like the hit record's vertex buffer and in
+ *     that buffer's space (xyz = the first 3 floats of each stride_bytes element), NULL for a rigid instance;
+ *   object_to_previous_world maps that space into the previous frame's world: prevObjectToWorld_i, times the geometry's
+ *     transform3x4 if the BLAS was built with one.  Only its 3x3 is applied.
+ * For a primary hit P on primitive prim with barycentrics (bu, bv), record indices i0 i1 i2 and record vertex positions
+ * v_k (this frame's vertex buffer: the one the refitted BLAS was built from, as the reference assumes for normals), in
+ * fp32 operation by operation:
+ *   b0 = (1 - bu) - bv, b1 = bu, b2 = bv                 (interpolate_normal's weights)
+ *   d_k = previous_positions[i_k] - v_k                  (per component)
+ *   D = (d0*b0 + d1*b1) + d2*b2
+ *   Dw_r = (m_r0*D.x + m_r1*D.y) + m_r2*D.z              (r = 0..2, m = object_to_previous_world)
+ *   P' = [rt_set_instance_motion's rule: M_i * (P, 1), or P] + Dw
+ * That follows from prevO2W * (X + D) = M_i * P + L(prevO2W) * D with M_i = prevO2W * inverse(O2W), so it composes with
+ * rigid motion.  Dw is left out (P' is exactly the value above) when nothing is bound, i >= n or previous_positions is
+ * NULL.  It is also left out, and rt_get_status reports RT_ERR_INVALID_ARG (as for a missing hit record), when an index
+ * is >= vertex_count or stride_bytes is < 12 or not a multiple of 4.  Previous positions equal to the current ones
+ * therefore give the AOV without the binding bit for bit, except that a coordinate of -0 may come out +0.  The scope is
+ * per-vertex linear motion within each triangle: the hit point moves with the barycentric blend of its vertices'
+ * displacements; topology changes (other vertex or index counts) are not described.  Context state like
+ * rt_set_instance_motion, read only by dispatches that write PREVIOUS_POSITION; the caller keeps descs and the arrays
+ * it points to alive and unchanged until they are done.  NULL with n = 0 unbinds.  RT_ERR_INVALID_ARG: NULL with n > 0
+ * or a pointer with n = 0, descs not 16-byte aligned, n > 2^24 - 1. */
+int rt_set_instance_deformation(rt_context *ctx, const rt_deformation_desc *descs, uint32_t n);
 /* Adaptive sampling of the progressive program (new work: the reference has no counterpart; it accumulates every pixel
  * with the one global accumCount).  counts is a DEVICE array of width x height uint32 in image order (y * width + x):
  * bits 0-30 hold n_p, the samples accumulated into pixel p, and bit 31 (RT_ADAPTIVE_CONVERGED) marks p converged.
@@ -384,15 +410,16 @@ int rt_denoise_temporal(rt_context *ctx, const float *beauty, const float *albed
                         float *history /* 4 * width * height RGBA fp32 */, float *tmp /* 2 * width * height RGBA fp32 */,
                         float *out, uint32_t width, uint32_t height, const rt_temporal_denoise_params *params);
 /* rt_denoise_temporal for scenes whose instances move between frames.  previous_position = RT_AOV_PREVIOUS_POSITION
- * (Q = .xyz: where this frame's primary hit point was in the previous frame's world, rt_set_instance_motion).  Q takes
+ * (Q = .xyz: where this frame's primary hit point was in the previous frame's world, rt_set_instance_motion and
+ * rt_set_instance_deformation).  Q takes
  * the place of Pp in exactly two places of the rule above:
  *   the reprojection: r = Q - o';
  *   the position test: a tap is dropped when |Pq - Q| > position_tolerance*|Q - o'|.
  * Everything else is unchanged: the normal test compares this frame's normal AOV with the history's (the normal AOV is
  * object-space, so a rigid instance motion leaves it unchanged), and history plane 3 stores this frame's P, which the
  * next frame's Pq is.  previous_position == position therefore gives rt_denoise_temporal's out and history bit for bit.
- * A deforming mesh (a BLAS refit with moved vertices) has no motion here: its pixels fail the position test as under
- * rt_denoise_temporal.  previous_position is required; its alignment and overlap rules are those of the other inputs,
+ * A deforming mesh (a BLAS refit with moved vertices) keeps its history when its previous positions are bound with
+ * rt_set_instance_deformation; the normal test still sees its changed normals.  previous_position is required; its alignment and overlap rules are those of the other inputs,
  * and it is only read.  Launches and RT_ERR_INVALID_ARG cases otherwise as rt_denoise_temporal. */
 int rt_denoise_temporal_motion(rt_context *ctx, const float *beauty, const float *albedo, const float *normal,
                                const float *position, const float *previous_position, const rt_camera_params *prev_camera,

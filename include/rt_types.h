@@ -123,6 +123,14 @@ typedef struct rt_adaptive_params {
 /* Bit 31 of a sample count: the pixel has converged and dispatches skip it. */
 #define RT_ADAPTIVE_CONVERGED 0x80000000u
 
+/* rt_set_instance_deformation (rt_core.h); new work, no reference counterpart.  One per InstanceIndex(). */
+typedef struct rt_deformation_desc {
+    const float *previous_positions;   /* DEVICE; NULL = the instance is rigid */
+    uint32_t stride_bytes;             /* >= 12, a multiple of 4: xyz are the first 3 floats of an element */
+    uint32_t vertex_count;             /* elements of previous_positions */
+    float object_to_previous_world[12]; /* row-major 3x4; only its 3x3 is applied */
+} rt_deformation_desc; /* 64 B, 16-byte aligned in an array */
+
 /* Interleaved vertex the hit shaders read: libs/DXRFramework/RtModel.cpp:13-17 (stride 24). */
 typedef struct rt_vertex {
     float position[3];
